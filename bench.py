@@ -67,7 +67,13 @@ def parse():
   p.add_argument("--no-concurrent", action="store_true", help="skip the search + concurrent learner section")
   p.add_argument("--ref-moves-per-step", type=int, default=2,
                  help="reference arm: moves each worker plays per step")
-  return p.parse_args()
+  p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                 help="after the timed steps, write what the last timed move returned for rank 0's games (actions, "
+                      "root_value, child_visits, init_value) as DIR/<name>.npy, to compare two builds output for output")
+  args = p.parse_args()
+  if args.dump_outputs is not None and args.impl != "b200":
+    p.error("--dump-outputs needs --impl b200")
+  return args
 
 
 def search_config(args):
@@ -385,6 +391,8 @@ def run_b200(args):
   barrier()
   ms_total = timed(fs.run, args.steps)
   barrier()
+  # later sections run fs again (the concurrent learner also hands it new weights): keep this move's outputs now
+  outputs = search_outputs(fs) if args.dump_outputs is not None and rank == 0 else None
   # end-to-end: host buffers in, host buffers out, through the public call
   pinned = fs.pinned_inputs()  # the engine's own pinned staging views: the host writes a move's inputs here
   for name, src in (("obs_u8", h_obs_u8), ("noise", h_noise), ("uniforms", h_u), ("temperature", h_t)):
@@ -558,9 +566,35 @@ def run_b200(args):
     }
     if cpu_baseline is not None:
       line["cpu_baseline"] = cpu_baseline
+    if outputs is not None:
+      dump_outputs(args.dump_outputs, outputs)
     emit(line)
   if world > 1:
     dist.destroy_process_group()
+
+
+DUMP_BYTES = 60 << 20  # under 64 MB with the .npy headers
+
+
+def search_outputs(fs):
+  """The arrays FCSearch.search_host returns for the move in fs's device buffers, as float64 / float32 numpy arrays
+  (the int32 actions as float64, exactly)."""
+  return {"actions": fs.actions.cpu().numpy().astype(np.float64), "root_value": fs.root_value.cpu().numpy(),
+          "child_visits": fs.child_visits.cpu().numpy(), "init_value": fs.init_value.cpu().numpy()}
+
+
+def dump_outputs(path, outputs):
+  """Writes every per-game array as path/<name>.npy.  Past DUMP_BYTES in all, a fixed seeded sample of the games is
+  written instead: the same games in every array, their indices as game_index.npy."""
+  games = len(outputs["actions"])
+  row_bytes = sum(a[:1].nbytes for a in outputs.values())
+  if games * row_bytes > DUMP_BYTES:
+    keep = np.sort(np.random.default_rng(0).choice(games, DUMP_BYTES // (row_bytes + 8), replace=False))
+    outputs = {name: a[keep] for name, a in outputs.items()}
+    outputs["game_index"] = keep.astype(np.float64)
+  os.makedirs(path, exist_ok=True)
+  for name, a in outputs.items():
+    np.save(os.path.join(path, name + ".npy"), a)
 
 
 def bench_other_configs(args, torch, dev, timed):

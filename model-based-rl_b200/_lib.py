@@ -4,6 +4,7 @@ There is no fallback: if the CUDA library is missing or a call fails, this raise
 """
 import ctypes as C
 import os
+import shutil
 import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -221,9 +222,21 @@ EXPORTED_SYMBOLS = sorted(_SIGNATURES)
 _lib = None
 
 
+def nvcc_path():
+  """$NVCC, else nvcc on PATH, else the toolkit under $CUDA_HOME or /usr/local/cuda: a login shell's PATH often
+  lacks the CUDA bin directory."""
+  found = os.environ.get("NVCC") or shutil.which("nvcc")
+  if found:
+    return found
+  for root in (os.environ.get("CUDA_HOME"), "/usr/local/cuda"):
+    if root and os.access(os.path.join(root, "bin", "nvcc"), os.X_OK):
+      return os.path.join(root, "bin", "nvcc")
+  raise MzError("nvcc not found: put the CUDA toolkit's bin directory on PATH or set CUDA_HOME")
+
+
 def build(force=False, verbose=False):
   """Compiles csrc/*.cu for sm_100a into libmzb200.so (nvcc cross-compiles without a GPU)."""
-  cmd = ["make", "-C", CSRC, "-j8"] + (["-B"] if force else [])
+  cmd = ["make", "-C", CSRC, "-j8", "NVCC=" + nvcc_path()] + (["-B"] if force else [])
   out = None if verbose else subprocess.DEVNULL
   subprocess.check_call(cmd, stdout=out)
   return LIB_PATH

@@ -46,10 +46,14 @@ def _sub(v):
   return v[::max(1, v.numel() // 1024)] if v.numel() > 2048 else v
 
 
-def _check_against_golden(g, learner, net, tol):
+def _check_against_golden(g, learner, net, tol, exact_first_step=None):
+  """exact_first_step: (losses, errors) the first step must reproduce bit for bit."""
   from model_based_rl_b200 import learners  # noqa: F401  (imported by the caller; keeps flake quiet)
   for step in range(2):
     losses = learner.update_weights(_batch(g, step))
+    if step == 0 and exact_first_step is not None:
+      np.testing.assert_array_equal(losses.cpu().numpy(), exact_first_step[0])
+      np.testing.assert_array_equal(learner.last_errors.cpu().numpy(), exact_first_step[1])
     np.testing.assert_allclose(losses.cpu().numpy(), g["s%d_losses" % step], rtol=tol, atol=0)
     np.testing.assert_allclose(learner.last_errors.cpu().numpy(), g["s%d_new_errors" % step], rtol=0,
                                atol=max(tol * 40, 5e-4))  # h^-1 cancels in float32 (DESIGN.md section 2)
@@ -83,14 +87,18 @@ def test_oracle_learner_step_matches_reference_golden(case):
                                              torch.from_numpy(t_r), torch.from_numpy(t_p), torch.from_numpy(is_w))
   net.zero_grad()
   losses.sum().backward()
-  np.testing.assert_allclose(losses.detach().numpy(), g["s0_losses"], rtol=1e-12)
-  np.testing.assert_array_equal(errs.numpy(), g["s0_new_errors"])
+  # torch's CPU kernels (MKL GEMM, ATen's vectorised loops) are picked by the CPU's instruction set, and another kernel
+  # groups the float32 sums differently: the reference's run is reproduced bit for bit only on a CPU that picks the
+  # same kernels, elsewhere to float32 rounding (losses up to 3e-8 relative; h^-1 amplifies it in the priorities).
+  np.testing.assert_allclose(losses.detach().numpy(), g["s0_losses"], rtol=1e-7)
+  np.testing.assert_allclose(errs.numpy(), g["s0_new_errors"], rtol=0, atol=5e-4)
   for k, p in net.named_parameters():
     gr = p.grad
     np.testing.assert_allclose(float(gr.double().pow(2).sum().sqrt()), float(g["s0_gnorm_" + k]), rtol=1e-6)
     np.testing.assert_allclose(_sub(gr).numpy(), g["s0_g_" + k], rtol=0, atol=1e-7, err_msg=k)
   net.zero_grad()
-  _check_against_golden(g, learner, net, tol=1e-6)
+  # on the same CPU the Learner's first step is the restatement above, bit for bit
+  _check_against_golden(g, learner, net, tol=1e-6, exact_first_step=(losses.detach().numpy(), errs.numpy()))
 
 
 @pytest.mark.parametrize("case", CASES)
