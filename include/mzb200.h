@@ -250,7 +250,8 @@ int mz_fc_recurrent_tf32x3(const mz_fc_weights* w, int32_t batch, const float* h
  * shared-memory image the MMA consumes:
  *   packed: mz_fc_tc_packed_bytes(A) bytes, tail: mz_fc_tc_tail_floats() floats (caller-allocated).
  * mz_fc_recurrent_tc has the arguments of mz_fc_recurrent_f32 plus the packed buffers; `w` is only
- * read for its integer fields.  Limits: A <= 32, value/reward bins <= 32.
+ * read for its integer fields.  Limits: A <= 32, value/reward bins <= 32.  Hidden rows are read
+ * as float2, so hidden_in must be 8-byte aligned and in_row_stride even (MZ_ERR_BAD_ARG otherwise).
  */
 int64_t mz_fc_tc_packed_bytes(int32_t num_actions);
 /* Diagnostics: when set to a device buffer of >= 512 int64, CTA 0 of every following

@@ -666,6 +666,8 @@ int mz_fc_recurrent_tc(const mz_fc_weights* w, const void* packed, const float* 
   if (!w || !packed || !tail || batch < 1 || !hidden_in || !actions || !hidden_out || !value ||
       !reward || !logits)
     return MZ_ERR_BAD_ARG;
+  // the epilogue reads hidden rows as float2: every row start must be 8-byte aligned
+  if ((in_row_stride & 1) || ((uintptr_t)hidden_in & 7)) return MZ_ERR_BAD_ARG;
   if (w->num_actions < 1 || w->num_actions > 32 || w->value_bins > 32 || w->reward_bins > 32 || w->no_support)
     return MZ_ERR_UNSUPPORTED;
   TcParams p;

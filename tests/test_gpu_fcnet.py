@@ -283,15 +283,17 @@ def test_fc_search_tf32x3_replays_bit_exact_in_oracle():
   assert np.allclose(visits["tf32x3"][1][same], visits["f32"][1][same], rtol=1e-3, atol=1e-3)
 
 
-def _search_cfg(S, A, two_players=False, discount=0.997, known_bounds=(None, None)):
+def _search_cfg(S, A, two_players=False, discount=0.997, known_bounds=(None, None), value_support=(-15, 15),
+                reward_support=(-15, 15), no_target_transform=False):
   return types.SimpleNamespace(
       num_simulations=S, action_space=A, two_players=two_players, discount=discount, pb_c_base=19652,
       pb_c_init=1.25, init_value_score=0.0, known_bounds=list(known_bounds), root_exploration_fraction=0.25,
-      value_support=[-15, 15], reward_support=[-15, 15], no_support=False, no_target_transform=False)
+      value_support=list(value_support), reward_support=list(reward_support), no_support=False,
+      no_target_transform=no_target_transform)
 
 
 @pytest.mark.parametrize("cluster,engine", [(2, 0), (4, 0), (4, 1)])
-@pytest.mark.parametrize("shape", ["atari18", "ttt9", "lunar4", "wide32", "ties6"])
+@pytest.mark.parametrize("shape", ["atari18", "ttt9", "lunar4", "wide32", "ties6", "asym5_nott"])
 def test_fused_search_equals_per_launch_search(cluster, engine, shape):
   """mz_fc_search (the whole move in one persistent kernel, clusters of 2 or 4 CTAs) against the
   per-simulation launches of mz_tree_step + mz_fc_recurrent_tc on the same inputs: identical network
@@ -300,18 +302,24 @@ def test_fused_search_equals_per_launch_search(cluster, engine, shape):
   actions -- bit for bit -- and the same trees (priors, children, value sums, visit counts, rewards).
   Game counts are not multiples of the 128-game tile (absent rows), TTT has legal masks, two players
   and known bounds; `ties6` runs a network whose policy head is zero (all priors equal at every node: every
-  unexpanded-child choice is a tie broken by the action index).  engine 0 = dense tree walk, 1 = sparse
-  node-parallel ranking (csrc/mz_fcs_sparse.cuh)."""
+  unexpanded-child choice is a tie broken by the action index); `asym5_nott` has a 32-bin value support
+  [-4, 27], a 9-bin reward support [-2, 6] and raw expectations (no_target_transform), with support logits
+  spread x16.  engine 0 = dense tree walk, 1 = sparse node-parallel ranking (csrc/mz_fcs_sparse.cuh)."""
   from model_based_rl_b200 import _lib
   from model_based_rl_b200.networks import FCNetwork, FCSearch, random_state_dict
   G, A, S, D, two, disc, kb = {"atari18": (300, 18, 50, 128, False, 0.997, (None, None)),
                                "ttt9": (130, 9, 30, 9, True, 1.0, (-1, 1)),
                                "lunar4": (257, 4, 30, 8, False, 0.997, (None, None)),
                                "wide32": (100, 32, 20, 16, False, 0.99, (None, None)),
-                               "ties6": (140, 6, 40, 12, False, 0.997, (None, None))}[shape]
-  cfg = _search_cfg(S, A, two, disc, kb)
+                               "ties6": (140, 6, 40, 12, False, 0.997, (None, None)),
+                               "asym5_nott": (150, 5, 25, 10, False, 0.997, (None, None))}[shape]
+  vs, rs, nott = ((-4, 27), (-2, 6), True) if shape == "asym5_nott" else ((-15, 15), (-15, 15), False)
+  cfg = _search_cfg(S, A, two, disc, kb, vs, rs, nott)
   net = FCNetwork(D, A, "cuda", cfg)
-  sd = random_state_dict(D, A, seed=11)
+  sd = random_state_dict(D, A, vs[1] - vs[0] + 1, rs[1] - rs[0] + 1, seed=11)
+  if shape == "asym5_nott":
+    for k in ("value_head.value", "reward_head.reward"):
+      sd[k + ".weight"], sd[k + ".bias"] = sd[k + ".weight"] * 16, sd[k + ".bias"] * 16
   if shape == "ties6":
     sd["policy_head.policy.weight"] = torch.zeros_like(sd["policy_head.policy.weight"])
     sd["policy_head.policy.bias"] = torch.zeros_like(sd["policy_head.policy.bias"])
