@@ -289,19 +289,18 @@ int mz_fc_initial_tc(const mz_fc_weights* w, const void* packed, const float* ta
 /* backpropagate (mcts.py:47-55, 126-143), handed from phase to phase through mbarriers in          */
 /* (distributed) shared memory, and the root statistics of game.py:106-111 at the end.  Same       */
 /* arithmetic as mz_tree_step + mz_fc_recurrent_tc (bit-identical results); the tree uses its own    */
-/* layout (node record = node statistics + per-action {child id, child visits, prior, child q}, so  */
-/* a level of the descent is one memory round trip) and the hidden pool is bf16 [G][S+1][64].       */
+/* layout (csrc/mz_fcs_sparse.cuh) and the hidden pool is bf16 [G][S+1][64].                        */
+/* Shapes: 1 <= A <= 32, 1 <= S <= 63, and (S, A) within the kernel's shared-memory plan, as        */
+/* mz_fc_search_supported reports; mz_fc_search returns MZ_ERR_UNSUPPORTED for any other shape.     */
 /* ------------------------------------------------------------------------------------------- */
 typedef struct mz_fc_search_args {
   const mz_fc_weights* weights;  /* dims, supports (the float32 pointers are not read) */
   const void* packed;            /* mz_fc_tc_pack image */
   const float* tail;
   int32_t num_games;             /* G */
-  int32_t num_simulations;       /* S <= 253   config.num_simulations mcts.py:66 */
+  int32_t num_simulations;       /* S <= 63    config.num_simulations mcts.py:66 */
   int32_t two_players;           /*            config.two_players     mcts.py:73 */
   int32_t prior_sum_mode;        /* as in mz_tree */
-  int32_t node_bytes;            /* mz_fc_search_node_bytes(A) */
-  int32_t reserved;
   int64_t game_bytes;            /* >= mz_fc_search_game_bytes(S, A) */
   double discount, init_value_score, min_bound, max_bound;  /* as in mz_tree */
   double noise_frac;             /* config.root_exploration_fraction (used when noise != NULL) */
@@ -327,7 +326,6 @@ typedef struct mz_fc_search_args {
   int32_t* error_flag;           /* set before the kernel traps on a protocol time-out, or NULL */
 } mz_fc_search_args;
 
-int32_t mz_fc_search_node_bytes(int32_t num_actions);
 int64_t mz_fc_search_game_bytes(int32_t num_simulations, int32_t num_actions);
 int32_t mz_fc_search_pool_row(void);                         /* bf16 elements per pool row (64) */
 int mz_fc_search_supported(int32_t num_simulations, int32_t num_actions); /* 1: shapes fit the kernel */
@@ -335,15 +333,6 @@ int mz_fc_search(const mz_fc_search_args* a, void* stream);
 /* one game's tree as the arrays of mz_tree_export (+ the cached child q [S+1][A]) */
 int mz_fc_search_export(const mz_fc_search_args* a, int32_t game, double* prior, int32_t* child,
                         double* vsum, int32_t* visit, float* reward, double* q, void* stream);
-/* cluster size of mz_fc_search: 2 (rank 0 = reward + value heads, rank 1 = transition + policy, weights
- * streamed per simulation), 4 (one head per CTA, weights resident in shared memory), 0 = default
- * (MZ_FS_CLUSTER in the environment, else 4). */
-int mz_fc_search_set_cluster(int32_t cluster);
-/* tree engine of mz_fc_search: 0 = dense (four lanes per game walk the tree level by level, every action of a
- * node scored), 1 = sparse (clusters of four, S <= 63: every expanded node ranks only its expanded children and
- * its best unexpanded child, all nodes in parallel, then the descent is a pointer chase), -1 = default
- * (MZ_FS_ENGINE in the environment, else sparse whenever the shape allows).  Same results bit for bit. */
-int mz_fc_search_set_engine(int32_t engine);
 
 /* ------------------------------------------------------------------------------------------- */
 /* Scalar transforms and supports (config.py:27-68), float32 in torch's op order.                */

@@ -50,9 +50,8 @@ class FcSearchArgs(C.Structure):
   """struct mz_fc_search_args"""
   _fields_ = [("weights", C.POINTER(FcWeights)), ("packed", C.c_void_p), ("tail", C.c_void_p),
               ("num_games", C.c_int32), ("num_simulations", C.c_int32), ("two_players", C.c_int32),
-              ("prior_sum_mode", C.c_int32), ("node_bytes", C.c_int32), ("reserved", C.c_int32),
-              ("game_bytes", C.c_int64), ("discount", C.c_double), ("init_value_score", C.c_double),
-              ("min_bound", C.c_double), ("max_bound", C.c_double), ("noise_frac", C.c_double),
+              ("prior_sum_mode", C.c_int32), ("game_bytes", C.c_int64), ("discount", C.c_double),
+              ("init_value_score", C.c_double), ("min_bound", C.c_double), ("max_bound", C.c_double), ("noise_frac", C.c_double),
               ("games", C.c_void_p), ("pb_c_table", C.c_void_p), ("pool", C.c_void_p),
               ("root_logits", C.c_void_p), ("legal_mask", C.c_void_p), ("noise", C.c_void_p),
               ("root_to_play", C.c_void_p), ("root_hidden", C.c_void_p), ("visits", C.c_void_p),
@@ -151,14 +150,11 @@ _SIGNATURES = {
     "mz_fc_tc_initial_packed_bytes": (C.c_int64, [C.c_int32]),
     "mz_fc_tc_pack_initial": (C.c_int, [C.POINTER(FcWeights), _V, _V, _V]),
     "mz_fc_initial_tc": (C.c_int, [C.POINTER(FcWeights), _V, _V, C.c_int32, _V, _V, C.c_int64, _V, _V, _V]),
-    "mz_fc_search_node_bytes": (C.c_int32, [C.c_int32]),
     "mz_fc_search_game_bytes": (C.c_int64, [C.c_int32, C.c_int32]),
     "mz_fc_search_pool_row": (C.c_int32, []),
     "mz_fc_search_supported": (C.c_int, [C.c_int32, C.c_int32]),
     "mz_fc_search": (C.c_int, [C.POINTER(FcSearchArgs), _V]),
     "mz_fc_search_export": (C.c_int, [C.POINTER(FcSearchArgs), C.c_int32, _V, _V, _V, _V, _V, _V, _V]),
-    "mz_fc_search_set_cluster": (C.c_int, [C.c_int32]),
-    "mz_fc_search_set_engine": (C.c_int, [C.c_int32]),
     "mz_scalar_transform": (C.c_int, [C.c_int64, _V, _V, _V]),
     "mz_scalar_to_support": (C.c_int, [C.c_int64, _V, C.c_int32, C.c_int32, C.c_int32, _V, _V]),
     "mz_support_to_scalar": (C.c_int, [C.c_int64, _V, C.c_int32, C.c_int32, C.c_int32, _V, _V]),

@@ -1,4 +1,4 @@
-// Sparse, node-parallel tree engine of the persistent search kernel (mz_fcsearch.cu, cluster size 4).
+// Tree engine of the persistent search kernel (mz_fcsearch.cu): sparse and node-parallel.
 //
 // What bounds the search is the length of ONE game's dependent instruction stream per simulation (a warp
 // issues ~1 dependent instruction per 10 cycles), so this engine shortens that stream instead of packing
@@ -15,7 +15,7 @@
 //    descent (mcts.py:87-92) is then a pointer chase through the per-node winners in shared memory --
 //    a handful of instructions per level instead of a full score evaluation per level.
 //
-// Arithmetic per score is the one of mz_tree.cu / the dense engine (IEEE binary64, reference operation order);
+// Arithmetic per score is the one of mz_tree.cu (IEEE binary64, reference operation order);
 // results are bit-identical (tests/test_gpu_fcnet.py::test_fused_search_equals_per_launch_search).
 //
 // Per-game block in global memory (L2):   S1 = round_up(S + 1, 2) node slots, A2 = round_up(A, 2)
@@ -151,7 +151,9 @@ MZ_DEV void top_unexpanded(const double (&pv)[NS][AL], const uint32_t (&xmask)[N
   }
 }
 
-// Node.expand priors for the eight lanes of a game (see fs_prior_sum in mz_fcsearch.cu: same sum order)
+// Node.expand priors (mcts.py:52-55) for the eight lanes of a game: p_a = exp(logit_a) / sum over the legal actions
+// in ascending order, the sum evaluated like CPython's builtin sum() (prior_sum_mode 1: Neumaier).  Every lane
+// returns the sum; pexp[t] holds exp(logit) of action 8 t + sub (0 where illegal / absent).
 template <int AL>
 MZ_DEV double prior_sum(const FsParams& p, const Smem& sm, const Game& gm, const float* logits, uint32_t legal_bits,
                         double (&pexp)[AL]) {

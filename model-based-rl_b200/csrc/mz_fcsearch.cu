@@ -1,6 +1,6 @@
 // The whole MCTS move of the FCNetwork engine in ONE persistent kernel (MCTS.run, mcts.py:78-102).
 //
-// A cluster of CL (2 or 4) CTAs owns a tile of 128 games for all S simulations of a move:
+// A cluster of four CTAs owns a tile of 128 games for all S simulations of a move:
 //
 //   per simulation   tree phase  : expand + backpropagate of the previous simulation (mcts.py:47-55,
 //                                  126-143), pUCT descent of this one (mcts.py:87-92, 104-124), gather of
@@ -15,26 +15,17 @@
 //   reward / value / policy epilogues --st.async--> output slots of the CTA that owns the game (out_full)
 //   h' rows --> bf16 hidden pool in global memory (L2), released to the cluster with the out_full arrival
 //
-// CL = 2: rank 0 = reward + value heads, rank 1 = transition + policy heads (weights streamed through a
-// shared-memory ring once per simulation, as in mz_fcnet_tc.cu); CL = 4: one head per CTA, its packed
-// weights resident in shared memory for the whole move.  The eight epilogue warps of a CTA double as the
-// tree engine of the 128 / CL games the CTA owns: four lanes per game, lane `sub` owns actions sub,
-// sub + 4, ...  The two phases of a tile are serial by data dependence, so sharing the warps costs nothing.
+// One head per CTA (rank 0 reward, 1 transition, 2 value, 3 policy), its packed weights resident in shared
+// memory for the whole move.  The eight epilogue warps of a CTA double as the tree engine of the 32 games the
+// CTA owns (mz_fcs_sparse.cuh: eight lanes per game, its own tree layout; mz_fc_search_export converts a game
+// to the arrays of mz_tree_export).  The two phases of a tile are serial by data dependence, so sharing the
+// warps costs nothing.  All score arithmetic is IEEE binary64 in the reference's operation order (explicit
+// *_rn intrinsics), bit-identical to mz_tree.cu.
 //
-// Tree layout (this kernel only; mz_fcs_export converts a game to the arrays of mz_tree_export):
-//   game block  = header 64 B (f64 min, f64 max) | node record x (S + 1)       node n is created by sim n-1
-//   node record = f64 value_sum | i32 visit_count | f32 reward                      (the node itself)
-//               | u16 meta[4][8]    meta[a & 3][a >> 2] = child id (255 unexpanded, 254 illegal) | visits << 8
-//               | {f64 prior, f64 q}[A]   q = reward -/+ discount * value() of the CHILD reached by action a
-//   node_bytes  = round_up(80 + 16 A, 64)
-// Everything select_child needs of a node's children sits in the node's own record: one L2 round trip per
-// level (the per-launch kernels chase child index -> child record).  All score arithmetic is IEEE binary64
-// in the reference's operation order (explicit *_rn intrinsics), bit-identical to mz_tree.cu.
+// Shapes: A <= 32, S <= 63 (fs2::MAX_S), and the shared-memory plan (fs_layout) within kFsMaxSmem; the
+// caller runs every other shape on the per-launch kernels (mz_fc_search_supported).
 #include <cuda_bf16.h>
 #include <math.h>
-#include <stdlib.h>
-
-#include <type_traits>
 
 #include "mz_common.cuh"
 #include "mz_exp.cuh"
@@ -46,9 +37,8 @@ namespace {
 using namespace mzfc;
 
 constexpr int FS_THREADS = TC_THREADS;  // warp 0 producer, 1 layer-1 MMA, 2..9 epilogue + tree, 10 layer-2 MMA, 11 store
-constexpr int FS_HDR = 64;              // game header bytes
-constexpr int FS_META = 16, FS_PQ = 80; // offsets inside a node record
-constexpr int CH_UNEXP = 255, CH_ILLEGAL = 254;
+constexpr int FS_CL = 4;                // CTAs per cluster: one network head each
+constexpr int FS_GP = ROWS / FS_CL;     // games whose tree a CTA runs
 constexpr int POOL_ROW = 64;            // bf16 elements per hidden-pool row (128 bytes, one line)
 constexpr int SP_STRIDE = 33;           // doubles per game of the expansion scratch (>= 32 actions; odd: conflict free)
 
@@ -56,14 +46,13 @@ struct FsParams {
   // network (same packed image as mz_fc_recurrent_tc)
   const uint8_t* chunks;
   const float* tail;
-  int k1, A, value_min, reward_min, no_tt, stages, cl;
+  int k1, A, value_min, reward_min, no_tt;
   // search
   int G, S, two_players, prior_sum_mode;
   double discount, init_score, min_bound, max_bound, noise_frac;
   const double* pb_c;  // [(S+1)^2]
   uint8_t* games;
   long long game_bytes;
-  int node_bytes;
   __nv_bfloat16* pool;  // [G][S+1][64]
   // root
   const float* root_logits;
@@ -114,6 +103,11 @@ MZ_DEV void fs_wait_cluster(uint64_t* bar, uint32_t parity, int* err, int code) 
   while (!mbar_try_wait_cluster(bar, parity))
     if (clock64() - t0 > 6000000000ll) fs_timeout(err, code);
 }
+MZ_DEV uint32_t cluster_nctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
+  return r;
+}
 MZ_DEV void mbar_arrive_remote_release(uint32_t remote_bar) {
   asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(remote_bar) : "memory");
 }
@@ -145,16 +139,6 @@ MZ_DEV bool fs_divisor_ok(double d) {
   const unsigned h = (unsigned)__double2hiint(d), l = (unsigned)__double2loint(d);
   return fs_exp_in_fast_range(d) && !(((h & 0xfffffu) == 0xfffffu) && l == 0xffffffffu);
 }
-MZ_DEV double shfl4_xor_f64(double v, int m) {
-  int lo = __double2loint(v), hi = __double2hiint(v);
-  lo = __shfl_xor_sync(MZ_FULL, lo, m, 4);
-  hi = __shfl_xor_sync(MZ_FULL, hi, m, 4);
-  return __hiloint2double(hi, lo);
-}
-MZ_DEV uint32_t meta_at(const uint4& mw, int t) {  // u16 number t of a lane's meta words
-  const uint32_t w = t < 2 ? mw.x : (t < 4 ? mw.y : (t < 6 ? mw.z : mw.w));
-  return (w >> (16 * (t & 1))) & 0xffffu;
-}
 
 // exp() of mz_exp.cuh with the 2 KB table in shared memory: this kernel's shared-memory footprint leaves almost no
 // L1, so the table lookups of the global-memory version are L2 round trips on the expansion's critical path.
@@ -181,412 +165,6 @@ MZ_DEV double fs_exp(double x, const unsigned long long* tab) {
   return __fma_rn(scale, tmp, scale);
 }
 
-// ---- shared-memory map of the tree engine (per CTA: GP = 128 / CL games) --------------------------------
-struct FsTreeSmem {
-  float* logit;     // [GP][A4]   policy logits of the last network evaluation (st.async from the policy head)
-  float* val;       // [GP]
-  float* rew;       // [GP]
-  double* sp;       // [GP][25]   exp(logit) / reward scratch of the expansion
-  double* mm;       // [GP][2]    MinMaxStats (mcts.py:6-25)
-  const double* pbc;  // lower-triangular pb_c table: entry N (N + 1) / 2 + n
-  const unsigned long long* exp_tab;  // mz_exp_tab in shared memory
-  uint8_t* path_n;  // [GP][PS]  node ids of the current search path
-  uint8_t* path_a;  // [GP][PS]  action taken at each level
-  uint8_t* depth;   // [GP]
-  int ps;           // path stride
-  int a4;           // logits row stride (floats)
-};
-
-struct FsGame {  // per-thread view of the game this lane works on
-  bool valid;
-  int g, gl, sub;
-  uint8_t* base;  // game block in global memory
-};
-
-MZ_DEV uint8_t* fs_node(const FsGame& gm, int node_bytes, int n) { return gm.base + FS_HDR + (size_t)n * node_bytes; }
-MZ_DEV int fs_meta_off(int a) { return FS_META + 16 * (a & 3) + 2 * (a >> 2); }
-
-// ------------------------------------------------------------------------------------------------------
-// Node.expand priors (mcts.py:52-55) for the four lanes of a game: p_a = exp(logit_a) / sum over the legal
-// actions in ascending order, the sum evaluated like CPython's builtin sum() (prior_sum_mode 1: Neumaier).
-// Every lane returns the sum; pexp[t] holds exp(logit) of action 4 t + sub (0 where illegal / absent).
-// ------------------------------------------------------------------------------------------------------
-template <int T>
-MZ_DEV double fs_prior_sum(const FsParams& p, const FsTreeSmem& sm, const FsGame& gm, const float* logits,
-                           uint32_t legal_bits, double (&pexp)[T]) {
-  const int A = p.A;
-  double* sp = sm.sp + gm.gl * SP_STRIDE;
-#pragma unroll
-  for (int t = 0; t < T; ++t) {
-    const int a = 4 * t + gm.sub;
-    double e = 0.0;
-    if (a < A && ((legal_bits >> a) & 1u)) e = fs_exp((double)logits[a], sm.exp_tab);
-    pexp[t] = e;
-    if (a < A) sp[a] = e;
-  }
-  __syncwarp();
-  double f = 0.0, c = 0.0;
-  bool first = true;
-#pragma unroll 1
-  for (int a = 0; a < A; ++a) {
-    if (!((legal_bits >> a) & 1u)) continue;
-    const double x = sp[a];
-    if (first) {
-      f = x;  // int 0 + x
-      first = false;
-    } else if (p.prior_sum_mode == 0) {
-      f = __dadd_rn(f, x);
-    } else {  // Neumaier step, CPython >= 3.12 Python/bltinmodule.c
-      const double s = __dadd_rn(f, x);
-      const bool big = fabs(f) >= fabs(x);
-      const double hi = big ? f : x, lo = big ? x : f;
-      c = __dadd_rn(c, __dadd_rn(__dsub_rn(hi, s), lo));
-      f = s;
-    }
-  }
-  if (p.prior_sum_mode != 0 && c != 0.0 && isfinite(c)) f = __dadd_rn(f, c);
-  __syncwarp();
-  return f;
-}
-
-// Root set-up: Node.expand over the legal actions + add_exploration_noise (mcts.py:47-61) + MinMaxStats.reset
-// (mcts.py:79); the root's hidden state goes to pool slot 0 as bf16.
-template <int T>
-MZ_DEV void fs_set_root(const FsParams& p, const FsTreeSmem& sm, const FsGame& gm) {
-  const int A = p.A;
-  uint32_t lm = 0u;  // lanes of absent games take the same path with nothing legal and no memory traffic
-  if (gm.valid) {
-    lm = p.legal ? p.legal[gm.g] : 0xffffffffu;
-    if (A < 32) lm &= (1u << A) - 1u;
-  }
-  double pexp[T];
-  const double f = fs_prior_sum<T>(p, sm, gm, p.root_logits + (size_t)(gm.valid ? gm.g : 0) * A, lm, pexp);
-  if (!gm.valid) return;
-  uint8_t* rec = fs_node(gm, p.node_bytes, 0);
-  uint32_t mwords[4] = {0u, 0u, 0u, 0u};
-#pragma unroll
-  for (int t = 0; t < 8; ++t) {
-    const int a = 4 * t + gm.sub;
-    const bool legal = a < A && ((lm >> a) & 1u);
-    if (t < T && a < A) {
-      double prior = legal ? __ddiv_rn(pexp[t < T ? t : 0], f) : 0.0;
-      if (p.noise && legal) {  // noise is dense over the root's children in action order
-        const int j = __popc(lm & ((1u << a) - 1u));
-        const double nz = p.noise[(size_t)gm.g * A + j];
-        prior = __dadd_rn(__dmul_rn(prior, __dsub_rn(1.0, p.noise_frac)), __dmul_rn(nz, p.noise_frac));
-      }
-      *reinterpret_cast<double2*>(rec + FS_PQ + 16 * a) = make_double2(prior, 0.0);
-    }
-    mwords[t >> 1] |= (uint32_t)(legal ? CH_UNEXP : CH_ILLEGAL) << (16 * (t & 1));
-  }
-  *reinterpret_cast<uint4*>(rec + FS_META + 16 * gm.sub) = make_uint4(mwords[0], mwords[1], mwords[2], mwords[3]);
-  if (gm.sub == 0) {
-    *reinterpret_cast<uint4*>(rec) = make_uint4(0u, 0u, 0u, 0u);  // value_sum 0.0, visit_count 0, reward 0.0f
-    sm.mm[2 * gm.gl] = p.min_bound;
-    sm.mm[2 * gm.gl + 1] = p.max_bound;
-  }
-  // hidden state of the root: float32 [50] -> bf16 [64] (zero padded), pool slot 0
-  const float* h = p.root_hidden + (size_t)gm.g * H;
-  __nv_bfloat16* row = p.pool + (size_t)gm.g * (p.S + 1) * POOL_ROW;
-#pragma unroll
-  for (int kb = 0; kb < 2; ++kb) {
-    const int k0 = 16 * gm.sub + 8 * kb;
-    uint32_t w[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int k = k0 + 2 * j;
-      const float lo = k < H ? h[k] : 0.0f, hi = k + 1 < H ? h[k + 1] : 0.0f;
-      w[j] = pack_bf16(lo, hi);
-    }
-    *reinterpret_cast<uint4*>(row + k0) = make_uint4(w[0], w[1], w[2], w[3]);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------------
-// descent: while node.expanded(): select_child (mcts.py:87-92, 104-124).  One L2 round trip per level: the
-// lane's meta words and its {prior, q} pairs of the current node; ucb_score in binary64; argmax over
-// (score, action) tuples (ties -> larger action) inside the lane, then across the four lanes.
-// ------------------------------------------------------------------------------------------------------
-template <int T>
-MZ_DEV void fs_descend(const FsParams& p, const FsTreeSmem& sm, const FsGame& gm, int sim, int& out_parent,
-                       int& out_action) {
-  const int A = p.A, NB = p.node_bytes;
-  const double init_score = p.init_score;
-  const double mn = sm.mm[2 * gm.gl], mx = sm.mm[2 * gm.gl + 1];
-  const double d = __dsub_rn(mx, mn);
-  int mode = 0;
-  double r = 0.0;
-  if (mx > mn) {
-    if (fs_divisor_ok(d)) {
-      mode = 2;
-      r = __drcp_rn(d);
-    } else {
-      mode = 3;
-    }
-  } else if (mx == mn) {
-    mode = 1;
-  }
-  uint8_t* pn = sm.path_n + gm.gl * sm.ps;
-  uint8_t* pa = sm.path_a + gm.gl * sm.ps;
-  int node = 0, N = sim, depth = 0, parent = 0, action = 0;  // root.visit_count == completed simulations
-  bool done = !gm.valid;
-  if (gm.valid && gm.sub == 0) pn[0] = 0;
-  while (__any_sync(MZ_FULL, !done)) {
-    double best_s = 0.0;
-    int best_a = -1;
-    uint4 mw = make_uint4(0u, 0u, 0u, 0u);
-    if (!done) {
-      const uint8_t* rec = gm.base + FS_HDR + (size_t)node * NB;
-      mw = ldg16(rec + FS_META + 16 * gm.sub);
-      double2 pq[T];
-#pragma unroll
-      for (int t = 0; t < T; ++t) {
-        const int a = 4 * t + gm.sub;
-        pq[t] = make_double2(0.0, 0.0);
-        if (a < A) pq[t] = *reinterpret_cast<const double2*>(rec + FS_PQ + 16 * a);
-      }
-      const double* row = sm.pbc + (N * (N + 1)) / 2;
-#pragma unroll
-      for (int t = 0; t < T; ++t) {
-        const int a = 4 * t + gm.sub;
-        const uint32_t mt = meta_at(mw, t);
-        const int ch = (int)(mt & 0xffu), n = (int)(mt >> 8);
-        const bool cand = a < A && ch != CH_ILLEGAL;
-        double score;
-        if (N == 0) {  // mcts.py:105-108: an unvisited (root) node ranks children by prior
-          score = pq[t].x;
-        } else {       // ucb_score mcts.py:115-124
-          const double pb_c = row[cand ? n : 0];
-          double value_score = init_score;
-          if (n > 0) {
-            const double q = pq[t].y;
-            if (mode == 2) {
-              const double x = __dsub_rn(q, mn);
-              value_score = fs_div_by_const(x, d, r);
-              const unsigned hx = (unsigned)__double2hiint(x);  // x >= 0 because min <= q
-              if (__builtin_expect(hx - 0x33700000u > 0x19000000u, 0)) value_score = (x == 0.0) ? 0.0 : __ddiv_rn(x, d);
-            } else if (mode == 3) {
-              value_score = __ddiv_rn(__dsub_rn(q, mn), d);
-            } else if (mode == 1) {
-              value_score = 1.0;
-            } else {
-              value_score = q;
-            }
-          }
-          score = __dadd_rn(__dmul_rn(pb_c, pq[t].x), value_score);
-        }
-        if (cand && (best_a < 0 || score >= best_s)) {  // the lane's actions ascend: >= keeps the larger action
-          best_s = score;
-          best_a = a;
-        }
-      }
-    }
-    // across the four lanes of the game: max over (score, action), ties -> larger action (mcts.py:106-112)
-#pragma unroll
-    for (int m = 1; m < 4; m <<= 1) {
-      const double os = shfl4_xor_f64(best_s, m);
-      const int oa = __shfl_xor_sync(MZ_FULL, best_a, m, 4);
-      if (oa >= 0 && (best_a < 0 || os > best_s || (os == best_s && oa > best_a))) {
-        best_s = os;
-        best_a = oa;
-      }
-    }
-    const int ba = best_a < 0 ? 0 : best_a;
-    const uint32_t mt_b = __shfl_sync(MZ_FULL, meta_at(mw, ba >> 2), ba & 3, 4);
-    if (!done) {
-      depth++;
-      const int ch_b = (int)(mt_b & 0xffu);
-      if (gm.sub == 0) pa[depth - 1] = (uint8_t)ba;
-      if (ch_b >= CH_ILLEGAL) {  // child not expanded: this is the leaf
-        parent = node;
-        action = ba;
-        done = true;
-      } else {
-        node = ch_b;
-        N = (int)(mt_b >> 8);
-        if (gm.sub == 0) pn[depth] = (uint8_t)node;
-      }
-    }
-  }
-  if (gm.valid && gm.sub == 0) {
-    sm.depth[gm.gl] = (uint8_t)depth;
-    if (p.trace_parent) p.trace_parent[(size_t)sim * p.G + gm.g] = parent;
-    if (p.trace_action) p.trace_action[(size_t)sim * p.G + gm.g] = action;
-    if (p.trace_depth) p.trace_depth[(size_t)sim * p.G + gm.g] = depth;
-  }
-  out_parent = parent;
-  out_action = action;
-}
-
-// ------------------------------------------------------------------------------------------------------
-// expand (mcts.py:47-55) + backpropagate (mcts.py:126-143) of simulation `sim` with the network outputs the
-// output slots hold.  Path position k is node path_n[k] (k < depth) or the new node (k == depth); lane `sub`
-// owns positions k = 4 m + sub.  The value recurrence runs redundantly in the four lanes (rewards through the
-// scratch row); every lane then updates its positions: the node's own (value_sum, visit_count) and the edge
-// (q, visits) in its parent's record.
-// ------------------------------------------------------------------------------------------------------
-template <int T>
-MZ_DEV void fs_expand_backup(const FsParams& p, const FsTreeSmem& sm, const FsGame& gm, int sim) {
-  const int A = p.A, NB = p.node_bytes;
-  const bool two = p.two_players != 0;
-  const double disc = p.discount;
-  const int newn = sim + 1;
-  const float* logits = sm.logit + gm.gl * sm.a4;
-  const float value_f = sm.val[gm.gl], reward_in = sm.rew[gm.gl];
-  const float node_reward_new = (reward_in != 0.0f) ? reward_in : 0.0f;  // `if network_output.reward:`
-  const uint8_t* pn = sm.path_n + gm.gl * sm.ps;
-  const uint8_t* pa = sm.path_a + gm.gl * sm.ps;
-  const int depth = gm.valid ? (int)sm.depth[gm.gl] : 0;
-  if (gm.valid) {
-    if (gm.sub == 0) {
-      if (p.rec_value) p.rec_value[(size_t)sim * p.G + gm.g] = value_f;
-      if (p.rec_reward) p.rec_reward[(size_t)sim * p.G + gm.g] = reward_in;
-    }
-    if (p.rec_logits) {
-#pragma unroll
-      for (int t = 0; t < T; ++t) {
-        const int a = 4 * t + gm.sub;
-        if (a < A) p.rec_logits[((size_t)sim * p.G + gm.g) * A + a] = logits[a];
-      }
-    }
-  }
-  // the lane's path positions of the deepest chunk: issue the loads before the expansion arithmetic
-  int dmax = depth;
-#pragma unroll
-  for (int m = 16; m > 0; m >>= 1) dmax = max(dmax, __shfl_xor_sync(MZ_FULL, dmax, m));
-
-  // ---- expand: priors of the new node (every action is legal below the root, mcts.py:72, 97) ----
-  double pexp[T];
-  const uint32_t all = A < 32 ? (1u << A) - 1u : 0xffffffffu;
-  const double f = fs_prior_sum<T>(p, sm, gm, logits, gm.valid ? all : 0u, pexp);
-  if (gm.valid) {
-    uint8_t* rec = fs_node(gm, NB, newn);
-    uint32_t mwords[4] = {0u, 0u, 0u, 0u};
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-      const int a = 4 * t + gm.sub;
-      if (t < T && a < A)
-        *reinterpret_cast<double2*>(rec + FS_PQ + 16 * a) = make_double2(__ddiv_rn(pexp[t < T ? t : 0], f), 0.0);
-      mwords[t >> 1] |= (uint32_t)(a < A ? CH_UNEXP : CH_ILLEGAL) << (16 * (t & 1));
-    }
-    *reinterpret_cast<uint4*>(rec + FS_META + 16 * gm.sub) = make_uint4(mwords[0], mwords[1], mwords[2], mwords[3]);
-  }
-
-  // ---- backup ----
-  float* scratch = reinterpret_cast<float*>(sm.sp + gm.gl * SP_STRIDE);  // 32 rewards of the chunk
-  double value = (double)value_f;
-  double lmin = INFINITY, lmax = -INFINITY;
-  for (int base = (dmax >> 5) << 5; base >= 0; base -= 32) {
-    double vs[8], myval[8];
-    int vc[8];
-    float rw[8];
-#pragma unroll
-    for (int m = 0; m < 8; ++m) {
-      const int kk = base + 4 * m + gm.sub;
-      vs[m] = 0.0;
-      vc[m] = 0;
-      rw[m] = node_reward_new;
-      myval[m] = 0.0;
-      if (base + 4 * m <= dmax && gm.valid && kk < depth) {
-        const uint4 o = ldg16(fs_node(gm, NB, (int)pn[kk]));
-        vs[m] = u2d(o.x, o.y);
-        vc[m] = (int)o.z;
-        rw[m] = __uint_as_float(o.w);
-      }
-      if (base + 4 * m <= dmax && gm.valid && kk <= depth) scratch[4 * m + gm.sub] = rw[m];
-    }
-    __syncwarp();
-#pragma unroll
-    for (int m = 7; m >= 0; --m) {
-      if (base + 4 * m > dmax) continue;  // warp uniform
-#pragma unroll
-      for (int jj = 3; jj >= 0; --jj) {
-        const int kk = base + 4 * m + jj;
-        if (gm.valid && kk <= depth) {
-          const float rj = scratch[4 * m + jj];
-          if (jj == gm.sub) myval[m] = value;
-          // value = (-reward if two_players and node.to_play == to_play else reward) + discount * value
-          const bool same = two ? (((depth - kk) & 1) == 0) : false;
-          value = __dadd_rn((double)(same ? -rj : rj), __dmul_rn(disc, value));
-        }
-      }
-    }
-    __syncwarp();
-#pragma unroll
-    for (int m = 0; m < 8; ++m) {
-      const int kk = base + 4 * m + gm.sub;
-      if (base + 4 * m <= dmax && gm.valid && kk <= depth) {
-        // value_sum += value if node.to_play == to_play else -value
-        const bool same = two ? (((depth - kk) & 1) == 0) : true;
-        const double nvs = __dadd_rn(vs[m], same ? myval[m] : -myval[m]);
-        const int nvc = vc[m] + 1;
-        const int nid = kk < depth ? (int)pn[kk] : newn;
-        uint8_t* rec = fs_node(gm, NB, nid);
-        *reinterpret_cast<uint4*>(rec) = make_uint4((uint32_t)__double2loint(nvs), (uint32_t)__double2hiint(nvs),
-                                                    (uint32_t)nvc, __float_as_uint(rw[m]));
-        if (kk > 0) {  // mcts.py:136-141
-          const double dq = __dmul_rn(disc, __ddiv_rn(nvs, (double)nvc));
-          const double new_q = two ? __dsub_rn((double)rw[m], dq) : __dadd_rn((double)rw[m], dq);
-          lmin = fmin(lmin, new_q);
-          lmax = fmax(lmax, new_q);
-          // the edge in the parent's record: q and the child's visit count (child id too for the new node)
-          uint8_t* prec = fs_node(gm, NB, (int)pn[kk - 1]);
-          const int a = (int)pa[kk - 1];
-          *reinterpret_cast<double*>(prec + FS_PQ + 16 * a + 8) = new_q;
-          if (kk == depth) *reinterpret_cast<uint16_t*>(prec + fs_meta_off(a)) = (uint16_t)(newn | (nvc << 8));
-          else *(prec + fs_meta_off(a) + 1) = (uint8_t)nvc;
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int m = 1; m < 4; m <<= 1) {
-    lmin = fmin(lmin, shfl4_xor_f64(lmin, m));
-    lmax = fmax(lmax, shfl4_xor_f64(lmax, m));
-  }
-  if (gm.valid && gm.sub == 0 && depth > 0) {  // MinMaxStats.update mcts.py:11-14
-    if (lmin < sm.mm[2 * gm.gl]) sm.mm[2 * gm.gl] = lmin;
-    if (lmax > sm.mm[2 * gm.gl + 1]) sm.mm[2 * gm.gl + 1] = lmax;
-  }
-  __syncwarp();  // the descent that follows reads what other lanes of the game just stored
-}
-
-// game.py:106-111 + Node.value (mcts.py:42-45): visit counts, child-visit distribution, root value, MinMax
-MZ_DEV void fs_root_stats(const FsParams& p, const FsTreeSmem& sm, const FsGame& gm) {
-  const int A = p.A;
-  uint4 mw = make_uint4(0u, 0u, 0u, 0u);
-  const uint8_t* rec = gm.base + FS_HDR;
-  if (gm.valid) mw = ldg16(rec + FS_META + 16 * gm.sub);
-  int sum = 0;
-#pragma unroll
-  for (int t = 0; t < 8; ++t)
-    if (4 * t + gm.sub < A) sum += (int)(meta_at(mw, t) >> 8);
-  sum += __shfl_xor_sync(MZ_FULL, sum, 1, 4);
-  sum += __shfl_xor_sync(MZ_FULL, sum, 2, 4);
-  if (!gm.valid) return;
-#pragma unroll
-  for (int t = 0; t < 8; ++t) {
-    const int a = 4 * t + gm.sub;
-    if (a < A) {
-      const uint32_t mt = meta_at(mw, t);
-      const int v = (int)(mt >> 8);
-      if (p.visits) p.visits[(size_t)gm.g * A + a] = v;
-      if (p.child_visits)
-        p.child_visits[(size_t)gm.g * A + a] = (mt & 0xffu) != CH_ILLEGAL ? __ddiv_rn((double)v, (double)sum) : 0.0;
-    }
-  }
-  if (gm.sub == 0) {
-    const uint4 o = ldg16(rec);
-    const int n = (int)o.z;
-    if (p.root_value) p.root_value[gm.g] = n == 0 ? 0.0 : __ddiv_rn(u2d(o.x, o.y), (double)n);
-    if (p.minmax) {
-      p.minmax[2 * gm.g] = sm.mm[2 * gm.gl];
-      p.minmax[2 * gm.g + 1] = sm.mm[2 * gm.gl + 1];
-    }
-    *reinterpret_cast<double2*>(gm.base) = make_double2(sm.mm[2 * gm.gl], sm.mm[2 * gm.gl + 1]);
-  }
-}
-
 }  // namespace
 
 #include "mz_fcs_sparse.cuh"
@@ -594,82 +172,66 @@ MZ_DEV void fs_root_stats(const FsParams& p, const FsTreeSmem& sm, const FsGame&
 namespace {
 
 // shared-memory plan (bytes).  Everything a peer CTA addresses (barriers, output slots, A1 / A3 images) sits at
-// the same offset in every CTA of the cluster.  In clusters of four no CTA owns both a dynamics and a prediction
-// head, so the A3 image shares the A1 region.
+// the same offset in every CTA of the cluster.  No CTA owns both a dynamics and a prediction head, so the A3
+// image shares the A1 region.
 __host__ __device__ inline size_t fs_align16(size_t x) { return (x + 15) & ~(size_t)15; }
 struct FsLayout {
-  size_t a1, w, a3, bars, tail, sh, logit, val, rew, sp, mm, pbc, path_n, path_a, depth, total;
-  size_t best_ca, node, xmask, links;  // sparse engine
+  size_t a1, w, bars, tail, sh, logit, val, rew, sp, mm, path_n, path_a, depth, total;
+  size_t best_ca, node, xmask, links;
   size_t exp_tab, rcp, pbf;
-  int ps, a4, gp, s1;
+  int ps, a4, s1;
 };
-__host__ __device__ inline FsLayout fs_layout(int k1, int stages, int cl, int A, int S, bool sparse) {
+__host__ __device__ inline FsLayout fs_layout(int k1, int A, int S) {
   FsLayout L;
-  L.gp = ROWS / cl;
   L.a4 = (A + 3) / 4 * 4;
   L.ps = (S + 2 + 15) / 16 * 16;
   L.s1 = (S + 2) & ~1;
   size_t off = 0;
   L.a1 = off; off += (size_t)ROWS * k1 * 2;
-  L.w = off; off += (size_t)stages * stage_bytes_for(k1);
-  if (cl == 4) {
-    L.a3 = L.a1;
-  } else {
-    L.a3 = off; off += (size_t)ROWS * K3 * 2;
-  }
+  L.w = off; off += (size_t)4 * stage_bytes_for(k1);  // the four chunks of the CTA's head, resident
   L.bars = off; off += 32 * sizeof(uint64_t);
   L.tail = off; off += TAIL_FLOATS * sizeof(float);
   L.sh = off; off += (size_t)ROWS * 128;
-  L.logit = off; off += fs_align16((size_t)L.gp * L.a4 * 4);
-  L.val = off; off += fs_align16((size_t)L.gp * 4);
-  L.rew = off; off += fs_align16((size_t)L.gp * 4);
-  L.mm = off; off += (size_t)L.gp * 16;
-  L.path_n = off; off += (size_t)L.gp * L.ps;
-  L.path_a = off; off += (size_t)L.gp * L.ps;
-  L.depth = off; off += fs_align16((size_t)L.gp);
+  L.logit = off; off += fs_align16((size_t)FS_GP * L.a4 * 4);
+  L.val = off; off += fs_align16((size_t)FS_GP * 4);
+  L.rew = off; off += fs_align16((size_t)FS_GP * 4);
+  L.mm = off; off += (size_t)FS_GP * 16;
+  L.path_n = off; off += (size_t)FS_GP * L.ps;
+  L.path_a = off; off += (size_t)FS_GP * L.ps;
+  L.depth = off; off += fs_align16((size_t)FS_GP);
   L.exp_tab = off; off += 256 * 8;
   L.rcp = off; off += 64 * 8;
   L.pbf = off; off += 64 * 8;
-  L.pbc = L.best_ca = L.node = L.xmask = L.links = 0;
-  if (sparse) {
-    // exp / reward scratch and the per-node maxima are used in different phases: one region
-    const int row = L.s1 > SP_STRIDE ? L.s1 : SP_STRIDE;  // doubles per game (fs2::Smem::row)
-    L.sp = off; off += fs_align16((size_t)L.gp * row * 8);
-    L.best_ca = off; off += (size_t)L.gp * L.s1 * 2;
-    L.links = off; off += fs_align16((size_t)L.gp * L.s1 * 2);
-    L.node = off; off += (size_t)L.gp * L.s1 * 4;
-    L.xmask = off; off += (size_t)L.gp * L.s1 * 4;
-  } else {
-    L.sp = off; off += fs_align16((size_t)L.gp * SP_STRIDE * 8);
-    L.pbc = off; off += fs_align16((size_t)(S + 1) * (S + 2) / 2 * 8);
-  }
+  // exp / reward scratch and the per-node maxima are used in different phases: one region
+  const int row = L.s1 > SP_STRIDE ? L.s1 : SP_STRIDE;  // doubles per game (fs2::Smem::row)
+  L.sp = off; off += fs_align16((size_t)FS_GP * row * 8);
+  L.best_ca = off; off += (size_t)FS_GP * L.s1 * 2;
+  L.links = off; off += fs_align16((size_t)FS_GP * L.s1 * 2);
+  L.node = off; off += (size_t)FS_GP * L.s1 * 4;
+  L.xmask = off; off += (size_t)FS_GP * L.s1 * 4;
   L.total = off;
   return L;
 }
 
 // ======================================================================================================
-// T: actions per lane of the dense engine (four lanes per game); AL > 0 selects the sparse engine (eight lanes
-// per game, AL actions per lane at expansion; clusters of four only)
-template <int T, int AL>
+// AL: actions per lane of the tree engine at expansion (eight lanes per game)
+template <int AL>
 __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
-  constexpr bool SPARSE = AL > 0;
-  constexpr int LANES = SPARSE ? fs2::L : 4;
+  constexpr int LANES = fs2::L;
   extern __shared__ __align__(1024) uint8_t smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int k1 = p.k1, cl = p.cl, S = p.S, A = p.A;
+  const int k1 = p.k1, S = p.S, A = p.A;
   const int stage_bytes = stage_bytes_for(k1);
   const int rank = (int)cluster_ctarank();
-  const int tile = (int)blockIdx.x / cl;
-  const int GP = ROWS / cl;
-  const int STAGES = p.stages;
-  // head -> rank: CL = 2: reward, value on rank 0, transition, policy on rank 1; CL = 4: one head per rank
-  const int rank_value = cl == 2 ? 0 : 2, rank_policy = cl == 2 ? 1 : 3;
-  const bool has_dyn = rank < 2, has_pred = cl == 2 || rank >= 2;
+  const int tile = (int)blockIdx.x / FS_CL;
+  // games whose tree this CTA runs (FS_GP), read from the launched cluster size rather than folded from the constant:
+  // with the constant nvcc schedules the tree engine of the 17..24-action instantiation worse (C4 on a B200 at
+  // 1000 W: 198 vs 214 M expansions/s)
+  const int GP = ROWS / (int)cluster_nctarank();
+  // head -> rank: 0 reward, 1 transition (the dynamics heads), 2 value, 3 policy (the prediction heads)
+  constexpr int rank_value = 2, rank_policy = 3;
+  const bool has_dyn = rank < 2;
   const bool own_reward = rank == 0, own_trans = rank == 1, own_value = rank == rank_value, own_policy = rank == rank_policy;
-  const int nch = cl == 2 ? 8 : 4;  // chunks this CTA runs per simulation
-  const bool resident = nch <= STAGES;  // the CTA's weights fit the ring: loaded once
-  const int c_pred = has_dyn ? 4 : 0;   // first chunk of the prediction head
-  auto canon = [&](int c) { return cl == 2 ? (c < 4 ? 4 * rank + c : 8 + 4 * rank + (c - 4)) : 4 * rank + c; };
   int* const err = p.error_flag;
 
   if (p.timeline && blockIdx.x == 0 && threadIdx.x == 64) {  // diagnostics: kernel entry (cycles, ns)
@@ -678,75 +240,59 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
     p.timeline[27] = clock64();
     p.timeline[29] = (long long)ns;
   }
-  const FsLayout L = fs_layout(k1, STAGES, cl, A, S, SPARSE);
-  uint8_t* sA1 = smem + L.a1;
+  const FsLayout L = fs_layout(k1, A, S);
+  uint8_t* sA1 = smem + L.a1;  // A1 image on the dynamics ranks, A3 (h') image on the prediction ranks
   uint8_t* sW = smem + L.w;
-  uint8_t* sA3 = smem + L.a3;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L.bars);
   uint64_t* w_full = bars;            // [4]
-  uint64_t* w_empty = bars + 4;       // [4]
-  uint64_t* d1_full = bars + 8;       // [2]
-  uint64_t* d1_empty = bars + 10;     // [2]
-  uint64_t* a2_full = bars + 12;      // [2]
-  uint64_t* a2_empty = bars + 14;     // [2]
-  uint64_t* a1_full = bars + 16;      // tx: the tile's A1 rows have arrived (st.async from the tree lanes)
-  uint64_t* a1_ready = bars + 17;     // epilogue warps -> layer-1 issuer (after the async-proxy fence)
-  uint64_t* a3_full = bars + 18;      // tx: h' rows from the transition head
-  uint64_t* a3_ready = bars + 19;
-  uint64_t* d2_full = bars + 20;
-  uint64_t* h_staged = bars + 21;     // transition rank: h' rows are in the staging area
-  uint64_t* out_full = bars + 22;     // tx: value / reward / logits of this CTA's games + the pool rows' release
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 24);
+  uint64_t* d1_full = bars + 4;       // [2]
+  uint64_t* d1_empty = bars + 6;      // [2]
+  uint64_t* a2_full = bars + 8;       // [2]
+  uint64_t* a2_empty = bars + 10;     // [2]
+  uint64_t* a1_full = bars + 12;      // tx: the tile's A1 rows have arrived (st.async from the tree lanes)
+  uint64_t* a1_ready = bars + 13;     // epilogue warps -> layer-1 issuer (after the async-proxy fence)
+  uint64_t* a3_full = bars + 14;      // tx: h' rows from the transition head
+  uint64_t* a3_ready = bars + 15;
+  uint64_t* d2_full = bars + 16;
+  uint64_t* h_staged = bars + 17;     // transition rank: h' rows are in the staging area
+  uint64_t* out_full = bars + 18;     // tx: value / reward / logits of this CTA's games + the pool rows' release
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 20);
   float* sTail = reinterpret_cast<float*>(smem + L.tail);
   uint8_t* sH = smem + L.sh;  // [128][8 x 16 B], block index XOR (row & 7)
-  FsTreeSmem sm;
+  fs2::Smem sm;
   sm.logit = reinterpret_cast<float*>(smem + L.logit);
   sm.val = reinterpret_cast<float*>(smem + L.val);
   sm.rew = reinterpret_cast<float*>(smem + L.rew);
-  sm.sp = reinterpret_cast<double*>(smem + L.sp);
   sm.mm = reinterpret_cast<double*>(smem + L.mm);
-  double* pbc_w = reinterpret_cast<double*>(smem + L.pbc);
-  sm.pbc = pbc_w;
+  sm.sp = reinterpret_cast<double*>(smem + L.sp);
+  sm.best_key = reinterpret_cast<unsigned long long*>(smem + L.sp);
+  sm.best_ca = reinterpret_cast<uint16_t*>(smem + L.best_ca);
+  sm.first = smem + L.links;
+  sm.next = smem + L.links + (size_t)GP * L.s1;
+  sm.node = reinterpret_cast<uint32_t*>(smem + L.node);
+  sm.xmask = reinterpret_cast<uint32_t*>(smem + L.xmask);
   sm.path_n = smem + L.path_n;
   sm.path_a = smem + L.path_a;
   sm.depth = smem + L.depth;
-  sm.ps = L.ps;
-  sm.a4 = L.a4;
+  sm.ps = L.ps; sm.a4 = L.a4; sm.s1 = L.s1;
+  sm.row = L.s1 > SP_STRIDE ? L.s1 : SP_STRIDE;
   unsigned long long* exp_tab_w = reinterpret_cast<unsigned long long*>(smem + L.exp_tab);
   sm.exp_tab = exp_tab_w;
   for (int i = threadIdx.x; i < 256; i += FS_THREADS) exp_tab_w[i] = mz_exp_tab[i];
-  fs2::Smem sm2;
-  sm2.logit = sm.logit; sm2.val = sm.val; sm2.rew = sm.rew; sm2.mm = sm.mm; sm2.sp = sm.sp;
-  sm2.best_key = reinterpret_cast<unsigned long long*>(smem + L.sp);
-  sm2.best_ca = reinterpret_cast<uint16_t*>(smem + L.best_ca);
-  sm2.first = smem + L.links;
-  sm2.next = smem + L.links + (size_t)L.gp * L.s1;
-  sm2.node = reinterpret_cast<uint32_t*>(smem + L.node);
-  sm2.xmask = reinterpret_cast<uint32_t*>(smem + L.xmask);
-  sm2.path_n = sm.path_n; sm2.path_a = sm.path_a; sm2.depth = sm.depth;
-  sm2.ps = L.ps; sm2.a4 = L.a4; sm2.s1 = L.s1;
-  sm2.row = L.s1 > SP_STRIDE ? L.s1 : SP_STRIDE;
-  sm2.exp_tab = exp_tab_w;
   double* rcp_w = reinterpret_cast<double*>(smem + L.rcp);
-  sm2.rcp = rcp_w;
+  sm.rcp = rcp_w;
   for (int i = threadIdx.x; i < 64; i += FS_THREADS) rcp_w[i] = i > 0 ? __drcp_rn((double)i) : 0.0;
   double* pbc0_w = reinterpret_cast<double*>(smem + L.pbf);
-  sm2.pbc0 = pbc0_w;
+  sm.pbc0 = pbc0_w;
   for (int i = threadIdx.x; i < 64; i += FS_THREADS) pbc0_w[i] = i <= S ? p.pb_c[(size_t)i * (S + 1)] : 0.0;
-  const fs2::Geo geo2 = fs2::geo(S, A);
+  const fs2::Geo geo = fs2::geo(S, A);
 
   const uint32_t a1_bytes = (uint32_t)(ROWS * k1 * 2), a3_bytes = (uint32_t)(ROWS * K3 * 2);
   const uint32_t out_bytes = (uint32_t)(GP * (8 + 4 * L.a4));
 
   for (int i = threadIdx.x; i < TAIL_FLOATS; i += FS_THREADS) sTail[i] = p.tail[i];
-  if (!SPARSE) {
-    for (int i = threadIdx.x; i < (S + 1) * (S + 1); i += FS_THREADS) {
-      const int N = i / (S + 1), n = i % (S + 1);
-      if (n <= N) pbc_w[(N * (N + 1)) / 2 + n] = p.pb_c[i];
-    }
-  }
   if (threadIdx.x == 0) {
-    for (int i = 0; i < 4; ++i) { mbar_init(&w_full[i], 1); mbar_init(&w_empty[i], 1); }
+    for (int i = 0; i < 4; ++i) mbar_init(&w_full[i], 1);
     for (int i = 0; i < 2; ++i) {
       mbar_init(&d1_full[i], 1);
       mbar_init(&d1_empty[i], EPI_THREADS / 32);
@@ -773,81 +319,64 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
   const uint32_t tmem = *tmem_ptr;
 
   if (warp == 0) {
-    // ===== producer: weight chunks through the ring (once when the CTA's heads fit it) =====
+    // ===== producer: the four weight chunks of the CTA's head, loaded once for the whole move =====
     if (lane == 0) {
-      size_t offs[8];
-      int nbytes[8];
-      for (int c = 0; c < nch; ++c) {
-        offs[c] = chunk_offset(canon(c), k1);
-        nbytes[c] = chunk_geom(canon(c), k1).bytes;
-      }
-      const int total = resident ? nch : S * nch;
-      int st = 0, round = 0, c = 0;
-      for (int n = 0; n < total; ++n) {
-        fs_wait(&w_empty[st], (round & 1) ^ 1, err, 1);
-        mbar_arrive_expect_tx(&w_full[st], (uint32_t)nbytes[c]);
-        bulk_copy_g2s(sW + st * stage_bytes, p.chunks + offs[c], (uint32_t)nbytes[c], &w_full[st]);
-        if (++st == STAGES) { st = 0; ++round; }
-        if (++c == nch) c = 0;
+      for (int c = 0; c < 4; ++c) {
+        const int bytes = chunk_geom(4 * rank + c, k1).bytes;
+        mbar_arrive_expect_tx(&w_full[c], (uint32_t)bytes);
+        bulk_copy_g2s(sW + c * stage_bytes, p.chunks + chunk_offset(4 * rank + c, k1), (uint32_t)bytes, &w_full[c]);
       }
     }
   } else if (warp == 1) {
     // ===== layer-1 MMA issuer (converged warp, one elected lane issues) =====
-    const uint32_t a1_addr = smem_u32(sA1), a3_addr = smem_u32(sA3), w_addr = smem_u32(sW);
+    const uint32_t a1_addr = smem_u32(sA1), w_addr = smem_u32(sW);
     const uint32_t idesc1 = make_idesc(CHUNK);
     constexpr uint64_t KSTEP = (uint64_t)((2 * (CHUNK / 8) * 128) >> 4);
-    int st = 0, round = 0, gc = 0;
+    int gc = 0;
     for (int sim = 0; sim < S; ++sim) {
-      for (int c = 0; c < nch; ++c, ++gc) {
-        const int cc = canon(c);
-        if (!resident || sim == 0) fs_wait(&w_full[st], round & 1, err, 2);
-        if (has_dyn && c == 0) fs_wait(a1_ready, sim & 1, err, 3);
-        if (has_pred && c == c_pred) fs_wait(a3_ready, sim & 1, err, 4);
+      for (int c = 0; c < 4; ++c, ++gc) {
+        if (sim == 0) fs_wait(&w_full[c], 0, err, 2);
+        if (c == 0) {
+          if (has_dyn) fs_wait(a1_ready, sim & 1, err, 3);
+          else fs_wait(a3_ready, sim & 1, err, 4);
+        }
         fs_wait(&d1_empty[gc & 1], ((gc >> 1) & 1) ^ 1, err, 5);
         tc_fence_after();
         const uint32_t d1 = tmem + COL_D1 + (gc & 1) * CHUNK;
-        const uint64_t bd = make_desc(w_addr + st * stage_bytes, (CHUNK / 8) * 128, 128);
+        const uint64_t ad = make_desc(a1_addr, (ROWS / 8) * 128, 128);
+        const uint64_t bd = make_desc(w_addr + c * stage_bytes, (CHUNK / 8) * 128, 128);
         if (elect_one()) {
-          if (cc < 8) {  // dynamics: A = [h | onehot | 1] (K = k1)
-            const uint64_t ad = make_desc(a1_addr, (ROWS / 8) * 128, 128);
-            umma_ss<false>(d1, ad, bd, idesc1);
+          umma_ss<false>(d1, ad, bd, idesc1);
+          if (has_dyn) {  // dynamics: A = [h | onehot | 1] (K = k1)
 #pragma unroll 1
             for (int ks = 1; ks < k1 / 16; ++ks) umma_ss<true>(d1, ad + ks * KSTEP, bd + ks * KSTEP, idesc1);
-          } else {       // prediction: A = [h' | 1] (K = 64)
-            const uint64_t ad = make_desc(a3_addr, (ROWS / 8) * 128, 128);
-            umma_ss<false>(d1, ad, bd, idesc1);
+          } else {        // prediction: A = [h' | 1] (K = 64)
 #pragma unroll
             for (int ks = 1; ks < K3 / 16; ++ks) umma_ss<true>(d1, ad + ks * KSTEP, bd + ks * KSTEP, idesc1);
           }
           tc_commit(&d1_full[gc & 1]);
         }
         __syncwarp();
-        if (++st == STAGES) { st = 0; ++round; }
-        if (resident && c == nch - 1) st = 0;
       }
     }
   } else if (warp == MMA2_WARP) {
     // ===== layer-2 MMA issuer =====
     const uint32_t w_addr = smem_u32(sW);
-    const uint32_t w1_bytes_dyn = CHUNK * k1 * 2, w1_bytes_pred = CHUNK * K3 * 2;
-    int st = 0, gc = 0;
+    const uint32_t w1_bytes = has_dyn ? CHUNK * k1 * 2 : CHUNK * K3 * 2;
+    int gc = 0;
     for (int sim = 0; sim < S; ++sim) {
-      for (int c = 0; c < nch; ++c, ++gc) {
-        const int cc = canon(c), head = cc >> 2;
+      for (int c = 0; c < 4; ++c, ++gc) {
         fs_wait(&a2_full[gc & 1], (gc >> 1) & 1, err, 6);
         tc_fence_after();
         const uint32_t a_tm = tmem + COL_A2 + (gc & 1) * (CHUNK / 2);
-        const uint32_t b_addr = w_addr + st * stage_bytes + (cc < 8 ? w1_bytes_dyn : w1_bytes_pred);
+        const uint32_t b_addr = w_addr + c * stage_bytes + w1_bytes;
         if (elect_one()) {
-          if (head == 1) issue_mma2<N_HID>(tmem + COL_D2B, a_tm, b_addr, (cc & 3) == 0);
-          else issue_mma2<32>(tmem + ((head & 1) ? COL_D2B : COL_D2A), a_tm, b_addr, (cc & 3) == 0);
-          if (!resident) tc_commit(&w_empty[st]);
+          if (own_trans) issue_mma2<N_HID>(tmem + COL_D2B, a_tm, b_addr, c == 0);
+          else issue_mma2<32>(tmem + ((rank & 1) ? COL_D2B : COL_D2A), a_tm, b_addr, c == 0);
           tc_commit(&a2_empty[gc & 1]);
-          if ((c & 3) == 3) tc_commit(d2_full);
+          if (c == 3) tc_commit(d2_full);
         }
         __syncwarp();
-        if (++st == STAGES) st = 0;
-        if (resident && c == nch - 1) st = 0;
       }
     }
   } else if (warp == STORE_WARP) {
@@ -866,7 +395,7 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
           }
         }
         __syncwarp();
-        if (lane < cl) mbar_arrive_remote_release(map_to_cta(smem_u32(out_full), (uint32_t)lane));
+        if (lane < FS_CL) mbar_arrive_remote_release(map_to_cta(smem_u32(out_full), (uint32_t)lane));
         __syncwarp();
       }
     }
@@ -878,14 +407,12 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
     const int e = (warp - 2) * 32 + lane;         // 0..255
     const uint32_t lane_addr = tmem + ((uint32_t)(quarter * 32) << 16);
     const bool tree_role = e < LANES * GP;
-    FsGame gm;
+    fs2::Game gm;
     gm.gl = tree_role ? (e / LANES) : 0;
     gm.sub = e % LANES;
     gm.g = tile * ROWS + rank * GP + gm.gl;
     gm.valid = tree_role && gm.g < p.G;
     gm.base = p.games + (size_t)(gm.valid ? gm.g : 0) * p.game_bytes;
-    fs2::Game gm2;
-    gm2.valid = gm.valid; gm2.g = gm.g; gm2.gl = gm.gl; gm2.sub = gm.sub; gm2.base = gm.base;
     const int my_row = rank * GP + gm.gl;         // tile row of the game this lane works on
     const bool stamp = p.timeline && blockIdx.x == 0 && e == 0;
 #define FS_STAMP(sim_, slot_)                                           \
@@ -900,16 +427,13 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
     auto arm = [&]() {  // one thread arms this simulation's transaction barriers
       if (e == 0) {
         if (has_dyn) mbar_arrive_expect_tx(a1_full, a1_bytes);
-        if (has_pred) mbar_arrive_expect_tx(a3_full, a3_bytes);
+        else mbar_arrive_expect_tx(a3_full, a3_bytes);
         mbar_arrive_expect_tx(out_full, out_bytes);
       }
     };
     arm();
     FS_STAMP(0, 13);
-    if (tree_role) {
-      if constexpr (SPARSE) fs2::set_root<(AL > 0 ? AL : 1)>(p, sm2, gm2, geo2);
-      else fs_set_root<T>(p, sm, gm);
-    }
+    if (tree_role) fs2::set_root<AL>(p, sm, gm, geo);
     __syncwarp();
     FS_STAMP(0, 14);
 
@@ -948,29 +472,19 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
       FS_STAMP(sim < S ? sim : S - 1, sim < S ? 0 : 12);
       if (sim > 0) {
         if (tree_role) {
-          if constexpr (SPARSE) {
-            fs2::Pre pre;
-            fs2::pre_expand<(AL > 0 ? AL : 1)>(p, sm2, gm2, geo2, pre);  // overlaps the wait for the outputs
-            fs_wait_cluster(out_full, (sim - 1) & 1, err, 10);
-            if (sim < S) arm();
-            FS_STAMP(sim - 1, 10);
-            fs2::expand_backup<(AL > 0 ? AL : 1)>(p, sm2, gm2, geo2, sim - 1, pre,
-                                                  stamp ? p.timeline + (size_t)(sim - 1) * 32 : nullptr);
-          } else {
-            fs_wait_cluster(out_full, (sim - 1) & 1, err, 10);
-            if (sim < S) arm();
-            FS_STAMP(sim - 1, 10);
-            fs_expand_backup<T>(p, sm, gm, sim - 1);
-          }
+          fs2::Pre pre;
+          fs2::pre_expand<AL>(p, sm, gm, geo, pre);  // overlaps the wait for the outputs
+          fs_wait_cluster(out_full, (sim - 1) & 1, err, 10);
+          if (sim < S) arm();
+          FS_STAMP(sim - 1, 10);
+          fs2::expand_backup<AL>(p, sm, gm, geo, sim - 1, pre, stamp ? p.timeline + (size_t)(sim - 1) * 32 : nullptr);
           FS_STAMP(sim - 1, 11);
         }
       }
       if (sim == S) break;
       if (tree_role) {
         int parent, action;
-        if constexpr (SPARSE)
-          fs2::descend(p, sm2, gm2, geo2, sim, parent, action, stamp ? p.timeline + (size_t)sim * 32 : nullptr);
-        else fs_descend<T>(p, sm, gm, sim, parent, action);
+        fs2::descend(p, sm, gm, geo, sim, parent, action, stamp ? p.timeline + (size_t)sim * 32 : nullptr);
         FS_STAMP(sim, 1);
         // A1 row of the game: bf16([h (50) | onehot(action) (A) | 1 | 0]) as 16-byte blocks of the canonical
         // K-major image, sent to every CTA that owns a dynamics head (ranks 0 and 1)
@@ -1082,7 +596,7 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
           for (int j = H + 1; j < 64; ++j) hbuf[j] = 0.0f;
           // h' as bf16: the A operand of the prediction layer of the CTAs that own those heads, and the pool row
           const uint32_t pr0 = (uint32_t)rank_value, pr1 = (uint32_t)rank_policy;
-          const uint32_t a3_p0 = map_to_cta(smem_u32(sA3), pr0), a3_p1 = map_to_cta(smem_u32(sA3), pr1);
+          const uint32_t a3_p0 = map_to_cta(smem_u32(sA1), pr0), a3_p1 = map_to_cta(smem_u32(sA1), pr1);
           const uint32_t bar_p0 = map_to_cta(smem_u32(a3_full), pr0), bar_p1 = map_to_cta(smem_u32(a3_full), pr1);
           uint4 q[K3 / 8];
 #pragma unroll
@@ -1100,8 +614,7 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
           if (lane == 0) mbar_arrive(h_staged);  // the store warp takes it from here
         }
         FS_STAMP(sim, 5);
-      }
-      if (has_pred) {
+      } else {
         if (grp == 0) {
           fs_wait_cluster(a3_full, sim & 1, err, 13);
           fence_async_smem();
@@ -1140,10 +653,7 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
         FS_STAMP(sim, 8);
       }
     }
-    if (tree_role) {
-      if constexpr (SPARSE) fs2::root_stats(p, sm2, gm2, geo2);
-      else fs_root_stats(p, sm, gm);
-    }
+    if (tree_role) fs2::root_stats(p, sm, gm, geo);
     FS_STAMP(S - 1, 15);
 #undef FS_STAMP
   }
@@ -1163,26 +673,6 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
 }
 
 // one game of the fused engine's tree as the arrays of mz_tree_export (tests / the Node facade)
-__global__ void fs_export_kernel(const uint8_t* games, long long game_bytes, int node_bytes, int S, int A, int game,
-                                 double* prior, int32_t* child, double* vsum, int32_t* visit, float* reward,
-                                 double* q_out) {
-  const uint8_t* base = games + (size_t)game * game_bytes + FS_HDR;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < (S + 1) * A; i += gridDim.x * blockDim.x) {
-    const int n = i / A, a = i % A;
-    const uint8_t* rec = base + (size_t)n * node_bytes;
-    const uint16_t mt = *reinterpret_cast<const uint16_t*>(rec + fs_meta_off(a));
-    const int ch = mt & 0xff;
-    if (prior) prior[i] = *reinterpret_cast<const double*>(rec + FS_PQ + 16 * a);
-    if (q_out) q_out[i] = *reinterpret_cast<const double*>(rec + FS_PQ + 16 * a + 8);
-    if (child) child[i] = ch == CH_UNEXP ? MZ_CHILD_UNEXPANDED : (ch == CH_ILLEGAL ? MZ_CHILD_ILLEGAL : ch);
-    if (a == 0) {
-      if (vsum) vsum[n] = *reinterpret_cast<const double*>(rec);
-      if (visit) visit[n] = *reinterpret_cast<const int32_t*>(rec + 8);
-      if (reward) reward[n] = *reinterpret_cast<const float*>(rec + 12);
-    }
-  }
-}
-
 __global__ void fs2_export_kernel(const uint8_t* games, long long game_bytes, int S, int A, int game, double* prior,
                                   int32_t* child, double* vsum, int32_t* visit, float* reward, double* q_out) {
   const fs2::Geo G = fs2::geo(S, A);
@@ -1212,54 +702,28 @@ __global__ void fs2_export_kernel(const uint8_t* games, long long game_bytes, in
 int fs_k1_for(int A) { return (H + A + 1 + 15) / 16 * 16; }
 constexpr size_t kFsMaxSmem = 232448;
 
-int g_fs_cluster = 0;  // 0: from MZ_FS_CLUSTER (default 2)
-int fs_cluster() {
-  if (g_fs_cluster == 0) {
-    const char* e = getenv("MZ_FS_CLUSTER");
-    const int v = e ? atoi(e) : 4;
-    g_fs_cluster = (v == 2) ? 2 : 4;
-  }
-  return g_fs_cluster;
-}
-int g_fs_engine = -1;  // -1: from MZ_FS_ENGINE (default 1 = sparse when the shape allows), 0 dense, 1 sparse
-int fs_engine_pref() {
-  if (g_fs_engine < 0) {
-    const char* e = getenv("MZ_FS_ENGINE");
-    g_fs_engine = e ? (atoi(e) != 0 ? 1 : 0) : 1;
-  }
-  return g_fs_engine;
-}
-int fs_stages(int cl);
-bool fs_sparse_ok(int cl, int S, int A) {
-  if (cl != 4 || S > fs2::MAX_S) return false;
-  return fs_layout(fs_k1_for(A), fs_stages(cl), cl, A, S, true).total <= kFsMaxSmem;
-}
-bool fs_use_sparse(int cl, int S, int A) { return fs_engine_pref() == 1 && fs_sparse_ok(cl, S, A); }
-
-int fs_stages(int cl) {
-  const char* e = getenv("MZ_FS_STAGES");
-  const int v = e ? atoi(e) : 0;
-  if (v >= 2 && v <= 4) return v;
-  return cl == 4 ? 4 : 3;
+// the shapes the kernel takes: S <= 63 (fs2::MAX_S) and a shared-memory plan within the opt-in maximum
+bool fs_fits(int S, int A) {
+  return A >= 1 && A <= 32 && S >= 1 && S <= fs2::MAX_S && fs_layout(fs_k1_for(A), A, S).total <= kFsMaxSmem;
 }
 
-template <int T, int AL>
+template <int AL>
 int fs_launch(const FsParams& p, size_t smem, void* stream) {
   static bool attr = false;
   if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(fc_search_kernel<T, AL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFsMaxSmem);
+    cudaError_t e = cudaFuncSetAttribute(fc_search_kernel<AL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFsMaxSmem);
     if (e != cudaSuccess) return (int)e;
     attr = true;
   }
   const int tiles = (p.G + ROWS - 1) / ROWS;
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(tiles * p.cl);
+  cfg.gridDim = dim3(tiles * FS_CL);
   cfg.blockDim = dim3(FS_THREADS);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = (cudaStream_t)stream;
   cudaLaunchAttribute lattr[2];
   lattr[0].id = cudaLaunchAttributeClusterDimension;
-  lattr[0].val.clusterDim.x = p.cl;
+  lattr[0].val.clusterDim.x = FS_CL;
   lattr[0].val.clusterDim.y = 1;
   lattr[0].val.clusterDim.z = 1;
   lattr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -1268,7 +732,7 @@ int fs_launch(const FsParams& p, size_t smem, void* stream) {
   // (launching it as a programmatic dependent of the initial-inference kernel was measured: no gain -- 204.5 vs
   // 203.7 M expansions/s on C4, slightly slower on C1 / C3 -- so it is a plain launch)
   cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, fc_search_kernel<T, AL>, p);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, fc_search_kernel<AL>, p);
   if (e != cudaSuccess) return (int)e;
   MZ_LAUNCH_CHECK();
   return MZ_OK;
@@ -1278,40 +742,14 @@ int fs_launch(const FsParams& p, size_t smem, void* stream) {
 
 extern "C" {
 
-int mz_fc_search_set_cluster(int32_t cluster) {
-  if (cluster != 0 && cluster != 2 && cluster != 4) return MZ_ERR_BAD_ARG;
-  g_fs_cluster = cluster;
-  return MZ_OK;
-}
-
-int32_t mz_fc_search_node_bytes(int32_t A) {
-  if (A < 1 || A > 32) return MZ_ERR_UNSUPPORTED;
-  return (FS_PQ + 16 * A + 63) / 64 * 64;
-}
-
-int64_t mz_fc_search_game_bytes(int32_t S, int32_t A) {  // large enough for either engine's layout
-  if (A < 1 || A > 32 || S < 1 || S > 253) return MZ_ERR_UNSUPPORTED;
-  int64_t b = FS_HDR + (int64_t)(S + 1) * mz_fc_search_node_bytes(A);
-  b = (b + 127) / 128 * 128;
-  const int64_t b2 = fs2::geo(S, A).bytes;
-  return b > b2 ? b : b2;
-}
-
-int mz_fc_search_set_engine(int32_t engine) {
-  if (engine < -1 || engine > 1) return MZ_ERR_BAD_ARG;
-  g_fs_engine = engine;
-  return MZ_OK;
+int64_t mz_fc_search_game_bytes(int32_t S, int32_t A) {
+  if (!fs_fits(S, A)) return MZ_ERR_UNSUPPORTED;
+  return fs2::geo(S, A).bytes;
 }
 
 int32_t mz_fc_search_pool_row(void) { return POOL_ROW; }
 
-int mz_fc_search_supported(int32_t S, int32_t A) {
-  if (A < 1 || A > 32 || S < 1 || S > 253) return 0;
-  const int cl = fs_cluster();
-  if (fs_use_sparse(cl, S, A)) return 1;
-  const FsLayout L = fs_layout(fs_k1_for(A), fs_stages(cl), cl, A, S, false);
-  return L.total <= kFsMaxSmem ? 1 : 0;
-}
+int mz_fc_search_supported(int32_t S, int32_t A) { return fs_fits(S, A) ? 1 : 0; }
 
 int mz_fc_search(const mz_fc_search_args* a, void* stream) {
   if (!a || !a->weights || !a->packed || !a->tail || !a->games || !a->pb_c_table || !a->pool || !a->root_logits ||
@@ -1319,12 +757,9 @@ int mz_fc_search(const mz_fc_search_args* a, void* stream) {
     return MZ_ERR_BAD_ARG;
   const mz_fc_weights* w = a->weights;
   if (a->num_games < 1 || a->num_simulations < 1) return MZ_ERR_BAD_ARG;
-  if (w->num_actions < 1 || w->num_actions > 32 || w->value_bins > 32 || w->reward_bins > 32 ||
-      a->num_simulations > 253 || w->no_support)
+  if (w->value_bins > 32 || w->reward_bins > 32 || w->no_support || !fs_fits(a->num_simulations, w->num_actions))
     return MZ_ERR_UNSUPPORTED;
-  if (a->node_bytes != mz_fc_search_node_bytes(w->num_actions) ||
-      a->game_bytes < mz_fc_search_game_bytes(a->num_simulations, w->num_actions))
-    return MZ_ERR_BAD_ARG;
+  if (a->game_bytes < mz_fc_search_game_bytes(a->num_simulations, w->num_actions)) return MZ_ERR_BAD_ARG;
   FsParams p;
   p.chunks = (const uint8_t*)a->packed;
   p.tail = a->tail;
@@ -1333,8 +768,6 @@ int mz_fc_search(const mz_fc_search_args* a, void* stream) {
   p.value_min = w->value_min;
   p.reward_min = w->reward_min;
   p.no_tt = w->no_target_transform;
-  p.cl = fs_cluster();
-  p.stages = fs_stages(p.cl);
   p.G = a->num_games;
   p.S = a->num_simulations;
   p.two_players = a->two_players;
@@ -1347,7 +780,6 @@ int mz_fc_search(const mz_fc_search_args* a, void* stream) {
   p.pb_c = a->pb_c_table;
   p.games = a->games;
   p.game_bytes = a->game_bytes;
-  p.node_bytes = a->node_bytes;
   p.pool = (__nv_bfloat16*)a->pool;
   p.root_logits = a->root_logits;
   p.legal = a->legal_mask;
@@ -1366,35 +798,20 @@ int mz_fc_search(const mz_fc_search_args* a, void* stream) {
   p.rec_logits = a->rec_logits;
   p.timeline = (long long*)a->timeline;
   p.error_flag = a->error_flag;
-  const bool sparse = fs_use_sparse(p.cl, p.S, p.A);
-  const FsLayout L = fs_layout(p.k1, p.stages, p.cl, p.A, p.S, sparse);
-  if (L.total > kFsMaxSmem) return MZ_ERR_UNSUPPORTED;
-  if (sparse) {
-    const int AL = (p.A + fs2::L - 1) / fs2::L;
-    if (AL <= 1) return fs_launch<1, 1>(p, L.total, stream);
-    if (AL <= 2) return fs_launch<1, 2>(p, L.total, stream);
-    if (AL <= 3) return fs_launch<1, 3>(p, L.total, stream);
-    return fs_launch<1, 4>(p, L.total, stream);
-  }
-  const int T = (p.A + 3) / 4;
-  if (T <= 1) return fs_launch<1, 0>(p, L.total, stream);
-  if (T <= 2) return fs_launch<2, 0>(p, L.total, stream);
-  if (T <= 3) return fs_launch<3, 0>(p, L.total, stream);
-  if (T <= 5) return fs_launch<5, 0>(p, L.total, stream);
-  return fs_launch<8, 0>(p, L.total, stream);
+  const size_t smem = fs_layout(p.k1, p.A, p.S).total;
+  const int AL = (p.A + fs2::L - 1) / fs2::L;
+  if (AL <= 1) return fs_launch<1>(p, smem, stream);
+  if (AL <= 2) return fs_launch<2>(p, smem, stream);
+  if (AL <= 3) return fs_launch<3>(p, smem, stream);
+  return fs_launch<4>(p, smem, stream);
 }
 
 int mz_fc_search_export(const mz_fc_search_args* a, int32_t game, double* prior, int32_t* child, double* vsum,
                         int32_t* visit, float* reward, double* q, void* stream) {
   if (!a || !a->games || !a->weights || game < 0 || game >= a->num_games) return MZ_ERR_BAD_ARG;
-  if (fs_use_sparse(fs_cluster(), a->num_simulations, a->weights->num_actions))
-    fs2_export_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(a->games, a->game_bytes, a->num_simulations,
-                                                           a->weights->num_actions, game, prior, child, vsum, visit,
-                                                           reward, q);
-  else
-    fs_export_kernel<<<4, 128, 0, (cudaStream_t)stream>>>(a->games, a->game_bytes, a->node_bytes, a->num_simulations,
-                                                          a->weights->num_actions, game, prior, child, vsum, visit,
-                                                          reward, q);
+  fs2_export_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(a->games, a->game_bytes, a->num_simulations,
+                                                         a->weights->num_actions, game, prior, child, vsum, visit,
+                                                         reward, q);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }

@@ -303,7 +303,6 @@ class _FusedEngine(object):
     self.net, self.lib = fcnet, fcnet.lib
     G, S, A, dev = parent.G, parent.S, parent.A, fcnet.device
     self.G, self.S, self.A = G, S, A
-    self.node_bytes = int(self.lib.mz_fc_search_node_bytes(A))
     self.game_bytes = int(self.lib.mz_fc_search_game_bytes(S, A))
     self.games = torch.zeros(G * self.game_bytes, dtype=torch.uint8, device=dev)
     self.pool = torch.zeros((G, S + 1, int(self.lib.mz_fc_search_pool_row())), dtype=torch.bfloat16, device=dev)
@@ -318,7 +317,7 @@ class _FusedEngine(object):
     a = self.args
     a.num_games, a.num_simulations, a.two_players = G, S, int(bool(config.two_players))
     a.prior_sum_mode = default_prior_sum_mode()
-    a.node_bytes, a.game_bytes = self.node_bytes, self.game_bytes
+    a.game_bytes = self.game_bytes
     a.discount, a.init_value_score = float(config.discount), float(config.init_value_score)
     a.min_bound = math.inf if kb[0] is None else float(kb[0])
     a.max_bound = -math.inf if kb[1] is None else float(kb[1])
@@ -392,8 +391,10 @@ class FCSearch(object):
   def __init__(self, config, fcnet, num_games, noise_frac=None, use_graph=True, num_streams=1, fused=None):
     """fused: True = the whole move in one persistent kernel (`mz_fc_search`, csrc/mz_fcsearch.cu), False =
     one tree launch + one network launch per simulation on `num_streams` slices, None = fused whenever the
-    network runs in bf16, the shape fits the kernel and at most 8192 games play (MZ_FUSED=0 in the environment turns the default off).
-    Both give bit-identical searches (tests/test_gpu_fcnet.py)."""
+    network runs in bf16, at most 8192 games play and the shape fits the kernel: S <= 63 and (S, A) within its
+    shared-memory plan, as `mz_fc_search_supported` reports (S <= 63 for A <= 13, S <= 55 for A <= 20, S <= 53 for
+    A <= 29, S <= 19 for A <= 32).  Every other shape runs the per-launch path; MZ_FUSED=0 in the environment turns
+    the default off.  Both give bit-identical searches (tests/test_gpu_fcnet.py)."""
     self.net = fcnet
     G, A, dev = int(num_games), int(config.action_space), fcnet.device
     self.G, self.A, self.S = G, A, int(config.num_simulations)
@@ -429,8 +430,8 @@ class FCSearch(object):
       # few per cent from 16 384 games on, where the per-launch path has more games in flight per SM
       fused = can_fuse and os.environ.get("MZ_FUSED", "1") != "0" and G <= 8192
     elif fused and not can_fuse:
-      raise ValueError("the fused search kernel needs a bf16 FCNetwork with loaded weights, A <= 32 and a "
-                       "tree that fits its shared-memory plan")
+      raise ValueError("the fused search kernel needs a bf16 FCNetwork with loaded weights, A <= 32, S <= 63 "
+                       "and a tree that fits its shared-memory plan")
     self.fused = _FusedEngine(config, fcnet, self) if fused else None
     self.lanes = []
     self.eng = None
@@ -484,78 +485,6 @@ class FCSearch(object):
     """All launches of one move; lanes fork from / join back into the current stream."""
     if self.fused is not None:
       stream_ptr = torch.cuda.current_stream().cuda_stream
-      key = (bool(self.use_noise), float(self.noise_frac), stream_ptr)
-      if getattr(self, '_fused_plan_key', None) != key:
-        self._fused_plan = self.fused.plan(self, self.use_noise, self.noise_frac, C.c_void_p(stream_ptr))
-        self._fused_plan_key = key
-      for fn, args in self._fused_plan:
-        rc = fn(*args)
-        if rc:
-          _lib.check(rc, fn.__name__)
-      self.launches_per_move = len(self._fused_plan)
-      return
-    if len(self.lanes) == 1:
-      self.launches_per_move = self.lanes[0].enqueue(self.use_noise, self.noise_frac)
-      return
-    main = torch.cuda.current_stream()
-    fork = torch.cuda.Event()
-    fork.record(main)
-    n = 0
-    for lane in self.lanes:
-      lane.stream.wait_event(fork)
-      with torch.cuda.stream(lane.stream):
-        n += lane.enqueue(self.use_noise, self.noise_frac)
-        done = torch.cuda.Event()
-        done.record(lane.stream)
-      main.wait_event(done)
-    self.launches_per_move = n
-
-  @_lib.on_device
-  def run(self):
-    """One move for all games with inputs already in the device staging buffers."""
-    if not self.use_graph:
-      self._enqueue()
-      return
-    if self.graph is None:
-      # warm up once outside capture (lazy module loading, cudaFuncSetAttribute)
-      self._enqueue()
-      torch.cuda.synchronize()
-      self.graph = torch.cuda.CUDAGraph()
-      with torch.cuda.graph(self.graph):
-        self._enqueue()
-    self.graph.replay()
-
-  # -- end-to-end call: host buffers in, host buffers out ----------------------------------------
-  def _pinned(self):
-    if getattr(self, '_h', None) is None:
-      self._in_host, h = _carve(self._in_specs, pin_memory=True)
-      self._out_host, out = _carve(self._out_specs, pin_memory=True)
-      h.update(out)
-      h['obs'] = torch.zeros((self.G, self.net.input_dim), dtype=torch.float32, pin_memory=True)
-      h['legal'].fill_(_all_legal(self.A))
-      h['to_play'].fill_(1)
-      h['temperature'].fill_(1.0)
-      self._h = h
-    return self._h
-
-  def pinned_inputs(self):
-    """Pinned host views of the per-move inputs (one contiguous blob): 'obs_u8' [G, input_dim] uint8,
-    'noise' [G, A] f64, 'uniforms' [G] f64, 'temperature' [G] f64, 'legal' [G] i32 bit masks, 'to_play'
-    [G] i8.  Write the move's inputs here and call `search_pinned()`: no host-side staging copy."""
-    h = self._pinned()
-    return {name: h[name] for name, _, _ in self._in_specs}
-
-  @_lib.on_device
-  def search_pinned(self):
-    """search_host for inputs already written into `pinned_inputs()` (byte observations): ONE
-    host->device copy of the input blob, normalisation + the move's graph, ONE device->host copy of the
-    output blob.  Returns the pinned (actions, root_value, child_visits, init_value)."""
-    h = self._pinned()
-    mn, rg = getattr(self, '_obs_norm', (None, None))
-    if self.fused is not None and self.use_graph:
-      # ONE graph launch for the whole call: the input blob's copy, the normalisation, the move, the output blob's
-      # copy (tests/e2e_probe.py: 1081 -> 1048 us per call; copying the noise on a second branch under the initial
-      # inference was measured too and is not faster)
       key = (bool(self.use_noise), float(self.noise_frac), stream_ptr)
       if getattr(self, '_fused_plan_key', None) != key:
         self._fused_plan = self.fused.plan(self, self.use_noise, self.noise_frac, C.c_void_p(stream_ptr))

@@ -3,13 +3,9 @@ import sys, types
 import numpy as np
 import torch
 sys.path.insert(0, ".")
-from model_based_rl_b200 import _lib
 from model_based_rl_b200.networks import FCNetwork, FCSearch, random_state_dict
 
-cluster, engine, S, game = int(sys.argv[1]), int(sys.argv[2]), int(sys.argv[3]), int(sys.argv[4])
-lib = _lib.load()
-lib.mz_fc_search_set_cluster(cluster)
-lib.mz_fc_search_set_engine(engine)
+S, game = int(sys.argv[1]), int(sys.argv[2])
 G, A, D = 300, 18, 128
 cfg = types.SimpleNamespace(
     num_simulations=S, action_space=A, two_players=False, discount=0.997, pb_c_base=19652, pb_c_init=1.25,

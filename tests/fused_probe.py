@@ -1,17 +1,10 @@
-"""Bring-up / timing probe of the fused search kernel (not a pytest): python tests/fused_probe.py [cluster]"""
+"""Bring-up / timing probe of the fused search kernel (not a pytest): python tests/fused_probe.py"""
 import sys, types, time
 import numpy as np
 import torch
 sys.path.insert(0, ".")
-from model_based_rl_b200 import _lib
 from model_based_rl_b200.networks import FCNetwork, FCSearch, random_state_dict
 
-cluster = int(sys.argv[1]) if len(sys.argv) > 1 else 2
-engine = int(sys.argv[2]) if len(sys.argv) > 2 else 0
-lib = _lib.load()
-lib.mz_fc_search_set_cluster(cluster)
-lib.mz_fc_search_set_engine(engine)
-print("cluster %d engine %d" % (cluster, engine))
 
 
 def cfg_for(S, A):
@@ -59,8 +52,8 @@ def compare(G, S, A=18, D=128):
     if not torch.equal(x, y):
       ok = False
       print("  %s differs in %d entries" % (name, int((x != y).sum())))
-  print("compare G=%d S=%d A=%d cluster=%d: %s (err flag %d)" % (G, S, A, cluster, "IDENTICAL" if ok else "MISMATCH",
-                                                                 int(fb.fused.error_flag.item())))
+  print("compare G=%d S=%d A=%d: %s (err flag %d)" % (G, S, A, "IDENTICAL" if ok else "MISMATCH",
+                                                      int(fb.fused.error_flag.item())))
   return ok
 
 
@@ -84,8 +77,7 @@ def timing(G, S=50, A=18, D=128, moves=20):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / moves
-    print("timing G=%d fused=%s cluster=%d: %.3f ms/move  %.1f M expansions/s" % (G, fused, cluster, ms,
-                                                                               G * S / ms / 1e3))
+    print("timing G=%d fused=%s: %.3f ms/move  %.1f M expansions/s" % (G, fused, ms, G * S / ms / 1e3))
     if fused:
       fs.fused.enable_timeline()
       fs._fused_plan_key = None
@@ -124,12 +116,11 @@ def timing(G, S=50, A=18, D=128, moves=20):
           tl[-1, 15] - tl[-1, 12]))
       nxt = tl[1:, 0] - tl[:-1, 0]
       print("   sim period median %d cycles" % np.median(nxt))
-      if engine == 1:
-        d = lambda a, b: int(np.median((tl[:, a] - tl[:, b])[5:]))
-        print("   descent: reset %d | issue loads %d | rank items %d | winners %d | chase %d" % (
-            int(np.median((tl[1:, 16] - tl[:-1, 11])[5:])), d(17, 16), d(18, 17), d(19, 18), d(20, 19)))
-        print("   expand+backup: early loads %d | exp + prior sum %d | priors %d | top x2 + meta %d | backup %d | minmax %d" % (
-            d(22, 10), d(23, 22), d(24, 23), d(25, 24), d(26, 25), d(11, 26)))
+      d = lambda a, b: int(np.median((tl[:, a] - tl[:, b])[5:]))
+      print("   descent: reset %d | issue loads %d | rank items %d | winners %d | chase %d" % (
+          int(np.median((tl[1:, 16] - tl[:-1, 11])[5:])), d(17, 16), d(18, 17), d(19, 18), d(20, 19)))
+      print("   expand+backup: early loads %d | exp + prior sum %d | priors %d | top x2 + meta %d | backup %d | minmax %d" % (
+          d(22, 10), d(23, 22), d(24, 23), d(25, 24), d(26, 25), d(11, 26)))
       print("   next sim: wait for outputs %d, expand+backup %d, descent %d" % (
           np.median((tl[:-1, 10] - tl[1:, 0])[5:]), np.median((tl[:-1, 11] - tl[:-1, 10])[5:]),
           np.median((tl[1:, 1] - tl[:-1, 11])[5:])))

@@ -1,4 +1,5 @@
-"""Timing sweep (not a pytest): per-launch path vs the fused kernel's variants on the BASELINE shapes."""
+"""Timing sweep (not a pytest): per-launch path vs the fused kernel, with and without programmatic dependent
+launches, on the BASELINE shapes."""
 import sys, types
 import numpy as np
 import torch
@@ -23,11 +24,8 @@ def run(name, variant, moves=20):
   rng = np.random.default_rng(2)
   obs = rng.random((G, D)).astype(np.float32)
   noise, u, temp = rng.dirichlet([0.25] * A, size=G), rng.random(G), np.ones(G)
-  fused, cl, eng, pdl = variant
+  fused, pdl = variant
   lib.mz_set_programmatic_launch(pdl)
-  if fused:
-    lib.mz_fc_search_set_cluster(cl)
-    lib.mz_fc_search_set_engine(eng)
   fs = FCSearch(cfg, net, G, use_graph=True, num_streams=4, fused=bool(fused))
   fs.search_host(obs, noise, u, temp)
   for _ in range(3):
@@ -45,8 +43,7 @@ def run(name, variant, moves=20):
 
 
 if __name__ == "__main__":
-  variants = {"per-launch x4 streams": (0, 0, 0, 1), "fused cl4 sparse pdl": (1, 4, 1, 1), "fused cl4 sparse no-pdl": (1, 4, 1, 0),
-              "fused cl4 dense": (1, 4, 0, 1), "fused cl2 dense": (1, 2, 0, 1)}
+  variants = {"per-launch x4 streams": (0, 1), "fused pdl": (1, 1), "fused no-pdl": (1, 0)}
   for name in sys.argv[1:] or list(SHAPES):
     for vn, v in variants.items():
       ms, rate = run(name, v, moves=5 if name == "C4x4" else 20)

@@ -44,6 +44,8 @@ int main(void) {
          offsetof(mz_fc_weights, rep_w1), offsetof(mz_target_cfg, discounts));
   printf("%zu %zu %zu %zu %zu %zu %zu\n", sizeof(mz_pack_job), sizeof(mz_tc_head), sizeof(mz_tc_job), sizeof(mz_tc_chain),
          offsetof(mz_tc_job, dx), offsetof(mz_tc_chain, hook_scale), offsetof(mz_tc_chain, dyall));
+  printf("%zu %zu %zu\n", sizeof(mz_fc_search_args), offsetof(mz_fc_search_args, game_bytes),
+         offsetof(mz_fc_search_args, error_flag));
   return 0;
 }'''
   with tempfile.TemporaryDirectory() as d:
@@ -56,8 +58,22 @@ int main(void) {
                        C.sizeof(_lib.TargetCfg)]
   assert sizes[4:8] == [_lib.Tree.games.offset, _lib.Tree.leaf_action.offset,
                         _lib.FcWeights.rep_w1.offset, _lib.TargetCfg.discounts.offset]
-  assert sizes[8:] == [C.sizeof(_lib.PackJob), C.sizeof(_lib.TcHead), C.sizeof(_lib.TcJob), C.sizeof(_lib.TcChain),
-                       _lib.TcJob.dx.offset, _lib.TcChain.hook_scale.offset, _lib.TcChain.dyall.offset]
+  assert sizes[8:15] == [C.sizeof(_lib.PackJob), C.sizeof(_lib.TcHead), C.sizeof(_lib.TcJob), C.sizeof(_lib.TcChain),
+                         _lib.TcJob.dx.offset, _lib.TcChain.hook_scale.offset, _lib.TcChain.dyall.offset]
+  assert sizes[15:] == [C.sizeof(_lib.FcSearchArgs), _lib.FcSearchArgs.game_bytes.offset,
+                        _lib.FcSearchArgs.error_flag.offset]
+
+
+def test_fused_search_shape_boundary():
+  """The shapes the persistent search kernel takes: S <= 63 and a shared-memory plan within 232 448 bytes.  The
+  largest S is 63 up to 13 actions, 55 at 14..20 and 19 at 30..32; every other shape runs the per-launch path."""
+  lib = _lib.load()
+  for S, A in ((50, 18), (55, 18), (63, 13), (19, 32), (1, 1)):
+    assert lib.mz_fc_search_supported(S, A) == 1, (S, A)
+    assert lib.mz_fc_search_game_bytes(S, A) > 0, (S, A)
+  for S, A in ((56, 18), (64, 4), (20, 32), (253, 1), (0, 4), (10, 0), (10, 33)):
+    assert lib.mz_fc_search_supported(S, A) == 0, (S, A)
+    assert lib.mz_fc_search_game_bytes(S, A) == -2, (S, A)  # MZ_ERR_UNSUPPORTED
 
 
 def test_tree_geometry_and_pb_c_table_host_helpers():

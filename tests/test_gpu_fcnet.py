@@ -292,10 +292,9 @@ def _search_cfg(S, A, two_players=False, discount=0.997, known_bounds=(None, Non
       no_target_transform=no_target_transform)
 
 
-@pytest.mark.parametrize("cluster,engine", [(2, 0), (4, 0), (4, 1)])
-@pytest.mark.parametrize("shape", ["atari18", "ttt9", "lunar4", "wide32", "ties6", "asym5_nott"])
-def test_fused_search_equals_per_launch_search(cluster, engine, shape):
-  """mz_fc_search (the whole move in one persistent kernel, clusters of 2 or 4 CTAs) against the
+@pytest.mark.parametrize("shape", ["atari18", "ttt9", "lunar4", "wide32", "ties6", "asym5_nott", "edge13"])
+def test_fused_search_equals_per_launch_search(shape):
+  """mz_fc_search (the whole move in one persistent kernel, clusters of 4 CTAs) against the
   per-simulation launches of mz_tree_step + mz_fc_recurrent_tc on the same inputs: identical network
   outputs at every simulation (same MMA sequence on the same bf16 operands), identical (parent, action,
   depth) traces, visit counts, root values, MinMax bounds, child-visit distributions and selected
@@ -304,15 +303,16 @@ def test_fused_search_equals_per_launch_search(cluster, engine, shape):
   and known bounds; `ties6` runs a network whose policy head is zero (all priors equal at every node: every
   unexpanded-child choice is a tie broken by the action index); `asym5_nott` has a 32-bin value support
   [-4, 27], a 9-bin reward support [-2, 6] and raw expectations (no_target_transform), with support logits
-  spread x16.  engine 0 = dense tree walk, 1 = sparse node-parallel ranking (csrc/mz_fcs_sparse.cuh)."""
-  from model_based_rl_b200 import _lib
+  spread x16.  `wide32` (S = 19) and `edge13` (S = 63) are the largest trees the kernel takes at A = 32 and at
+  A = 13: `edge13` has the largest shared-memory plan of all shapes (217 248 of 232 448 bytes)."""
   from model_based_rl_b200.networks import FCNetwork, FCSearch, random_state_dict
   G, A, S, D, two, disc, kb = {"atari18": (300, 18, 50, 128, False, 0.997, (None, None)),
                                "ttt9": (130, 9, 30, 9, True, 1.0, (-1, 1)),
                                "lunar4": (257, 4, 30, 8, False, 0.997, (None, None)),
-                               "wide32": (100, 32, 20, 16, False, 0.99, (None, None)),
+                               "wide32": (100, 32, 19, 16, False, 0.99, (None, None)),
                                "ties6": (140, 6, 40, 12, False, 0.997, (None, None)),
-                               "asym5_nott": (150, 5, 25, 10, False, 0.997, (None, None))}[shape]
+                               "asym5_nott": (150, 5, 25, 10, False, 0.997, (None, None)),
+                               "edge13": (200, 13, 63, 24, False, 0.997, (None, None))}[shape]
   vs, rs, nott = ((-4, 27), (-2, 6), True) if shape == "asym5_nott" else ((-15, 15), (-15, 15), False)
   cfg = _search_cfg(S, A, two, disc, kb, vs, rs, nott)
   net = FCNetwork(D, A, "cuda", cfg)
@@ -336,27 +336,19 @@ def test_fused_search_equals_per_launch_search(cluster, engine, shape):
       n = bin(int(legal[i])).count("1")
       noise[i, :n] = rng.dirichlet([0.25] * n)
   u, temp = rng.random(G), rng.choice([0.0, 0.5, 1.0], size=G)
-  lib = _lib.load()
   outs = []
-  try:
-    for fused in (False, True):
-      if fused:
-        _lib.check(lib.mz_fc_search_set_cluster(cluster), "mz_fc_search_set_cluster")
-        _lib.check(lib.mz_fc_search_set_engine(engine), "mz_fc_search_set_engine")
-      fs = FCSearch(cfg, net, G, use_graph=False, num_streams=1, fused=fused)
-      fs.enable_record()
-      r = fs.search_host(obs, noise, u, temp, legal=legal, to_play=to_play)
-      torch.cuda.synchronize()
-      if fused:
-        assert int(fs.fused.error_flag.item()) == 0
-      eng = fs.fused if fused else fs.eng
-      trees = [eng.export_game(g) for g in (0, G // 2, G - 1)]
-      outs.append(dict(actions=r[0].clone(), root_value=r[1].clone(), child_visits=r[2].clone(),
-                       init_value=r[3].clone(), visits=fs.visits.cpu(), minmax=fs.minmax.cpu(),
-                       record=[t.cpu() for t in fs.record], trace=[t.cpu() for t in fs.trace], trees=trees))
-  finally:
-    lib.mz_fc_search_set_cluster(0)
-    lib.mz_fc_search_set_engine(-1)
+  for fused in (False, True):
+    fs = FCSearch(cfg, net, G, use_graph=False, num_streams=1, fused=fused)
+    fs.enable_record()
+    r = fs.search_host(obs, noise, u, temp, legal=legal, to_play=to_play)
+    torch.cuda.synchronize()
+    if fused:
+      assert int(fs.fused.error_flag.item()) == 0
+    eng = fs.fused if fused else fs.eng
+    trees = [eng.export_game(g) for g in (0, G // 2, G - 1)]
+    outs.append(dict(actions=r[0].clone(), root_value=r[1].clone(), child_visits=r[2].clone(),
+                     init_value=r[3].clone(), visits=fs.visits.cpu(), minmax=fs.minmax.cpu(),
+                     record=[t.cpu() for t in fs.record], trace=[t.cpu() for t in fs.trace], trees=trees))
   a, b = outs
   for i, name in enumerate(("value", "reward", "logits")):
     assert torch.equal(a["record"][i], b["record"][i]), "network %s differs" % name
@@ -367,6 +359,20 @@ def test_fused_search_equals_per_launch_search(cluster, engine, shape):
   for ta, tb in zip(a["trees"], b["trees"]):
     for k in ("prior", "child", "vsum", "visit", "reward"):
       assert np.array_equal(ta[k], tb[k]), "tree %s differs" % k
+
+
+def test_search_outside_fused_plan_runs_per_launch():
+  """A = 18, S = 60 lies outside the persistent kernel's plan (S <= 55 at 18 actions): the default engine is the
+  per-launch path, and asking for the fused kernel is an error."""
+  from model_based_rl_b200.networks import FCNetwork, FCSearch, random_state_dict
+  G, A, S, D = 130, 18, 60, 32
+  cfg = _search_cfg(S, A)
+  net = FCNetwork(D, A, "cuda", cfg)
+  net.load_weights(random_state_dict(D, A, seed=3))
+  fs = FCSearch(cfg, net, G, fused=None)
+  assert fs.fused is None and len(fs.lanes) == 1
+  with pytest.raises(ValueError):
+    FCSearch(cfg, net, G, fused=True)
 
 
 def test_search_after_load_weights_uses_new_weights():
