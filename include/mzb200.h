@@ -573,6 +573,18 @@ int mz_unroll_loss(const mz_loss_cfg* c, const float* value_logits, const float*
                    const float* t_policies, const double* is_weights, float* d_value_logits,
                    float* d_reward_logits, float* d_policy_logits, double* row_losses, double* losses,
                    float* new_errors, void* stream);
+/* The same pass for `--no_support` networks (config.py:95-96; learners.py:182-213 with utils.py:61-70), whose
+ * value and reward heads emit one scalar: value_out [K+1][B][1], reward_out [K][B][1] f32, the other inputs as
+ * above.  Value loss = sum over steps 0..K, reward loss = sum over steps 1..K of l(out, h(target)) (h skipped with
+ * no_target_transform), l = MSELoss (scalar_loss 0) or SmoothL1Loss with beta 1 (scalar_loss 1), reduction 'none';
+ * policy loss as above.  new_errors [B] = value_out[0] - t_values[:, 0] (raw output minus raw target, no inverse
+ * transform).  Gradients with the 1/K scale of learners.py:213, in the operation order of torch's
+ * mse_loss_backward / smooth_l1_loss_backward.  Only batch, num_unroll_steps (1..31), num_actions and
+ * no_target_transform of c are read.  -1 for a rejected size or scalar_loss, -2 for a NULL required pointer. */
+int mz_scalar_unroll_loss(const mz_loss_cfg* c, int32_t scalar_loss, const float* value_out, const float* reward_out,
+                          const float* policy_logits, const float* t_values, const float* t_rewards,
+                          const float* t_policies, const double* is_weights, float* d_value_out, float* d_reward_out,
+                          float* d_policy_logits, double* row_losses, double* losses, float* new_errors, void* stream);
 
 /* Diagnostics: compares the constant-divisor division used by the descent's MinMax normalisation
  * with IEEE division on blocks*256*per_thread pseudo-random operand pairs; adds the number of

@@ -205,6 +205,8 @@ _SIGNATURES = {
     "mz_conv_head": (C.c_int, [C.c_int32, _V, C.c_int32, _V, _V, C.c_int32, C.c_int32, C.c_int32,
                                C.c_int32, _V, C.c_int32, _V]),
     "mz_unroll_loss": (C.c_int, [C.POINTER(LossCfg), _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V]),
+    "mz_scalar_unroll_loss": (C.c_int, [C.POINTER(LossCfg), C.c_int32, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V,
+                                        _V, _V]),
     "mz_debug_div_check": (C.c_int, [C.c_uint64, C.c_int32, C.c_int32, _V, _V, _V]),
     "mz_set_programmatic_launch": (C.c_int, [C.c_int32]),
     "mz_tree_set_wide_step_max_games": (C.c_int, [C.c_int32]),

@@ -11,6 +11,7 @@ search kernels' `FCNetwork.load_weights` see the usual tensors.  `FusedLearner(p
     mz_chain_forward_tc       representation -> LN -> K x (dynamics -> LN)               1 launch
     mz_heads_forward_tc       value / policy / reward heads over all K + 1 steps         1 launch
     mz_unroll_loss            fused loss + logit gradients (csrc/mz_unroll_loss.cu)      2 launches
+                              (mz_scalar_unroll_loss for --no_support networks)
     mz_heads_backward_tc      the three output heads                                     1 launch
     mz_chain_backward_tc      the serial part: LN backward -> dH -> dX per step          1 launch
     mz_heads_backward_tc      parameter gradients of dynamics + representation           1 launch
@@ -23,10 +24,14 @@ search kernels' `FCNetwork.load_weights` see the usual tensors.  `FusedLearner(p
     transposes, 2 (K + 1) forward launches, 3 head launches, loss, 3 + 2 (K + 1) backward launches, optimiser.
 
 Both are captured in CUDA graphs.  SGD / RMSprop use the torch optimiser over the flat buffer (elementwise, the
-reference's arithmetic).  With torch.distributed initialised the gradients of the three output heads are all-reduced
+reference's arithmetic).  `--no_support` networks (one-unit value / reward heads, `config.scalar_loss` MSE or Huber,
+utils.py:61-70) run the same launches with d_out = 1 heads and the scalar loss kernel.  `save_state` writes the
+checkpoint dictionary of learners.py:72-83; `load_state` / `FusedLearner(state=...)` resume from it (weights, optimiser
+state, training_step, replay throughput), and a graph captured later keeps the restored optimiser state.  With torch.distributed initialised the gradients of the three output heads are all-reduced
 on a side stream while the recurrent part of the backward still runs; the rest follows before the optimiser step.
 """
 import ctypes as C
+import os
 
 import numpy as np
 import torch
@@ -49,13 +54,11 @@ class _Head(object):
 
 
 class FusedFCNetwork(object):
-  """The reference's FCNetwork in train mode (support logits) with flat parameter storage.  Heads in buffer order:
+  """The reference's FCNetwork in train mode (support logits, or one-unit value / reward heads with
+  config.no_support) with flat parameter storage.  Heads in buffer order:
   value, policy, reward (the gradient bucket that is complete first), transition, representation, LN."""
 
   def __init__(self, input_dim, action_space, device, config):
-    if getattr(config, 'no_support', False):
-      raise NotImplementedError("the fused learner kernels cover the support heads; train --no_support networks with "
-                                "learners.Learner (FCNetworkTrain + scalar_unroll_loss)")
     self.device = _lib.normalize_device(device)
     self.lib = _lib.load()
     self.input_dim, self.action_space = int(input_dim), int(action_space)
@@ -64,10 +67,11 @@ class FusedFCNetwork(object):
       raise ValueError("the fused learner kernels take at most 128 input features per head")
     vmin, vmax = [int(v) for v in config.value_support]
     rmin, rmax = [int(v) for v in config.reward_support]
+    no_support = bool(getattr(config, 'no_support', False))  # networks.py:135-136: one-unit scalar heads
     self.heads = {
-        'value_head': _Head('value_head', 'value', HIDDEN, vmax - vmin + 1),
+        'value_head': _Head('value_head', 'value', HIDDEN, 1 if no_support else vmax - vmin + 1),
         'policy_head': _Head('policy_head', 'policy', HIDDEN, A),
-        'reward_head': _Head('reward_head', 'reward', HIDDEN + A, rmax - rmin + 1),
+        'reward_head': _Head('reward_head', 'reward', HIDDEN + A, 1 if no_support else rmax - rmin + 1),
         'transition_head': _Head('transition_head', 'out', HIDDEN + A, HIDDEN),
         'representation_head': _Head('representation_head', 'out', self.input_dim, HIDDEN),
     }
@@ -169,9 +173,11 @@ class FusedFCNetwork(object):
 class FusedLearner(object):
   """`learners.Learner` with the step on this library's kernels.  Same `update_weights(batch)` on the tuple
   `PrioritizedReplay.sample_batch()` / `sample_batch_device()` returns, priority feedback, weight hand-off,
-  schedules and checkpoint keys."""
+  schedules, checkpoints (`save_state` / `load_state`, `state=`) and `--no_support` networks (MSE or Huber scalar
+  loss, config.scalar_loss)."""
 
-  def __init__(self, config, network, replay_buffer=None, search_network=None, use_graph=True, precision='bf16'):
+  def __init__(self, config, network, replay_buffer=None, search_network=None, use_graph=True, precision='bf16',
+               state=None):
     _lib.require_cuda()
     if not isinstance(network, FusedFCNetwork):
       raise TypeError("FusedLearner trains a FusedFCNetwork")
@@ -184,6 +190,12 @@ class FusedLearner(object):
     self.use_graph = bool(use_graph)
     self.K, self.A = int(config.num_unroll_steps), network.action_space
     self.loss_cfg = learners.loss_cfg(config)
+    self.scalar_loss = None  # support heads: mz_unroll_loss; no_support: 0 = MSE, 1 = Huber (mz_scalar_unroll_loss)
+    if getattr(config, 'no_support', False):
+      kind = getattr(config, 'scalar_loss', 'MSE')
+      if kind not in ('MSE', 'Huber'):
+        raise NotImplementedError("scalar_loss %r: the scalar loss kernel computes 'MSE' or 'Huber'" % (kind,))
+      self.scalar_loss = int(kind == 'Huber')
     self.training_step = 0
     self.losses_to_log = {'reward': 0., 'value': 0., 'policy': 0.}
     self.last_losses = self.last_errors = None
@@ -215,6 +227,8 @@ class FusedLearner(object):
     self._shape = None
     self._graphs = None
     self._comm = None
+    if state is not None:
+      self.load_state(state)
 
   # -- buffers of one batch shape ----------------------------------------------------------------------
   def _alloc(self, B):
@@ -282,6 +296,16 @@ class FusedLearner(object):
                                          _P(dy), ldy, None if dx is None else _P(dx), lddx, _P(h.g[0]), _P(h.g[1]),
                                          _P(h.g[2]), _P(h.g[3]), st), "mz_mlp2_backward")
 
+  def _loss(self, st):
+    """The loss and the gradient of every head output: support logits (mz_unroll_loss) or the scalar heads of a
+    no_support network (mz_scalar_unroll_loss)."""
+    args = (_P(self.v), _P(self.r), _P(self.p), _P(self.s_tv), _P(self.s_tr), _P(self.s_tp), _P(self.s_isw), _P(self.dv),
+            _P(self.dr), _P(self.dp), _P(self.rows), _P(self.losses), _P(self.new_errors), st)
+    if self.scalar_loss is None:
+      _lib.check(self.lib.mz_unroll_loss(self.c_loss, *args), "mz_unroll_loss")
+    else:
+      _lib.check(self.lib.mz_scalar_unroll_loss(self.c_loss, self.scalar_loss, *args), "mz_scalar_unroll_loss")
+
   def _forward_and_heads_backward(self):
     """Transposes, the K + 1 network evaluations (learners.py:175-206), the loss, and the backward of the three
     output heads (whose parameter gradients are then complete)."""
@@ -291,9 +315,7 @@ class FusedLearner(object):
       _lib.check(lib.mz_learner_pack(len(self.tc_first_jobs), self.tc_first_jobs, st), "mz_learner_pack")
       _lib.check(lib.mz_chain_forward_tc(self.tc_chain, st), "mz_chain_forward_tc")
       _lib.check(lib.mz_heads_forward_tc(len(self.tc_jobs), self.tc_jobs, st), "mz_heads_forward_tc")
-      _lib.check(lib.mz_unroll_loss(self.c_loss, _P(self.v), _P(self.r), _P(self.p), _P(self.s_tv), _P(self.s_tr),
-                                    _P(self.s_tp), _P(self.s_isw), _P(self.dv), _P(self.dr), _P(self.dp), _P(self.rows),
-                                    _P(self.losses), _P(self.new_errors), st), "mz_unroll_loss")
+      self._loss(st)
       _lib.check(lib.mz_heads_backward_tc(len(self.tc_jobs), self.tc_jobs, st), "mz_heads_backward_tc")
       return
     ln_w, ln_b = net.views['LN.weight'], net.views['LN.bias']
@@ -312,9 +334,7 @@ class FusedLearner(object):
     self._fwd('policy_head', (K + 1) * B, self.xs, ldx, self.p, A, st)
     if K > 0:
       self._fwd('reward_head', K * B, self.xs, ldx, self.r, self.r.shape[2], st)
-    _lib.check(lib.mz_unroll_loss(self.c_loss, _P(self.v), _P(self.r), _P(self.p), _P(self.s_tv), _P(self.s_tr), _P(self.s_tp),
-                                  _P(self.s_isw), _P(self.dv), _P(self.dr), _P(self.dp), _P(self.rows), _P(self.losses),
-                                  _P(self.new_errors), st), "mz_unroll_loss")
+    self._loss(st)
     self._bwd('value_head', (K + 1) * B, self.xs, ldx, self.dv, self.v.shape[2], self.dxs, ldx, st)
     self._bwd('policy_head', (K + 1) * B, self.xs, ldx, self.dp, A, self.dxs, ldx, st)
     if K > 0:
@@ -427,7 +447,14 @@ class FusedLearner(object):
     main.wait_stream(self._comm)
     apply()
 
+  def _optimizer_tensors(self):
+    if self.own_optimizer:
+      return [self.exp_avg, self.exp_avg_sq, self.opt_state]
+    return [v for st in self.optimizer.state.values() for v in st.values() if torch.is_tensor(v)]
+
   def _capture(self, world):
+    # the optimiser state as it stands (fresh, or restored by load_state): the warm-up step below changes it
+    saved = {id(t): t.clone() for t in self._optimizer_tensors()}
     # warm-up outside capture: kernel attributes, lazy module loading, optimiser state
     self._forward_and_heads_backward()
     self._recurrent_backward()
@@ -442,25 +469,18 @@ class FusedLearner(object):
     g3 = None
     if self.own_optimizer or self._graph_opt:
       if not self.own_optimizer:
-        # the torch optimiser initialises its state on the first step: take one with zero gradients, then restore
+        # the torch optimiser initialises its state on the first step: take one with zero gradients (restored below)
         self.network.grad.zero_()
         self.optimizer.step()
-        for st in self.optimizer.state.values():
-          for k, v in st.items():
-            if torch.is_tensor(v):
-              v.zero_()
       g3 = torch.cuda.CUDAGraph()
       with torch.cuda.graph(g3, pool=g1.pool()):
         self._apply(world)
-      if not self.own_optimizer:
-        for st in self.optimizer.state.values():
-          for k, v in st.items():
-            if torch.is_tensor(v):
-              v.zero_()
+    # in place, so that the captured step reads it: the state from before, zeros for state the warm-up step created
+    for t in self._optimizer_tensors():
+      if id(t) in saved:
+        t.copy_(saved[id(t)])
       else:
-        self.exp_avg.zero_()
-        self.exp_avg_sq.zero_()
-        self.opt_state[0] = 0.0
+        t.zero_()
     self.network.flat.copy_(snapshot)
     torch.cuda.synchronize()
     self._graphs = (g1, g2, g3)
@@ -489,27 +509,76 @@ class FusedLearner(object):
     if self.replay_buffer.size() < need:
       raise RuntimeError("replay buffer holds %d memories, config.stored_before_train is %d" %
                          (self.replay_buffer.size(), need))
+    save_every = int(getattr(self.config, 'save_state_frequency', 0) or 0)
     end = self.training_step + steps
     while self.training_step < end:
       self.update_weights(self.replay_buffer.sample_batch_device(False, ring=4))
       self.training_step += 1
       if self.training_step % self.config.send_weights_frequency == 0:
         self.send_weights()
+      if save_every and self.training_step % save_every == 0:  # learners.py:135-136
+        saves = (getattr(self, 'dirs', None) or {}).get('saves')
+        self.save_state(os.path.join(saves, str(self.training_step)) if saves else None)
     return self.training_step
 
   def save_state(self, path=None, actor_games=None, dirs=None):
-    """The checkpoint dictionary of learners.py:72-83 (see learners.Learner.save_state)."""
+    """The checkpoint dictionary of learners.py:72-83 (see learners.Learner.save_state); the optimiser entry is
+    {'exp_avg', 'exp_avg_sq', 'state' = (step, learning rate, scratch)} for the library's Adam / AdamW, else the torch
+    optimiser's state_dict.  `dirs` / `actor_games` default to the attributes of the same names."""
     tp = self.replay_buffer.get_throughput() if self.replay_buffer is not None else {'frames': 0, 'games': 0}
     if self.own_optimizer:
       opt = {'exp_avg': self.exp_avg.cpu(), 'exp_avg_sq': self.exp_avg_sq.cpu(), 'state': self.opt_state.cpu()}
     else:
       opt = self.optimizer.state_dict()
-    state = {'dirs': dict(dirs or {}), 'config': self.config, 'weights': self.network.get_weights(), 'optimizer': opt,
+    state = {'dirs': dict(dirs if dirs is not None else getattr(self, 'dirs', {}) or {}),
+             'config': self.config, 'weights': self.network.get_weights(), 'optimizer': opt,
              'training_step': self.training_step, 'total_games': tp['games'], 'total_frames': tp['frames'],
-             'actor_games': dict(actor_games or {})}
+             'actor_games': dict(actor_games if actor_games is not None else getattr(self, 'actor_games', {}) or {})}
     if path is not None:
       torch.save(state, path)
+    self.last_saved_state = state
     return state
+
+  def load_state(self, state):
+    """Resumes from a `save_state` checkpoint of a FusedLearner with the same optimiser and network (learners.py:59-70,
+    learners.Learner.load_state): weights, optimiser state, training_step and the replay throughput.  The library's
+    Adam state is copied in place (captured graphs stay valid); a torch optimiser's load_state_dict replaces its
+    tensors, so the step is captured again."""
+    opt, n = state['optimizer'], self.network.flat.numel()
+    own = isinstance(opt, dict) and 'exp_avg' in opt
+    saved_kind = getattr(state.get('config'), 'optimizer', self.config.optimizer)
+    if own != self.own_optimizer or saved_kind != self.config.optimizer:
+      raise ValueError("the checkpoint holds %s optimiser state, this learner runs %s" % (saved_kind, self.config.optimizer))
+    if own:
+      sizes = {opt['exp_avg'].numel(), opt['exp_avg_sq'].numel()}
+    else:
+      sizes = {v.numel() for st in opt['state'].values() for v in st.values() if torch.is_tensor(v) and v.dim() > 0}
+    if sizes - {n}:
+      raise ValueError("the checkpoint's optimiser state has %s elements per tensor, the flat buffer %d" % (sorted(sizes), n))
+    self.network.load_weights(state['weights'])
+    if own:
+      self.exp_avg.copy_(opt['exp_avg'])
+      self.exp_avg_sq.copy_(opt['exp_avg_sq'])
+      self.opt_state.copy_(opt['state'])
+      if isinstance(self.lr_scheduler, _ExponentialLR):  # the decay continues from the restored rate
+        self.lr_scheduler.lr = float(self.opt_state[1])
+    else:
+      group = dict(self.optimizer.param_groups[0])
+      self.optimizer.load_state_dict(opt)
+      # how this learner runs the step (captured or not, learning rate in a device scalar) is not the checkpoint's
+      g = self.optimizer.param_groups[0]
+      if torch.is_tensor(group['lr']):
+        group['lr'].fill_(float(g['lr']))
+        g['lr'] = group['lr']
+      if 'capturable' in group:
+        g['capturable'] = group['capturable']
+        for st in self.optimizer.state.values():
+          if torch.is_tensor(st.get('step')):
+            st['step'] = st['step'].to(self.device if g['capturable'] else 'cpu', torch.float32)
+      self._graphs = None
+    self.training_step = state['training_step']
+    if self.replay_buffer is not None and 'total_frames' in state:
+      self.replay_buffer.add_initial_throughput(state['total_frames'], state['total_games'])
 
 
 class _LrHandle(object):
