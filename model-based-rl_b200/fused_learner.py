@@ -40,6 +40,7 @@ from . import _lib, learners, parallel
 from .networks import HIDDEN
 
 WIDTH = _lib.FC_WIDTH
+MAX_SUPPORT_BINS = 64  # widest value / reward head: LMAXOUT in csrc/mz_learner.cu, head_ok in csrc/mz_learner_tc.cu
 _P = lambda t: C.c_void_p(t.data_ptr())
 
 
@@ -59,15 +60,20 @@ class FusedFCNetwork(object):
   value, policy, reward (the gradient bucket that is complete first), transition, representation, LN."""
 
   def __init__(self, input_dim, action_space, device, config):
+    vmin, vmax = [int(v) for v in config.value_support]
+    rmin, rmax = [int(v) for v in config.reward_support]
+    no_support = bool(getattr(config, 'no_support', False))  # networks.py:135-136: one-unit scalar heads
+    if not no_support:  # before the library or the device is touched: the first step would fail with MZ_ERR_BAD_ARG
+      for name, lo, hi in (('value_support', vmin, vmax), ('reward_support', rmin, rmax)):
+        if hi < lo or hi - lo + 1 > MAX_SUPPORT_BINS:
+          raise ValueError("%s [%d, %d]: the fused learner's head kernels take supports of 1 to %d bins "
+                           "(learners.Learner trains wider ones)" % (name, lo, hi, MAX_SUPPORT_BINS))
     self.device = _lib.normalize_device(device)
     self.lib = _lib.load()
     self.input_dim, self.action_space = int(input_dim), int(action_space)
     A = self.action_space
     if self.input_dim > 128 or HIDDEN + A > 128:
       raise ValueError("the fused learner kernels take at most 128 input features per head")
-    vmin, vmax = [int(v) for v in config.value_support]
-    rmin, rmax = [int(v) for v in config.reward_support]
-    no_support = bool(getattr(config, 'no_support', False))  # networks.py:135-136: one-unit scalar heads
     self.heads = {
         'value_head': _Head('value_head', 'value', HIDDEN, 1 if no_support else vmax - vmin + 1),
         'policy_head': _Head('policy_head', 'policy', HIDDEN, A),

@@ -200,6 +200,36 @@ def scalar_to_support(x, mn, mx):
   return out
 
 
+def scalar_transform_f32(x):
+  """mz_scalar_transform_f (csrc/mz_transforms.cuh) in numpy float32, same operation order: c = sqrt(|x| + 1) - 1,
+  then sign(x) * c + 0.001f * x, every operation rounded to float32.  numpy's float32 sqrt is correctly rounded (torch's
+  CPU sqrt is not), so this is the kernel's result bit for bit."""
+  x = np.asarray(x, dtype=np.float32)
+  c = np.sqrt(np.abs(x) + np.float32(1)) - np.float32(1)
+  return (np.sign(x) * c + np.float32(0.001) * x).astype(np.float32)
+
+
+def two_hot_f64(x, mn, mx, float32=False):
+  """Config.scalar_to_support (config.py:56-68) in binary64: x clamped to [mn, mx], p_hi = x - floor(x) at ceil(x),
+  then 1 - p_hi at floor(x) (1.0 at an integer).  Returns (clamped x, support[..., mx - mn + 1]).
+
+  float32=True gives the float32 two-hot of mz_two_hot (csrc/mz_transforms.cuh) bit for bit, as float32.  For float32
+  x both of its subtractions are exact in binary64, but x - floor(x) is not exact in float32 when x is a negative
+  non-integer (-0.24 + 1 needs the bits of both), and 1 - p_hi then starts from the rounded p_hi: so p_hi is rounded
+  to float32 before 1 - p_hi is formed, and each weight is rounded once, where the float32 operations round it."""
+  x = np.clip(np.asarray(x, dtype=np.float64), mn, mx)
+  lo = np.floor(x)
+  p_hi = x - lo
+  if float32:
+    p_hi = p_hi.astype(np.float32).astype(np.float64)
+  out = np.zeros(x.shape + (mx - mn + 1,), np.float64)
+  idx = (lo - mn).astype(np.int64)
+  hi = np.minimum(idx + 1, mx - mn)
+  np.put_along_axis(out, hi[..., None], p_hi[..., None], axis=-1)
+  np.put_along_axis(out, idx[..., None], (1.0 - p_hi)[..., None], axis=-1)  # the low bin wins on integers
+  return x, (out.astype(np.float32) if float32 else out)
+
+
 def inverse_transform(logits, mn, mx, no_target_transform=False):
   logits = np.ascontiguousarray(logits, dtype=np.float32)
   B, size = logits.shape

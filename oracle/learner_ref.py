@@ -14,12 +14,13 @@ def scalar_transform(x):
 
 
 def scalar_to_support(x, mn, mx):
-  """config.py:56-68 (clamp, p_high at ceil, then p_low at floor)."""
+  """config.py:56-68 (clamp, p_high at ceil, then p_low at floor).  The support has x's dtype and device, so that
+  float64 targets give a float64 reference."""
   x = x.clamp(mn, mx)
   floor, ceil = x.floor(), x.ceil()
   p_high = x - floor
   p_low = 1 - p_high
-  support = torch.zeros(x.shape[0], x.shape[1], mx - mn + 1)
+  support = torch.zeros(x.shape[0], x.shape[1], mx - mn + 1, dtype=x.dtype, device=x.device)
   support.scatter_(2, (ceil - mn).long().unsqueeze(-1), p_high.unsqueeze(-1))
   support.scatter_(2, (floor - mn).long().unsqueeze(-1), p_low.unsqueeze(-1))
   return support
