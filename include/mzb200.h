@@ -592,11 +592,6 @@ int mz_scalar_unroll_loss(const mz_loss_cfg* c, int32_t scalar_loss, const float
 int mz_debug_div_check(uint64_t seed, int32_t blocks, int32_t per_thread, uint64_t* mismatches,
                        uint64_t* tested, void* stream);
 
-/* mz_tree_step with at most 16 actions: batches of up to `max_games` games run on the warp-per-game kernel,
- * larger ones on the sub-warp-per-game kernels (8 / 4 / 2 games per warp).  Default: INT32_MAX -- the
- * warp-per-game kernel measured faster at every batch size; 0 = always sub-warps.  Results are identical. */
-int mz_tree_set_wide_step_max_games(int32_t max_games);
-
 /* Games (= warps) per CTA of the warp-per-game step kernel: 1, 2 or 4; 0 (default) = by launch size (one game per
  * CTA from 512 games per launch on: a CTA frees its staged image as soon as its own descent ends and fits beside a
  * network-kernel CTA; four below that).  Results are identical; the parity tests run both. */

@@ -209,7 +209,6 @@ _SIGNATURES = {
                                         _V, _V]),
     "mz_debug_div_check": (C.c_int, [C.c_uint64, C.c_int32, C.c_int32, _V, _V, _V]),
     "mz_set_programmatic_launch": (C.c_int, [C.c_int32]),
-    "mz_tree_set_wide_step_max_games": (C.c_int, [C.c_int32]),
     "mz_tree_set_games_per_block": (C.c_int, [C.c_int32]),
     "mz_version": (C.c_char_p, []),
     "mz_compiled_arch": (C.c_int32, []),

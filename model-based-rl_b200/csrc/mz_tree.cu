@@ -1,13 +1,12 @@
 // Tree kernels: root set-up, pUCT descent, expand + backup, root statistics, action selection.
 //
-// One sub-warp of LPG lanes (LPG = 4, 8, 16 or 32, the smallest >= A) owns one game; lane `a`
-// owns action `a`.  All score arithmetic is IEEE binary64 in the reference's operation order
-// (explicit __d*_rn intrinsics; this file is also compiled with -fmad=false), so that argmaxes --
-// and therefore visit counts -- are bit-identical to mcts.py executed by CPython.
+// One warp owns one game and lane `a` owns action `a` (A <= 32).  All score arithmetic is IEEE
+// binary64 in the reference's operation order (explicit __d*_rn intrinsics; this file is also
+// compiled with -fmad=false), so that argmaxes -- and therefore visit counts -- are bit-identical to
+// mcts.py executed by CPython.
 //
 // Reference: mcts.py:6-145, config.py:70-81, game.py:106-111 (JimOhman/model-based-rl).
 #include <math.h>
-#include <stdlib.h>
 
 #include <type_traits>
 
@@ -20,28 +19,16 @@ namespace {
 
 constexpr int kThreads = 128;
 
-
-// MinMaxStats.normalize mcts.py:16-21
-MZ_DEV double mm_normalize(double v, double mn, double mx) {
-  if (mx > mn) return __ddiv_rn(__dsub_rn(v, mn), __dsub_rn(mx, mn));
-  if (mx == mn) return 1.0;
-  return v;
-}
-
-// Node.expand priors mcts.py:52-55 for the lanes of one group: p_a = exp(logit_a) / sum(p) with the
+// Node.expand priors mcts.py:52-55 for the lanes of one warp: p_a = exp(logit_a) / sum(p) with the
 // sum evaluated like CPython's builtin sum() over the legal actions in ascending order.
-template <int LPG>
-MZ_DEV double group_priors(float logit, bool legal, int sum_mode, int A) {
+MZ_DEV double legal_priors(float logit, bool legal, int sum_mode, int A) {
   const double p = legal ? mz_exp((double)logit) : 0.0;
-  const unsigned lane = threadIdx.x & 31u;
-  const unsigned group_shift = lane & ~(unsigned)(LPG - 1);
-  const unsigned group_mask = (LPG == 32 ? 0xffffffffu : ((1u << LPG) - 1u)) << group_shift;
-  const unsigned legal_bits = (__ballot_sync(MZ_FULL, legal) & group_mask) >> group_shift;
+  const unsigned legal_bits = __ballot_sync(MZ_FULL, legal);
   double f = 0.0, c = 0.0;
   bool first = true;
 #pragma unroll 1
   for (int a = 0; a < A; ++a) {
-    const double x = shfl_f64<LPG>(p, a);
+    const double x = shfl_f64<32>(p, a);
     if (!((legal_bits >> a) & 1u)) continue;
     if (first) {
       f = x;  // int 0 + x
@@ -59,207 +46,17 @@ MZ_DEV double group_priors(float logit, bool legal, int sum_mode, int A) {
   return legal ? __ddiv_rn(p, f) : 0.0;
 }
 
-// ------------------------------------------------------------------------------------------------
-// descent: while node.expanded(): select_child  (mcts.py:87-92, 104-124)
-//
-// `rd` is the image the group reads the tree from: the game block staged in shared memory by one
-// bulk async copy (STAGED) or the block in global memory.  Per level: one load of (prior, child)
-// for the lane's action, one dependent load of the child's cached (q, visit), one pb_c table
-// lookup, a binary64 multiply / divide / add, and a two-step redux argmax.
-// ------------------------------------------------------------------------------------------------
+// ================================================================================================
+// Descent (while node.expanded(): select_child, mcts.py:87-92, 104-124) and expand + backup of one
+// game by a converged warp: every loop bound and branch is warp-uniform, the child's (q, visit,
+// reward) arrives in one 16-byte load, MinMax normalisation divides by a per-descent constant, and
+// the sequential loops run A / depth iterations.
+// ================================================================================================
 MZ_DEV unsigned long long sortable_key(double x) {  // monotone map double -> u64 (no NaNs)
   const unsigned long long b = (unsigned long long)__double_as_longlong(x);
   return b ^ ((unsigned long long)((long long)b >> 63) | 0x8000000000000000ull);
 }
 
-template <int LPG>
-MZ_DEV void descend(const mz_tree& t, const MzGame& rd, bool valid, int sub, unsigned gmask,
-                    int16_t* path, int& out_depth, int& out_parent, int& out_action) {
-  const int A = t.num_actions, SP1 = t.num_simulations + 1;
-  const double init_score = t.init_value_score;
-  const double mn = rd.mn(), mx = rd.mx();
-  const unsigned gshift = (threadIdx.x & 31u) & ~(unsigned)(LPG - 1);
-  int node = 0, depth = 0, parent = 0, action = 0;
-  int N = rd.node(0).visit();
-  bool done = !valid;
-  if (valid && sub == 0) path[0] = 0;
-  while (__any_sync(MZ_FULL, !done)) {
-    const MzNode nd = rd.node(node);
-    const bool lane_ok = sub < A;
-    double prior = 0.0;
-    int ch = MZ_CHILD_ILLEGAL;
-    if (lane_ok) {
-      prior = nd.prior()[sub];
-      ch = nd.child()[sub];
-    }
-    int n = 0;
-    double q = 0.0;
-    if (ch >= 0) {
-      const MzNode c = rd.node(ch);
-      n = c.visit();
-      q = c.q();  // reward + discount * (+/-)value(), cached by the last backup through the child
-    }
-    double score;
-    if (N == 0) {  // mcts.py:105-108: an unvisited (root) node ranks children by prior
-      score = prior;
-    } else {       // ucb_score mcts.py:115-124
-      const double pb_c = __ldg(&t.pb_c_table[(size_t)N * SP1 + n]);
-      const double prior_score = __dmul_rn(pb_c, prior);
-      const double value_score = n > 0 ? mm_normalize(q, mn, mx) : init_score;
-      score = __dadd_rn(prior_score, value_score);
-    }
-    // max over (score, action) tuples, ties -> larger action (mcts.py:106-112): compare the
-    // order-preserving 64-bit keys with two 32-bit redux steps, then take the highest lane.
-    const bool cand = lane_ok && ch != MZ_CHILD_ILLEGAL;
-    const unsigned long long key = cand ? sortable_key(score) : 0ull;
-    const unsigned hi = (unsigned)(key >> 32);
-    const unsigned hi_max = __reduce_max_sync(gmask, hi);
-    const unsigned lo = (cand && hi == hi_max) ? (unsigned)key : 0u;
-    const unsigned lo_max = __reduce_max_sync(gmask, lo);
-    const bool is_max = cand && hi == hi_max && (unsigned)key == lo_max;
-    const unsigned winners = (__ballot_sync(gmask, is_max) & gmask) >> gshift;
-    const int best = winners ? 31 - __clz(winners) : -1;
-    const int src = best < 0 ? 0 : best;
-    const int ch_b = __shfl_sync(gmask, ch, src, LPG);
-    const int n_b = __shfl_sync(gmask, n, src, LPG);
-    if (!done) {
-      depth++;
-      if (ch_b < 0) {  // child not expanded: this is the leaf
-        parent = node;
-        action = best;
-        done = true;
-      } else {
-        node = ch_b;
-        N = n_b;
-        if (sub == 0) path[depth] = (int16_t)node;
-      }
-    }
-  }
-  out_depth = depth;
-  out_parent = parent;
-  out_action = action;
-}
-
-// ------------------------------------------------------------------------------------------------
-// expand (mcts.py:47-55) + backpropagate (mcts.py:126-143).  Reads from `rd`; every store goes to
-// the global block `gl` and, when the image is staged, to `rd` as well (the descent of the next
-// simulation runs on it in the same launch).
-// ------------------------------------------------------------------------------------------------
-template <int LPG, bool STAGED>
-MZ_DEV void expand_backup(const mz_tree& t, const MzGame& rd, const MzGame& gl, bool valid, int sub,
-                          int sim, float value_f, float reward_f, float logit, int16_t* path,
-                          int depth, int parent, int action) {
-  const int A = t.num_actions;
-  const bool two = t.two_players != 0;
-  const double disc = t.discount;
-  const int newn = sim + 1;
-  const float node_reward_new = (reward_f != 0.0f) ? reward_f : 0.0f;  // `if network_output.reward:`
-
-  const double prior = group_priors<LPG>(logit, sub < A, t.prior_sum_mode, A);
-  if (valid) {
-    const MzNode ng = gl.node(newn), ns = rd.node(newn);
-    if (sub < A) {
-      ng.prior()[sub] = prior;
-      ng.child()[sub] = (int16_t)MZ_CHILD_UNEXPANDED;
-      if (STAGED) {
-        ns.prior()[sub] = prior;
-        ns.child()[sub] = (int16_t)MZ_CHILD_UNEXPANDED;
-      }
-    }
-    if (sub == 0) {
-      ng.reward() = node_reward_new;
-      gl.node(parent).child()[action] = (int16_t)newn;
-      if (STAGED) {
-        ns.reward() = node_reward_new;
-        rd.node(parent).child()[action] = (int16_t)newn;
-      }
-      path[depth] = (int16_t)newn;
-    }
-  }
-
-  // backup.  Position k on the path holds node path[k] (k < depth) or the new node (k == depth).
-  double value = (double)value_f;
-  double lmin = INFINITY, lmax = -INFINITY;
-  int dmax = valid ? depth : 0;
-#pragma unroll
-  for (int m = 16; m > 0; m >>= 1) dmax = max(dmax, __shfl_xor_sync(MZ_FULL, dmax, m));
-  for (int base = (dmax / LPG) * LPG; base >= 0; base -= LPG) {
-    const int k = base + sub;
-    const bool has = valid && k <= depth;
-    const int nid = has ? (k == depth ? newn : (int)path[k]) : 0;
-    const MzNode nd = rd.node(nid);
-    double vs = 0.0;
-    int vc = 0;
-    float rw = 0.0f;
-    if (has) {
-      if (k == depth) {
-        rw = node_reward_new;
-      } else {
-        vs = nd.vsum();
-        vc = nd.visit();
-        rw = nd.reward();
-      }
-    }
-    double myval = 0.0;
-    const int jtop = min(LPG - 1, dmax - base);  // deepest position any group of the warp holds
-#pragma unroll 1
-    for (int j = jtop; j >= 0; --j) {
-      const int kk = base + j;
-      const float rj = __shfl_sync(MZ_FULL, rw, j, LPG);
-      if (valid && kk <= depth) {
-        if (sub == j) myval = value;
-        const bool same = two ? (((depth - kk) & 1) == 0) : true;
-        const double nr = (double)rj;
-        const double r = (two && same) ? -nr : nr;
-        value = __dadd_rn(r, __dmul_rn(disc, value));
-      }
-    }
-    if (has) {
-      const bool same = two ? (((depth - k) & 1) == 0) : true;
-      vs = __dadd_rn(vs, same ? myval : -myval);
-      vc += 1;
-      double new_q = 0.0;
-      if (k > 0) {  // mcts.py:136-141
-        const double nv = __ddiv_rn(vs, (double)vc);
-        const double dq = __dmul_rn(disc, nv);
-        new_q = two ? __dsub_rn((double)rw, dq) : __dadd_rn((double)rw, dq);
-        lmin = fmin(lmin, new_q);
-        lmax = fmax(lmax, new_q);
-      }
-      const MzNode ng = gl.node(nid);
-      ng.vsum() = vs;
-      ng.q() = new_q;
-      ng.visit() = vc;
-      if (STAGED) {
-        nd.vsum() = vs;
-        nd.q() = new_q;
-        nd.visit() = vc;
-      }
-    }
-  }
-#pragma unroll
-  for (int m = LPG / 2; m > 0; m >>= 1) {
-    lmin = fmin(lmin, shfl_xor_f64<LPG>(lmin, m));
-    lmax = fmax(lmax, shfl_xor_f64<LPG>(lmax, m));
-  }
-  if (valid && sub == 0) {
-    if (lmin < rd.mn()) {
-      gl.mn() = lmin;
-      if (STAGED) rd.mn() = lmin;
-    }
-    if (lmax > rd.mx()) {
-      gl.mx() = lmax;
-      if (STAGED) rd.mx() = lmax;
-    }
-  }
-}
-
-// ================================================================================================
-// Warp-per-game fast path (LPG == 32, i.e. 17..32 actions: the Atari-scale sweep).  Same arithmetic
-// as descend<> / expand_backup<> above, restated for a converged warp: every loop bound and branch
-// is warp-uniform, the child's (q, visit, reward) arrives in one 16-byte load, MinMax normalisation
-// divides by a per-descent constant, and the sequential loops run A / depth iterations instead of 32.
-// ================================================================================================
 struct NodeHead {  // first 16 bytes of a node record
   double q;
   int32_t visit;
@@ -422,8 +219,8 @@ MZ_DEV void descend_loop(const mz_tree& t, typename ImgLoad<STAGED>::Addr nodes,
 }
 
 template <bool STAGED>
-MZ_DEV void descend_w32(const mz_tree& t, const uint8_t* img, int lane, int16_t* path, int& out_depth,
-                        int& out_parent, int& out_action) {
+MZ_DEV void descend(const mz_tree& t, const uint8_t* img, int lane, int16_t* path, int& out_depth,
+                    int& out_parent, int& out_action) {
   using L = ImgLoad<STAGED>;
   const int A = t.num_actions;
   const typename L::Addr base = L::base(img);
@@ -455,13 +252,13 @@ MZ_DEV void descend_w32(const mz_tree& t, const uint8_t* img, int lane, int16_t*
   }
 }
 
-// expand (mcts.py:47-55) + backpropagate (mcts.py:126-143) for one game per warp.  `img` is the
+// expand (mcts.py:47-55) + backpropagate (mcts.py:126-143).  `img` is the
 // image the warp reads (shared memory when STAGED, else the global block); stores go to the global
 // block and, when staged, to the image as well.
 template <bool STAGED>
-MZ_DEV void expand_backup_w32(const mz_tree& t, uint8_t* img, uint8_t* gbl, int lane, int sim,
-                              float value_f, float reward_f, float logit, int16_t* path, int depth,
-                              int parent, int action) {
+MZ_DEV void expand_backup(const mz_tree& t, uint8_t* img, uint8_t* gbl, int lane, int sim,
+                          float value_f, float reward_f, float logit, int16_t* path, int depth,
+                          int parent, int action) {
   const int A = t.num_actions, NB = t.node_bytes;
   const bool two = t.two_players != 0;
   const double disc = t.discount;
@@ -587,47 +384,45 @@ MZ_DEV void expand_backup_w32(const mz_tree& t, uint8_t* img, uint8_t* gbl, int 
   }
 }
 
-template <int LPG>
-MZ_DEV void copy_words(uint32_t* dst, const uint32_t* src, int words, int sub) {
-  for (int i = sub; i < words; i += LPG) dst[i] = src[i];
+MZ_DEV void copy_words(uint32_t* dst, const uint32_t* src, int words, int lane) {
+  for (int i = lane; i < words; i += 32) dst[i] = src[i];
 }
 
 // ------------------------------------------------------------------------------------------------
 // kernels
 // ------------------------------------------------------------------------------------------------
-template <int LPG>
 __global__ void __launch_bounds__(kThreads)
 set_root_kernel(mz_tree t, const float* __restrict__ root_logits,
                 const uint32_t* __restrict__ legal_mask, const double* __restrict__ noise,
                 double noise_frac, const int8_t* __restrict__ root_to_play,
                 const uint32_t* __restrict__ root_hidden, const double* __restrict__ root_priors) {
-  const int gidx = (blockIdx.x * kThreads + threadIdx.x) / LPG;
-  const int sub = threadIdx.x & (LPG - 1);
+  const int gidx = (blockIdx.x * kThreads + threadIdx.x) / 32;
+  const int lane = threadIdx.x & 31;
   const bool valid = gidx < t.num_games;
   const int g = valid ? gidx : t.num_games - 1;
   const int A = t.num_actions;
   const MzGame gm{t.games + (size_t)g * t.game_bytes, t.node_bytes, A};
   const uint32_t lm = legal_mask ? legal_mask[g] : 0xffffffffu;
-  const bool legal = sub < A && ((lm >> sub) & 1u);
+  const bool legal = lane < A && ((lm >> lane) & 1u);
   double prior;
   if (root_priors) {  // the caller ran Node.expand / add_exploration_noise itself
-    prior = legal ? root_priors[(size_t)g * A + sub] : 0.0;
+    prior = legal ? root_priors[(size_t)g * A + lane] : 0.0;
   } else {
-    const float logit = sub < A ? root_logits[(size_t)g * A + sub] : 0.0f;
-    prior = group_priors<LPG>(logit, legal, t.prior_sum_mode, A);
+    const float logit = lane < A ? root_logits[(size_t)g * A + lane] : 0.0f;
+    prior = legal_priors(logit, legal, t.prior_sum_mode, A);
   }
   if (noise && legal) {  // add_exploration_noise mcts.py:57-61; noise is dense over children
-    const int j = __popc(lm & ((1u << sub) - 1u));
+    const int j = __popc(lm & ((1u << lane) - 1u));
     const double nz = noise[(size_t)g * A + j];
     prior = __dadd_rn(__dmul_rn(prior, __dsub_rn(1.0, noise_frac)), __dmul_rn(nz, noise_frac));
   }
   if (!valid) return;
   const MzNode root = gm.node(0);
-  if (sub < A) {
-    root.prior()[sub] = prior;
-    root.child()[sub] = (int16_t)(legal ? MZ_CHILD_UNEXPANDED : MZ_CHILD_ILLEGAL);
+  if (lane < A) {
+    root.prior()[lane] = prior;
+    root.child()[lane] = (int16_t)(legal ? MZ_CHILD_UNEXPANDED : MZ_CHILD_ILLEGAL);
   }
-  if (sub == 0) {
+  if (lane == 0) {
     root.vsum() = 0.0;
     root.q() = 0.0;
     root.visit() = 0;
@@ -637,83 +432,14 @@ set_root_kernel(mz_tree t, const float* __restrict__ root_logits,
     gm.root_to_play() = root_to_play ? (int32_t)root_to_play[g] : 1;
   }
   if (root_hidden && t.hidden_words > 0)
-    copy_words<LPG>(t.hidden + (size_t)g * (t.num_simulations + 1) * t.hidden_words,
-                    root_hidden + (size_t)g * t.hidden_words, t.hidden_words, sub);
+    copy_words(t.hidden + (size_t)g * (t.num_simulations + 1) * t.hidden_words,
+               root_hidden + (size_t)g * t.hidden_words, t.hidden_words, lane);
 }
 
 // One launch per simulation boundary: [expand + backup of simulation `sim`] then [descent of
 // simulation sim + 1].  STAGED: the live part of each game block (header + nodes 0..sim) is brought
 // into shared memory with one cp.async.bulk (TMA unit) per game and both phases run on that image.
-// blockDim.x = LPG * games_per_block.
-template <int LPG, bool STAGED>
-__global__ void __launch_bounds__(kThreads)
-tree_step_kernel(mz_tree t, int sim, int do_backup, int do_select, int live_nodes, int stage_bytes,
-                 const float* __restrict__ value, const float* __restrict__ reward,
-                 const float* __restrict__ logits, const uint32_t* __restrict__ new_hidden,
-                 uint32_t* __restrict__ gathered_hidden, int32_t* __restrict__ trace_parent,
-                 int32_t* __restrict__ trace_action, int32_t* __restrict__ trace_depth) {
-  extern __shared__ __align__(128) uint8_t smem[];
-  const int gpb = blockDim.x / LPG;
-  const int grp = threadIdx.x / LPG;
-  const int gidx = blockIdx.x * gpb + grp;
-  const int sub = threadIdx.x & (LPG - 1);
-  const bool valid = gidx < t.num_games;
-  const int g = valid ? gidx : t.num_games - 1;
-  const int A = t.num_actions, SP1 = t.num_simulations + 1, HW = t.hidden_words;
-  const unsigned lane = threadIdx.x & 31u;
-  const unsigned gmask = (LPG == 32 ? 0xffffffffu : ((1u << LPG) - 1u)) << (lane & ~(unsigned)(LPG - 1));
-  const MzGame gl{t.games + (size_t)g * t.game_bytes, t.node_bytes, A};
-  MzGame rd = gl;
-  int16_t* path = t.path + (size_t)g * (t.num_simulations + 2);
-
-  if (STAGED) {
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)gpb * stage_bytes);
-    if (threadIdx.x == 0) {
-      for (int i = 0; i < gpb; ++i) mbar_init(&bars[i], 1);
-      mbar_fence_init();
-    }
-    __syncthreads();
-    uint8_t* image = smem + (size_t)grp * stage_bytes;
-    // nodes 0..live_nodes-1 exist before this launch (a backup creates node `sim + 1` in place)
-    const uint32_t live = MZ_GAME_HEADER_BYTES + (uint32_t)live_nodes * (uint32_t)t.node_bytes;
-    if (sub == 0) {
-      mbar_arrive_expect_tx(&bars[grp], live);
-      bulk_copy_g2s(image, gl.base, live, &bars[grp]);
-    }
-    mbar_wait(&bars[grp], 0);
-    rd = MzGame{image, t.node_bytes, A};
-  }
-
-  if (do_backup) {
-    const int depth = t.path_len[g], parent = t.leaf_parent[g], action = t.leaf_action[g];
-    const float logit = sub < A ? logits[(size_t)g * A + sub] : 0.0f;
-    expand_backup<LPG, STAGED>(t, rd, gl, valid, sub, sim, value[g], reward[g], logit, path, depth,
-                               parent, action);
-    if (valid && new_hidden && HW > 0)
-      copy_words<LPG>(t.hidden + ((size_t)g * SP1 + sim + 1) * HW, new_hidden + (size_t)g * HW, HW,
-                      sub);
-    __syncwarp();
-  }
-  if (do_select) {
-    int depth, parent, action;
-    descend<LPG>(t, rd, valid, sub, gmask, path, depth, parent, action);
-    if (valid) {
-      if (sub == 0) {
-        t.path_len[g] = depth;
-        t.leaf_parent[g] = parent;
-        t.leaf_action[g] = action;
-        if (trace_parent) trace_parent[g] = parent;
-        if (trace_action) trace_action[g] = action;
-        if (trace_depth) trace_depth[g] = depth;
-      }
-      if (gathered_hidden && HW > 0)
-        copy_words<LPG>(gathered_hidden + (size_t)g * HW,
-                        t.hidden + ((size_t)g * SP1 + parent) * HW, HW, sub);
-    }
-  }
-}
-
-// Warp-per-game variant of tree_step_kernel (17..32 actions).  blockDim.x = 32 * games_per_block.
+// blockDim.x = 32 * games_per_block.
 template <bool STAGED>
 __global__ void __launch_bounds__(kThreads)
 tree_step_w32_kernel(mz_tree t, int sim, int do_backup, int do_select, int live_nodes, int stage_bytes,
@@ -756,9 +482,9 @@ tree_step_w32_kernel(mz_tree t, int sim, int do_backup, int do_select, int live_
     const float logit = lane < A ? logits[(size_t)g * A + lane] : 0.0f;
     const float v = value[g], r = reward[g];
     if (STAGED) mbar_wait(&bars[warp], 0);
-    expand_backup_w32<STAGED>(t, img, gbl, lane, sim, v, r, logit, path, depth, parent, action);
+    expand_backup<STAGED>(t, img, gbl, lane, sim, v, r, logit, path, depth, parent, action);
     if (new_hidden && HW > 0)
-      copy_words<32>(t.hidden + ((size_t)g * SP1 + sim + 1) * HW, new_hidden + (size_t)g * HW, HW, lane);
+      copy_words(t.hidden + ((size_t)g * SP1 + sim + 1) * HW, new_hidden + (size_t)g * HW, HW, lane);
     __syncwarp();
   } else {
     pdl_wait();
@@ -767,7 +493,7 @@ tree_step_w32_kernel(mz_tree t, int sim, int do_backup, int do_select, int live_
   }
   if (do_select) {
     int depth, parent, action;
-    descend_w32<STAGED>(t, img, lane, path, depth, parent, action);
+    descend<STAGED>(t, img, lane, path, depth, parent, action);
     if (lane == 0) {
       t.path_len[g] = depth;
       t.leaf_parent[g] = parent;
@@ -777,8 +503,7 @@ tree_step_w32_kernel(mz_tree t, int sim, int do_backup, int do_select, int live_
       if (trace_depth) trace_depth[g] = depth;
     }
     if (gathered_hidden && HW > 0)
-      copy_words<32>(gathered_hidden + (size_t)g * HW, t.hidden + ((size_t)g * SP1 + parent) * HW, HW,
-                     lane);
+      copy_words(gathered_hidden + (size_t)g * HW, t.hidden + ((size_t)g * SP1 + parent) * HW, HW, lane);
   }
 }
 
@@ -973,46 +698,20 @@ int check_tree(const mz_tree* t) {
   return MZ_OK;
 }
 
-int g_w32_max_games = 0x7fffffff;  // mz_tree_set_wide_step_max_games
-
 // Games (= warps) per CTA of the warp-per-game step kernel.  One game per CTA from 512 games per launch on: a CTA
 // gives its shared memory back as soon as ITS game's descent ends (a four-game CTA holds 4 images until the
 // deepest of them is done), 21 instead of 20 images fit an SM at the last simulation, and a one-game CTA fits
 // beside a network-kernel CTA (16 KB of shared memory left there).  Measured on one box, 30 timed moves, 4 / 2 / 1
 // games per CTA: C4 136.9-137.3 / 135.9 / 139.1-139.3 M expansions/s, 16 384 games 191.6-194.8 / 196.5 / 209.6 M,
 // C3 shape 188.5-189.6 / 186.5 / 205.9-208.7 M; 256-game launches (C2 shape) prefer four: 60.1-60.3 vs 57.6-59.0 M.
-// mz_tree_set_games_per_block(1|2|4) (or MZ_W32_GPB in the environment) forces one value, 0 = by launch size.
-int g_w32_gpb = -1;
+// mz_tree_set_games_per_block(1|2|4) forces one value, 0 = by launch size.
+int g_w32_gpb = 0;
 int w32_games_per_block(int num_games) {
-  if (g_w32_gpb < 0) {
-    const char* e = getenv("MZ_W32_GPB");
-    const int v = e ? atoi(e) : 0;
-    g_w32_gpb = (v == 1 || v == 2 || v == 4) ? v : 0;
-  }
   if (g_w32_gpb) return g_w32_gpb;
   return num_games >= 512 ? 1 : kThreads / 32;
 }
 
-template <typename F>
-int dispatch_lpg(int A, F&& f) {
-  if (A <= 4) return f(std::integral_constant<int, 4>());
-  if (A <= 8) return f(std::integral_constant<int, 8>());
-  if (A <= 16) return f(std::integral_constant<int, 16>());
-  return f(std::integral_constant<int, 32>());
-}
-
 constexpr int kMaxStageSmem = 200 * 1024;
-
-template <int LPG, bool STAGED>
-int set_smem_attr_once() {
-  static int rc = -1;
-  if (rc < 0) {
-    cudaError_t e = cudaFuncSetAttribute(tree_step_kernel<LPG, STAGED>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxStageSmem + 1024);
-    rc = (int)e;
-  }
-  return rc;
-}
 
 template <bool STAGED>
 int set_smem_attr_w32_once() {
@@ -1026,59 +725,34 @@ int set_smem_attr_w32_once() {
 int launch_step(const mz_tree* t, int sim, int live_nodes, int do_backup, int do_select, const float* value,
                 const float* reward, const float* logits, const uint32_t* new_hidden,
                 uint32_t* gathered_hidden, int32_t* tp, int32_t* ta, int32_t* td, void* stream) {
-  // Few actions: a sub-warp per game packs 8 / 4 / 2 games into a warp, but the games of a warp wait for each
-  // other's descents and the code is not warp-uniform.  Measured (A = 4, 50 simulations): the converged
-  // warp-per-game kernel is faster at every batch size -- 13.9 vs 32.0 us per step at 4096 games, 27.8 vs
-  // 44.5 us at 16 k, 83 vs 122 us at 64 k -- so it serves every action count up to 32; the sub-warp kernels
-  // stay selectable (g_w32_max_games = 0) and covered by the parity tests.
-  const int step_actions = (t->num_games <= g_w32_max_games) ? 32 : t->num_actions;
-  return dispatch_lpg(step_actions, [&](auto lpg) {
-    constexpr int LPG = decltype(lpg)::value;
-    // image: header + nodes 0..sim+1 (the new node is built in place)
-    const int nodes = live_nodes + (do_backup ? 1 : 0);
-    const int stage_bytes = MZ_GAME_HEADER_BYTES + nodes * t->node_bytes;
-    int gpb = kThreads / LPG;
-    if (LPG == 32) gpb = w32_games_per_block(t->num_games);
-    while (gpb > 1 && (size_t)gpb * stage_bytes > 96 * 1024) gpb >>= 1;
-    const bool staged = (size_t)gpb * stage_bytes <= kMaxStageSmem;
-    if (LPG == 32) {  // one game per warp: the converged-warp kernel
-      if (!staged) gpb = kThreads / 32;
-      const int grid = (t->num_games + gpb - 1) / gpb;
-      if (staged) {
-        int rc = set_smem_attr_w32_once<true>();
-        if (rc) return rc;
-        cudaError_t e = mz_launch(tree_step_w32_kernel<true>, dim3(grid), dim3(gpb * 32),
-                                  (size_t)gpb * stage_bytes + sizeof(uint64_t) * gpb, (cudaStream_t)stream,
-                                  do_backup != 0, *t, sim, do_backup, do_select, live_nodes, stage_bytes, value,
-                                  reward, logits, new_hidden, gathered_hidden, tp, ta, td);
-        if (e != cudaSuccess) return (int)e;
-      } else {
-        cudaError_t e = mz_launch(tree_step_w32_kernel<false>, dim3(grid), dim3(gpb * 32), 0,
-                                  (cudaStream_t)stream, do_backup != 0, *t, sim, do_backup, do_select,
-                                  live_nodes, 0, value, reward, logits, new_hidden, gathered_hidden, tp, ta, td);
-        if (e != cudaSuccess) return (int)e;
-      }
-      MZ_LAUNCH_CHECK();
-      return MZ_OK;
-    }
-    if (staged) {
-      int rc = set_smem_attr_once<LPG, true>();
-      if (rc) return rc;
-      const int grid = (t->num_games + gpb - 1) / gpb;
-      const size_t smem = (size_t)gpb * stage_bytes + sizeof(uint64_t) * gpb;
-      tree_step_kernel<LPG, true><<<grid, gpb * LPG, smem, (cudaStream_t)stream>>>(
-          *t, sim, do_backup, do_select, live_nodes, stage_bytes, value, reward, logits, new_hidden,
-          gathered_hidden, tp, ta, td);
-    } else {  // tree too large for shared memory: run on the global block directly
-      gpb = kThreads / LPG;
-      const int grid = (t->num_games + gpb - 1) / gpb;
-      tree_step_kernel<LPG, false><<<grid, gpb * LPG, 0, (cudaStream_t)stream>>>(
-          *t, sim, do_backup, do_select, live_nodes, 0, value, reward, logits, new_hidden,
-          gathered_hidden, tp, ta, td);
-    }
-    MZ_LAUNCH_CHECK();
-    return MZ_OK;
-  });
+  // One warp per game at every action count.  Packing 8 / 4 / 2 games of few actions into a warp makes the games
+  // of a warp wait for each other's descents, and the code is not warp-uniform.  Measured (A = 4, 50 simulations):
+  // the converged warp-per-game kernel is faster at every batch size -- 13.9 vs 32.0 us per step at 4096 games,
+  // 27.8 vs 44.5 us at 16 k, 83 vs 122 us at 64 k.
+  // image: header + nodes 0..sim+1 (the new node is built in place)
+  const int nodes = live_nodes + (do_backup ? 1 : 0);
+  const int stage_bytes = MZ_GAME_HEADER_BYTES + nodes * t->node_bytes;
+  int gpb = w32_games_per_block(t->num_games);
+  while (gpb > 1 && (size_t)gpb * stage_bytes > 96 * 1024) gpb >>= 1;
+  const bool staged = (size_t)gpb * stage_bytes <= kMaxStageSmem;
+  if (!staged) gpb = kThreads / 32;
+  const int grid = (t->num_games + gpb - 1) / gpb;
+  if (staged) {
+    int rc = set_smem_attr_w32_once<true>();
+    if (rc) return rc;
+    cudaError_t e = mz_launch(tree_step_w32_kernel<true>, dim3(grid), dim3(gpb * 32),
+                              (size_t)gpb * stage_bytes + sizeof(uint64_t) * gpb, (cudaStream_t)stream,
+                              do_backup != 0, *t, sim, do_backup, do_select, live_nodes, stage_bytes, value,
+                              reward, logits, new_hidden, gathered_hidden, tp, ta, td);
+    if (e != cudaSuccess) return (int)e;
+  } else {  // tree too large for shared memory: run on the global block directly
+    cudaError_t e = mz_launch(tree_step_w32_kernel<false>, dim3(grid), dim3(gpb * 32), 0,
+                              (cudaStream_t)stream, do_backup != 0, *t, sim, do_backup, do_select,
+                              live_nodes, 0, value, reward, logits, new_hidden, gathered_hidden, tp, ta, td);
+    if (e != cudaSuccess) return (int)e;
+  }
+  MZ_LAUNCH_CHECK();
+  return MZ_OK;
 }
 
 }  // namespace
@@ -1115,15 +789,11 @@ int mz_tree_set_root(const mz_tree* t, const float* root_logits, const uint32_t*
   int rc = check_tree(t);
   if (rc) return rc;
   if (!root_logits) return MZ_ERR_BAD_ARG;
-  return dispatch_lpg(t->num_actions, [&](auto lpg) {
-    constexpr int LPG = decltype(lpg)::value;
-    const int gpb = kThreads / LPG;
-    const int grid = (t->num_games + gpb - 1) / gpb;
-    set_root_kernel<LPG><<<grid, kThreads, 0, (cudaStream_t)stream>>>(
-        *t, root_logits, legal_mask, noise, noise_frac, root_to_play, root_hidden, nullptr);
-    MZ_LAUNCH_CHECK();
-    return MZ_OK;
-  });
+  const int grid = (t->num_games + 3) / 4;  // a warp per game
+  set_root_kernel<<<grid, kThreads, 0, (cudaStream_t)stream>>>(*t, root_logits, legal_mask, noise, noise_frac,
+                                                               root_to_play, root_hidden, nullptr);
+  MZ_LAUNCH_CHECK();
+  return MZ_OK;
 }
 
 int mz_tree_set_root_priors(const mz_tree* t, const double* root_priors, const uint32_t* legal_mask,
@@ -1131,15 +801,11 @@ int mz_tree_set_root_priors(const mz_tree* t, const double* root_priors, const u
   int rc = check_tree(t);
   if (rc) return rc;
   if (!root_priors) return MZ_ERR_BAD_ARG;
-  return dispatch_lpg(t->num_actions, [&](auto lpg) {
-    constexpr int LPG = decltype(lpg)::value;
-    const int gpb = kThreads / LPG;
-    const int grid = (t->num_games + gpb - 1) / gpb;
-    set_root_kernel<LPG><<<grid, kThreads, 0, (cudaStream_t)stream>>>(
-        *t, nullptr, legal_mask, nullptr, 0.0, root_to_play, root_hidden, root_priors);
-    MZ_LAUNCH_CHECK();
-    return MZ_OK;
-  });
+  const int grid = (t->num_games + 3) / 4;  // a warp per game
+  set_root_kernel<<<grid, kThreads, 0, (cudaStream_t)stream>>>(*t, nullptr, legal_mask, nullptr, 0.0,
+                                                               root_to_play, root_hidden, root_priors);
+  MZ_LAUNCH_CHECK();
+  return MZ_OK;
 }
 
 int mz_tree_select(const mz_tree* t, int32_t sim, uint32_t* gathered_hidden, int32_t* trace_parent,
@@ -1219,11 +885,6 @@ int mz_debug_div_check(uint64_t seed, int32_t blocks, int32_t per_thread, uint64
   div_check_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(
       seed, per_thread, (unsigned long long*)mismatches, (unsigned long long*)tested);
   MZ_LAUNCH_CHECK();
-  return MZ_OK;
-}
-
-int mz_tree_set_wide_step_max_games(int32_t max_games) {
-  g_w32_max_games = max_games;
   return MZ_OK;
 }
 

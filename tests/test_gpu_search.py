@@ -50,17 +50,15 @@ def _run_golden(g):
   return eng, res
 
 
-@pytest.fixture(params=["wide", "wide_1_game_per_cta", "subwarp"])
+@pytest.fixture(params=["wide", "wide_1_game_per_cta"])
 def step_kernel(request):
-  """Trees with <= 16 actions have two step kernels (warp per game, the default; sub-warp per game beyond
-  mz_tree_set_wide_step_max_games), and the warp-per-game kernel runs four games per CTA or one (the choice
-  large launches get, mz_tree_set_games_per_block): run the parity tests through all of them."""
+  """The step kernel runs four games per CTA or one (the choice large launches get,
+  mz_tree_set_games_per_block): run the parity tests through both, since the golden batches are too small to
+  reach one game per CTA by launch size."""
   from model_based_rl_b200 import _lib
   lib = _lib.load()
-  lib.mz_tree_set_wide_step_max_games(0 if request.param == "subwarp" else 0x7fffffff)
-  lib.mz_tree_set_games_per_block(1 if request.param == "wide_1_game_per_cta" else (4 if request.param == "wide" else 0))
+  lib.mz_tree_set_games_per_block(1 if request.param == "wide_1_game_per_cta" else 4)
   yield request.param
-  lib.mz_tree_set_wide_step_max_games(0x7fffffff)
   lib.mz_tree_set_games_per_block(0)
 
 
