@@ -35,7 +35,7 @@ extern "C" {
 #define MZ_ERR_BAD_ARG (-1)
 #define MZ_ERR_UNSUPPORTED (-2)
 
-#define MZ_MAX_ACTIONS 32      /* one lane per action, one (sub-)warp per game */
+#define MZ_MAX_ACTIONS 64      /* one warp per game; lane l owns action l and, when A > 32, action l + 32 */
 #define MZ_CHILD_UNEXPANDED (-1)
 #define MZ_CHILD_ILLEGAL (-2)  /* action absent from root.children (illegal move) */
 #define MZ_GAME_HEADER_BYTES 32
@@ -53,6 +53,10 @@ extern "C" {
 /*               value(), the quantity backpropagate feeds to MinMaxStats (mcts.py:136-141) and   */
 /*               ucb_score normalises (mcts.py:120-121), cached at backup time)                   */
 /* node_bytes  = round_up(24 + 10 * A, 16);  game_bytes = round_up(32 + (S+1) * node_bytes, 128)  */
+/* ------------------------------------------------------------------------------------------- */
+/* Legal masks (mz_tree_set_root, mz_tree_set_root_priors, mz_select_action, mz_dirichlet_noise):  */
+/* W = ceil(A / 32) u32 words per game, row-major [G][W]; bit b of word w set <=> action 32 w + b  */
+/* is legal.  Bits at or beyond A are ignored.  For A <= 32 this is one word per game.             */
 /* ------------------------------------------------------------------------------------------- */
 typedef struct mz_tree {
   int32_t num_games;        /* G */
@@ -92,7 +96,7 @@ int mz_fill_pb_c_table(int32_t num_simulations, double pb_c_base, double pb_c_in
  * actors.py:142), Node.add_exploration_noise (mcts.py:57-61, actors.py:143) and
  * MinMaxStats.reset (mcts.py:79).
  *   root_logits [G][A] f32   initial_inference().policy_logits
- *   legal_mask  [G] u32      bit a set <=> a in legal_actions; NULL = all legal
+ *   legal_mask  [G][W] u32   legal-action mask (layout above); NULL = all legal
  *   noise       [G][A] f64   Dirichlet sample, dense over the root's children in action order
  *                            (what np.random.dirichlet returns at mcts.py:59); NULL = no noise
  *   root_to_play[G] i8       game.to_play; NULL = 1
@@ -105,7 +109,7 @@ int mz_tree_set_root(const mz_tree* t, const float* root_logits, const uint32_t*
 /*
  * Node.add_exploration_noise's draw (mcts.py:59: np.random.dirichlet([root_dirichlet_alpha] * len(actions))) for
  * every game of a move, made on the device into the `noise` layout of mz_tree_set_root / mz_fc_search: row g holds
- * one value per legal action of game g (legal_mask[g] bit a = action a is legal; NULL = all), dense from column 0,
+ * one value per legal action of game g (legal_mask [G][W], layout above; NULL = all), dense from column 0,
  * zeros behind.  Same distribution, another stream than numpy's: Philox4x32-10 keyed by (seed, game, action) and
  * advanced by `move`; the host-supplied buffer stays the bit-exact path.
  */
@@ -164,7 +168,7 @@ int mz_tree_root_stats(const mz_tree* t, int32_t* visits, double* child_visits, 
 
 /*
  * Config.select_action (config.py:70-81) for G roots with host-supplied randomness.
- *   visits [G][A] i32, legal_mask [G] u32 or NULL, temperature [G] f64, uniforms [G] f64 in [0,1)
+ *   visits [G][A] i32, legal_mask [G][W] u32 or NULL, temperature [G] f64, uniforms [G] f64 in [0,1)
  *   T > 0 : p = visits**(1/T) / sum; action = children[searchsorted(cumsum(p)/cumsum(p)[-1], u,
  *           'right')]  (what np.random.choice(len, p=p) does with one uniform draw)
  *   T == 0: uniform over the argmax ties, tie index = floor(u * n_ties)
@@ -596,6 +600,10 @@ int mz_debug_div_check(uint64_t seed, int32_t blocks, int32_t per_thread, uint64
  * CTA from 512 games per launch on: a CTA frees its staged image as soon as its own descent ends and fits beside a
  * network-kernel CTA; four below that).  Results are identical; the parity tests run both. */
 int mz_tree_set_games_per_block(int32_t games);
+
+/* Where the step kernel reads a game's tree: 0 (default) = a shared-memory image of its live part whenever the
+ * images fit, 1 = the global block directly.  Results are identical; for measurements. */
+int mz_debug_set_tree_staging(int32_t mode);
 
 /* The per-simulation kernels (tree step, recurrent network) are launched as programmatic dependents
  * (their prologues overlap the predecessor's tail; griddepcontrol.wait before the first dependent

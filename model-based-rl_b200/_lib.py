@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmzb200.so")
 CSRC = os.path.join(_HERE, "csrc")
 
-MZ_MAX_ACTIONS = 32
+MZ_MAX_ACTIONS = 64  # one warp per game; lane l owns action l and, when A > 32, action l + 32
 CHILD_UNEXPANDED = -1
 CHILD_ILLEGAL = -2
 GAME_HEADER_BYTES = 32
@@ -210,6 +210,7 @@ _SIGNATURES = {
     "mz_debug_div_check": (C.c_int, [C.c_uint64, C.c_int32, C.c_int32, _V, _V, _V]),
     "mz_set_programmatic_launch": (C.c_int, [C.c_int32]),
     "mz_tree_set_games_per_block": (C.c_int, [C.c_int32]),
+    "mz_debug_set_tree_staging": (C.c_int, [C.c_int32]),
     "mz_version": (C.c_char_p, []),
     "mz_compiled_arch": (C.c_int32, []),
 }

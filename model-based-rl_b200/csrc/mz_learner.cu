@@ -281,7 +281,9 @@ __global__ void ln_relu_forward_kernel(int rows, int d, const float* __restrict_
   float* out = X_out + (size_t)r * ldx;
   if (lane < d) out[lane] = fmaxf(c0 * rstd * gamma[lane] + beta[lane], 0.0f);
   if (lane + 32 < d) out[lane + 32] = fmaxf(c1 * rstd * gamma[lane + 32] + beta[lane + 32], 0.0f);
-  if (lane < A) out[d + lane] = (actions != nullptr && actions[(size_t)r * action_stride] == lane) ? 1.0f : 0.0f;
+  const int act = actions != nullptr ? actions[(size_t)r * action_stride] : -1;
+  if (lane < A) out[d + lane] = act == lane ? 1.0f : 0.0f;
+  if (lane + 32 < A) out[d + lane + 32] = act == lane + 32 ? 1.0f : 0.0f;
   if (lane == 0) {
     mean_out[r] = mean;
     rstd_out[r] = rstd;
@@ -435,7 +437,7 @@ int mz_mlp2_backward(int32_t rows, int32_t d_in, int32_t ldx, const float* X, co
 int mz_ln_relu_forward(int32_t rows, int32_t d, const float* Y, const float* gamma, const float* beta,
                        const int32_t* actions, int32_t action_stride, int32_t num_actions, float* X_out, int32_t ldx,
                        float* mean, float* rstd, void* stream) {
-  if (rows < 1 || d < 1 || d > 64 || num_actions < 0 || num_actions > 32 || ldx < d + num_actions || !Y || !gamma || !beta ||
+  if (rows < 1 || d < 1 || d > 64 || num_actions < 0 || num_actions > 64 || ldx < d + num_actions || !Y || !gamma || !beta ||
       !X_out || !mean || !rstd)
     return MZ_ERR_BAD_ARG;
   ln_relu_forward_kernel<<<(rows + 7) / 8, 256, 0, (cudaStream_t)stream>>>(rows, d, Y, gamma, beta, actions, action_stride,

@@ -35,24 +35,37 @@ MZ_DEV double gamma_variate(curandStatePhilox4_32_10_t* st, double alpha) {
   return out;
 }
 
-// a warp per game, lane = rank of the legal action (A <= 32)
+// a warp per game, lane l draws for the legal actions of ranks l and l + 32.  The Philox subsequence is
+// g * 32 + rank for A <= 32 and g * 64 + rank above.
 __global__ void dirichlet_noise_kernel(int G, int A, double alpha, const int32_t* __restrict__ legal,
                                        unsigned long long seed, unsigned long long move, double* __restrict__ noise) {
   const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (g >= G) return;
-  uint32_t mask = legal ? (uint32_t)legal[g] : 0xffffffffu;
-  if (A < 32) mask &= (1u << A) - 1u;
-  const int n = __popc(mask);
-  double x = 0.0;
-  if (lane < n) {
-    curandStatePhilox4_32_10_t st;
-    curand_init(seed, (unsigned long long)g * 32 + lane, move * 64, &st);
-    x = gamma_variate(&st, alpha);
+  const int W = (A + 31) >> 5;
+  int n = 0;
+  for (int w = 0; w < W; ++w) {
+    uint32_t mask = legal ? (uint32_t)legal[(size_t)g * W + w] : 0xffffffffu;
+    if (A < 32 * (w + 1)) mask &= (1u << (A - 32 * w)) - 1u;
+    n += __popc(mask);
   }
-  double sum = x;
+  double x[2] = {0.0, 0.0};
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const int rank = lane + 32 * h;
+    if (h < W && rank < n) {
+      curandStatePhilox4_32_10_t st;
+      curand_init(seed, (unsigned long long)g * 32 * W + rank, move * 64, &st);
+      x[h] = gamma_variate(&st, alpha);
+    }
+  }
+  double sum = W > 1 ? x[0] + x[1] : x[0];
 #pragma unroll
   for (int m = 16; m > 0; m >>= 1) sum += shfl_xor_f64<32>(sum, m);
-  if (lane < A) noise[(size_t)g * A + lane] = lane < n ? (sum > 0.0 ? x / sum : 1.0 / n) : 0.0;
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const int rank = lane + 32 * h;
+    if (h < W && rank < A) noise[(size_t)g * A + rank] = rank < n ? (sum > 0.0 ? x[h] / sum : 1.0 / n) : 0.0;
+  }
 }
 
 }  // namespace
@@ -61,7 +74,8 @@ extern "C" {
 
 int mz_dirichlet_noise(int32_t num_games, int32_t num_actions, double alpha, const int32_t* legal_mask,
                        uint64_t seed, uint64_t move, double* noise, void* stream) {
-  if (num_games < 1 || num_actions < 1 || num_actions > 32 || !(alpha > 0.0) || !noise) return MZ_ERR_BAD_ARG;
+  if (num_games < 1 || num_actions < 1 || num_actions > MZ_MAX_ACTIONS || !(alpha > 0.0) || !noise)
+    return MZ_ERR_BAD_ARG;
   dirichlet_noise_kernel<<<(num_games + 3) / 4, 128, 0, (cudaStream_t)stream>>>(num_games, num_actions, alpha, legal_mask,
                                                                                 seed, move, noise);
   MZ_LAUNCH_CHECK();

@@ -1,6 +1,9 @@
 // Tree kernels: root set-up, pUCT descent, expand + backup, root statistics, action selection.
 //
-// One warp owns one game and lane `a` owns action `a` (A <= 32).  All score arithmetic is IEEE
+// One warp owns one game.  Lane l owns action l, and action l + 32 as well when A > 32: the kernels are
+// instantiated for APL (actions per lane) = 1 (A <= 32) and 2 (32 < A <= 64), chosen from A at launch, and every
+// sequential pass over the actions (prior sums, argmax ties) runs over ascending action indices, the low half
+// (owned as action l) before the high half (action l + 32).  All score arithmetic is IEEE
 // binary64 in the reference's operation order (explicit __d*_rn intrinsics; this file is also
 // compiled with -fmad=false), so that argmaxes -- and therefore visit counts -- are bit-identical to
 // mcts.py executed by CPython.
@@ -19,31 +22,48 @@ namespace {
 
 constexpr int kThreads = 128;
 
+// Actions [32 h, end) of the game are held by the lanes as their action `lane + 32 h`.
+template <int APL>
+MZ_DEV int half_end(int A, int h) {
+  return APL == 1 ? A : min(A, 32 * h + 32);
+}
+
 // Node.expand priors mcts.py:52-55 for the lanes of one warp: p_a = exp(logit_a) / sum(p) with the
 // sum evaluated like CPython's builtin sum() over the legal actions in ascending order.
-MZ_DEV double legal_priors(float logit, bool legal, int sum_mode, int A) {
-  const double p = legal ? mz_exp((double)logit) : 0.0;
-  const unsigned legal_bits = __ballot_sync(MZ_FULL, legal);
+template <int APL>
+MZ_DEV void legal_priors(const float (&logit)[APL], const bool (&legal)[APL], int sum_mode, int A,
+                         double (&prior)[APL]) {
+  double p[APL];
+  unsigned legal_bits[APL];
+#pragma unroll
+  for (int h = 0; h < APL; ++h) {
+    p[h] = legal[h] ? mz_exp((double)logit[h]) : 0.0;
+    legal_bits[h] = __ballot_sync(MZ_FULL, legal[h]);
+  }
   double f = 0.0, c = 0.0;
   bool first = true;
+#pragma unroll
+  for (int h = 0; h < APL; ++h) {
 #pragma unroll 1
-  for (int a = 0; a < A; ++a) {
-    const double x = shfl_f64<32>(p, a);
-    if (!((legal_bits >> a) & 1u)) continue;
-    if (first) {
-      f = x;  // int 0 + x
-      first = false;
-    } else if (sum_mode == 0) {
-      f = __dadd_rn(f, x);
-    } else {  // Neumaier step, CPython >= 3.12 Python/bltinmodule.c
-      const double t = __dadd_rn(f, x);
-      if (fabs(f) >= fabs(x)) c = __dadd_rn(c, __dadd_rn(__dsub_rn(f, t), x));
-      else c = __dadd_rn(c, __dadd_rn(__dsub_rn(x, t), f));
-      f = t;
+    for (int a = 32 * h; a < half_end<APL>(A, h); ++a) {
+      const double x = shfl_f64<32>(p[h], a - 32 * h);
+      if (!((legal_bits[h] >> (a - 32 * h)) & 1u)) continue;
+      if (first) {
+        f = x;  // int 0 + x
+        first = false;
+      } else if (sum_mode == 0) {
+        f = __dadd_rn(f, x);
+      } else {  // Neumaier step, CPython >= 3.12 Python/bltinmodule.c
+        const double t = __dadd_rn(f, x);
+        if (fabs(f) >= fabs(x)) c = __dadd_rn(c, __dadd_rn(__dsub_rn(f, t), x));
+        else c = __dadd_rn(c, __dadd_rn(__dsub_rn(x, t), f));
+        f = t;
+      }
     }
   }
   if (sum_mode != 0 && c != 0.0 && isfinite(c)) f = __dadd_rn(f, c);
-  return legal ? __ddiv_rn(p, f) : 0.0;
+#pragma unroll
+  for (int h = 0; h < APL; ++h) prior[h] = legal[h] ? __ddiv_rn(p[h], f) : 0.0;
 }
 
 // ================================================================================================
@@ -148,61 +168,90 @@ struct ImgLoad {
   }
 };
 
-// (score, action) argmax over the lanes of a converged warp, ties -> larger action
-// (mcts.py:106-112): returns the winning lane or -1 when no lane is a candidate.
-MZ_DEV int warp_argmax(double score, bool cand) {
-  const unsigned long long key = cand ? sortable_key(score) : 0ull;
-  const unsigned long long best_key = warp_max_key(key);
-  const unsigned winners = __ballot_sync(MZ_FULL, cand && key == best_key);
-  return winners ? 31 - __clz(winners) : -1;
+// (score, action) argmax over the actions of a converged warp, ties -> larger action
+// (mcts.py:106-112): returns the winning action or -1 when no action is a candidate.
+template <int APL>
+MZ_DEV int warp_argmax(const double (&score)[APL], const bool (&cand)[APL]) {
+  if constexpr (APL == 1) {
+    const unsigned long long key = cand[0] ? sortable_key(score[0]) : 0ull;
+    const unsigned long long best_key = warp_max_key(key);
+    const unsigned winners = __ballot_sync(MZ_FULL, cand[0] && key == best_key);
+    return winners ? 31 - __clz(winners) : -1;
+  } else {
+    // the lane's own pair first (a tie goes to action lane + 32), then the warp; every high-half action is
+    // larger than every low-half one, so a high-half winner takes the ties across lanes
+    const unsigned long long k0 = cand[0] ? sortable_key(score[0]) : 0ull;
+    const unsigned long long k1 = cand[1] ? sortable_key(score[1]) : 0ull;
+    const bool hi = cand[1] && k1 >= k0;
+    const unsigned long long key = hi ? k1 : k0;  // 0 <=> neither action is a candidate
+    const unsigned long long best_key = warp_max_key(key);
+    const bool win = key != 0ull && key == best_key;
+    const unsigned win_hi = __ballot_sync(MZ_FULL, win && hi), win_lo = __ballot_sync(MZ_FULL, win && !hi);
+    if (win_hi) return 63 - __clz(win_hi);
+    return win_lo ? 31 - __clz(win_lo) : -1;
+  }
 }
 
 // MODE: MinMaxStats.normalize (mcts.py:16-21) hoisted out of the loop -- 2 = (v - min) / (max - min)
 // through the constant-divisor division, 3 = same through IEEE division, 1 = constant 1.0, 0 = raw.
-template <bool STAGED, int MODE>
+template <bool STAGED, int MODE, int APL>
 MZ_DEV void descend_loop(const mz_tree& t, typename ImgLoad<STAGED>::Addr nodes, int lane, int16_t* path,
                          int N, double mn, double d, double r, int& out_depth, int& out_parent,
                          int& out_action) {
   using L = ImgLoad<STAGED>;
   const int A = t.num_actions, SP1 = t.num_simulations + 1, NB = t.node_bytes;
   const double init_score = t.init_value_score;
-  const bool lane_ok = lane < A;
-  const int sp = lane_ok ? lane : A - 1;
-  const int prior_off = MZ_NODE_STATS_BYTES + 8 * sp, child_off = MZ_NODE_STATS_BYTES + 8 * A + 2 * sp;
+  bool lane_ok[APL];
+  int prior_off[APL], child_off[APL];
+#pragma unroll
+  for (int h = 0; h < APL; ++h) {
+    lane_ok[h] = lane + 32 * h < A;
+    const int sp = lane_ok[h] ? lane + 32 * h : A - 1;
+    prior_off[h] = MZ_NODE_STATS_BYTES + 8 * sp;
+    child_off[h] = MZ_NODE_STATS_BYTES + 8 * A + 2 * sp;
+  }
   const double* table = t.pb_c_table;
   int node = 0, depth = 0, parent, action;
   const double* row = table + N * SP1;  // pb_c[N][.] of the node being expanded (warp-uniform)
   for (;;) {
     const typename L::Addr rec = nodes + node * NB;
-    const double prior = L::f64(rec + prior_off);
-    int ch = L::s16(rec + child_off);
-    if (!lane_ok) ch = MZ_CHILD_ILLEGAL;
-    const NodeHead c = L::head(nodes + max(ch, 0) * NB);
-    const int n = ch >= 0 ? c.visit : 0;
-    // ucb_score mcts.py:115-124
-    const double pb_c = __ldg(row + n);
-    double value_score;
-    if (MODE == 0) {
-      value_score = c.q;
-    } else if (MODE == 1) {
-      value_score = 1.0;
-    } else if (MODE == 3) {
-      value_score = __ddiv_rn(__dsub_rn(c.q, mn), d);
-    } else {
-      // every lane evaluates the constant-divisor division (lanes without a visited child discard it);
-      // only a visited child outside [2^-200, 2^200] (or exactly at the minimum) takes the IEEE path
-      const double x = __dsub_rn(c.q, mn);
-      value_score = div_by_const(x, d, r);
-      const unsigned hx = (unsigned)__double2hiint(x);  // x >= 0 because min <= q
-      if (__builtin_expect(n > 0 && hx - 0x33700000u > 0x19000000u, 0))
-        value_score = (x == 0.0) ? 0.0 : __ddiv_rn(x, d);
+    double score[APL];
+    bool cand[APL];
+    int ch[APL], n[APL];
+#pragma unroll
+    for (int h = 0; h < APL; ++h) {
+      const double prior = L::f64(rec + prior_off[h]);
+      ch[h] = L::s16(rec + child_off[h]);
+      if (!lane_ok[h]) ch[h] = MZ_CHILD_ILLEGAL;
+      const NodeHead c = L::head(nodes + max(ch[h], 0) * NB);
+      n[h] = ch[h] >= 0 ? c.visit : 0;
+      // ucb_score mcts.py:115-124
+      const double pb_c = __ldg(row + n[h]);
+      double value_score;
+      if (MODE == 0) {
+        value_score = c.q;
+      } else if (MODE == 1) {
+        value_score = 1.0;
+      } else if (MODE == 3) {
+        value_score = __ddiv_rn(__dsub_rn(c.q, mn), d);
+      } else {
+        // every lane evaluates the constant-divisor division (lanes without a visited child discard it);
+        // only a visited child outside [2^-200, 2^200] (or exactly at the minimum) takes the IEEE path
+        const double x = __dsub_rn(c.q, mn);
+        value_score = div_by_const(x, d, r);
+        const unsigned hx = (unsigned)__double2hiint(x);  // x >= 0 because min <= q
+        if (__builtin_expect(n[h] > 0 && hx - 0x33700000u > 0x19000000u, 0))
+          value_score = (x == 0.0) ? 0.0 : __ddiv_rn(x, d);
+      }
+      if (n[h] <= 0) value_score = init_score;
+      score[h] = __dadd_rn(__dmul_rn(pb_c, prior), value_score);
+      cand[h] = ch[h] != MZ_CHILD_ILLEGAL;
     }
-    if (n <= 0) value_score = init_score;
-    const double score = __dadd_rn(__dmul_rn(pb_c, prior), value_score);
-    const int best = warp_argmax(score, ch != MZ_CHILD_ILLEGAL);
-    const int src = best < 0 ? 0 : best;
-    const int ch_b = __shfl_sync(MZ_FULL, ch, src);
-    const int n_b = __shfl_sync(MZ_FULL, n, src);
+    const int best = warp_argmax<APL>(score, cand);
+    const int src = best < 0 ? 0 : (APL == 1 ? best : best & 31);
+    const bool high = APL == 2 && best >= 32;  // warp-uniform
+    const int ch_b = __shfl_sync(MZ_FULL, high ? ch[APL - 1] : ch[0], src);
+    const int n_b = __shfl_sync(MZ_FULL, high ? n[APL - 1] : n[0], src);
     depth++;
     if (ch_b < 0) {  // child not expanded: this is the leaf
       parent = node;
@@ -218,7 +267,7 @@ MZ_DEV void descend_loop(const mz_tree& t, typename ImgLoad<STAGED>::Addr nodes,
   out_action = action;
 }
 
-template <bool STAGED>
+template <bool STAGED, int APL>
 MZ_DEV void descend(const mz_tree& t, const uint8_t* img, int lane, int16_t* path, int& out_depth,
                     int& out_parent, int& out_action) {
   using L = ImgLoad<STAGED>;
@@ -231,11 +280,17 @@ MZ_DEV void descend(const mz_tree& t, const uint8_t* img, int lane, int16_t* pat
   if (N == 0) {
     // mcts.py:105-108: an unvisited root (simulation 0) ranks its children by prior; none of them
     // is expanded yet, so the first step already reaches the leaf
-    const bool lane_ok = lane < A;
-    const int sp = lane_ok ? lane : A - 1;
-    const double prior = L::f64(nodes + MZ_NODE_STATS_BYTES + 8 * sp);
-    const int ch = L::s16(nodes + MZ_NODE_STATS_BYTES + 8 * A + 2 * sp);
-    const int best = warp_argmax(prior, lane_ok && ch != MZ_CHILD_ILLEGAL);
+    double prior[APL];
+    bool cand[APL];
+#pragma unroll
+    for (int h = 0; h < APL; ++h) {
+      const bool lane_ok = lane + 32 * h < A;
+      const int sp = lane_ok ? lane + 32 * h : A - 1;
+      prior[h] = L::f64(nodes + MZ_NODE_STATS_BYTES + 8 * sp);
+      const int ch = L::s16(nodes + MZ_NODE_STATS_BYTES + 8 * A + 2 * sp);
+      cand[h] = lane_ok && ch != MZ_CHILD_ILLEGAL;
+    }
+    const int best = warp_argmax<APL>(prior, cand);
     out_depth = 1;
     out_parent = 0;
     out_action = best;
@@ -243,21 +298,21 @@ MZ_DEV void descend(const mz_tree& t, const uint8_t* img, int lane, int16_t* pat
   }
   const double d = __dsub_rn(mx, mn);
   if (mx > mn) {
-    if (divisor_ok(d)) descend_loop<STAGED, 2>(t, nodes, lane, path, N, mn, d, __drcp_rn(d), out_depth, out_parent, out_action);
-    else descend_loop<STAGED, 3>(t, nodes, lane, path, N, mn, d, 0.0, out_depth, out_parent, out_action);
+    if (divisor_ok(d)) descend_loop<STAGED, 2, APL>(t, nodes, lane, path, N, mn, d, __drcp_rn(d), out_depth, out_parent, out_action);
+    else descend_loop<STAGED, 3, APL>(t, nodes, lane, path, N, mn, d, 0.0, out_depth, out_parent, out_action);
   } else if (mx == mn) {
-    descend_loop<STAGED, 1>(t, nodes, lane, path, N, mn, d, 0.0, out_depth, out_parent, out_action);
+    descend_loop<STAGED, 1, APL>(t, nodes, lane, path, N, mn, d, 0.0, out_depth, out_parent, out_action);
   } else {
-    descend_loop<STAGED, 0>(t, nodes, lane, path, N, mn, d, 0.0, out_depth, out_parent, out_action);
+    descend_loop<STAGED, 0, APL>(t, nodes, lane, path, N, mn, d, 0.0, out_depth, out_parent, out_action);
   }
 }
 
 // expand (mcts.py:47-55) + backpropagate (mcts.py:126-143).  `img` is the
 // image the warp reads (shared memory when STAGED, else the global block); stores go to the global
 // block and, when staged, to the image as well.
-template <bool STAGED>
+template <bool STAGED, int APL>
 MZ_DEV void expand_backup(const mz_tree& t, uint8_t* img, uint8_t* gbl, int lane, int sim,
-                          float value_f, float reward_f, float logit, int16_t* path, int depth,
+                          float value_f, float reward_f, const float (&logit)[APL], int16_t* path, int depth,
                           int parent, int action) {
   const int A = t.num_actions, NB = t.node_bytes;
   const bool two = t.two_players != 0;
@@ -266,7 +321,6 @@ MZ_DEV void expand_backup(const mz_tree& t, uint8_t* img, uint8_t* gbl, int lane
   const float node_reward_new = (reward_f != 0.0f) ? reward_f : 0.0f;  // `if network_output.reward:`
   uint8_t* nodes_s = img + MZ_GAME_HEADER_BYTES;
   uint8_t* nodes_g = gbl + MZ_GAME_HEADER_BYTES;
-  const bool lane_ok = lane < A;
 
   // the path positions this lane owns in the first (deepest) chunk: issue the loads early
   const int top = (depth >> 5) << 5;
@@ -275,32 +329,44 @@ MZ_DEV void expand_backup(const mz_tree& t, uint8_t* img, uint8_t* gbl, int lane
 
   // priors: p_a = exp(logit_a) / sum(p), the sum evaluated like CPython's builtin sum()
   // (every action is legal below the root, mcts.py:72, 97)
-  const double p = lane_ok ? mz_exp((double)logit) : 0.0;
-  double f = shfl_f64<32>(p, 0), c = 0.0;
+  double p[APL];
+#pragma unroll
+  for (int h = 0; h < APL; ++h) p[h] = lane + 32 * h < A ? mz_exp((double)logit[h]) : 0.0;
+  double f = shfl_f64<32>(p[0], 0), c = 0.0;
   if (t.prior_sum_mode == 0) {
+#pragma unroll
+    for (int h = 0; h < APL; ++h) {
 #pragma unroll 1
-    for (int a = 1; a < A; ++a) f = __dadd_rn(f, shfl_f64<32>(p, a));
+      for (int a = h == 0 ? 1 : 32; a < half_end<APL>(A, h); ++a) f = __dadd_rn(f, shfl_f64<32>(p[h], a - 32 * h));
+    }
   } else {  // Neumaier step, CPython >= 3.12 Python/bltinmodule.c
+#pragma unroll
+    for (int h = 0; h < APL; ++h) {
 #pragma unroll 1
-    for (int a = 1; a < A; ++a) {
-      const double x = shfl_f64<32>(p, a);
-      const double s = __dadd_rn(f, x);
-      const bool big = fabs(f) >= fabs(x);
-      const double hi = big ? f : x, lo = big ? x : f;
-      c = __dadd_rn(c, __dadd_rn(__dsub_rn(hi, s), lo));
-      f = s;
+      for (int a = h == 0 ? 1 : 32; a < half_end<APL>(A, h); ++a) {
+        const double x = shfl_f64<32>(p[h], a - 32 * h);
+        const double s = __dadd_rn(f, x);
+        const bool big = fabs(f) >= fabs(x);
+        const double hi = big ? f : x, lo = big ? x : f;
+        c = __dadd_rn(c, __dadd_rn(__dsub_rn(hi, s), lo));
+        f = s;
+      }
     }
     if (c != 0.0 && isfinite(c)) f = __dadd_rn(f, c);
   }
-  if (lane_ok) {
-    const double prior = __ddiv_rn(p, f);
-    const int po = newn * NB + MZ_NODE_STATS_BYTES + 8 * lane;
-    const int co = newn * NB + MZ_NODE_STATS_BYTES + 8 * A + 2 * lane;
-    *reinterpret_cast<double*>(nodes_g + po) = prior;
-    *reinterpret_cast<int16_t*>(nodes_g + co) = (int16_t)MZ_CHILD_UNEXPANDED;
-    if (STAGED) {
-      *reinterpret_cast<double*>(nodes_s + po) = prior;
-      *reinterpret_cast<int16_t*>(nodes_s + co) = (int16_t)MZ_CHILD_UNEXPANDED;
+#pragma unroll
+  for (int h = 0; h < APL; ++h) {
+    const int a = lane + 32 * h;
+    if (a < A) {
+      const double prior = __ddiv_rn(p[h], f);
+      const int po = newn * NB + MZ_NODE_STATS_BYTES + 8 * a;
+      const int co = newn * NB + MZ_NODE_STATS_BYTES + 8 * A + 2 * a;
+      *reinterpret_cast<double*>(nodes_g + po) = prior;
+      *reinterpret_cast<int16_t*>(nodes_g + co) = (int16_t)MZ_CHILD_UNEXPANDED;
+      if (STAGED) {
+        *reinterpret_cast<double*>(nodes_s + po) = prior;
+        *reinterpret_cast<int16_t*>(nodes_s + co) = (int16_t)MZ_CHILD_UNEXPANDED;
+      }
     }
   }
   if (lane == 0) {
@@ -391,6 +457,7 @@ MZ_DEV void copy_words(uint32_t* dst, const uint32_t* src, int words, int lane) 
 // ------------------------------------------------------------------------------------------------
 // kernels
 // ------------------------------------------------------------------------------------------------
+template <int APL>
 __global__ void __launch_bounds__(kThreads)
 set_root_kernel(mz_tree t, const float* __restrict__ root_logits,
                 const uint32_t* __restrict__ legal_mask, const double* __restrict__ noise,
@@ -402,25 +469,40 @@ set_root_kernel(mz_tree t, const float* __restrict__ root_logits,
   const int g = valid ? gidx : t.num_games - 1;
   const int A = t.num_actions;
   const MzGame gm{t.games + (size_t)g * t.game_bytes, t.node_bytes, A};
-  const uint32_t lm = legal_mask ? legal_mask[g] : 0xffffffffu;
-  const bool legal = lane < A && ((lm >> lane) & 1u);
-  double prior;
-  if (root_priors) {  // the caller ran Node.expand / add_exploration_noise itself
-    prior = legal ? root_priors[(size_t)g * A + lane] : 0.0;
-  } else {
-    const float logit = lane < A ? root_logits[(size_t)g * A + lane] : 0.0f;
-    prior = legal_priors(logit, legal, t.prior_sum_mode, A);
+  uint32_t lm[APL];  // legal-mask words of the game (APL = ceil(A / 32))
+  bool legal[APL];
+  double prior[APL];
+#pragma unroll
+  for (int h = 0; h < APL; ++h) {
+    lm[h] = legal_mask ? legal_mask[(size_t)g * APL + h] : 0xffffffffu;
+    legal[h] = lane + 32 * h < A && ((lm[h] >> lane) & 1u);
   }
-  if (noise && legal) {  // add_exploration_noise mcts.py:57-61; noise is dense over children
-    const int j = __popc(lm & ((1u << lane) - 1u));
-    const double nz = noise[(size_t)g * A + j];
-    prior = __dadd_rn(__dmul_rn(prior, __dsub_rn(1.0, noise_frac)), __dmul_rn(nz, noise_frac));
+  if (root_priors) {  // the caller ran Node.expand / add_exploration_noise itself
+#pragma unroll
+    for (int h = 0; h < APL; ++h) prior[h] = legal[h] ? root_priors[(size_t)g * A + lane + 32 * h] : 0.0;
+  } else {
+    float logit[APL];
+#pragma unroll
+    for (int h = 0; h < APL; ++h) logit[h] = lane + 32 * h < A ? root_logits[(size_t)g * A + lane + 32 * h] : 0.0f;
+    legal_priors<APL>(logit, legal, t.prior_sum_mode, A, prior);
+  }
+#pragma unroll
+  for (int h = 0; h < APL; ++h) {
+    if (noise && legal[h]) {  // add_exploration_noise mcts.py:57-61; noise is dense over children
+      // every bit of the low word is an action when A > 32
+      const int j = (h ? __popc(lm[0]) : 0) + __popc(lm[h] & ((1u << lane) - 1u));
+      const double nz = noise[(size_t)g * A + j];
+      prior[h] = __dadd_rn(__dmul_rn(prior[h], __dsub_rn(1.0, noise_frac)), __dmul_rn(nz, noise_frac));
+    }
   }
   if (!valid) return;
   const MzNode root = gm.node(0);
-  if (lane < A) {
-    root.prior()[lane] = prior;
-    root.child()[lane] = (int16_t)(legal ? MZ_CHILD_UNEXPANDED : MZ_CHILD_ILLEGAL);
+#pragma unroll
+  for (int h = 0; h < APL; ++h) {
+    if (lane + 32 * h < A) {
+      root.prior()[lane + 32 * h] = prior[h];
+      root.child()[lane + 32 * h] = (int16_t)(legal[h] ? MZ_CHILD_UNEXPANDED : MZ_CHILD_ILLEGAL);
+    }
   }
   if (lane == 0) {
     root.vsum() = 0.0;
@@ -440,7 +522,7 @@ set_root_kernel(mz_tree t, const float* __restrict__ root_logits,
 // simulation sim + 1].  STAGED: the live part of each game block (header + nodes 0..sim) is brought
 // into shared memory with one cp.async.bulk (TMA unit) per game and both phases run on that image.
 // blockDim.x = 32 * games_per_block.
-template <bool STAGED>
+template <bool STAGED, int APL>
 __global__ void __launch_bounds__(kThreads)
 tree_step_w32_kernel(mz_tree t, int sim, int do_backup, int do_select, int live_nodes, int stage_bytes,
                      const float* __restrict__ value, const float* __restrict__ reward,
@@ -479,10 +561,12 @@ tree_step_w32_kernel(mz_tree t, int sim, int do_backup, int do_select, int live_
     const int depth = t.path_len[g], parent = t.leaf_parent[g], action = t.leaf_action[g];
     pdl_wait();     // the network kernel's outputs (and nothing before this line) depend on it
     pdl_trigger();
-    const float logit = lane < A ? logits[(size_t)g * A + lane] : 0.0f;
+    float logit[APL];
+#pragma unroll
+    for (int h = 0; h < APL; ++h) logit[h] = lane + 32 * h < A ? logits[(size_t)g * A + lane + 32 * h] : 0.0f;
     const float v = value[g], r = reward[g];
     if (STAGED) mbar_wait(&bars[warp], 0);
-    expand_backup<STAGED>(t, img, gbl, lane, sim, v, r, logit, path, depth, parent, action);
+    expand_backup<STAGED, APL>(t, img, gbl, lane, sim, v, r, logit, path, depth, parent, action);
     if (new_hidden && HW > 0)
       copy_words(t.hidden + ((size_t)g * SP1 + sim + 1) * HW, new_hidden + (size_t)g * HW, HW, lane);
     __syncwarp();
@@ -493,7 +577,7 @@ tree_step_w32_kernel(mz_tree t, int sim, int do_backup, int do_select, int live_
   }
   if (do_select) {
     int depth, parent, action;
-    descend<STAGED>(t, img, lane, path, depth, parent, action);
+    descend<STAGED, APL>(t, img, lane, path, depth, parent, action);
     if (lane == 0) {
       t.path_len[g] = depth;
       t.leaf_parent[g] = parent;
@@ -508,8 +592,9 @@ tree_step_w32_kernel(mz_tree t, int sim, int do_backup, int do_select, int live_
 }
 
 // game.py:106-111 + Node.value mcts.py:42-45
-// One warp per game, lane = action (the per-action loads are two dependent L2 accesses: child index ->
-// child's visit count; a thread per game serialised 2 A of them).
+// One warp per game, a lane per action (two above 32 actions; the per-action loads are two dependent L2
+// accesses: child index -> child's visit count; a thread per game serialised 2 A of them).
+template <int APL>
 __global__ void root_stats_kernel(mz_tree t, int32_t* __restrict__ visits,
                                   double* __restrict__ child_visits, double* __restrict__ root_value,
                                   double* __restrict__ minmax) {
@@ -518,16 +603,26 @@ __global__ void root_stats_kernel(mz_tree t, int32_t* __restrict__ visits,
   const int A = t.num_actions;
   const MzGame gm{t.games + (size_t)g * t.game_bytes, t.node_bytes, A};
   const MzNode root = gm.node(0);
-  int ch = MZ_CHILD_ILLEGAL, v = 0;
-  if (lane < A) {
-    ch = root.child()[lane];
-    v = ch >= 0 ? gm.node(ch).visit() : 0;
+  int ch[APL], v[APL], mine = 0;
+#pragma unroll
+  for (int h = 0; h < APL; ++h) {
+    ch[h] = MZ_CHILD_ILLEGAL;
+    v[h] = 0;
+    if (lane + 32 * h < A) {
+      ch[h] = root.child()[lane + 32 * h];
+      v[h] = ch[h] >= 0 ? gm.node(ch[h]).visit() : 0;
+    }
+    mine += v[h];
   }
-  const int sum = __reduce_add_sync(MZ_FULL, v);  // integer: order does not matter
-  if (lane < A) {
-    if (visits) visits[(size_t)g * A + lane] = v;
-    if (child_visits)
-      child_visits[(size_t)g * A + lane] = ch != MZ_CHILD_ILLEGAL ? __ddiv_rn((double)v, (double)sum) : 0.0;
+  const int sum = __reduce_add_sync(MZ_FULL, mine);  // integer: order does not matter
+#pragma unroll
+  for (int h = 0; h < APL; ++h) {
+    const int a = lane + 32 * h;
+    if (a < A) {
+      if (visits) visits[(size_t)g * A + a] = v[h];
+      if (child_visits)
+        child_visits[(size_t)g * A + a] = ch[h] != MZ_CHILD_ILLEGAL ? __ddiv_rn((double)v[h], (double)sum) : 0.0;
+    }
   }
   if (lane == 0) {
     if (root_value) {
@@ -559,40 +654,54 @@ __device__ double np_pairwise_sum(const double* a, int n) {
   return res;
 }
 
-// Config.select_action config.py:70-81.  One warp per game: the legal actions are compacted to lanes
-// 0..n-1 (action order, like the dict of children); pow, the two divisions and the comparison run one
-// candidate per lane, the two float64 sums keep numpy's order (pairwise add.reduce, sequential cumsum).
+// Config.select_action config.py:70-81.  One warp per game: the legal actions are compacted to
+// candidates 0..n-1 (action order, like the dict of children), candidate i on lane i % 32; pow, the two
+// divisions and the comparison run per candidate, the two float64 sums keep numpy's order (pairwise
+// add.reduce, sequential cumsum).
+template <int APL>
 __global__ void select_action_kernel(int G, int A, const int32_t* __restrict__ visits,
                                      const uint32_t* __restrict__ legal_mask,
                                      const double* __restrict__ temperature,
                                      const double* __restrict__ uniforms,
                                      int32_t* __restrict__ actions) {
-  __shared__ double s_d[4][MZ_MAX_ACTIONS];
+  __shared__ double s_d[4][32 * APL];
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int g = blockIdx.x * 4 + w;
   if (g >= G) return;
-  uint32_t lm = legal_mask ? legal_mask[g] : 0xffffffffu;
-  if (A < 32) lm &= (1u << A) - 1u;
-  const int n = __popc(lm);
+  uint32_t lm[APL];
+#pragma unroll
+  for (int h = 0; h < APL; ++h) lm[h] = legal_mask ? legal_mask[(size_t)g * APL + h] : 0xffffffffu;
+  if (A < 32 * APL) lm[APL - 1] &= (1u << (A - 32 * (APL - 1))) - 1u;
+  const int n0 = __popc(lm[0]);
+  const int n = APL == 1 ? n0 : n0 + __popc(lm[APL - 1]);
   if (n == 0) {
     if (lane == 0) actions[g] = -1;
     return;
   }
-  // lane i < n holds the i-th legal action
-  const int my_act = lane < n ? __fns(lm, 0, lane + 1) : 0;
-  const int cnt = lane < n ? visits[(size_t)g * A + my_act] : 0;
+  // candidate i = lane + 32 h < n is the i-th legal action
+  int my_act[APL], cnt[APL];
+#pragma unroll
+  for (int h = 0; h < APL; ++h) {
+    const int i = lane + 32 * h;
+    my_act[h] = i >= n ? 0 : (APL == 1 || i < n0) ? __fns(lm[0], 0, i + 1) : 32 + __fns(lm[APL - 1], 0, i - n0 + 1);
+    cnt[h] = i < n ? visits[(size_t)g * A + my_act[h]] : 0;
+  }
   const double T = temperature[g], u = uniforms[g];
   double* d = s_d[w];
   int idx = 0;
   if (T != 0.0) {
     const double inv_t = __ddiv_rn(1.0, T);
-    if (lane < n) d[lane] = pow((double)cnt, inv_t);
+#pragma unroll
+    for (int h = 0; h < APL; ++h)
+      if (lane + 32 * h < n) d[lane + 32 * h] = pow((double)cnt[h], inv_t);
     __syncwarp();
     double s = 0.0;
     if (lane == 0) s = np_pairwise_sum(d, n);
     s = shfl_f64<32>(s, 0);
     __syncwarp();
-    if (lane < n) d[lane] = __ddiv_rn(d[lane], s);  // distribution / sum
+#pragma unroll
+    for (int h = 0; h < APL; ++h)
+      if (lane + 32 * h < n) d[lane + 32 * h] = __ddiv_rn(d[lane + 32 * h], s);  // distribution / sum
     __syncwarp();
     if (lane == 0) {  // cumsum
       double acc = d[0];
@@ -603,19 +712,31 @@ __global__ void select_action_kernel(int G, int A, const int32_t* __restrict__ v
     }
     __syncwarp();
     const double last = d[n - 1];
-    const bool le = lane < n && __ddiv_rn(d[lane], last) <= u;  // searchsorted(side='right')
-    const unsigned m = __ballot_sync(MZ_FULL, le);
-    idx = m ? 32 - __clz(m) : 0;  // (last index with cdf <= u) + 1, as the sequential scan leaves it
+    unsigned m[APL];
+#pragma unroll
+    for (int h = 0; h < APL; ++h) {
+      const int i = lane + 32 * h;
+      m[h] = __ballot_sync(MZ_FULL, i < n && __ddiv_rn(d[i], last) <= u);  // searchsorted(side='right')
+    }
+    // (last index with cdf <= u) + 1, as the sequential scan leaves it
+    idx = (APL == 2 && m[APL - 1]) ? 64 - __clz(m[APL - 1]) : m[0] ? 32 - __clz(m[0]) : 0;
     if (idx >= n) idx = n - 1;
   } else {
-    const int mx = __reduce_max_sync(MZ_FULL, lane < n ? cnt : -1);
-    const unsigned tie = __ballot_sync(MZ_FULL, lane < n && cnt == mx);
-    const int ties = __popc(tie);
+    int c = lane < n ? cnt[0] : -1;
+    if (APL == 2) c = max(c, lane + 32 < n ? cnt[APL - 1] : -1);
+    const int mx = __reduce_max_sync(MZ_FULL, c);
+    unsigned tie[APL];
+#pragma unroll
+    for (int h = 0; h < APL; ++h) tie[h] = __ballot_sync(MZ_FULL, lane + 32 * h < n && cnt[h] == mx);
+    const int t0 = __popc(tie[0]);
+    const int ties = APL == 1 ? t0 : t0 + __popc(tie[APL - 1]);
     int pick = (int)floor(__dmul_rn(u, (double)ties));
     if (pick >= ties) pick = ties - 1;
-    idx = __fns(tie, 0, pick + 1);  // the pick-th tie in action order
+    // the pick-th tie in action order
+    idx = (APL == 1 || pick < t0) ? __fns(tie[0], 0, pick + 1) : 32 + __fns(tie[APL - 1], 0, pick - t0 + 1);
   }
-  const int chosen = __shfl_sync(MZ_FULL, my_act, idx);
+  const int chosen = __shfl_sync(MZ_FULL, (APL == 2 && idx >= 32) ? my_act[APL - 1] : my_act[0],
+                                   APL == 1 ? idx : idx & 31);
   if (lane == 0) actions[g] = chosen;
 }
 
@@ -713,13 +834,47 @@ int w32_games_per_block(int num_games) {
 
 constexpr int kMaxStageSmem = 200 * 1024;
 
-template <bool STAGED>
+// Shared-memory image of the step kernel: 0 = staged whenever the images fit (default), 1 = never staged
+// (mz_debug_set_tree_staging; for measurements).
+int g_tree_staging = 0;
+
+template <bool STAGED, int APL>
 int set_smem_attr_w32_once() {
   static int rc = -1;
   if (rc < 0)
-    rc = (int)cudaFuncSetAttribute(tree_step_w32_kernel<STAGED>,
+    rc = (int)cudaFuncSetAttribute(tree_step_w32_kernel<STAGED, APL>,
                                    cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxStageSmem + 1024);
   return rc;
+}
+
+template <int APL>
+int launch_step_apl(const mz_tree* t, int sim, int live_nodes, int do_backup, int do_select, const float* value,
+                    const float* reward, const float* logits, const uint32_t* new_hidden,
+                    uint32_t* gathered_hidden, int32_t* tp, int32_t* ta, int32_t* td, void* stream) {
+  // image: header + nodes 0..sim+1 (the new node is built in place)
+  const int nodes = live_nodes + (do_backup ? 1 : 0);
+  const int stage_bytes = MZ_GAME_HEADER_BYTES + nodes * t->node_bytes;
+  int gpb = w32_games_per_block(t->num_games);
+  while (gpb > 1 && (size_t)gpb * stage_bytes > 96 * 1024) gpb >>= 1;
+  const bool staged = g_tree_staging == 0 && (size_t)gpb * stage_bytes <= kMaxStageSmem;
+  if (!staged) gpb = kThreads / 32;
+  const int grid = (t->num_games + gpb - 1) / gpb;
+  if (staged) {
+    int rc = set_smem_attr_w32_once<true, APL>();
+    if (rc) return rc;
+    cudaError_t e = mz_launch(tree_step_w32_kernel<true, APL>, dim3(grid), dim3(gpb * 32),
+                              (size_t)gpb * stage_bytes + sizeof(uint64_t) * gpb, (cudaStream_t)stream,
+                              do_backup != 0, *t, sim, do_backup, do_select, live_nodes, stage_bytes, value,
+                              reward, logits, new_hidden, gathered_hidden, tp, ta, td);
+    if (e != cudaSuccess) return (int)e;
+  } else {  // tree too large for shared memory: run on the global block directly
+    cudaError_t e = mz_launch(tree_step_w32_kernel<false, APL>, dim3(grid), dim3(gpb * 32), 0,
+                              (cudaStream_t)stream, do_backup != 0, *t, sim, do_backup, do_select,
+                              live_nodes, 0, value, reward, logits, new_hidden, gathered_hidden, tp, ta, td);
+    if (e != cudaSuccess) return (int)e;
+  }
+  MZ_LAUNCH_CHECK();
+  return MZ_OK;
 }
 
 int launch_step(const mz_tree* t, int sim, int live_nodes, int do_backup, int do_select, const float* value,
@@ -728,31 +883,12 @@ int launch_step(const mz_tree* t, int sim, int live_nodes, int do_backup, int do
   // One warp per game at every action count.  Packing 8 / 4 / 2 games of few actions into a warp makes the games
   // of a warp wait for each other's descents, and the code is not warp-uniform.  Measured (A = 4, 50 simulations):
   // the converged warp-per-game kernel is faster at every batch size -- 13.9 vs 32.0 us per step at 4096 games,
-  // 27.8 vs 44.5 us at 16 k, 83 vs 122 us at 64 k.
-  // image: header + nodes 0..sim+1 (the new node is built in place)
-  const int nodes = live_nodes + (do_backup ? 1 : 0);
-  const int stage_bytes = MZ_GAME_HEADER_BYTES + nodes * t->node_bytes;
-  int gpb = w32_games_per_block(t->num_games);
-  while (gpb > 1 && (size_t)gpb * stage_bytes > 96 * 1024) gpb >>= 1;
-  const bool staged = (size_t)gpb * stage_bytes <= kMaxStageSmem;
-  if (!staged) gpb = kThreads / 32;
-  const int grid = (t->num_games + gpb - 1) / gpb;
-  if (staged) {
-    int rc = set_smem_attr_w32_once<true>();
-    if (rc) return rc;
-    cudaError_t e = mz_launch(tree_step_w32_kernel<true>, dim3(grid), dim3(gpb * 32),
-                              (size_t)gpb * stage_bytes + sizeof(uint64_t) * gpb, (cudaStream_t)stream,
-                              do_backup != 0, *t, sim, do_backup, do_select, live_nodes, stage_bytes, value,
-                              reward, logits, new_hidden, gathered_hidden, tp, ta, td);
-    if (e != cudaSuccess) return (int)e;
-  } else {  // tree too large for shared memory: run on the global block directly
-    cudaError_t e = mz_launch(tree_step_w32_kernel<false>, dim3(grid), dim3(gpb * 32), 0,
-                              (cudaStream_t)stream, do_backup != 0, *t, sim, do_backup, do_select,
-                              live_nodes, 0, value, reward, logits, new_hidden, gathered_hidden, tp, ta, td);
-    if (e != cudaSuccess) return (int)e;
-  }
-  MZ_LAUNCH_CHECK();
-  return MZ_OK;
+  // 27.8 vs 44.5 us at 16 k, 83 vs 122 us at 64 k.  More than 32 actions: two per lane.
+  return t->num_actions > 32
+             ? launch_step_apl<2>(t, sim, live_nodes, do_backup, do_select, value, reward, logits, new_hidden,
+                                  gathered_hidden, tp, ta, td, stream)
+             : launch_step_apl<1>(t, sim, live_nodes, do_backup, do_select, value, reward, logits, new_hidden,
+                                  gathered_hidden, tp, ta, td, stream);
 }
 
 }  // namespace
@@ -790,8 +926,12 @@ int mz_tree_set_root(const mz_tree* t, const float* root_logits, const uint32_t*
   if (rc) return rc;
   if (!root_logits) return MZ_ERR_BAD_ARG;
   const int grid = (t->num_games + 3) / 4;  // a warp per game
-  set_root_kernel<<<grid, kThreads, 0, (cudaStream_t)stream>>>(*t, root_logits, legal_mask, noise, noise_frac,
-                                                               root_to_play, root_hidden, nullptr);
+  if (t->num_actions > 32)
+    set_root_kernel<2><<<grid, kThreads, 0, (cudaStream_t)stream>>>(*t, root_logits, legal_mask, noise, noise_frac,
+                                                                  root_to_play, root_hidden, nullptr);
+  else
+    set_root_kernel<1><<<grid, kThreads, 0, (cudaStream_t)stream>>>(*t, root_logits, legal_mask, noise, noise_frac,
+                                                                  root_to_play, root_hidden, nullptr);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }
@@ -802,8 +942,12 @@ int mz_tree_set_root_priors(const mz_tree* t, const double* root_priors, const u
   if (rc) return rc;
   if (!root_priors) return MZ_ERR_BAD_ARG;
   const int grid = (t->num_games + 3) / 4;  // a warp per game
-  set_root_kernel<<<grid, kThreads, 0, (cudaStream_t)stream>>>(*t, nullptr, legal_mask, nullptr, 0.0,
-                                                               root_to_play, root_hidden, root_priors);
+  if (t->num_actions > 32)
+    set_root_kernel<2><<<grid, kThreads, 0, (cudaStream_t)stream>>>(*t, nullptr, legal_mask, nullptr, 0.0, root_to_play,
+                                                                  root_hidden, root_priors);
+  else
+    set_root_kernel<1><<<grid, kThreads, 0, (cudaStream_t)stream>>>(*t, nullptr, legal_mask, nullptr, 0.0, root_to_play,
+                                                                  root_hidden, root_priors);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }
@@ -843,8 +987,10 @@ int mz_tree_root_stats(const mz_tree* t, int32_t* visits, double* child_visits, 
   int rc = check_tree(t);
   if (rc) return rc;
   const int threads = 128, grid = (t->num_games + 3) / 4;  // a warp per game
-  root_stats_kernel<<<grid, threads, 0, (cudaStream_t)stream>>>(*t, visits, child_visits, root_value,
-                                                               minmax);
+  if (t->num_actions > 32)
+    root_stats_kernel<2><<<grid, threads, 0, (cudaStream_t)stream>>>(*t, visits, child_visits, root_value, minmax);
+  else
+    root_stats_kernel<1><<<grid, threads, 0, (cudaStream_t)stream>>>(*t, visits, child_visits, root_value, minmax);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }
@@ -855,8 +1001,12 @@ int mz_select_action(int32_t G, int32_t A, const int32_t* visits, const uint32_t
   if (G < 1 || A < 1 || A > MZ_MAX_ACTIONS || !visits || !temperature || !uniforms || !actions)
     return MZ_ERR_BAD_ARG;
   const int threads = 128, grid = (G + 3) / 4;  // a warp per game
-  select_action_kernel<<<grid, threads, 0, (cudaStream_t)stream>>>(G, A, visits, legal_mask,
-                                                                  temperature, uniforms, actions);
+  if (A > 32)
+    select_action_kernel<2><<<grid, threads, 0, (cudaStream_t)stream>>>(G, A, visits, legal_mask, temperature,
+                                                                       uniforms, actions);
+  else
+    select_action_kernel<1><<<grid, threads, 0, (cudaStream_t)stream>>>(G, A, visits, legal_mask, temperature,
+                                                                       uniforms, actions);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }
@@ -891,6 +1041,12 @@ int mz_debug_div_check(uint64_t seed, int32_t blocks, int32_t per_thread, uint64
 int mz_tree_set_games_per_block(int32_t games) {
   if (games != 0 && games != 1 && games != 2 && games != 4) return MZ_ERR_BAD_ARG;
   g_w32_gpb = games;
+  return MZ_OK;
+}
+
+int mz_debug_set_tree_staging(int32_t mode) {
+  if (mode != 0 && mode != 1) return MZ_ERR_BAD_ARG;
+  g_tree_staging = mode;
   return MZ_OK;
 }
 

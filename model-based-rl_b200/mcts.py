@@ -106,6 +106,44 @@ SearchResult = namedtuple('SearchResult', ('visits', 'child_visits', 'root_value
                                            'trace_parent', 'trace_action', 'trace_depth'))
 
 
+def legal_words(legal_mask, num_games, num_actions):
+  """Host legal masks -> the kernels' layout (include/mzb200.h): int32 [G, W], W = ceil(A / 32), bit b of word w
+  set <=> action 32 w + b is legal.
+
+  Accepts one mask per game as integers (Python ints, or an int64 / uint64 / uint32 array [G]: bit a <=> action a;
+  at A = 64 action 63 is the sign bit of an int64), a bool array [G, A], or integer words [G, W] already in the
+  kernels' layout.  Bits at or beyond A are passed on; the kernels ignore them."""
+  G, A = int(num_games), int(num_actions)
+  W = (A + 31) // 32
+  if torch.is_tensor(legal_mask):
+    m = legal_mask.cpu().numpy()
+  elif isinstance(legal_mask, np.ndarray):
+    m = legal_mask
+  else:  # a sequence: Python ints with bit 63 set would become float64 (or fail) under numpy's inference
+    m = np.asarray(legal_mask, dtype=object)
+    if m.ndim == 1 and not isinstance(m[0], (bool, np.bool_)):
+      m = np.array([int(x) & 0xffffffffffffffff for x in m], np.uint64)
+    else:
+      m = np.array(m.tolist())
+  if m.dtype == object:
+    m = np.array([int(x) & 0xffffffffffffffff for x in m.ravel()], np.uint64).reshape(m.shape)
+  if m.dtype == np.bool_:
+    if m.shape != (G, A):
+      raise ValueError("expected a bool legal mask of shape %s, got %s" % ((G, A), m.shape))
+    bits = np.zeros((G, 32 * W), np.bool_)
+    bits[:, :A] = m
+    return np.packbits(bits.reshape(G, W, 32), axis=-1, bitorder='little').reshape(G, 4 * W).view('<i4').copy()
+  if m.ndim == 2:
+    if m.shape != (G, W):
+      raise ValueError("expected legal-mask words of shape %s, got %s" % ((G, W), m.shape))
+    return np.ascontiguousarray(m.astype(np.int64).astype(np.int32))
+  if m.shape != (G,):
+    raise ValueError("expected shape %s, got %s" % ((G,), m.shape))
+  u = m.astype(np.uint64) if m.dtype.kind == 'u' else m.astype(np.int64).view(np.uint64)
+  words = [(u >> np.uint64(32 * w)) & np.uint64(0xffffffff) for w in range(W)]
+  return np.ascontiguousarray(np.stack(words, axis=1).astype(np.uint32).view(np.int32))
+
+
 def pb_c_table(num_simulations, pb_c_base, pb_c_init):
   """[(S+1), (S+1)] float64: entry [N, n] is pb_c after the two statements at mcts.py:116-117,
   evaluated with the interpreter's own math.log / math.sqrt (so it is what the reference computes)."""
@@ -135,6 +173,7 @@ class BatchedMCTS(object):
     self.A = int(config.action_space)
     if not 1 <= self.A <= _lib.MZ_MAX_ACTIONS:
       raise ValueError("action_space must be in [1, %d]" % _lib.MZ_MAX_ACTIONS)
+    self.W = (self.A + 31) // 32  # legal-mask words per game
     self.two_players = bool(config.two_players)
     self.discount = float(config.discount)
     self.init_value_score = float(config.init_value_score)
@@ -311,14 +350,20 @@ class BatchedMCTS(object):
     return x
 
   def _mask(self, legal_mask):
+    """Legal masks in the kernels' form: an int32 device tensor [G, W] (`legal_words`; [G] when A <= 32)."""
     if legal_mask is None:
       return None
+    kernel_shape = (self.G,) if self.W == 1 else (self.G, self.W)
     if (torch.is_tensor(legal_mask) and legal_mask.dtype == torch.int32 and
-        legal_mask.device == self.device and tuple(legal_mask.shape) == (self.G,)):
-      return legal_mask.contiguous()  # already in kernel form (bit a set <=> action a legal)
-    if not torch.is_tensor(legal_mask):
-      legal_mask = torch.as_tensor(np.asarray(legal_mask).astype(np.int64))
-    return self._dev(legal_mask.to(torch.int64), torch.int64, (self.G,)).to(torch.int32)
+        legal_mask.device == self.device and tuple(legal_mask.shape) == kernel_shape):
+      return legal_mask.contiguous()  # already in kernel form (bit b of word w set <=> action 32 w + b legal)
+    if torch.is_tensor(legal_mask) and legal_mask.dim() == 1 and legal_mask.dtype != torch.bool:
+      m = self._dev(legal_mask.to(torch.int64), torch.int64, (self.G,))  # one integer per game
+      if self.W == 1:
+        return m.to(torch.int32)
+      return torch.stack([m & 0xffffffff, (m >> 32) & 0xffffffff], dim=1).to(torch.int32).contiguous()
+    words = legal_words(legal_mask, self.G, self.A)
+    return self._dev(words.reshape(kernel_shape), torch.int32, kernel_shape)
 
   def _hidden_words(self, h):
     if h is None or self.hidden_words == 0:
@@ -379,7 +424,8 @@ class MCTS(object):
       priors[0, a] = child.prior
       mask |= 1 << a
     to_play = np.array([root.to_play], np.int8)
-    res = eng.search(network, None, hidden, legal_mask=np.array([mask], np.int64), to_play=to_play,
+    # uint64: at A = 64 bit 63 (action 63) does not fit an int64
+    res = eng.search(network, None, hidden, legal_mask=np.array([mask], np.uint64), to_play=to_play,
                      root_priors=priors)
     mm = res.minmax.cpu().numpy()
     self.min_max_stats.minimum, self.min_max_stats.maximum = float(mm[0, 0]), float(mm[0, 1])

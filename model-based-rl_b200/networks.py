@@ -408,7 +408,7 @@ class FCSearch(object):
     self.obs = torch.zeros((G, fcnet.input_dim), dtype=torch.float32, device=dev)
     # host-visible inputs / outputs live in two blobs so that the end-to-end call moves each with ONE copy
     self._in_specs = [('noise', torch.float64, (G, A)), ('uniforms', torch.float64, (G,)),
-                      ('temperature', torch.float64, (G,)), ('legal', torch.int32, (G,)),
+                      ('temperature', torch.float64, (G,)), ('legal', torch.int32, _legal_shape(G, A)),
                       ('to_play', torch.int8, (G,)), ('obs_u8', torch.uint8, (G, fcnet.input_dim))]
     self._out_specs = [('root_value', torch.float64, (G,)), ('child_visits', torch.float64, (G, A)),
                        ('actions', torch.int32, (G,)), ('init_value', torch.float32, (G,))]
@@ -416,7 +416,7 @@ class FCSearch(object):
     self.__dict__.update(views)
     self._out_dev, views = _carve(self._out_specs, device=dev)
     self.__dict__.update(views)
-    self.legal.fill_(_all_legal(A))
+    _fill_all_legal(self.legal, A)
     self.to_play.fill_(1)
     self.temperature.fill_(1.0)
     self.root_logits = torch.zeros((G, A), dtype=torch.float32, device=dev)
@@ -533,7 +533,7 @@ class FCSearch(object):
       self._out_host, out = _carve(self._out_specs, pin_memory=True)
       h.update(out)
       h['obs'] = torch.zeros((self.G, self.net.input_dim), dtype=torch.float32, pin_memory=True)
-      h['legal'].fill_(_all_legal(self.A))
+      _fill_all_legal(h['legal'], self.A)
       h['to_play'].fill_(1)
       h['temperature'].fill_(1.0)
       self._h = h
@@ -541,8 +541,8 @@ class FCSearch(object):
 
   def pinned_inputs(self):
     """Pinned host views of the per-move inputs (one contiguous blob): 'obs_u8' [G, input_dim] uint8,
-    'noise' [G, A] f64, 'uniforms' [G] f64, 'temperature' [G] f64, 'legal' [G] i32 bit masks, 'to_play'
-    [G] i8.  Write the move's inputs here and call `search_pinned()`: no host-side staging copy."""
+    'noise' [G, A] f64, 'uniforms' [G] f64, 'temperature' [G] f64, 'legal' [G] i32 bit masks ([G, W] words when
+    A > 32, layout of mcts.legal_words), 'to_play' [G] i8.  Write the move's inputs here and call `search_pinned()`: no host-side staging copy."""
     h = self._pinned()
     return {name: h[name] for name, _, _ in self._in_specs}
 
@@ -612,7 +612,8 @@ class FCSearch(object):
     `set_obs_normalization`, default 0 / 255) runs on the device in the same float32 arithmetic --, Dirichlet noise
     [G, A] float64 (row g: one value per legal action of game g, in action order), uniforms [G]
     float64 (action sampling), temperature [G] float64, and optionally the roots' legal-action bit
-    masks [G] (bit a = action a is legal, actors.py:141-142) and to_play [G] (+1 / -1).  Returns
+    masks (actors.py:141-142; any form mcts.legal_words takes: [G] integers with bit a = action a, a bool [G, A]
+    array, or [G, W] words) and to_play [G] (+1 / -1).  Returns
     pinned host tensors: actions [G] i32, root_value [G] f64, child_visits [G, A] f64, and the
     initial-inference value [G] f32 (the priority seed `error = root.value() - value`,
     actors.py:147).  Host->device and device->host copies are part of the call.  With `dirichlet_alpha` set and no
@@ -642,7 +643,8 @@ class FCSearch(object):
     stage('uniforms', uniforms, self.uniforms)
     stage('temperature', temperature, self.temperature)
     if legal is not None:
-      stage('legal', np.ascontiguousarray(np.asarray(legal).astype(np.int64).astype(np.int32)), self.legal)
+      from .mcts import legal_words
+      stage('legal', legal_words(legal, self.G, self.A).reshape(self.legal.shape), self.legal)
     if to_play is not None:
       stage('to_play', np.ascontiguousarray(np.asarray(to_play, dtype=np.int8)), self.to_play)
     self.use_noise = noise is not None or self.use_noise
@@ -683,8 +685,17 @@ class FCSearch(object):
 
 
 def _all_legal(A):
-  """int32 bit mask with the low A bits set (A = 32: all ones = -1 as a signed word)."""
-  return -1 if A >= 32 else (1 << A) - 1
+  """int32 legal-mask words with the low A bits set (a full word: all ones = -1 as a signed word)."""
+  return [-1 if A >= 32 * (w + 1) else (1 << (A - 32 * w)) - 1 for w in range((A + 31) // 32)]
+
+
+def _legal_shape(G, A):
+  """Legal masks of the per-launch path: one int32 word per game up to 32 actions, [G, W] words above."""
+  return (G,) if A <= 32 else (G, (A + 31) // 32)
+
+
+def _fill_all_legal(legal, A):
+  legal.view(legal.shape[0], -1).copy_(torch.tensor(_all_legal(A), dtype=torch.int32).expand(legal.shape[0], -1))
 
 
 def _carve(specs, **alloc):

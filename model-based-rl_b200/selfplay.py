@@ -21,7 +21,7 @@ import collections
 import numpy as np
 import torch
 
-from .mcts import BatchedMCTS
+from .mcts import BatchedMCTS, legal_words
 
 HistorySlice = collections.namedtuple(
     "HistorySlice", "observations child_visits root_values actions rewards errors dones steps env_states "
@@ -52,6 +52,15 @@ class _Game(object):
     return out
 
 
+def _legal_count(legal, i, A):
+  """Legal actions of game i in env.legal_mask()'s result: one integer per game, [G, W] words or a bool [G, A]
+  array (mcts.legal_words)."""
+  if A <= 32 and np.ndim(legal[i]) == 0:
+    return bin(int(legal[i])).count("1")
+  words = legal_words(np.asarray(legal[i:i + 1]) if isinstance(legal, np.ndarray) else legal[i:i + 1], 1, A)
+  return int(np.unpackbits(words.view(np.uint8), bitorder='little')[:A].sum())
+
+
 class BatchedActor(object):
 
   def __init__(self, config, network, env, replay_buffer=None, device=None, temperature=1.0, search=None):
@@ -80,7 +89,7 @@ class BatchedActor(object):
     if noise is None:  # Node.add_exploration_noise (mcts.py:57-61): one draw per root over its children
       noise = np.zeros((G, A))
       for i in range(G):
-        n = bin(int(legal[i])).count("1")
+        n = _legal_count(legal, i, A)
         noise[i, :n] = np.random.dirichlet([cfg.root_dirichlet_alpha] * n)
     if uniforms is None:
       uniforms = np.random.random(G)
@@ -223,7 +232,7 @@ class DeviceActor(object):
       else:
         noise = np.zeros((G, A))
         for i in range(G):
-          n = bin(int(legal[i])).count("1")
+          n = _legal_count(legal, i, A)
           noise[i, :n] = np.random.dirichlet([cfg.root_dirichlet_alpha] * n)
     if uniforms is None:
       uniforms = np.random.random(G)
