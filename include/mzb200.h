@@ -251,12 +251,19 @@ int mz_fc_recurrent_tf32x3(const mz_fc_weights* w, int32_t batch, const float* h
 /*
  * bf16 tensor-core path (tcgen05.mma, accumulators in TMEM, fp32 accumulation) of
  * recurrent_inference.  The weights are first re-packed once per weight update into the
- * shared-memory image the MMA consumes:
- *   packed: mz_fc_tc_packed_bytes(A) bytes, tail: mz_fc_tc_tail_floats() floats (caller-allocated).
+ * shared-memory image the MMA consumes (packed bytes and tail floats caller-allocated).
  * mz_fc_recurrent_tc has the arguments of mz_fc_recurrent_f32 plus the packed buffers; `w` is only
- * read for its integer fields.  Limits: A <= 32, value/reward bins <= 32.  Hidden rows are read
- * as float2, so hidden_in must be 8-byte aligned and in_row_stride even (MZ_ERR_BAD_ARG otherwise).
+ * read for its integer fields.  Limits: 1 <= A <= 64, value/reward bins 1..64, no no_support
+ * (MZ_ERR_UNSUPPORTED otherwise).  Hidden rows are read as float2, so hidden_in must be 8-byte aligned
+ * and in_row_stride even (MZ_ERR_BAD_ARG otherwise).
+ * Two image geometries: narrow (A <= 32 and both supports <= 32 bins; the image mz_fc_search reads) and
+ * wide (anything up to 64).  mz_fc_tc_sizes gives the sizes of both images and of the tail for `w`:
+ * recurrent packed bytes, initial-inference packed bytes (MZ_ERR_UNSUPPORTED in that slot when obs_dim is
+ * too wide for the kernel: use mz_fc_initial_f32), tail floats.  mz_fc_tc_packed_bytes(A),
+ * mz_fc_tc_initial_packed_bytes(obs_dim) and mz_fc_tc_tail_floats() give the narrow image's sizes.
  */
+int mz_fc_tc_sizes(const mz_fc_weights* w, int64_t* recurrent_bytes, int64_t* initial_bytes,
+                   int32_t* tail_floats);
 int64_t mz_fc_tc_packed_bytes(int32_t num_actions);
 /* Diagnostics: when set to a device buffer of >= 512 int64, CTA 0 of every following
  * mz_fc_recurrent_tc launch stores clock64() stamps of its pipeline phases there (NULL disables). */

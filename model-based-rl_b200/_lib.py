@@ -143,6 +143,8 @@ _SIGNATURES = {
     "mz_debug_set_targets_tma": (C.c_int, [C.c_int32, C.c_int32]),
     "mz_debug_set_tc_trace_block": (C.c_int, [C.c_int32]),
     "mz_fc_tc_tail_floats": (C.c_int32, []),
+    "mz_fc_tc_sizes": (C.c_int, [C.POINTER(FcWeights), C.POINTER(C.c_int64), C.POINTER(C.c_int64),
+                                 C.POINTER(C.c_int32)]),
     "mz_fc_tc_pack": (C.c_int, [C.POINTER(FcWeights), _V, _V, _V]),
     "mz_fc_recurrent_tc": (C.c_int, [C.POINTER(FcWeights), _V, _V, C.c_int32, _V, C.c_int64, _V, _V, _V,
                                      C.c_int64, C.c_int64, _V, _V, _V, _V]),

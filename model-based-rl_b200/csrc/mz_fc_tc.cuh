@@ -34,6 +34,24 @@ constexpr int T_REW_B = 0, T_DYN_B = 32, T_LN_W = 96, T_LN_B = 160, T_VAL_B = 22
 constexpr int TAIL_FLOATS = 288;
 constexpr int OUT_STRIDE = 51;        // odd row stride of the output staging area (bank-conflict free)
 
+// Second-layer head geometry.  Narrow: A <= 32 and both supports <= 32 bins, reward / value / policy second
+// layers padded to N = 32 (the constants above; the persistent search kernel knows only this one).  Wide: any of
+// them above 32 (up to 64), all three padded to N = 64, with the TMEM columns and the tail laid out for 64.
+struct NarrowGeom {
+  static constexpr int NB = 32;  // padded reward / value / policy width
+  static constexpr int COL_D2A = mzfc::COL_D2A, COL_D2B = mzfc::COL_D2B;
+  static constexpr int T_REW_B = mzfc::T_REW_B, T_DYN_B = mzfc::T_DYN_B, T_LN_W = mzfc::T_LN_W, T_LN_B = mzfc::T_LN_B,
+                       T_VAL_B = mzfc::T_VAL_B, T_POL_B = mzfc::T_POL_B, TAIL_FLOATS = mzfc::TAIL_FLOATS;
+};
+struct WideGeom {
+  static constexpr int NB = 64;
+  static constexpr int COL_D2A = 384;  // 64: reward / value logits
+  static constexpr int COL_D2B = 448;  // 64: next hidden / policy logits (ends at TMEM_COLS)
+  static constexpr int T_REW_B = 0, T_DYN_B = 64, T_LN_W = 128, T_LN_B = 192, T_VAL_B = 256, T_POL_B = 320;
+  static constexpr int TAIL_FLOATS = 384;
+};
+static_assert(WideGeom::COL_D2B + N_HID == TMEM_COLS, "the wide column map fills the allocation");
+
 struct ChunkGeom {  // byte geometry of one packed chunk: [W1 | W2]; the first-layer bias is folded
                     // into W1 as the weight of a constant-1 input column (index kin)
   int k;            // K of the first layer (K1 or K3)
@@ -41,23 +59,26 @@ struct ChunkGeom {  // byte geometry of one packed chunk: [W1 | W2]; the first-l
   int w1_bytes, w2_bytes, bytes;
 };
 
+template <class G = NarrowGeom>
 __host__ __device__ inline ChunkGeom chunk_geom(int c, int k1) {
   ChunkGeom g;
   const int head = c >> 2;  // 0 reward, 1 transition, 2 value, 3 policy
   g.k = head < 2 ? k1 : K3;
-  g.n2 = head == 0 ? N_REW : (head == 1 ? N_HID : (head == 2 ? N_VAL : N_POL));
+  g.n2 = head == 0 ? G::NB : (head == 1 ? N_HID : G::NB);
   g.w1_bytes = CHUNK * g.k * 2;
   g.w2_bytes = g.n2 * CHUNK * 2;
   g.bytes = g.w1_bytes + g.w2_bytes;
   return g;
 }
+template <class G = NarrowGeom>
 __host__ __device__ inline size_t chunk_offset(int c, int k1) {
   size_t off = 0;
-  for (int i = 0; i < c; ++i) off += chunk_geom(i, k1).bytes;
+  for (int i = 0; i < c; ++i) off += chunk_geom<G>(i, k1).bytes;
   return off;
 }
+template <class G = NarrowGeom>
 __host__ __device__ inline int stage_bytes_for(int k1) {  // largest chunk: a k1-wide head or a prediction head
-  const int a = chunk_geom(4, k1).bytes, b = chunk_geom(8, k1).bytes;
+  const int a = chunk_geom<G>(4, k1).bytes, b = chunk_geom<G>(8, k1).bytes;
   return a > b ? a : b;
 }
 
@@ -222,6 +243,40 @@ MZ_DEV float support_to_scalar_regs(const uint32_t (&v)[32], const float* bias, 
   }
   const float2 d2 = __fadd2_rn(den[0], den[1]), n2 = __fadd2_rn(num[0], num[1]);
   const float mean = __fdividef(n2.x + n2.y, d2.x + d2.y) + (float)mn;  // sum_j (mn + j) softmax_j
+  return no_tt ? mean : mz_inverse_scalar_transform_f(mean);
+}
+
+// support_to_scalar_regs over 64 columns (wide geometry): columns 0..31 in v, 32..63 in v2.  At 64 bins there
+// is no padding column, as at 32 bins in the narrow geometry.
+MZ_DEV float support_to_scalar_regs(const uint32_t (&v)[32], const uint32_t (&v2)[32], const float* bias, int mn,
+                                    int no_tt) {
+  float2 x[32];
+  const float4* b4 = reinterpret_cast<const float4*>(bias);
+#pragma unroll
+  for (int k = 0; k < 8; ++k) {
+    const float4 b = b4[k], c = b4[8 + k];
+    x[2 * k] = __fadd2_rn(make_float2(__uint_as_float(v[4 * k]), __uint_as_float(v[4 * k + 1])), make_float2(b.x, b.y));
+    x[2 * k + 1] = __fadd2_rn(make_float2(__uint_as_float(v[4 * k + 2]), __uint_as_float(v[4 * k + 3])), make_float2(b.z, b.w));
+    x[16 + 2 * k] = __fadd2_rn(make_float2(__uint_as_float(v2[4 * k]), __uint_as_float(v2[4 * k + 1])), make_float2(c.x, c.y));
+    x[17 + 2 * k] = __fadd2_rn(make_float2(__uint_as_float(v2[4 * k + 2]), __uint_as_float(v2[4 * k + 3])), make_float2(c.z, c.w));
+  }
+  float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
+#pragma unroll
+  for (int k = 0; k < 32; ++k) m4[k & 3] = fmaxf(m4[k & 3], fmaxf(x[k].x, x[k].y));
+  const float m = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
+  const float l2e = 1.4426950408889634f;
+  const float2 scale = make_float2(l2e, l2e), shift = make_float2(-m * l2e, -m * l2e);
+  float2 den[2] = {make_float2(0.0f, 0.0f), make_float2(0.0f, 0.0f)};
+  float2 num[2] = {make_float2(0.0f, 0.0f), make_float2(0.0f, 0.0f)};
+#pragma unroll
+  for (int k = 0; k < 32; ++k) {
+    const float2 t = __ffma2_rn(x[k], scale, shift);
+    const float2 e = make_float2(ex2_approx(t.x), ex2_approx(t.y));
+    den[k & 1] = __fadd2_rn(den[k & 1], e);
+    num[k & 1] = __ffma2_rn(e, make_float2((float)(2 * k), (float)(2 * k + 1)), num[k & 1]);
+  }
+  const float2 d2 = __fadd2_rn(den[0], den[1]), n2 = __fadd2_rn(num[0], num[1]);
+  const float mean = __fdividef(n2.x + n2.y, d2.x + d2.y) + (float)mn;
   return no_tt ? mean : mz_inverse_scalar_transform_f(mean);
 }
 

@@ -5,6 +5,10 @@
 //   LayerNorm + ReLU on h'  (fp32, one thread per row), reward = softmax-expectation + h^-1
 //   prediction : h' (K3 = 64) --W3--> 2 x 512 --relu--> W4 --> value logits (32), policy logits (32)
 //
+// That is the narrow head geometry (A <= 32, supports <= 32 bins).  The wide one (mzfc::WideGeom: more actions or
+// bins, up to 64) pads reward, value and policy logits to 64 columns each; the kernel and the packing are
+// templated on the geometry, and the host picks it from the weights (tc_geometry).
+//
 // The 512-wide hidden layers are processed in 16 chunks of 128 features.  Per chunk c:
 //   MMA1(c): D1[c&1] (TMEM, 128 lanes x 128 cols) = A(128 x K) * W1c^T          (tcgen05.mma)
 //   EPI(c) : D1[c&1] -> registers (tcgen05.ld) -> relu, bf16 -> A2[c&1] back in TMEM (tcgen05.st)
@@ -67,6 +71,7 @@ struct TcParams {
   } while (0)
 
 
+template <class G>
 __global__ void __maxnreg__(152) fc_recurrent_tc_kernel(TcParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -76,7 +81,7 @@ __global__ void __maxnreg__(152) fc_recurrent_tc_kernel(TcParams p) {
     p.trace[256 + 2 * blockIdx.x] = (long long)tns;
   }
   const int k1 = p.k1;
-  const int stage_bytes = stage_bytes_for(k1);
+  const int stage_bytes = stage_bytes_for<G>(k1);
   const bool split = p.split != 0;
   const int rank = split ? (int)cluster_ctarank() : 0;
   const int tile = split ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;  // which 128 rows
@@ -120,9 +125,9 @@ __global__ void __maxnreg__(152) fc_recurrent_tc_kernel(TcParams p) {
   uint64_t* h_stored = bars + 21;     // the store warp is done with sOut (the logits reuse it)
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 22);
   float* sTail = reinterpret_cast<float*>(bars + 24);   // 16-byte aligned: second-layer biases + LayerNorm affine
-  float* sOut = sTail + TAIL_FLOATS;                    // [128][51]: row-major staging of h'
+  float* sOut = sTail + G::TAIL_FLOATS;                 // [128][51]: row-major staging of h'
   float* sLog = sOut;                                   // [128][A]: the logits reuse it at the very end
-  for (int i = threadIdx.x; i < TAIL_FLOATS; i += TC_THREADS) sTail[i] = p.tail[i];
+  for (int i = threadIdx.x; i < G::TAIL_FLOATS; i += TC_THREADS) sTail[i] = p.tail[i];
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < MAX_STAGES; ++i) { mbar_init(&w_full[i], 1); mbar_init(&w_empty[i], 1); }
@@ -155,15 +160,15 @@ __global__ void __maxnreg__(152) fc_recurrent_tc_kernel(TcParams p) {
   if (warp == 0) {
     // ===== producer: stream the 16 weight chunks through the ring =====
     if (lane == 0) {
-      const size_t base = chunk_offset(c0, k1);
+      const size_t base = chunk_offset<G>(c0, k1);
       int st = 0, n = 0;  // ring slot and round, advanced incrementally (STAGES is a run-time value)
       for (int c = 0; c < nch; ++c, st = (st + 1 == STAGES ? 0 : st + 1), n += (st == 0)) {
         const int cc = canon(c);
-        const ChunkGeom g = chunk_geom(cc, k1);
+        const ChunkGeom g = chunk_geom<G>(cc, k1);
         mbar_wait(&w_empty[st], (n & 1) ^ 1);
         TC_STAMP(192 + c);
         mbar_arrive_expect_tx(&w_full[st], (uint32_t)g.bytes);
-        bulk_copy_g2s(sW + st * stage_bytes, p.chunks + (chunk_offset(cc, k1) - base), (uint32_t)g.bytes,
+        bulk_copy_g2s(sW + st * stage_bytes, p.chunks + (chunk_offset<G>(cc, k1) - base), (uint32_t)g.bytes,
                       &w_full[st]);
       }
     }
@@ -217,8 +222,8 @@ __global__ void __maxnreg__(152) fc_recurrent_tc_kernel(TcParams p) {
       const uint32_t a_tm = tmem + COL_A2 + (c & 1) * (CHUNK / 2);
       const uint32_t b_addr = w_addr + st * stage_bytes + (cc < 8 ? w1_bytes_dyn : w1_bytes_pred);
       if (elect_one()) {
-        if (head == 1) issue_mma2<N_HID>(tmem + COL_D2B, a_tm, b_addr, (cc & 3) == 0);
-        else issue_mma2<32>(tmem + ((head & 1) ? COL_D2B : COL_D2A), a_tm, b_addr, (cc & 3) == 0);
+        if (head == 1) issue_mma2<N_HID>(tmem + G::COL_D2B, a_tm, b_addr, (cc & 3) == 0);
+        else issue_mma2<G::NB>(tmem + ((head & 1) ? G::COL_D2B : G::COL_D2A), a_tm, b_addr, (cc & 3) == 0);
         tc_commit(&w_empty[st]);       // chunk c's weights are no longer needed
         tc_commit(&a2_empty[c & 1]);   // A2 buffer may be overwritten
         if (c == c_mid - 1 || c == nch - 1) tc_commit(d2_full);
@@ -374,21 +379,28 @@ __global__ void __maxnreg__(152) fc_recurrent_tc_kernel(TcParams p) {
     if (stamp) TC_STAMP(40);
     if (grp == 1) {
       if (c0 == 0 && own_reward) {  // initial_inference has no reward (networks.py:29 returns 0)
-        tmem_ld32(lane_addr + COL_D2A, v);
-        tmem_wait_ld();
-        const float rew = support_to_scalar_regs(v, sTail + T_REW_B, p.reward_min, p.no_tt);
+        float rew;
+        tmem_ld32(lane_addr + G::COL_D2A, v);
+        if constexpr (G::NB == 64) {
+          tmem_ld32(lane_addr + G::COL_D2A + 32, v2);
+          tmem_wait_ld();
+          rew = support_to_scalar_regs(v, v2, sTail + G::T_REW_B, p.reward_min, p.no_tt);
+        } else {
+          tmem_wait_ld();
+          rew = support_to_scalar_regs(v, sTail + G::T_REW_B, p.reward_min, p.no_tt);
+        }
         if (live) p.reward[g] = rew;
       }
     } else if (own_hidden) {
       float hbuf[64];
-      tmem_ld32(lane_addr + COL_D2B, v);
-      tmem_ld32(lane_addr + COL_D2B + 32, v2);
+      tmem_ld32(lane_addr + G::COL_D2B, v);
+      tmem_ld32(lane_addr + G::COL_D2B + 32, v2);
       tmem_wait_ld();
       // LayerNorm over the 50 state features in packed float32x2 arithmetic (25 pairs; this thread is one
       // in-order stream on the kernel's critical path, the instruction count is its cost)
       float2 h2[H / 2];
       {
-        const float4* b4 = reinterpret_cast<const float4*>(sTail + T_DYN_B);
+        const float4* b4 = reinterpret_cast<const float4*>(sTail + G::T_DYN_B);
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
           const float4 b = b4[k];
@@ -401,7 +413,7 @@ __global__ void __maxnreg__(152) fc_recurrent_tc_kernel(TcParams p) {
           h2[16 + 2 * k] = __fadd2_rn(make_float2(__uint_as_float(v2[4 * k]), __uint_as_float(v2[4 * k + 1])), make_float2(b.x, b.y));
           h2[16 + 2 * k + 1] = __fadd2_rn(make_float2(__uint_as_float(v2[4 * k + 2]), __uint_as_float(v2[4 * k + 3])), make_float2(b.z, b.w));
         }
-        const float2 b = *reinterpret_cast<const float2*>(sTail + T_DYN_B + 48);
+        const float2 b = *reinterpret_cast<const float2*>(sTail + G::T_DYN_B + 48);
         h2[24] = __fadd2_rn(make_float2(__uint_as_float(v2[16]), __uint_as_float(v2[17])), b);
       }
       float2 s2[4] = {make_float2(0.0f, 0.0f), make_float2(0.0f, 0.0f), make_float2(0.0f, 0.0f), make_float2(0.0f, 0.0f)};
@@ -420,8 +432,8 @@ __global__ void __maxnreg__(152) fc_recurrent_tc_kernel(TcParams p) {
       const float rstd = rsqrtf((qt.x + qt.y) * (1.0f / (float)H) + 1e-5f);
       const float2 rstd2 = make_float2(rstd, rstd);
       {
-        const float2* w2 = reinterpret_cast<const float2*>(sTail + T_LN_W);
-        const float2* b2 = reinterpret_cast<const float2*>(sTail + T_LN_B);
+        const float2* w2 = reinterpret_cast<const float2*>(sTail + G::T_LN_W);
+        const float2* b2 = reinterpret_cast<const float2*>(sTail + G::T_LN_B);
 #pragma unroll
         for (int k = 0; k < H / 2; ++k) {
           const float2 y = __ffma2_rn(__fmul2_rn(h2[k], rstd2), w2[k], b2[k]);
@@ -478,20 +490,34 @@ __global__ void __maxnreg__(152) fc_recurrent_tc_kernel(TcParams p) {
     if (stamp) TC_STAMP(42);
     if (grp == 0) {
       if (own_value) {
-        tmem_ld32(lane_addr + COL_D2A, v);
-        tmem_wait_ld();
-        const float val = support_to_scalar_regs(v, sTail + T_VAL_B, p.value_min, p.no_tt);
+        float val;
+        tmem_ld32(lane_addr + G::COL_D2A, v);
+        if constexpr (G::NB == 64) {
+          tmem_ld32(lane_addr + G::COL_D2A + 32, v2);
+          tmem_wait_ld();
+          val = support_to_scalar_regs(v, v2, sTail + G::T_VAL_B, p.value_min, p.no_tt);
+        } else {
+          tmem_wait_ld();
+          val = support_to_scalar_regs(v, sTail + G::T_VAL_B, p.value_min, p.no_tt);
+        }
         if (live) p.value[g] = val;
       }
     } else if (own_logits) {
-      tmem_ld32(lane_addr + COL_D2B, v);
+      tmem_ld32(lane_addr + G::COL_D2B, v);
       tmem_wait_ld();
       // logits [rows][A] of this CTA are one contiguous block: stage row-major, store linearly
       const int A = p.num_actions;
       mbar_wait(h_stored, 0);  // the staging area is free again
 #pragma unroll
       for (int j = 0; j < 32; ++j)
-        if (j < A) sLog[row * A + j] = __uint_as_float(v[j]) + sTail[T_POL_B + j];
+        if (j < A) sLog[row * A + j] = __uint_as_float(v[j]) + sTail[G::T_POL_B + j];
+      if constexpr (G::NB == 64) {  // second half of the 64 policy columns
+        tmem_ld32(lane_addr + G::COL_D2B + 32, v);
+        tmem_wait_ld();
+#pragma unroll
+        for (int j = 0; j < 32; ++j)
+          if (32 + j < A) sLog[row * A + 32 + j] = __uint_as_float(v[j]) + sTail[G::T_POL_B + 32 + j];
+      }
       asm volatile("bar.sync 1, 128;" ::: "memory");  // the four warps of this group
       const int rows_here = min(ROWS, p.batch - tile * ROWS);
       float* dl = p.logits + (size_t)tile * ROWS * A;
@@ -517,12 +543,13 @@ __global__ void __maxnreg__(152) fc_recurrent_tc_kernel(TcParams p) {
 // ---- packing: f32 reference-layout weights -> bf16 chunk images + tail parameters ---------------
 // chunk0 = 0: the recurrent image (reward, transition, value, policy heads); chunk0 = 4: the
 // initial-inference image (representation in place of the transition head, then value, policy)
+template <class G>
 __global__ void fc_tc_pack_kernel(mz_fc_weights w, int k1, int chunk0, uint8_t* chunks, float* tail) {
   const int A = w.num_actions;
   const bool init = chunk0 != 0;
   for (int c = chunk0; c < NCHUNK; ++c) {
-    const ChunkGeom g = chunk_geom(c, k1);
-    uint8_t* base = chunks + (chunk_offset(c, k1) - chunk_offset(chunk0, k1));
+    const ChunkGeom g = chunk_geom<G>(c, k1);
+    uint8_t* base = chunks + (chunk_offset<G>(c, k1) - chunk_offset<G>(chunk0, k1));
     const int head = c >> 2, f0 = (c & 3) * CHUNK;
     const float* dyn_w1 = init ? w.rep_w1 : w.dyn_w1;
     const float* dyn_b1 = init ? w.rep_b1 : w.dyn_b1;
@@ -545,14 +572,14 @@ __global__ void fc_tc_pack_kernel(mz_fc_weights w, int k1, int chunk0, uint8_t* 
       *reinterpret_cast<__nv_bfloat16*>(base + g.w1_bytes + canon_off(o, k, g.n2)) = __float2bfloat16_rn(x);
     }
   }
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < TAIL_FLOATS; i += gridDim.x * blockDim.x) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < G::TAIL_FLOATS; i += gridDim.x * blockDim.x) {
     float x = 0.0f;
-    if (i < T_DYN_B) x = i < w.reward_bins ? w.rew_b2[i] : -INFINITY;  // padding columns: see support_to_scalar_regs
-    else if (i < T_LN_W) x = (i - T_DYN_B) < H ? (init ? w.rep_b2 : w.dyn_b2)[i - T_DYN_B] : 0.0f;
-    else if (i < T_LN_B) x = (i - T_LN_W) < H ? w.ln_w[i - T_LN_W] : 0.0f;
-    else if (i < T_VAL_B) x = (i - T_LN_B) < H ? w.ln_b[i - T_LN_B] : 0.0f;
-    else if (i < T_POL_B) x = (i - T_VAL_B) < w.value_bins ? w.val_b2[i - T_VAL_B] : -INFINITY;
-    else x = (i - T_POL_B) < A ? w.pol_b2[i - T_POL_B] : 0.0f;
+    if (i < G::T_DYN_B) x = i < w.reward_bins ? w.rew_b2[i] : -INFINITY;  // padding columns: see support_to_scalar_regs
+    else if (i < G::T_LN_W) x = (i - G::T_DYN_B) < H ? (init ? w.rep_b2 : w.dyn_b2)[i - G::T_DYN_B] : 0.0f;
+    else if (i < G::T_LN_B) x = (i - G::T_LN_W) < H ? w.ln_w[i - G::T_LN_W] : 0.0f;
+    else if (i < G::T_VAL_B) x = (i - G::T_LN_B) < H ? w.ln_b[i - G::T_LN_B] : 0.0f;
+    else if (i < G::T_POL_B) x = (i - G::T_VAL_B) < w.value_bins ? w.val_b2[i - G::T_VAL_B] : -INFINITY;
+    else x = (i - G::T_POL_B) < A ? w.pol_b2[i - G::T_POL_B] : 0.0f;
     tail[i] = x;
   }
 }
@@ -577,19 +604,35 @@ int recurrent_stages() {
 
 int k1_obs(int obs_dim) { return (obs_dim + 1 + 15) / 16 * 16; }  // observation + bias column
 
-size_t tc_smem_bytes(int k1, int stages) {
-  return (size_t)ROWS * k1 * 2 + (size_t)stages * stage_bytes_for(k1) +
-         (size_t)ROWS * K3 * 2 + 24 * sizeof(uint64_t) + TAIL_FLOATS * sizeof(float) +
-         ROWS * OUT_STRIDE * sizeof(float);
+// the staging area holds h' ([128][51]) and then the logits ([128][A]: larger from A = 52 on)
+template <class G>
+size_t tc_smem_bytes(int k1, int stages, int A) {
+  return (size_t)ROWS * k1 * 2 + (size_t)stages * stage_bytes_for<G>(k1) +
+         (size_t)ROWS * K3 * 2 + 24 * sizeof(uint64_t) + G::TAIL_FLOATS * sizeof(float) +
+         ROWS * (A > OUT_STRIDE ? A : OUT_STRIDE) * sizeof(float);
 }
 
 constexpr size_t kTcMaxSmem = 232448;
 
+// Geometry of a network's bf16 images: 0 = not supported, 1 = narrow, 2 = wide.
+int tc_geometry(const mz_fc_weights& w) {
+  if (w.num_actions < 1 || w.num_actions > 64 || w.value_bins < 1 || w.value_bins > 64 || w.reward_bins < 1 ||
+      w.reward_bins > 64 || w.no_support)
+    return 0;
+  return (w.num_actions > 32 || w.value_bins > 32 || w.reward_bins > 32) ? 2 : 1;
+}
+
+// The wide recurrent kernel runs a three-stage ring at every k1: its larger tail does not leave room for a fourth
+// stage at k1 = 96 (A 30..45), and k1 = 112 / 128 (A 46..64) have no room for one with either tail.
+template <class G>
+int stages_for() { return G::NB == 64 && recurrent_stages() > 3 ? 3 : recurrent_stages(); }
+
+template <class G>
 int launch_tc(const TcParams& p, void* stream) {
-  const size_t smem = tc_smem_bytes(p.k1, p.stages);
+  const size_t smem = tc_smem_bytes<G>(p.k1, p.stages, p.num_actions);
   static bool attr = false;
   if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(fc_recurrent_tc_kernel,
+    cudaError_t e = cudaFuncSetAttribute(fc_recurrent_tc_kernel<G>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcMaxSmem);
     if (e != cudaSuccess) return (int)e;
     attr = true;
@@ -617,7 +660,7 @@ int launch_tc(const TcParams& p, void* stream) {
   }
   cfg.attrs = lattr;
   cfg.numAttrs = na;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, fc_recurrent_tc_kernel, p);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, fc_recurrent_tc_kernel<G>, p);
   if (e != cudaSuccess) return (int)e;
   MZ_LAUNCH_CHECK();
   return MZ_OK;
@@ -647,14 +690,41 @@ int64_t mz_fc_tc_packed_bytes(int32_t num_actions) {
   return (int64_t)chunk_offset(NCHUNK, k1_for(num_actions));
 }
 
+int mz_fc_tc_sizes(const mz_fc_weights* w, int64_t* recurrent_bytes, int64_t* initial_bytes, int32_t* tail_floats) {
+  if (!w || !recurrent_bytes || !initial_bytes || !tail_floats) return MZ_ERR_BAD_ARG;
+  const int geom = tc_geometry(*w);
+  if (geom == 0) return MZ_ERR_UNSUPPORTED;
+  const int k1 = k1_for(w->num_actions), k1i = k1_obs(w->obs_dim);
+  if (geom == 1) {
+    *recurrent_bytes = (int64_t)chunk_offset<NarrowGeom>(NCHUNK, k1);
+    *tail_floats = NarrowGeom::TAIL_FLOATS;
+  } else {
+    *recurrent_bytes = (int64_t)chunk_offset<WideGeom>(NCHUNK, k1);
+    *tail_floats = WideGeom::TAIL_FLOATS;
+  }
+  if (w->obs_dim < 1)
+    *initial_bytes = MZ_ERR_BAD_ARG;
+  else if ((geom == 1 ? tc_smem_bytes<NarrowGeom>(k1i, 2, w->num_actions)
+                      : tc_smem_bytes<WideGeom>(k1i, 2, w->num_actions)) > kTcMaxSmem)
+    *initial_bytes = MZ_ERR_UNSUPPORTED;
+  else
+    *initial_bytes = (int64_t)(geom == 1 ? chunk_offset<NarrowGeom>(NCHUNK, k1i) - chunk_offset<NarrowGeom>(4, k1i)
+                                         : chunk_offset<WideGeom>(NCHUNK, k1i) - chunk_offset<WideGeom>(4, k1i));
+  return MZ_OK;
+}
+
 int32_t mz_fc_tc_tail_floats(void) { return TAIL_FLOATS; }
 
 int mz_fc_tc_pack(const mz_fc_weights* w, void* packed, float* tail, void* stream) {
   if (!w || !packed || !tail) return MZ_ERR_BAD_ARG;
-  if (w->num_actions < 1 || w->num_actions > 32 || w->value_bins < 1 || w->value_bins > 32 ||
-      w->reward_bins < 1 || w->reward_bins > 32 || w->no_support)
-    return MZ_ERR_UNSUPPORTED;
-  fc_tc_pack_kernel<<<64, 256, 0, (cudaStream_t)stream>>>(*w, k1_for(w->num_actions), 0, (uint8_t*)packed, tail);
+  const int geom = tc_geometry(*w);
+  if (geom == 0) return MZ_ERR_UNSUPPORTED;
+  if (geom == 1)
+    fc_tc_pack_kernel<NarrowGeom><<<64, 256, 0, (cudaStream_t)stream>>>(*w, k1_for(w->num_actions), 0,
+                                                                        (uint8_t*)packed, tail);
+  else
+    fc_tc_pack_kernel<WideGeom><<<64, 256, 0, (cudaStream_t)stream>>>(*w, k1_for(w->num_actions), 0,
+                                                                      (uint8_t*)packed, tail);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }
@@ -668,8 +738,8 @@ int mz_fc_recurrent_tc(const mz_fc_weights* w, const void* packed, const float* 
     return MZ_ERR_BAD_ARG;
   // the epilogue reads hidden rows as float2: every row start must be 8-byte aligned
   if ((in_row_stride & 1) || ((uintptr_t)hidden_in & 7)) return MZ_ERR_BAD_ARG;
-  if (w->num_actions < 1 || w->num_actions > 32 || w->value_bins > 32 || w->reward_bins > 32 || w->no_support)
-    return MZ_ERR_UNSUPPORTED;
+  const int geom = tc_geometry(*w);
+  if (geom == 0) return MZ_ERR_UNSUPPORTED;
   TcParams p;
   p.chunks = (const uint8_t*)packed;
   p.tail = tail;
@@ -693,28 +763,34 @@ int mz_fc_recurrent_tc(const mz_fc_weights* w, const void* packed, const float* 
   p.logits = logits;
   p.trace = g_tc_trace;
   p.chunk0 = 0;
-  p.stages = recurrent_stages();
+  p.stages = geom == 1 ? stages_for<NarrowGeom>() : stages_for<WideGeom>();
   p.obs = nullptr;
   p.obs_dim = 0;
   p.split = g_tc_split;
   p.trace_block = g_tc_trace_block;
-  return launch_tc(p, stream);
+  return geom == 1 ? launch_tc<NarrowGeom>(p, stream) : launch_tc<WideGeom>(p, stream);
 }
 
 /* Initial-inference image: representation head (K = obs_dim + bias column) + value + policy. */
 int64_t mz_fc_tc_initial_packed_bytes(int32_t obs_dim) {
   if (obs_dim < 1) return MZ_ERR_BAD_ARG;
   const int k1 = k1_obs(obs_dim);
-  if (tc_smem_bytes(k1, 2) > kTcMaxSmem) return MZ_ERR_UNSUPPORTED;
+  if (tc_smem_bytes<NarrowGeom>(k1, 2, 32) > kTcMaxSmem) return MZ_ERR_UNSUPPORTED;
   return (int64_t)(chunk_offset(NCHUNK, k1) - chunk_offset(4, k1));
 }
 
 int mz_fc_tc_pack_initial(const mz_fc_weights* w, void* packed, float* tail, void* stream) {
   if (!w || !packed || !tail) return MZ_ERR_BAD_ARG;
-  if (w->num_actions < 1 || w->num_actions > 32 || w->value_bins < 1 || w->value_bins > 32 || w->no_support)
-    return MZ_ERR_UNSUPPORTED;
-  if (tc_smem_bytes(k1_obs(w->obs_dim), 2) > kTcMaxSmem) return MZ_ERR_UNSUPPORTED;
-  fc_tc_pack_kernel<<<64, 256, 0, (cudaStream_t)stream>>>(*w, k1_obs(w->obs_dim), 4, (uint8_t*)packed, tail);
+  const int geom = tc_geometry(*w);
+  if (geom == 0) return MZ_ERR_UNSUPPORTED;
+  const int k1 = k1_obs(w->obs_dim);
+  if (geom == 1) {
+    if (tc_smem_bytes<NarrowGeom>(k1, 2, w->num_actions) > kTcMaxSmem) return MZ_ERR_UNSUPPORTED;
+    fc_tc_pack_kernel<NarrowGeom><<<64, 256, 0, (cudaStream_t)stream>>>(*w, k1, 4, (uint8_t*)packed, tail);
+  } else {
+    if (tc_smem_bytes<WideGeom>(k1, 2, w->num_actions) > kTcMaxSmem) return MZ_ERR_UNSUPPORTED;
+    fc_tc_pack_kernel<WideGeom><<<64, 256, 0, (cudaStream_t)stream>>>(*w, k1, 4, (uint8_t*)packed, tail);
+  }
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }
@@ -723,7 +799,8 @@ int mz_fc_initial_tc(const mz_fc_weights* w, const void* packed, const float* ta
                      const float* obs, float* hidden_out, int64_t out_row_stride, float* value,
                      float* logits, void* stream) {
   if (!w || !packed || !tail || batch < 1 || !obs || !hidden_out || !value || !logits) return MZ_ERR_BAD_ARG;
-  if (w->num_actions < 1 || w->num_actions > 32 || w->value_bins > 32 || w->no_support) return MZ_ERR_UNSUPPORTED;
+  const int geom = tc_geometry(*w);
+  if (geom == 0) return MZ_ERR_UNSUPPORTED;
   TcParams p;
   p.chunks = (const uint8_t*)packed;
   p.tail = tail;
@@ -752,7 +829,7 @@ int mz_fc_initial_tc(const mz_fc_weights* w, const void* packed, const float* ta
   p.obs_dim = w->obs_dim;
   p.split = 0;
   p.trace_block = 0;
-  return launch_tc(p, stream);
+  return geom == 1 ? launch_tc<NarrowGeom>(p, stream) : launch_tc<WideGeom>(p, stream);
 }
 
 }  // extern "C"

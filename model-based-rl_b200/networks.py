@@ -45,7 +45,7 @@ class FCNetwork(object):
 
   def __init__(self, input_dim, action_space, device, config, precision='bf16'):
     """precision: 'bf16' = tcgen05 tensor-core kernel for recurrent_inference (bf16 operands, fp32
-    accumulation); 'f32' = CUDA-core float32 kernel (reference precision, used for parity); 'tf32x3' =
+    accumulation; A <= 64 and supports of at most 64 bins); 'f32' = CUDA-core float32 kernel (reference precision, used for parity); 'tf32x3' =
     reference precision on the tensor cores (three TF32 instructions per product on split operands,
     float32 accumulation: the results of 'f32' within float32 rounding)."""
     _lib.require_cuda()
@@ -111,16 +111,17 @@ class FCNetwork(object):
       self._tc_packed = self._tc_tail = None
       self._tc_init_packed = self._tc_init_tail = None
       if self.precision == 'bf16':
-        if self.action_space > 32 or self.value_bins > 32 or self.reward_bins > 32:
-          raise NotImplementedError("the tensor-core kernel supports A <= 32 and supports <= 32 bins; "
+        if self.action_space > 64 or self.value_bins > 64 or self.reward_bins > 64:
+          raise NotImplementedError("the tensor-core kernel supports A <= 64 and supports <= 64 bins; "
                                     "use precision='f32'")
-        nbytes = int(self.lib.mz_fc_tc_packed_bytes(self.action_space))
-        self._tc_packed = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
-        self._tc_tail = torch.zeros(int(self.lib.mz_fc_tc_tail_floats()), dtype=torch.float32,
-                                    device=self.device)
+        rec, init, tail = C.c_int64(), C.c_int64(), C.c_int32()
+        _lib.check(self.lib.mz_fc_tc_sizes(self.weights, C.byref(rec), C.byref(init), C.byref(tail)),
+                   "mz_fc_tc_sizes")
+        self._tc_packed = torch.zeros(rec.value, dtype=torch.uint8, device=self.device)
+        self._tc_tail = torch.zeros(tail.value, dtype=torch.float32, device=self.device)
         # initial_inference image (representation + prediction heads); observations too wide for
         # the kernel's shared-memory budget stay on the float32 kernel
-        nbytes = int(self.lib.mz_fc_tc_initial_packed_bytes(self.input_dim))
+        nbytes = init.value
         if nbytes > 0:
           self._tc_init_packed = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
           self._tc_init_tail = torch.zeros_like(self._tc_tail)
@@ -391,8 +392,8 @@ class FCSearch(object):
   def __init__(self, config, fcnet, num_games, noise_frac=None, use_graph=True, num_streams=1, fused=None):
     """fused: True = the whole move in one persistent kernel (`mz_fc_search`, csrc/mz_fcsearch.cu), False =
     one tree launch + one network launch per simulation on `num_streams` slices, None = fused whenever the
-    network runs in bf16, at most 8192 games play and the shape fits the kernel: S <= 63 and (S, A) within its
-    shared-memory plan, as `mz_fc_search_supported` reports (S <= 63 for A <= 13, S <= 55 for A <= 20, S <= 53 for
+    network runs in bf16 with supports of at most 32 bins, at most 8192 games play and the shape fits the kernel:
+    S <= 63 and (S, A) within its shared-memory plan, as `mz_fc_search_supported` reports (S <= 63 for A <= 13, S <= 55 for A <= 20, S <= 53 for
     A <= 29, S <= 19 for A <= 32).  Every other shape runs the per-launch path; MZ_FUSED=0 in the environment turns
     the default off.  Both give bit-identical searches (tests/test_gpu_fcnet.py)."""
     self.net = fcnet
@@ -422,7 +423,9 @@ class FCSearch(object):
     self.root_logits = torch.zeros((G, A), dtype=torch.float32, device=dev)
     self.visits = torch.zeros((G, A), dtype=torch.int32, device=dev)
     self.minmax = torch.zeros((G, 2), dtype=torch.float64, device=dev)
+    # the persistent kernel reads the narrow bf16 image only: supports of at most 32 bins
     can_fuse = (fcnet.precision == 'bf16' and fcnet.weights is not None and
+                fcnet.value_bins <= 32 and fcnet.reward_bins <= 32 and
                 int(fcnet.lib.mz_fc_search_supported(self.S, A)) == 1)
     if fused is None:
       # measured (profiles/r02l_fused_sweep.log): the persistent kernel wins wherever one wave of clusters holds
@@ -430,8 +433,8 @@ class FCSearch(object):
       # few per cent from 16 384 games on, where the per-launch path has more games in flight per SM
       fused = can_fuse and os.environ.get("MZ_FUSED", "1") != "0" and G <= 8192
     elif fused and not can_fuse:
-      raise ValueError("the fused search kernel needs a bf16 FCNetwork with loaded weights, A <= 32, S <= 63 "
-                       "and a tree that fits its shared-memory plan")
+      raise ValueError("the fused search kernel needs a bf16 FCNetwork with loaded weights, A <= 32, value and "
+                       "reward supports of at most 32 bins, S <= 63 and a tree that fits its shared-memory plan")
     self.fused = _FusedEngine(config, fcnet, self) if fused else None
     self.lanes = []
     self.eng = None
