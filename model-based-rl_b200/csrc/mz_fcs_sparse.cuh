@@ -246,9 +246,13 @@ MZ_DEV void set_root(const FsParams& p, const Smem& sm, const Game& gm, const Ge
   *reinterpret_cast<uint4*>(row + 8 * gm.sub) = make_uint4(w[0], w[1], w[2], w[3]);
 }
 
+// phase stamps of the instrumented instantiation (TL: FsParams::timeline set); the production one has none, so
+// no stamp splits its code into separate basic blocks
 #define FS2_STAMP(slot_)                    \
   do {                                      \
-    if (tl) tl[(slot_)] = clock64();        \
+    if constexpr (TL) {                     \
+      if (tl) tl[(slot_)] = clock64();      \
+    }                                       \
   } while (0)
 
 // ------------------------------------------------------------------------------------------------------
@@ -285,6 +289,7 @@ MZ_DEV Norm make_norm(double mn, double mx) {
   return n;
 }
 
+template <bool TL>
 MZ_DEV void descend(const FsParams& p, const Smem& sm, const Game& gm, const Geo& G, int sim, int& out_parent,
                     int& out_action, long long* tl) {
   const int A = p.A, SP1 = p.S + 1;
@@ -607,7 +612,7 @@ MZ_DEV void pre_expand(const FsParams& p, const Smem& sm, const Game& gm, const 
   pre.xm_par = xm_par;
 }
 
-template <int AL>
+template <bool TL, int AL>
 MZ_DEV void expand_backup(const FsParams& p, const Smem& sm, const Game& gm, const Geo& G, int sim, const Pre& pre,
                           long long* tl) {
   const int A = p.A;

@@ -214,8 +214,9 @@ __host__ __device__ inline FsLayout fs_layout(int k1, int A, int S) {
 }
 
 // ======================================================================================================
-// AL: actions per lane of the tree engine at expansion (eight lanes per game)
-template <int AL>
+// AL: actions per lane of the tree engine at expansion (eight lanes per game); TL: the instrumented instantiation
+// that writes the clock64 phase stamps of FsParams::timeline (launched only when it is set)
+template <int AL, bool TL>
 __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
   constexpr int LANES = fs2::L;
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -234,7 +235,7 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
   const bool own_reward = rank == 0, own_trans = rank == 1, own_value = rank == rank_value, own_policy = rank == rank_policy;
   int* const err = p.error_flag;
 
-  if (p.timeline && blockIdx.x == 0 && threadIdx.x == 64) {  // diagnostics: kernel entry (cycles, ns)
+  if (TL && blockIdx.x == 0 && threadIdx.x == 64) {  // diagnostics: kernel entry (cycles, ns)
     unsigned long long ns;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
     p.timeline[27] = clock64();
@@ -414,10 +415,12 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
     gm.valid = tree_role && gm.g < p.G;
     gm.base = p.games + (size_t)(gm.valid ? gm.g : 0) * p.game_bytes;
     const int my_row = rank * GP + gm.gl;         // tile row of the game this lane works on
-    const bool stamp = p.timeline && blockIdx.x == 0 && e == 0;
-#define FS_STAMP(sim_, slot_)                                           \
-  do {                                                                  \
-    if (stamp) p.timeline[(size_t)(sim_) * 32 + (slot_)] = clock64();   \
+    const bool stamp = TL && blockIdx.x == 0 && e == 0;
+#define FS_STAMP(sim_, slot_)                                             \
+  do {                                                                    \
+    if constexpr (TL) {                                                   \
+      if (stamp) p.timeline[(size_t)(sim_) * 32 + (slot_)] = clock64();   \
+    }                                                                     \
   } while (0)
     // output slots of the game a ROW belongs to (the epilogues send there)
     const uint32_t owner = (uint32_t)(row / GP);
@@ -477,14 +480,14 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
           fs_wait_cluster(out_full, (sim - 1) & 1, err, 10);
           if (sim < S) arm();
           FS_STAMP(sim - 1, 10);
-          fs2::expand_backup<AL>(p, sm, gm, geo, sim - 1, pre, stamp ? p.timeline + (size_t)(sim - 1) * 32 : nullptr);
+          fs2::expand_backup<TL, AL>(p, sm, gm, geo, sim - 1, pre, stamp ? p.timeline + (size_t)(sim - 1) * 32 : nullptr);
           FS_STAMP(sim - 1, 11);
         }
       }
       if (sim == S) break;
       if (tree_role) {
         int parent, action;
-        fs2::descend(p, sm, gm, geo, sim, parent, action, stamp ? p.timeline + (size_t)sim * 32 : nullptr);
+        fs2::descend<TL>(p, sm, gm, geo, sim, parent, action, stamp ? p.timeline + (size_t)sim * 32 : nullptr);
         FS_STAMP(sim, 1);
         // A1 row of the game: bf16([h (50) | onehot(action) (A) | 1 | 0]) as 16-byte blocks of the canonical
         // K-major image, sent to every CTA that owns a dynamics head (ranks 0 and 1)
@@ -660,7 +663,7 @@ __global__ void __maxnreg__(152) fc_search_kernel(FsParams p) {
 
   __syncthreads();
   cluster_sync_all();  // no CTA leaves while a peer may still address its shared memory
-  if (p.timeline && blockIdx.x == 0 && threadIdx.x == 64) {  // diagnostics: kernel exit
+  if (TL && blockIdx.x == 0 && threadIdx.x == 64) {  // diagnostics: kernel exit
     unsigned long long ns;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
     p.timeline[28] = clock64();
@@ -707,11 +710,11 @@ bool fs_fits(int S, int A) {
   return A >= 1 && A <= 32 && S >= 1 && S <= fs2::MAX_S && fs_layout(fs_k1_for(A), A, S).total <= kFsMaxSmem;
 }
 
-template <int AL>
+template <int AL, bool TL>
 int fs_launch(const FsParams& p, size_t smem, void* stream) {
   static bool attr = false;
   if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(fc_search_kernel<AL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFsMaxSmem);
+    cudaError_t e = cudaFuncSetAttribute(fc_search_kernel<AL, TL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFsMaxSmem);
     if (e != cudaSuccess) return (int)e;
     attr = true;
   }
@@ -732,7 +735,7 @@ int fs_launch(const FsParams& p, size_t smem, void* stream) {
   // (launching it as a programmatic dependent of the initial-inference kernel was measured: no gain -- 204.5 vs
   // 203.7 M expansions/s on C4, slightly slower on C1 / C3 -- so it is a plain launch)
   cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, fc_search_kernel<AL>, p);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, fc_search_kernel<AL, TL>, p);
   if (e != cudaSuccess) return (int)e;
   MZ_LAUNCH_CHECK();
   return MZ_OK;
@@ -800,10 +803,16 @@ int mz_fc_search(const mz_fc_search_args* a, void* stream) {
   p.error_flag = a->error_flag;
   const size_t smem = fs_layout(p.k1, p.A, p.S).total;
   const int AL = (p.A + fs2::L - 1) / fs2::L;
-  if (AL <= 1) return fs_launch<1>(p, smem, stream);
-  if (AL <= 2) return fs_launch<2>(p, smem, stream);
-  if (AL <= 3) return fs_launch<3>(p, smem, stream);
-  return fs_launch<4>(p, smem, stream);
+  if (p.timeline) {
+    if (AL <= 1) return fs_launch<1, true>(p, smem, stream);
+    if (AL <= 2) return fs_launch<2, true>(p, smem, stream);
+    if (AL <= 3) return fs_launch<3, true>(p, smem, stream);
+    return fs_launch<4, true>(p, smem, stream);
+  }
+  if (AL <= 1) return fs_launch<1, false>(p, smem, stream);
+  if (AL <= 2) return fs_launch<2, false>(p, smem, stream);
+  if (AL <= 3) return fs_launch<3, false>(p, smem, stream);
+  return fs_launch<4, false>(p, smem, stream);
 }
 
 int mz_fc_search_export(const mz_fc_search_args* a, int32_t game, double* prior, int32_t* child, double* vsum,
