@@ -625,13 +625,16 @@ int32_t mz_compiled_arch(void); /* 100 for sm_100a */
 /* Learner network forward / backward for the FCNetwork architecture (learners.py:164-230,      */
 /* networks.py:55-174), float32 like the reference.  Weights: torch layout W1 [512][d_in], W2     */
 /* [d_out][512] in the flat parameter buffer, plus k-major copies W1T [d_in][512], W2T            */
-/* [512][d_out] (mz_learner_transpose) for the forward.  d_in <= 128, d_out <= 64.                */
+/* [512][d_out] (mz_learner_transpose) for the forward.  d_in <= 1024, d_out <= 64; dX only for   */
+/* d_in <= 128.  A head wider than 128 inputs is the representation head (networks.py:55-68) on   */
+/* a wide observation, whose input needs no gradient: its X goes through the kernels' input tile  */
+/* in slices of 128 features.                                                                     */
 /* ------------------------------------------------------------------------------------------- */
 /* Y[r][0:d_out] = W2 relu(W1 X[r][0:d_in] + b1) + b2 -- one head (networks.py:55-119) over `rows` rows. */
 int mz_mlp2_forward(int32_t rows, int32_t d_in, int32_t ldx, const float* X, const float* W1T, const float* b1,
                     const float* W2T, const float* b2, int32_t d_out, float* Y, int32_t ldy, void* stream);
-/* Backward of the same head: dX[r][0:d_in] += ... (NULL: not needed), gW1 / gb1 / gW2 / gb2 += (atomics, torch
- * layouts); the 512-wide activation is recomputed from X. */
+/* Backward of the same head: dX[r][0:d_in] += ... (NULL: not needed; must be NULL for d_in > 128), gW1 / gb1 / gW2 /
+ * gb2 += (atomics, torch layouts); the 512-wide activation is recomputed from X. */
 int mz_mlp2_backward(int32_t rows, int32_t d_in, int32_t ldx, const float* X, const float* W1T, const float* b1,
                      const float* W1, const float* W2, int32_t d_out, const float* dY, int32_t ldy, float* dX,
                      int32_t lddx, float* gW1, float* gb1, float* gW2, float* gb2, void* stream);
@@ -673,7 +676,9 @@ int64_t mz_learner_packed_words(int32_t n, int32_t k);
  * clears n 32-bit words at dst instead (the gradient buffers a step accumulates into), so one launch prepares the step. */
 int mz_learner_pack(int32_t njobs, const mz_pack_job* jobs, void* stream);
 
-/* One head Linear(d_in, 512) -> ReLU -> Linear(512, d_out) (networks.py:55-119); d_in <= 128, d_out <= 64.
+/* One head Linear(d_in, 512) -> ReLU -> Linear(512, d_out) (networks.py:55-119); d_in <= 1024, d_out <= 64.
+ * d_in > 128 is the representation head (networks.py:55-68) on a wide observation: layer 1 and gw1 run over slices
+ * of 128 input features, and there is no dX (w1tp may be NULL).
  * Packed images of W1 [512][d_in] and W2 [d_out][512] (torch layouts):
  *   w1p  (N = 512, K = d_in;  src W1, stride_n d_in, stride_k 1)    layer 1
  *   w2p  (N = d_out, K = 512; src W2, stride_n 512, stride_k 1)     layer 2
@@ -687,7 +692,8 @@ typedef struct mz_tc_head {
   int32_t d_in, d_out;
 } mz_tc_head;
 /* One head over `rows` rows.  Forward: y[r][0:d_out] = head(x[r][0:d_in]).  Backward: dy in, parameter gradients
- * accumulated, dx[r][0:d_in] += (atomics: several heads may share the rows; NULL = not needed). */
+ * accumulated, dx[r][0:d_in] += (atomics: several heads may share the rows; NULL = not needed; a job with
+ * head.d_in > 128 must pass NULL, else MZ_ERR_BAD_ARG). */
 typedef struct mz_tc_job {
   mz_tc_head head;
   int32_t rows, ldx, ldy, lddx;
@@ -700,7 +706,8 @@ typedef struct mz_tc_job {
 int mz_heads_forward_tc(int32_t njobs, const mz_tc_job* jobs, void* stream);
 int mz_heads_backward_tc(int32_t njobs, const mz_tc_job* jobs, void* stream);
 
-/* The recurrent part: step 0 = `first` (representation) on x0, steps 1..steps-1 = `next` (dynamics) on the row
+/* The recurrent part: step 0 = `first` (representation, d_in <= 1024; x0 rows of ldx0 floats) on x0, steps
+ * 1..steps-1 = `next` (dynamics, d_in = d + num_actions <= 128) on the row
  * [hidden | one_hot(action)] the step before produced.  Per step s: yall[s] = head output (pre-LayerNorm),
  * mean / rstd[s], xs[s][r] = [relu(LN(yall[s][r])) (d values) | one_hot(actions[r * action_stride + s]) for
  * s < action_steps, zeros after]; relu_mask (NULL in inference): the sign bits of the dynamics heads' 512-wide

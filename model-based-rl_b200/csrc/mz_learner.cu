@@ -30,7 +30,8 @@ constexpr int LW = 512;   // hidden width of every head (networks.py:55-119)
 constexpr int LR = 32;    // rows per CTA
 constexpr int LT = 256;   // threads per CTA
 constexpr int LDH = 36;   // floats per row of the transposed [feature][row] tiles: 32 rows + 4 (bank spread)
-constexpr int LMAXIN = 128, LMAXOUT = 64;
+constexpr int LMAXIN = 128, LMAXOUT = 64;  // widest input tile (features per slice of X), widest output
+constexpr int LMAXD = 1024;                // widest head input: the representation head's slices of LMAXIN features
 
 // X tile -> shared memory, transposed: Xs[k * LDH + r] = X[(row0 + r) * ldx + k], zeros behind the last row
 MZ_DEV void load_tile_T(float* Xs, const float* __restrict__ X, int ldx, int row0, int rows, int d) {
@@ -41,27 +42,40 @@ MZ_DEV void load_tile_T(float* Xs, const float* __restrict__ X, int ldx, int row
 }
 
 // H = relu(W1 X + b1) for the tile: thread t owns hidden units t and t + 256, 32 rows each, and leaves them in
-// Hs[j * LDH + r]
-MZ_DEV void hidden_layer(const float* Xs, float* Hs, const float* __restrict__ W1T, const float* __restrict__ b1, int d_in) {
+// Hs[j * LDH + r].  Narrow (d_in <= LMAXIN): X is already in Xs.  WIDE: X goes through Xs in slices of LMAXIN
+// features, the accumulators kept across slices (the same sums in the same order as one pass); Xs holds the last
+// slice on return.
+template <bool WIDE>
+MZ_DEV void hidden_layer(float* Xs, float* Hs, const float* __restrict__ X, int ldx, int row0, int rows,
+                         const float* __restrict__ W1T, const float* __restrict__ b1, int d_in) {
   const int j0 = threadIdx.x, j1 = threadIdx.x + LT;
   float a0[LR], a1[LR];
 #pragma unroll
   for (int r = 0; r < LR; ++r) a0[r] = a1[r] = 0.0f;
-  for (int k = 0; k < d_in; ++k) {
-    const float w0 = __ldg(W1T + (size_t)k * LW + j0), w1 = __ldg(W1T + (size_t)k * LW + j1);
-    const float4* xr = reinterpret_cast<const float4*>(Xs + k * LDH);
-#pragma unroll
-    for (int q = 0; q < LR / 4; ++q) {
-      const float4 x = xr[q];
-      a0[4 * q + 0] = fmaf(w0, x.x, a0[4 * q + 0]);
-      a0[4 * q + 1] = fmaf(w0, x.y, a0[4 * q + 1]);
-      a0[4 * q + 2] = fmaf(w0, x.z, a0[4 * q + 2]);
-      a0[4 * q + 3] = fmaf(w0, x.w, a0[4 * q + 3]);
-      a1[4 * q + 0] = fmaf(w1, x.x, a1[4 * q + 0]);
-      a1[4 * q + 1] = fmaf(w1, x.y, a1[4 * q + 1]);
-      a1[4 * q + 2] = fmaf(w1, x.z, a1[4 * q + 2]);
-      a1[4 * q + 3] = fmaf(w1, x.w, a1[4 * q + 3]);
+  for (int k0 = 0; k0 < d_in; k0 += LMAXIN) {
+    const int dk = WIDE ? min(LMAXIN, d_in - k0) : d_in;
+    if (WIDE) {
+      if (k0) __syncthreads();  // every thread is done with the slice before
+      load_tile_T(Xs, X + k0, ldx, row0, rows, dk);
+      __syncthreads();
     }
+    for (int k = 0; k < dk; ++k) {
+      const float w0 = __ldg(W1T + (size_t)(k0 + k) * LW + j0), w1 = __ldg(W1T + (size_t)(k0 + k) * LW + j1);
+      const float4* xr = reinterpret_cast<const float4*>(Xs + k * LDH);
+#pragma unroll
+      for (int q = 0; q < LR / 4; ++q) {
+        const float4 x = xr[q];
+        a0[4 * q + 0] = fmaf(w0, x.x, a0[4 * q + 0]);
+        a0[4 * q + 1] = fmaf(w0, x.y, a0[4 * q + 1]);
+        a0[4 * q + 2] = fmaf(w0, x.z, a0[4 * q + 2]);
+        a0[4 * q + 3] = fmaf(w0, x.w, a0[4 * q + 3]);
+        a1[4 * q + 0] = fmaf(w1, x.x, a1[4 * q + 0]);
+        a1[4 * q + 1] = fmaf(w1, x.y, a1[4 * q + 1]);
+        a1[4 * q + 2] = fmaf(w1, x.z, a1[4 * q + 2]);
+        a1[4 * q + 3] = fmaf(w1, x.w, a1[4 * q + 3]);
+      }
+    }
+    if (!WIDE) break;
   }
   const float c0 = __ldg(b1 + j0), c1 = __ldg(b1 + j1);
   float4* h0 = reinterpret_cast<float4*>(Hs + j0 * LDH);
@@ -75,17 +89,20 @@ MZ_DEV void hidden_layer(const float* Xs, float* Hs, const float* __restrict__ W
   }
 }
 
+template <bool WIDE>  // d_in > LMAXIN
 __global__ void __launch_bounds__(LT)
 mlp2_forward_kernel(int rows, int d_in, int ldx, const float* __restrict__ X, const float* __restrict__ W1T,
                     const float* __restrict__ b1, const float* __restrict__ W2T, const float* __restrict__ b2, int d_out,
                     float* __restrict__ Y, int ldy) {
   extern __shared__ __align__(16) float lsm[];
-  float* Xs = lsm;                  // [d_in][LDH]
+  float* Xs = lsm;                  // [LMAXIN][LDH]: a slice of X
   float* Hs = lsm + LMAXIN * LDH;   // [LW][LDH]
   const int row0 = blockIdx.x * LR;
-  load_tile_T(Xs, X, ldx, row0, rows, d_in);
-  __syncthreads();
-  hidden_layer(Xs, Hs, W1T, b1, d_in);
+  if (!WIDE) {
+    load_tile_T(Xs, X, ldx, row0, rows, d_in);
+    __syncthreads();
+  }
+  hidden_layer<WIDE>(Xs, Hs, X, ldx, row0, rows, W1T, b1, d_in);
   __syncthreads();
   // Y = H W2^T + b2: thread (og, rg) owns outputs og, og + 16, og + 32, og + 48 of rows 2 rg, 2 rg + 1
   const int og = threadIdx.x & 15, rg = threadIdx.x >> 4;
@@ -120,22 +137,25 @@ mlp2_forward_kernel(int rows, int d_in, int ldx, const float* __restrict__ X, co
 }
 
 // Backward of the two-layer head over one tile.  W1T / W2T: the k-major copies (recompute); W1 [512][d_in], W2
-// [d_out][512]: torch layout (dH, dX).  dX (nullable): accumulated, columns [0, d_in).  Gradients: atomics.
+// [d_out][512]: torch layout (dH, dX).  dX (nullable, d_in <= LMAXIN): accumulated, columns [0, d_in).  Gradients:
+// atomics.  Shared memory: one LMAXIN-feature slice of X, H, dH, dY -- 171 KB; X wider than a slice (the
+// representation head) goes through the slice tile twice, for the recomputed H and for gW1.
+template <bool WIDE>  // d_in > LMAXIN
 __global__ void __launch_bounds__(LT)
 mlp2_backward_kernel(int rows, int d_in, int ldx, const float* __restrict__ X, const float* __restrict__ W1T,
                      const float* __restrict__ b1, const float* __restrict__ W1, const float* __restrict__ W2, int d_out,
                      const float* __restrict__ dY, int ldy, float* __restrict__ dX, int lddx, float* __restrict__ gW1,
                      float* __restrict__ gb1, float* __restrict__ gW2, float* __restrict__ gb2) {
   extern __shared__ __align__(16) float lsm[];
-  float* Xs = lsm;                              // [d_in][LDH]
+  float* Xs = lsm;                              // [LMAXIN][LDH]: a slice of X
   float* Hs = Xs + LMAXIN * LDH;                // [LW][LDH]   relu(W1 X + b1)
   float* dHs = Hs + LW * LDH;                   // [LW][LDH]
   float* dYs = dHs + LW * LDH;                  // [d_out][LDH]
   const int row0 = blockIdx.x * LR;
-  load_tile_T(Xs, X, ldx, row0, rows, d_in);
+  if (!WIDE) load_tile_T(Xs, X, ldx, row0, rows, d_in);
   load_tile_T(dYs, dY, ldy, row0, rows, d_out);
-  __syncthreads();
-  hidden_layer(Xs, Hs, W1T, b1, d_in);
+  if (!WIDE) __syncthreads();
+  hidden_layer<WIDE>(Xs, Hs, X, ldx, row0, rows, W1T, b1, d_in);
   // thread t: hidden units j0, j1.  One pass over the outputs: dH[r][j] = sum_o dY[r][o] W2[o][j] and
   // gW2[o][j] = sum_r dY[r][o] H[r][j]
   {
@@ -234,28 +254,38 @@ mlp2_backward_kernel(int rows, int d_in, int ldx, const float* __restrict__ X, c
       if (i < nr && row < rows) dX[(size_t)row * lddx + k] += acc[i];
     }
   }
-  if (k < d_in) {  // gW1[j][k] = sum_r dH[r][j] X[r][k], hidden units [g * LW / NG, (g + 1) * LW / NG)
-    float x[LR];
-    const float4* xp = reinterpret_cast<const float4*>(Xs + k * LDH);
-#pragma unroll
-    for (int q = 0; q < LR / 4; ++q) {
-      const float4 v = xp[q];
-      x[4 * q] = v.x; x[4 * q + 1] = v.y; x[4 * q + 2] = v.z; x[4 * q + 3] = v.w;
+  // gW1[j][k] = sum_r dH[r][j] X[r][k], hidden units [g * LW / NG, (g + 1) * LW / NG), per slice of X
+  for (int k0 = 0;; k0 += LMAXIN) {  // d_in >= 1: at least one pass
+    const int dk = WIDE ? min(LMAXIN, d_in - k0) : d_in;
+    if (WIDE) {
+      __syncthreads();
+      load_tile_T(Xs, X + k0, ldx, row0, rows, dk);
+      __syncthreads();
     }
-    const int nj = LW / NG;
-    for (int j = g * nj; j < (g + 1) * nj; ++j) {
-      const float4* dr = reinterpret_cast<const float4*>(dHs + j * LDH);
-      float s = 0.0f;
+    if (k < dk) {
+      float x[LR];
+      const float4* xp = reinterpret_cast<const float4*>(Xs + k * LDH);
 #pragma unroll
       for (int q = 0; q < LR / 4; ++q) {
-        const float4 v = dr[q];
-        s = fmaf(x[4 * q + 0], v.x, s);
-        s = fmaf(x[4 * q + 1], v.y, s);
-        s = fmaf(x[4 * q + 2], v.z, s);
-        s = fmaf(x[4 * q + 3], v.w, s);
+        const float4 v = xp[q];
+        x[4 * q] = v.x; x[4 * q + 1] = v.y; x[4 * q + 2] = v.z; x[4 * q + 3] = v.w;
       }
-      atomicAdd(gW1 + (size_t)j * d_in + k, s);
+      const int nj = LW / NG;
+      for (int j = g * nj; j < (g + 1) * nj; ++j) {
+        const float4* dr = reinterpret_cast<const float4*>(dHs + j * LDH);
+        float s = 0.0f;
+#pragma unroll
+        for (int q = 0; q < LR / 4; ++q) {
+          const float4 v = dr[q];
+          s = fmaf(x[4 * q + 0], v.x, s);
+          s = fmaf(x[4 * q + 1], v.y, s);
+          s = fmaf(x[4 * q + 2], v.z, s);
+          s = fmaf(x[4 * q + 3], v.w, s);
+        }
+        atomicAdd(gW1 + (size_t)j * d_in + k0 + k, s);
+      }
     }
+    if (!WIDE || k0 + LMAXIN >= d_in) break;
   }
 }
 
@@ -394,12 +424,14 @@ __global__ void counter_inc_kernel(float* state) { state[0] += 1.0f; }
 bool g_learner_attr = false;
 int learner_attrs() {
   if (g_learner_attr) return 0;
-  cudaError_t e = cudaFuncSetAttribute(mlp2_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)((LMAXIN + LW) * LDH * sizeof(float)));
-  if (e != cudaSuccess) return (int)e;
-  e = cudaFuncSetAttribute(mlp2_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (int)((LMAXIN + 2 * LW + LMAXOUT) * LDH * sizeof(float)));
-  if (e != cudaSuccess) return (int)e;
+  const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
+  const int fwd = (int)((LMAXIN + LW) * LDH * sizeof(float)), bwd = (int)((LMAXIN + 2 * LW + LMAXOUT) * LDH * sizeof(float));
+  cudaError_t e;
+  if ((e = cudaFuncSetAttribute(mlp2_forward_kernel<false>, attr, fwd)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mlp2_forward_kernel<true>, attr, fwd)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mlp2_backward_kernel<false>, attr, bwd)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(mlp2_backward_kernel<true>, attr, bwd)) != cudaSuccess)
+    return (int)e;
   g_learner_attr = true;
   return 0;
 }
@@ -410,12 +442,17 @@ extern "C" {
 
 int mz_mlp2_forward(int32_t rows, int32_t d_in, int32_t ldx, const float* X, const float* W1T, const float* b1,
                     const float* W2T, const float* b2, int32_t d_out, float* Y, int32_t ldy, void* stream) {
-  if (rows < 1 || d_in < 1 || d_in > LMAXIN || d_out < 1 || d_out > LMAXOUT || ldx < d_in || ldy < d_out || !X || !W1T ||
+  if (rows < 1 || d_in < 1 || d_in > LMAXD || d_out < 1 || d_out > LMAXOUT || ldx < d_in || ldy < d_out || !X || !W1T ||
       !b1 || !W2T || !b2 || !Y)
     return MZ_ERR_BAD_ARG;
   if (int rc = learner_attrs()) return rc;
-  mlp2_forward_kernel<<<(rows + LR - 1) / LR, LT, (LMAXIN + LW) * LDH * sizeof(float), (cudaStream_t)stream>>>(
-      rows, d_in, ldx, X, W1T, b1, W2T, b2, d_out, Y, ldy);
+  const size_t smem = (LMAXIN + LW) * LDH * sizeof(float);
+  if (d_in > LMAXIN)
+    mlp2_forward_kernel<true><<<(rows + LR - 1) / LR, LT, smem, (cudaStream_t)stream>>>(rows, d_in, ldx, X, W1T, b1, W2T, b2,
+                                                                                      d_out, Y, ldy);
+  else
+    mlp2_forward_kernel<false><<<(rows + LR - 1) / LR, LT, smem, (cudaStream_t)stream>>>(rows, d_in, ldx, X, W1T, b1, W2T, b2,
+                                                                                       d_out, Y, ldy);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }
@@ -423,13 +460,17 @@ int mz_mlp2_forward(int32_t rows, int32_t d_in, int32_t ldx, const float* X, con
 int mz_mlp2_backward(int32_t rows, int32_t d_in, int32_t ldx, const float* X, const float* W1T, const float* b1,
                      const float* W1, const float* W2, int32_t d_out, const float* dY, int32_t ldy, float* dX,
                      int32_t lddx, float* gW1, float* gb1, float* gW2, float* gb2, void* stream) {
-  if (rows < 1 || d_in < 1 || d_in > LMAXIN || d_out < 1 || d_out > LMAXOUT || ldx < d_in || ldy < d_out || !X || !W1T ||
-      !b1 || !W1 || !W2 || !dY || !gW1 || !gb1 || !gW2 || !gb2 || (dX && lddx < d_in))
+  if (rows < 1 || d_in < 1 || d_in > LMAXD || d_out < 1 || d_out > LMAXOUT || ldx < d_in || ldy < d_out || !X || !W1T ||
+      !b1 || !W1 || !W2 || !dY || !gW1 || !gb1 || !gW2 || !gb2 || (dX && (lddx < d_in || d_in > LMAXIN)))
     return MZ_ERR_BAD_ARG;
   if (int rc = learner_attrs()) return rc;
-  mlp2_backward_kernel<<<(rows + LR - 1) / LR, LT, (LMAXIN + 2 * LW + LMAXOUT) * LDH * sizeof(float),
-                         (cudaStream_t)stream>>>(rows, d_in, ldx, X, W1T, b1, W1, W2, d_out, dY, ldy, dX, lddx, gW1, gb1,
-                                                 gW2, gb2);
+  const size_t smem = (LMAXIN + 2 * LW + LMAXOUT) * LDH * sizeof(float);
+  if (d_in > LMAXIN)
+    mlp2_backward_kernel<true><<<(rows + LR - 1) / LR, LT, smem, (cudaStream_t)stream>>>(
+        rows, d_in, ldx, X, W1T, b1, W1, W2, d_out, dY, ldy, dX, lddx, gW1, gb1, gW2, gb2);
+  else
+    mlp2_backward_kernel<false><<<(rows + LR - 1) / LR, LT, smem, (cudaStream_t)stream>>>(
+        rows, d_in, ldx, X, W1T, b1, W1, W2, d_out, dY, ldy, dX, lddx, gW1, gb1, gW2, gb2);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }

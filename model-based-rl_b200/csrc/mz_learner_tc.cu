@@ -35,6 +35,8 @@ constexpr int NTH = 32 * NW;       // threads per CTA
 constexpr int CW = LW / NW;        // hidden units per warp: warp w owns [CW w, CW w + CW)
 constexpr int NTW = CW / 8;        // n-tiles per warp
 constexpr int XLD = 136;   // bf16 per row of the input tile (<= 128 features; 272 B: ldmatrix rows 16 B apart mod 128)
+constexpr int SLICE = 128;  // features per pass through the input tile: a wider head's input is staged in K slices
+constexpr int MAXIN = 1024; // widest head input (the representation head on a wide observation; no dX above SLICE)
 constexpr int HLD = 520;   // bf16 per row of the activation tiles
 constexpr int DYLD = 72;   // bf16 per row of the output-gradient tile (<= 64 outputs)
 constexpr int FLD = 68;    // floats per row of the float32 tile (layer-2 output / dX of the dynamics head)
@@ -113,20 +115,21 @@ __global__ void pack_kernel(PackParams p) {
   }
 }
 
-// acc[MT][NTW][4] += A (16 MT rows x 32 KQ, row-major bf16 in shared memory) * B (packed; n-tiles nt0 .. nt0 + NTW - 1)
+// acc[MT][NTW][4] += A (16 MT rows x 32 KQ, row-major bf16 in shared memory) * B (packed; n-tiles nt0 .. nt0 + NTW - 1).
+// ldq: k-step pairs per n-tile of the packed image (KQ, or more when Bp points at a K slice of a wider image).
 template <int MT>
 MZ_DEV void gemm_wide(float (&acc)[MT][NTW][4], const __nv_bfloat16* As, int lda, const uint32_t* __restrict__ Bp, int KQ,
-                      int nt0, int lane) {
+                      int nt0, int lane, int ldq) {
   const int arow = (lane & 7) + ((lane >> 3) & 1) * 8, acol = (lane >> 4) * 8;
-  const uint4* bp = reinterpret_cast<const uint4*>(Bp) + (size_t)nt0 * KQ * 32 + lane;
+  const uint4* bp = reinterpret_cast<const uint4*>(Bp) + (size_t)nt0 * ldq * 32 + lane;
   uint4 b[NTW];
 #pragma unroll
-  for (int n = 0; n < NTW; ++n) b[n] = __ldg(bp + (size_t)n * KQ * 32);
+  for (int n = 0; n < NTW; ++n) b[n] = __ldg(bp + (size_t)n * ldq * 32);
   for (int kq = 0; kq < KQ; ++kq) {
     uint4 bn[NTW];
     if (kq + 1 < KQ) {
 #pragma unroll
-      for (int n = 0; n < NTW; ++n) bn[n] = __ldg(bp + ((size_t)n * KQ + kq + 1) * 32);
+      for (int n = 0; n < NTW; ++n) bn[n] = __ldg(bp + ((size_t)n * ldq + kq + 1) * 32);
     }
     uint32_t a[2][MT][4];
 #pragma unroll
@@ -145,6 +148,11 @@ MZ_DEV void gemm_wide(float (&acc)[MT][NTW][4], const __nv_bfloat16* As, int lda
       for (int n = 0; n < NTW; ++n) b[n] = bn[n];
     }
   }
+}
+template <int MT>
+MZ_DEV void gemm_wide(float (&acc)[MT][NTW][4], const __nv_bfloat16* As, int lda, const uint32_t* __restrict__ Bp, int KQ,
+                      int nt0, int lane) {
+  gemm_wide<MT>(acc, As, lda, Bp, KQ, nt0, lane, KQ);
 }
 
 // acc[MT][4] = A (16 MT rows x 512, row-major bf16 in shared memory) * B (packed, KQ = 16; n-tile nt)
@@ -244,18 +252,10 @@ MZ_DEV void tile_add(float* __restrict__ dst, int ld, int rows_ok, int cols, con
   }
 }
 
-// H = relu(W1 X + b1) for the warp's CW hidden units -> Hs (bf16); returns the sign bits (bit 4 n + c of mask[mt])
+// H = relu(acc + b1) for the warp's CW hidden units -> Hs (bf16); returns the sign bits (bit 4 n + c of mask[mt])
 template <int MT>
-MZ_DEV void hidden_phase(const mz_tc_head& h, const __nv_bfloat16* Xs, __nv_bfloat16* Hs, uint32_t (&mask)[MT], int warp,
-                         int lane) {
-  float acc[MT][NTW][4];
-#pragma unroll
-  for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-    for (int n = 0; n < NTW; ++n)
-#pragma unroll
-      for (int c = 0; c < 4; ++c) acc[mt][n][c] = 0.0f;
-  gemm_wide(acc, Xs, XLD, h.w1p, round_up32(h.d_in) >> 5, NTW * warp, lane);
+MZ_DEV void hidden_epilogue(const mz_tc_head& h, const float (&acc)[MT][NTW][4], __nv_bfloat16* Hs, uint32_t (&mask)[MT],
+                            int warp, int lane) {
   const int g = lane >> 2, t = lane & 3;
 #pragma unroll
   for (int mt = 0; mt < MT; ++mt) mask[mt] = 0u;
@@ -273,6 +273,47 @@ MZ_DEV void hidden_phase(const mz_tc_head& h, const __nv_bfloat16* Xs, __nv_bflo
       *reinterpret_cast<uint32_t*>(Hs + (16 * mt + g + 8) * HLD + j) = pack2(v2, v3);
     }
   }
+}
+
+// H = relu(W1 X + b1) for the warp's CW hidden units, X in Xs (d_in <= SLICE)
+template <int MT>
+MZ_DEV void hidden_phase(const mz_tc_head& h, const __nv_bfloat16* Xs, __nv_bfloat16* Hs, uint32_t (&mask)[MT], int warp,
+                         int lane) {
+  float acc[MT][NTW][4];
+#pragma unroll
+  for (int mt = 0; mt < MT; ++mt)
+#pragma unroll
+    for (int n = 0; n < NTW; ++n)
+#pragma unroll
+      for (int c = 0; c < 4; ++c) acc[mt][n][c] = 0.0f;
+  gemm_wide(acc, Xs, XLD, h.w1p, round_up32(h.d_in) >> 5, NTW * warp, lane);
+  hidden_epilogue<MT>(h, acc, Hs, mask, warp, lane);
+}
+
+// The same for any d_in <= MAXIN, X read from global memory (rows row0 .. row0 + 16 MT of `rows`): layer 1 runs over
+// K slices of up to SLICE features, each staged through Xs (16 MT x XLD) by the whole CTA, with the accumulators kept
+// across slices -- the k-steps in the order of one pass, so the same sums.  Xs holds the last slice on return.  Every
+// thread of the CTA calls it (barriers inside).
+template <int MT>
+MZ_DEV void hidden_phase_sliced(const mz_tc_head& h, const float* __restrict__ X, int ldx, int row0, int rows,
+                                __nv_bfloat16* Xs, __nv_bfloat16* Hs, uint32_t (&mask)[MT], int warp, int lane) {
+  float acc[MT][NTW][4];
+#pragma unroll
+  for (int mt = 0; mt < MT; ++mt)
+#pragma unroll
+    for (int n = 0; n < NTW; ++n)
+#pragma unroll
+      for (int c = 0; c < 4; ++c) acc[mt][n][c] = 0.0f;
+  const int KQ = round_up32(h.d_in) >> 5;
+  for (int k0 = 0; k0 < h.d_in; k0 += SLICE) {
+    const int w = min(SLICE, h.d_in - k0);
+    if (k0) __syncthreads();  // every warp is done with the slice before
+    load_rows<16 * MT>(Xs, XLD, X + k0, ldx, row0, rows, w, round_up32(w));
+    __syncthreads();
+    // k-step pair k0 / 32 of every n-tile: 128 words per pair
+    gemm_wide<MT>(acc, Xs, XLD, h.w1p + (size_t)k0 * 4, round_up32(w) >> 5, NTW * warp, lane, KQ);
+  }
+  hidden_epilogue<MT>(h, acc, Hs, mask, warp, lane);
 }
 
 // Y = H W2^T + b2: warp w < ceil(d_out / 8) owns outputs [8 w, 8 w + 8).  To global memory (Y != nullptr) or to the
@@ -303,13 +344,49 @@ MZ_DEV void output_phase(const mz_tc_head& h, const __nv_bfloat16* Hs, float* __
   }
 }
 
+// gW1[j][k] += sum_r dH[r][j] X[r][k] for columns [0, cols) of the X tiles in Xs, to gw1[j * ld + k]: M = the warp's
+// hidden units, N = input features in chunks of 64, K = the CTA's rows.  One slice of a WIDE head's input; narrow heads
+// run the same loop inline over all of X (as one function it changes their register allocation).
+template <int TILES>
+MZ_DEV void gw1_phase(float* gw1, int ld, int cols, const __nv_bfloat16* Xs, const __nv_bfloat16* dHs, float* stage,
+                      int warp, int lane) {
+  const int lrow = lane & 7, lsel = lane >> 3;  // ldmatrix.trans: lanes 8 i .. 8 i + 7 address matrix i
+  for (int mt = 0; mt < CW / 16; ++mt) {
+    for (int chunk = 0; 64 * chunk < cols; ++chunk) {
+      float acc[8][4];
+#pragma unroll
+      for (int n = 0; n < 8; ++n)
+#pragma unroll
+        for (int c = 0; c < 4; ++c) acc[n][c] = 0.0f;
+#pragma unroll
+      for (int ks = 0; ks < 2 * TILES; ++ks) {
+        uint32_t a[4];
+        ldsm4t(a, dHs + (16 * ks + lrow + (lsel >> 1) * 8) * HLD + CW * warp + 16 * mt + (lsel & 1) * 8);
+#pragma unroll
+        for (int np = 0; np < 4; ++np) {
+          if (64 * chunk + 16 * np < cols) {  // warp-uniform; the tile is zero padded to a multiple of 32 columns
+            uint32_t b[4];
+            ldsm4t(b, Xs + (16 * ks + lrow + (lsel & 1) * 8) * XLD + 64 * chunk + 16 * np + (lsel >> 1) * 8);
+            mma16816(acc[2 * np], a, b[0], b[1]);
+            mma16816(acc[2 * np + 1], a, b[2], b[3]);
+          }
+        }
+      }
+      tile_add<8>(gw1 + (size_t)(CW * warp + 16 * mt) * ld + 64 * chunk, ld, 16, min(64, cols - 64 * chunk), acc, stage, lane);
+    }
+  }
+}
+
 // Backward of one head over the CTA's TILES tiles of 32 rows.  In: Xs (input rows, bf16), dYs (output gradient, bf16,
 // zero padded to a multiple of 32 columns).  Out: the four parameter gradients (vector reductions: one per weight and
 // CTA, so two tiles per CTA halve that traffic), and dX (columns [0, dx_cols)) accumulated into global memory.
-template <int TILES>
-MZ_DEV void backward_tiles(const mz_tc_head& h, const __nv_bfloat16* Xs, const __nv_bfloat16* dYs, __nv_bfloat16* Hs,
-                           __nv_bfloat16* dHs, float* __restrict__ dX, int lddx, int dx_cols, int row0, int rows,
-                           float* stage, int warp, int lane) {
+// WIDE (heads up to MAXIN inputs, no dX above SLICE): Xs is not loaded by the caller; the recomputed activation and gW1
+// each stream X (rows of `ldx` floats) through Xs in slices of SLICE features, so the shared-memory plan is that of a
+// narrow head (heads_bwd_smem).
+template <int TILES, bool WIDE>
+MZ_DEV void backward_tiles(const mz_tc_head& h, const float* __restrict__ X, int ldx, __nv_bfloat16* Xs,
+                           const __nv_bfloat16* dYs, __nv_bfloat16* Hs, __nv_bfloat16* dHs, float* __restrict__ dX, int lddx,
+                           int dx_cols, int row0, int rows, float* stage, int warp, int lane) {
   const int g = lane >> 2, t = lane & 3;
   TC_T(1, 0, 1);
   float s0[NTW], s1[NTW];  // column sums of the gated dH: gb1
@@ -322,7 +399,10 @@ MZ_DEV void backward_tiles(const mz_tc_head& h, const __nv_bfloat16* Xs, const _
     __nv_bfloat16* Ht = Hs + tile * RT * HLD;
     __nv_bfloat16* dHt = dHs + tile * RT * HLD;
     uint32_t mask[2];
-    hidden_phase<2>(h, Xt, Ht, mask, warp, lane);
+    if (WIDE)
+      hidden_phase_sliced<2>(h, X, ldx, row0 + RT * tile, rows, Xs + tile * RT * XLD, Ht, mask, warp, lane);
+    else
+      hidden_phase<2>(h, Xt, Ht, mask, warp, lane);
     // dH = dY W2 for the warp's hidden units, masked by the ReLU -> dHs
     float acc[2][NTW][4];
 #pragma unroll
@@ -408,6 +488,7 @@ MZ_DEV void backward_tiles(const mz_tc_head& h, const __nv_bfloat16* Xs, const _
     tile_add<NTW>(h.gw2 + (size_t)(16 * mt) * LW + CW * warp, LW, h.d_out - 16 * mt, CW, acc, stage, lane);
   }
   TC_T(1, 0, 5);
+  if (!WIDE) {
   // gW1[j][k] = sum_r dH[r][j] X[r][k]: M = the warp's hidden units, N = input features in chunks of 64, K = rows
   for (int mt = 0; mt < CW / 16; ++mt) {
     for (int chunk = 0; 64 * chunk < h.d_in; ++chunk) {
@@ -434,6 +515,19 @@ MZ_DEV void backward_tiles(const mz_tc_head& h, const __nv_bfloat16* Xs, const _
                   stage, lane);
     }
   }
+  } else {
+    for (int k0 = 0; k0 < h.d_in; k0 += SLICE) {
+      const int w = min(SLICE, h.d_in - k0);
+      if (h.d_in > SLICE) {  // one slice: still in Xs from the hidden phase
+        __syncthreads();
+#pragma unroll
+        for (int tile = 0; tile < TILES; ++tile)
+          load_rows(Xs + tile * RT * XLD, XLD, X + k0, ldx, row0 + RT * tile, rows, w, round_up32(w));
+        __syncthreads();
+      }
+      gw1_phase<TILES>(h.gw1 + k0, h.d_in, w, Xs, dHs, stage, warp, lane);
+    }
+  }
   TC_T(1, 0, 6);
 }
 
@@ -454,6 +548,8 @@ MZ_DEV Tiles carve(unsigned char* base) {  // the forward kernels' tiles
 }
 
 // ---- the output heads: one job per blockIdx.y --------------------------------------------------------------------
+// WIDE: some job has d_in > SLICE; every job's layer 1 then runs over slices (hidden_phase_sliced)
+template <bool WIDE>
 __global__ void __launch_bounds__(NTH) heads_fwd_kernel(PlainParams p) {
   extern __shared__ __align__(16) unsigned char tc_smem[];
   const mz_tc_job& job = p.jobs[blockIdx.y];
@@ -461,15 +557,23 @@ __global__ void __launch_bounds__(NTH) heads_fwd_kernel(PlainParams p) {
   if (row0 >= job.rows) return;
   const Tiles s = carve(tc_smem);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  load_rows(s.Xs, XLD, job.x, job.ldx, row0, job.rows, job.head.d_in, round_up32(job.head.d_in));
-  __syncthreads();
   uint32_t mask[2];
-  hidden_phase<2>(job.head, s.Xs, s.Hs, mask, warp, lane);
+  if (WIDE) {
+    hidden_phase_sliced<2>(job.head, job.x, job.ldx, row0, job.rows, s.Xs, s.Hs, mask, warp, lane);
+  } else {
+    load_rows(s.Xs, XLD, job.x, job.ldx, row0, job.rows, job.head.d_in, round_up32(job.head.d_in));
+    __syncthreads();
+    hidden_phase<2>(job.head, s.Xs, s.Hs, mask, warp, lane);
+  }
   __syncthreads();
   output_phase(job.head, s.Hs, job.y, job.ldy, row0, job.rows, nullptr, warp, lane);
 }
 
-template <int TILES>
+// Shared memory: TILES x 32 rows of X (XLD), H and dH (HLD), dY (DYLD) in bf16, plus NW staging areas -- 112 KB at
+// TILES = 1, 190 KB at TILES = 2 of the 227 KB.  Full-width X tiles of a 1024-feature head (64.5 KB per 32 rows instead
+// of 8.5 KB) would not fit at TILES = 2, so WIDE streams X through the same XLD tiles in slices of SLICE features
+// (backward_tiles): the same plan, the same heads_bwd_smem, for every width.
+template <int TILES, bool WIDE>
 __global__ void __launch_bounds__(NTH) heads_bwd_kernel(PlainParams p) {
   extern __shared__ __align__(16) unsigned char tc_smem[];
   const mz_tc_job& job = p.jobs[blockIdx.y];
@@ -486,7 +590,7 @@ __global__ void __launch_bounds__(NTH) heads_bwd_kernel(PlainParams p) {
   TC_T(1, 0, 0);
 #pragma unroll
   for (int tile = 0; tile < TILES; ++tile) {
-    load_rows(Xs + tile * RT * XLD, XLD, job.x, job.ldx, row0 + RT * tile, job.rows, h.d_in, round_up32(h.d_in));
+    if (!WIDE) load_rows(Xs + tile * RT * XLD, XLD, job.x, job.ldx, row0 + RT * tile, job.rows, h.d_in, round_up32(h.d_in));
     load_rows(dYs + tile * RT * DYLD, DYLD, job.dy, job.ldy, row0 + RT * tile, job.rows, h.d_out, round_up32(h.d_out));
   }
   if ((int)threadIdx.x < h.d_out) {  // gb2[o] = sum_r dY[r][o]
@@ -497,8 +601,8 @@ __global__ void __launch_bounds__(NTH) heads_bwd_kernel(PlainParams p) {
     atomicAdd(h.gb2 + threadIdx.x, (part[0] + part[1]) + (part[2] + part[3]));
   }
   __syncthreads();
-  backward_tiles<TILES>(h, Xs, dYs, Hs, dHs, job.dx, job.lddx, job.dx != nullptr ? h.d_in : 0, row0, job.rows,
-                        stage + warp * STAGE, warp, lane);
+  backward_tiles<TILES, WIDE>(h, job.x, job.ldx, Xs, dYs, Hs, dHs, job.dx, job.lddx, job.dx != nullptr ? h.d_in : 0, row0,
+                               job.rows, stage + warp * STAGE, warp, lane);
 }
 constexpr size_t heads_bwd_smem(int tiles) {
   return (size_t)tiles * RT * (XLD + 2 * HLD + DYLD) * 2 + (size_t)NW * STAGE * 4;
@@ -519,7 +623,9 @@ struct ChainGeo {
   static constexpr size_t BWD_SMEM = (size_t)ROWS * DYLD * 2 + (size_t)ROWS * HLD * 2 + (size_t)ROWS * FLD * 4 + 2 * 64 * 4;
 };
 
-template <int MT>
+// WIDE: first.d_in > SLICE -- step 0 streams x0 through Xs in slices (hidden_phase_sliced); the LayerNorm epilogues
+// write the next step's input into Xs as for a narrow first head
+template <int MT, bool WIDE>
 __global__ void __launch_bounds__(NTH) chain_fwd_kernel(mz_tc_chain c) {
   using G = ChainGeo<MT>;
   constexpr int ROWS = G::ROWS, LPR = G::LPR, CPL = G::CPL;
@@ -541,15 +647,20 @@ __global__ void __launch_bounds__(NTH) chain_fwd_kernel(mz_tc_chain c) {
     gam[i] = col < d ? __ldg(c.gamma + col) : 0.0f;
     bet[i] = col < d ? __ldg(c.beta + col) : 0.0f;
   }
-  load_rows<ROWS>(Xs, XLD, c.x0, c.ldx0, row0, c.rows, c.first.d_in, round_up32(c.first.d_in));
-  __syncthreads();
+  if (!WIDE) {
+    load_rows<ROWS>(Xs, XLD, c.x0, c.ldx0, row0, c.rows, c.first.d_in, round_up32(c.first.d_in));
+    __syncthreads();
+  }
   for (int step = 0; step < c.steps; ++step) {
     const mz_tc_head& h = step ? c.next : c.first;
     const int act = (live && c.actions != nullptr && step < c.action_steps)
                         ? __ldg(c.actions + (size_t)row * c.action_stride + step) : -1;  // in flight during the head
     TC_T(0, step, 0);
     uint32_t mask[MT];
-    hidden_phase<MT>(h, Xs, Hs, mask, warp, lane);
+    if (WIDE && step == 0)
+      hidden_phase_sliced<MT>(h, c.x0, c.ldx0, row0, c.rows, Xs, Hs, mask, warp, lane);
+    else
+      hidden_phase<MT>(h, Xs, Hs, mask, warp, lane);
     TC_T(0, step, 1);
     if (step && c.relu_mask != nullptr)  // the backward chain gates dH with these bits instead of recomputing the layer
       reinterpret_cast<uint2*>(c.relu_mask)[((size_t)step * gridDim.x + blockIdx.x) * NTH + threadIdx.x] =
@@ -773,11 +884,16 @@ int tc_attrs() {
   if (g_tc_attr) return 0;
   cudaError_t e;
   const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-  if ((e = cudaFuncSetAttribute(heads_fwd_kernel, attr, (int)FWD_SMEM)) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(chain_fwd_kernel<1>, attr, (int)ChainGeo<1>::FWD_SMEM)) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(chain_fwd_kernel<2>, attr, (int)ChainGeo<2>::FWD_SMEM)) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(heads_bwd_kernel<1>, attr, (int)heads_bwd_smem(1))) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(heads_bwd_kernel<2>, attr, (int)heads_bwd_smem(2))) != cudaSuccess ||
+  if ((e = cudaFuncSetAttribute(heads_fwd_kernel<false>, attr, (int)FWD_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(heads_fwd_kernel<true>, attr, (int)FWD_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(chain_fwd_kernel<1, false>, attr, (int)ChainGeo<1>::FWD_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(chain_fwd_kernel<2, false>, attr, (int)ChainGeo<2>::FWD_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(chain_fwd_kernel<1, true>, attr, (int)ChainGeo<1>::FWD_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(chain_fwd_kernel<2, true>, attr, (int)ChainGeo<2>::FWD_SMEM)) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(heads_bwd_kernel<1, false>, attr, (int)heads_bwd_smem(1))) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(heads_bwd_kernel<2, false>, attr, (int)heads_bwd_smem(2))) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(heads_bwd_kernel<1, true>, attr, (int)heads_bwd_smem(1))) != cudaSuccess ||
+      (e = cudaFuncSetAttribute(heads_bwd_kernel<2, true>, attr, (int)heads_bwd_smem(2))) != cudaSuccess ||
       (e = cudaFuncSetAttribute(chain_bwd_kernel<1>, attr, (int)ChainGeo<1>::BWD_SMEM)) != cudaSuccess ||
       (e = cudaFuncSetAttribute(chain_bwd_kernel<2>, attr, (int)ChainGeo<2>::BWD_SMEM)) != cudaSuccess)
     return (int)e;
@@ -789,9 +905,10 @@ int tc_attrs() {
 // step must agree: the ReLU bits are stored per CTA and thread)
 int chain_mt(int rows) { return (rows + 15) / 16 <= 148 ? 1 : 2; }
 
+// (w1tp only feeds dX, which a head wider than SLICE does not have: its image need not exist)
 bool head_ok(const mz_tc_head& h, bool backward) {
-  if (h.d_in < 1 || h.d_in > 128 || h.d_out < 1 || h.d_out > 64 || !h.w1p || !h.w2p || !h.b1 || !h.b2) return false;
-  if (backward && (!h.w2tp || !h.w1tp || !h.gw1 || !h.gb1 || !h.gw2 || !h.gb2)) return false;
+  if (h.d_in < 1 || h.d_in > MAXIN || h.d_out < 1 || h.d_out > 64 || !h.w1p || !h.w2p || !h.b1 || !h.b2) return false;
+  if (backward && (!h.w2tp || (h.d_in <= SLICE && !h.w1tp) || !h.gw1 || !h.gb1 || !h.gw2 || !h.gb2)) return false;
   if (backward && (((uintptr_t)h.gw1 | (uintptr_t)h.gw2) & 15)) return false;  // weight gradients leave as red.v4
   return true;
 }
@@ -851,14 +968,20 @@ int mz_heads_forward_tc(int32_t njobs, const mz_tc_job* jobs, void* stream) {
   if (njobs < 1 || njobs > MAXJOBS || !jobs) return MZ_ERR_BAD_ARG;
   PlainParams p;
   int most = 0;
+  bool wide = false;
   for (int i = 0; i < njobs; ++i) {
     const mz_tc_job& j = jobs[i];
     if (!head_ok(j.head, false) || j.rows < 1 || !j.x || !j.y || j.ldx < j.head.d_in || j.ldy < j.head.d_out) return MZ_ERR_BAD_ARG;
     p.jobs[i] = j;
     most = j.rows > most ? j.rows : most;
+    wide = wide || j.head.d_in > SLICE;
   }
   if (int rc = tc_attrs()) return rc;
-  heads_fwd_kernel<<<dim3((most + RT - 1) / RT, njobs), NTH, FWD_SMEM, (cudaStream_t)stream>>>(p);
+  const dim3 grid((most + RT - 1) / RT, njobs);
+  if (wide)
+    heads_fwd_kernel<true><<<grid, NTH, FWD_SMEM, (cudaStream_t)stream>>>(p);
+  else
+    heads_fwd_kernel<false><<<grid, NTH, FWD_SMEM, (cudaStream_t)stream>>>(p);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }
@@ -867,22 +990,30 @@ int mz_heads_backward_tc(int32_t njobs, const mz_tc_job* jobs, void* stream) {
   if (njobs < 1 || njobs > MAXJOBS || !jobs) return MZ_ERR_BAD_ARG;
   PlainParams p;
   int most = 0;
+  bool wide = false;
   for (int i = 0; i < njobs; ++i) {
     const mz_tc_job& j = jobs[i];
     if (!head_ok(j.head, true) || j.rows < 1 || !j.x || !j.dy || j.ldx < j.head.d_in || j.ldy < j.head.d_out ||
-        (j.dx && j.lddx < j.head.d_in))
+        (j.dx && (j.lddx < j.head.d_in || j.head.d_in > SLICE)))
       return MZ_ERR_BAD_ARG;
     p.jobs[i] = j;
     most = j.rows > most ? j.rows : most;
+    wide = wide || j.head.d_in > SLICE;
   }
   if (int rc = tc_attrs()) return rc;
   // more CTAs than one wave of single-tile CTAs: two tiles per CTA (half the weight-gradient reductions, one wave)
   int ctas = 0;
   for (int i = 0; i < njobs; ++i) ctas += (jobs[i].rows + RT - 1) / RT;
-  if (ctas > 148)
-    heads_bwd_kernel<2><<<dim3((most + 2 * RT - 1) / (2 * RT), njobs), NTH, heads_bwd_smem(2), (cudaStream_t)stream>>>(p);
+  const dim3 grid2((most + 2 * RT - 1) / (2 * RT), njobs), grid1((most + RT - 1) / RT, njobs);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (ctas > 148 && wide)
+    heads_bwd_kernel<2, true><<<grid2, NTH, heads_bwd_smem(2), st>>>(p);
+  else if (ctas > 148)
+    heads_bwd_kernel<2, false><<<grid2, NTH, heads_bwd_smem(2), st>>>(p);
+  else if (wide)
+    heads_bwd_kernel<1, true><<<grid1, NTH, heads_bwd_smem(1), st>>>(p);
   else
-    heads_bwd_kernel<1><<<dim3((most + RT - 1) / RT, njobs), NTH, heads_bwd_smem(1), (cudaStream_t)stream>>>(p);
+    heads_bwd_kernel<1, false><<<grid1, NTH, heads_bwd_smem(1), st>>>(p);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }
@@ -890,10 +1021,16 @@ int mz_heads_backward_tc(int32_t njobs, const mz_tc_job* jobs, void* stream) {
 int mz_chain_forward_tc(const mz_tc_chain* chain, void* stream) {
   if (!chain_ok(chain, false)) return MZ_ERR_BAD_ARG;
   if (int rc = tc_attrs()) return rc;
-  if (chain_mt(chain->rows) == 1)
-    chain_fwd_kernel<1><<<(chain->rows + 15) / 16, NTH, ChainGeo<1>::FWD_SMEM, (cudaStream_t)stream>>>(*chain);
+  const bool wide = chain->first.d_in > SLICE;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (chain_mt(chain->rows) == 1 && wide)
+    chain_fwd_kernel<1, true><<<(chain->rows + 15) / 16, NTH, ChainGeo<1>::FWD_SMEM, st>>>(*chain);
+  else if (chain_mt(chain->rows) == 1)
+    chain_fwd_kernel<1, false><<<(chain->rows + 15) / 16, NTH, ChainGeo<1>::FWD_SMEM, st>>>(*chain);
+  else if (wide)
+    chain_fwd_kernel<2, true><<<(chain->rows + 31) / 32, NTH, ChainGeo<2>::FWD_SMEM, st>>>(*chain);
   else
-    chain_fwd_kernel<2><<<(chain->rows + 31) / 32, NTH, ChainGeo<2>::FWD_SMEM, (cudaStream_t)stream>>>(*chain);
+    chain_fwd_kernel<2, false><<<(chain->rows + 31) / 32, NTH, ChainGeo<2>::FWD_SMEM, st>>>(*chain);
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }

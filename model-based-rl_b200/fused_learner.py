@@ -24,10 +24,11 @@ search kernels' `FCNetwork.load_weights` see the usual tensors.  `FusedLearner(p
     transposes, 2 (K + 1) forward launches, 3 head launches, loss, 3 + 2 (K + 1) backward launches, optimiser.
 
 Both are captured in CUDA graphs.  SGD / RMSprop use the torch optimiser over the flat buffer (elementwise, the
-reference's arithmetic).  `--no_support` networks (one-unit value / reward heads, `config.scalar_loss` MSE or Huber,
-utils.py:61-70) run the same launches with d_out = 1 heads and the scalar loss kernel.  `save_state` writes the
-checkpoint dictionary of learners.py:72-83; `load_state` / `FusedLearner(state=...)` resume from it (weights, optimiser
-state, training_step, replay throughput), and a graph captured later keeps the restored optimiser state.  With torch.distributed initialised the gradients of the three output heads are all-reduced
+reference's arithmetic).  Observations of up to 1024 features (MAX_INPUT_DIM) train in both precisions: the
+representation head's input goes through the kernels' 128-feature input tiles in slices.  `--no_support` networks
+(one-unit value / reward heads, `config.scalar_loss` MSE or Huber, utils.py:61-70) run the same launches with
+d_out = 1 heads and the scalar loss kernel.  `save_state` writes the checkpoint dictionary of learners.py:72-83;
+`load_state` / `FusedLearner(state=...)` resume from it (weights, optimiser state, training_step, replay throughput), and a graph captured later keeps the restored optimiser state.  With torch.distributed initialised the gradients of the three output heads are all-reduced
 on a side stream while the recurrent part of the backward still runs; the rest follows before the optimiser step.
 """
 import ctypes as C
@@ -41,6 +42,8 @@ from .networks import HIDDEN
 
 WIDTH = _lib.FC_WIDTH
 MAX_SUPPORT_BINS = 64  # widest value / reward head: LMAXOUT in csrc/mz_learner.cu, head_ok in csrc/mz_learner_tc.cu
+MAX_INPUT_DIM = 1024   # widest observation: LMAXD in csrc/mz_learner.cu, MAXIN in csrc/mz_learner_tc.cu
+SLICE = 128            # input features per pass of the kernels' X tile: a wider (representation) head has no dX image
 _P = lambda t: C.c_void_p(t.data_ptr())
 
 
@@ -63,6 +66,9 @@ class FusedFCNetwork(object):
     vmin, vmax = [int(v) for v in config.value_support]
     rmin, rmax = [int(v) for v in config.reward_support]
     no_support = bool(getattr(config, 'no_support', False))  # networks.py:135-136: one-unit scalar heads
+    if not 1 <= int(input_dim) <= MAX_INPUT_DIM:  # before the library or the device is touched
+      raise ValueError("input_dim %d: the fused learner's kernels take observations of 1 to %d features "
+                       "(learners.Learner trains wider ones)" % (int(input_dim), MAX_INPUT_DIM))
     if not no_support:  # before the library or the device is touched: the first step would fail with MZ_ERR_BAD_ARG
       for name, lo, hi in (('value_support', vmin, vmax), ('reward_support', rmin, rmax)):
         if hi < lo or hi - lo + 1 > MAX_SUPPORT_BINS:
@@ -72,8 +78,8 @@ class FusedFCNetwork(object):
     self.lib = _lib.load()
     self.input_dim, self.action_space = int(input_dim), int(action_space)
     A = self.action_space
-    if self.input_dim > 128 or HIDDEN + A > 128:
-      raise ValueError("the fused learner kernels take at most 128 input features per head")
+    if HIDDEN + A > SLICE:  # the dynamics / reward heads' input [hidden | one-hot action] needs a dX
+      raise ValueError("action_space %d: the fused learner kernels take at most %d actions" % (A, SLICE - HIDDEN))
     self.heads = {
         'value_head': _Head('value_head', 'value', HIDDEN, 1 if no_support else vmax - vmin + 1),
         'policy_head': _Head('policy_head', 'policy', HIDDEN, A),
@@ -111,9 +117,11 @@ class FusedFCNetwork(object):
       h.p = [self.views[k] for k in h.keys]
       h.g = [self.grads[k] for k in h.keys]
     # bf16 mma B-operand images of the same matrices for the tensor-core kernels (csrc/mz_learner_tc.cu), refreshed
-    # every step from the float32 master weights by ONE launch
+    # every step from the float32 master weights by ONE launch.  w1tp only feeds dX, which a head wider than SLICE
+    # (the representation head, whose input is the observation) never needs: no image for it.
     words = lambda n, k: int(self.lib.mz_learner_packed_words(n, k))
-    shapes = lambda h: [(WIDTH, h.d_in), (h.d_out, WIDTH), (WIDTH, h.d_out), (h.d_in, WIDTH)]  # (N, K) of w1p w2p w2tp w1tp
+    # (N, K) of w1p w2p w2tp w1tp
+    shapes = lambda h: [(WIDTH, h.d_in), (h.d_out, WIDTH), (WIDTH, h.d_out), (h.d_in, WIDTH)][:4 if h.d_in <= SLICE else 3]
     self.packed = torch.zeros(sum(words(n, k) for h in self.heads.values() for n, k in shapes(h)), dtype=torch.int32,
                               device=self.device)
     jobs, off = [], 0
@@ -160,7 +168,8 @@ class FusedFCNetwork(object):
   def tc_head(self, name):
     """struct mz_tc_head of one head: packed images, float32 biases, gradient views."""
     h = self.heads[name]
-    return _lib.TcHead(h.images[0].data_ptr(), h.images[1].data_ptr(), h.images[2].data_ptr(), h.images[3].data_ptr(),
+    w1tp = h.images[3].data_ptr() if len(h.images) > 3 else None
+    return _lib.TcHead(h.images[0].data_ptr(), h.images[1].data_ptr(), h.images[2].data_ptr(), w1tp,
                        h.p[1].data_ptr(), h.p[3].data_ptr(), h.g[0].data_ptr(), h.g[1].data_ptr(), h.g[2].data_ptr(),
                        h.g[3].data_ptr(), h.d_in, h.d_out)
 
