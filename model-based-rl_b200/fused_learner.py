@@ -28,8 +28,11 @@ reference's arithmetic).  Observations of up to 1024 features (MAX_INPUT_DIM) tr
 representation head's input goes through the kernels' 128-feature input tiles in slices.  `--no_support` networks
 (one-unit value / reward heads, `config.scalar_loss` MSE or Huber, utils.py:61-70) run the same launches with
 d_out = 1 heads and the scalar loss kernel.  `save_state` writes the checkpoint dictionary of learners.py:72-83;
-`load_state` / `FusedLearner(state=...)` resume from it (weights, optimiser state, training_step, replay throughput), and a graph captured later keeps the restored optimiser state.  With torch.distributed initialised the gradients of the three output heads are all-reduced
-on a side stream while the recurrent part of the backward still runs; the rest follows before the optimiser step.
+`load_state` / `FusedLearner(state=...)` resume from it (weights, optimiser state, training_step, replay throughput), and a
+graph captured later keeps the restored optimiser state.  They take a `learners.Learner` checkpoint too: its
+per-parameter optimiser state is mapped onto the flat buffer by name (checkpoints.py), and `learners.Learner` resumes
+from a FusedLearner checkpoint the same way.  With torch.distributed initialised the gradients of the three output
+heads are all-reduced on a side stream while the recurrent part of the backward still runs; the rest follows before the optimiser step.
 """
 import ctypes as C
 import os
@@ -37,7 +40,7 @@ import os
 import numpy as np
 import torch
 
-from . import _lib, learners, parallel
+from . import _lib, checkpoints, learners, parallel
 from .networks import HIDDEN
 
 WIDTH = _lib.FC_WIDTH
@@ -52,9 +55,7 @@ class _Head(object):
 
   def __init__(self, name, out_name, d_in, d_out):
     self.name, self.out_name, self.d_in, self.d_out = name, out_name, d_in, d_out
-    self.keys = ["%s.fc1.weight" % name, "%s.fc1.bias" % name, "%s.%s.weight" % (name, out_name),
-                 "%s.%s.bias" % (name, out_name)]
-    self.shapes = [(WIDTH, d_in), (WIDTH,), (d_out, WIDTH), (d_out,)]
+    self.keys = [k for k, _ in checkpoints.head_params(name, out_name, d_in, d_out)]
 
 
 class FusedFCNetwork(object):
@@ -80,31 +81,19 @@ class FusedFCNetwork(object):
     A = self.action_space
     if HIDDEN + A > SLICE:  # the dynamics / reward heads' input [hidden | one-hot action] needs a dX
       raise ValueError("action_space %d: the fused learner kernels take at most %d actions" % (A, SLICE - HIDDEN))
-    self.heads = {
-        'value_head': _Head('value_head', 'value', HIDDEN, 1 if no_support else vmax - vmin + 1),
-        'policy_head': _Head('policy_head', 'policy', HIDDEN, A),
-        'reward_head': _Head('reward_head', 'reward', HIDDEN + A, 1 if no_support else rmax - rmin + 1),
-        'transition_head': _Head('transition_head', 'out', HIDDEN + A, HIDDEN),
-        'representation_head': _Head('representation_head', 'out', self.input_dim, HIDDEN),
-    }
-    specs = []
-    for h in self.heads.values():
-      specs += list(zip(h.keys, h.shapes))
-    specs += [('LN.weight', (HIDDEN,)), ('LN.bias', (HIDDEN,))]
+    self.heads = {h[0]: _Head(*h) for h in checkpoints.fc_heads(self.input_dim, A, config)}
     # every tensor starts on a 16-byte boundary of the flat buffers (the tensor-core backward adds weight gradients
     # with 16-byte vector reductions); the padding floats stay zero in parameters, gradients and optimiser state
-    pad4 = lambda m: (m + 3) & ~3
-    n = sum(pad4(int(np.prod(s))) for _, s in specs)
+    layout, n = checkpoints.flat_layout(self.input_dim, A, config)
     self.flat = torch.zeros(n, dtype=torch.float32, device=self.device)
     self.grad = torch.zeros(n, dtype=torch.float32, device=self.device)
-    self.views, self.grads, off = {}, {}, 0
-    for k, s in specs:
+    self.views, self.grads = {}, {}
+    for k, s, off in layout:
       m = int(np.prod(s))
       self.views[k] = self.flat[off:off + m].view(s)
       self.grads[k] = self.grad[off:off + m].view(s)
-      off += pad4(m)
       if k == 'reward_head.reward.bias':
-        self.bucket_split = off  # value, policy and reward heads: the gradient bucket that is complete first
+        self.bucket_split = off + checkpoints.pad4(m)  # value, policy and reward heads: the bucket that is complete first
     # k-major copies of the weight matrices (refreshed every step)
     nt = sum(WIDTH * h.d_in + WIDTH * h.d_out for h in self.heads.values())
     self.t_flat = torch.zeros(nt, dtype=torch.float32, device=self.device)
@@ -144,11 +133,12 @@ class FusedFCNetwork(object):
     missing = set(self.views) - set(weights)
     if missing:
       raise KeyError("missing weights: %s" % sorted(missing))
+    srcs = {k: torch.as_tensor(weights[k]) for k in self.views}
+    for k, v in self.views.items():  # every shape before the first copy: refused weights leave the network as it was
+      if tuple(srcs[k].shape) != tuple(v.shape):
+        raise ValueError("%s has shape %s, expected %s" % (k, tuple(srcs[k].shape), tuple(v.shape)))
     for k, v in self.views.items():
-      src = torch.as_tensor(weights[k])
-      if tuple(src.shape) != tuple(v.shape):
-        raise ValueError("%s has shape %s, expected %s" % (k, tuple(src.shape), tuple(v.shape)))
-      v.copy_(src.to(self.device, torch.float32))
+      v.copy_(srcs[k].to(self.device, torch.float32))
 
   def load_state_dict(self, weights):
     self.load_weights(weights)
@@ -555,15 +545,24 @@ class FusedLearner(object):
     return state
 
   def load_state(self, state):
-    """Resumes from a `save_state` checkpoint of a FusedLearner with the same optimiser and network (learners.py:59-70,
-    learners.Learner.load_state): weights, optimiser state, training_step and the replay throughput.  The library's
-    Adam state is copied in place (captured graphs stay valid); a torch optimiser's load_state_dict replaces its
-    tensors, so the step is captured again."""
-    opt, n = state['optimizer'], self.network.flat.numel()
-    own = isinstance(opt, dict) and 'exp_avg' in opt
+    """Resumes from a `save_state` checkpoint of a FusedLearner or of a `learners.Learner` with the same optimiser and
+    network (learners.py:59-70, learners.Learner.load_state): weights, optimiser state, training_step and the replay
+    throughput.  A learners.Learner checkpoint's per-parameter optimiser state is mapped onto the flat buffer first
+    (checkpoints.module_to_flat).  Every check runs before anything is written: a refused checkpoint raises ValueError
+    and leaves the learner as it was.  The library's Adam state is copied in place (captured graphs stay valid); a
+    torch optimiser's load_state_dict replaces its tensors, so the step is captured again."""
+    opt, n, net = state['optimizer'], self.network.flat.numel(), self.network
+    module_form = checkpoints.is_module_form(opt, net.input_dim, net.action_space, self.config)
     saved_kind = getattr(state.get('config'), 'optimizer', self.config.optimizer)
-    if own != self.own_optimizer or saved_kind != self.config.optimizer:
-      raise ValueError("the checkpoint holds %s optimiser state, this learner runs %s" % (saved_kind, self.config.optimizer))
+    if saved_kind != self.config.optimizer:
+      raise ValueError("the checkpoint of a %s holds %s optimiser state, this learner runs %s" % (
+          'learners.Learner' if module_form else 'FusedLearner', saved_kind, self.config.optimizer))
+    if module_form:
+      opt = checkpoints.module_to_flat(opt, self.config, net.input_dim, net.action_space)
+    own = isinstance(opt, dict) and 'exp_avg' in opt
+    if own != self.own_optimizer:
+      raise ValueError("the checkpoint holds %s optimiser state, this learner runs %s" % (
+          'the library Adam kernel\'s' if own else 'torch optimiser', self.config.optimizer))
     if own:
       sizes = {opt['exp_avg'].numel(), opt['exp_avg_sq'].numel()}
     else:
@@ -578,18 +577,7 @@ class FusedLearner(object):
       if isinstance(self.lr_scheduler, _ExponentialLR):  # the decay continues from the restored rate
         self.lr_scheduler.lr = float(self.opt_state[1])
     else:
-      group = dict(self.optimizer.param_groups[0])
-      self.optimizer.load_state_dict(opt)
-      # how this learner runs the step (captured or not, learning rate in a device scalar) is not the checkpoint's
-      g = self.optimizer.param_groups[0]
-      if torch.is_tensor(group['lr']):
-        group['lr'].fill_(float(g['lr']))
-        g['lr'] = group['lr']
-      if 'capturable' in group:
-        g['capturable'] = group['capturable']
-        for st in self.optimizer.state.values():
-          if torch.is_tensor(st.get('step')):
-            st['step'] = st['step'].to(self.device if g['capturable'] else 'cpu', torch.float32)
+      learners.load_optimizer_state(self.optimizer, opt, self.device)
       self._graphs = None
     self.training_step = state['training_step']
     if self.replay_buffer is not None and 'total_frames' in state:

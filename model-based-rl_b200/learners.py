@@ -228,6 +228,23 @@ def get_optimizer(config, parameters, capturable=False, lr=None):
   raise NotImplementedError(name)
 
 
+def load_optimizer_state(optimizer, state_dict, device):
+  """optimizer.load_state_dict(state_dict), keeping how this optimiser runs its step: a learning rate held in a device
+  scalar (which a captured step reads) stays that scalar, and `capturable` with it the place of the step counters
+  (on `device` when capturable, on the host otherwise) -- neither is the checkpoint's to decide."""
+  group = dict(optimizer.param_groups[0])
+  optimizer.load_state_dict(state_dict)
+  g = optimizer.param_groups[0]
+  if torch.is_tensor(group['lr']):
+    group['lr'].fill_(float(g['lr']))
+    g['lr'] = group['lr']
+  if 'capturable' in group:
+    g['capturable'] = group['capturable']
+    for st in optimizer.state.values():
+      if torch.is_tensor(st.get('step')):
+        st['step'] = st['step'].to(device if g['capturable'] else 'cpu', torch.float32)
+
+
 def _set_lr(optimizer, lr):
   for group in optimizer.param_groups:
     if torch.is_tensor(group["lr"]):
@@ -336,11 +353,46 @@ class Learner(object):
 
   # -- checkpoint (learners.py:59-82) ------------------------------------------------------------
   def load_state(self, state):
-    self.network.load_state_dict(state['weights'])
-    self.optimizer.load_state_dict(state['optimizer'])
+    """Resumes from a `save_state` checkpoint, or from a `fused_learner.FusedLearner` one: its flat optimiser state is
+    mapped onto FCNetworkTrain's parameters by name (checkpoints.flat_to_module), checked before anything is written,
+    and loaded the way this learner runs its step (capturable or not, learning rate in a device scalar or not)."""
+    from . import checkpoints  # checkpoints builds FCNetworkTrain: imported here, where learners is complete
+    opt = state['optimizer']
+    if checkpoints.is_flat_form(opt) and ('exp_avg' in opt or len(list(self.network.parameters())) != 1):
+      opt = self._module_state(checkpoints, state)
+      self.network.load_state_dict(state['weights'])
+      load_optimizer_state(self.optimizer, opt, self.device)
+      self._graphs = None  # the captured optimiser step read the replaced state tensors
+    else:
+      self.network.load_state_dict(state['weights'])
+      self.optimizer.load_state_dict(opt)
     self.training_step = state['training_step']
     if self.replay_buffer is not None and 'total_frames' in state:
       self.replay_buffer.add_initial_throughput(state['total_frames'], state['total_games'])
+
+  def _module_state(self, checkpoints, state):
+    """A FusedLearner checkpoint's optimiser state as this learner's, after every check that can refuse it."""
+    shapes = [(name, tuple(p.shape)) for name, p in self.network.named_parameters()]
+    geometry = dict(shapes)
+    try:
+      input_dim = geometry['representation_head.fc1.weight'][1]
+      action_space = geometry['policy_head.policy.weight'][0]
+    except KeyError:
+      input_dim = action_space = None
+    if input_dim is None or shapes != checkpoints.module_params(input_dim, action_space, self.config):
+      raise ValueError("flat optimiser state maps only onto the FCNetwork parameters (learners.FCNetworkTrain), "
+                       "this learner's network has others")
+    saved_kind = getattr(state.get('config'), 'optimizer', self.config.optimizer)
+    if saved_kind != self.config.optimizer:
+      raise ValueError("the checkpoint of a FusedLearner holds %s optimiser state, this learner runs %s" %
+                       (saved_kind, self.config.optimizer))
+    opt = checkpoints.flat_to_module(state['optimizer'], self.config, input_dim, action_space)
+    weights = state['weights']
+    for name, shape in shapes:
+      if name not in weights or tuple(weights[name].shape) != shape:
+        raise ValueError("the checkpoint's weight %s has shape %s, this network's %s" % (
+            name, tuple(weights[name].shape) if name in weights else None, shape))
+    return opt
 
   def save_state(self, path=None, actor_games=None, dirs=None):
     """The checkpoint dictionary of learners.py:72-83 with every key the reference's tooling reads
