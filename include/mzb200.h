@@ -558,6 +558,18 @@ int mz_conv_fc_tc(int32_t games, const void* x, const void* w_packed, const floa
 int mz_conv_head(int32_t games, const float* hidden, int32_t ldh, const float* w2, const float* b2,
                  int32_t outs, int32_t to_scalar, int32_t support_min, int32_t no_target_transform,
                  float* out, int32_t ldo, void* stream);
+/* Value / reward head of more than 32 bins on the tensor cores: the second head Linear(512 -> bins)
+ * (networks.py:438-440 fc2, 477-483 fc_value_o) followed by Config.inverse_transform (config.py:27-33:
+ * softmax expectation over [support_min, support_min + bins), then h^-1 unless no_target_transform):
+ * one float per game at out[g * ldo].
+ *   hidden  [games][ldh] f32 (the ReLU'd fc1 rows mz_conv_fc_tc writes), 16-byte aligned, ldh % 4 == 0;
+ *           rounded to bf16 (nearest even) inside the kernel
+ *   w2      [bins][512] bf16 row-major, 16-byte aligned;  b2 [bins] f32
+ * 33 <= bins <= 1024 (MZ_ERR_UNSUPPORTED otherwise; 32 bins and fewer are mz_conv_head's).  Float32
+ * accumulation, online softmax in a fixed column order: a given input gives the same bits on every run. */
+int mz_conv_support_head_tc(int32_t games, const float* hidden, int32_t ldh, const void* w2, const float* b2,
+                            int32_t bins, int32_t support_min, int32_t no_target_transform, float* out, int32_t ldo,
+                            void* stream);
 
 /* ------------------------------------------------------------------------------------------- */
 /* Learner unroll loss (Learner.update_weights, learners.py:182-213; utils.py:53-56)              */

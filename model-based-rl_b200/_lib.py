@@ -206,6 +206,8 @@ _SIGNATURES = {
     "mz_conv_fc_tc": (C.c_int, [C.c_int32, _V, _V, _V, C.c_int32, C.c_int32, _V, C.c_int32, _V]),
     "mz_conv_head": (C.c_int, [C.c_int32, _V, C.c_int32, _V, _V, C.c_int32, C.c_int32, C.c_int32,
                                C.c_int32, _V, C.c_int32, _V]),
+    "mz_conv_support_head_tc": (C.c_int, [C.c_int32, _V, C.c_int32, _V, _V, C.c_int32, C.c_int32, C.c_int32, _V,
+                                          C.c_int32, _V]),
     "mz_unroll_loss": (C.c_int, [C.POINTER(LossCfg), _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V]),
     "mz_scalar_unroll_loss": (C.c_int, [C.POINTER(LossCfg), C.c_int32, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V, _V,
                                         _V, _V]),

@@ -826,6 +826,209 @@ conv_pair_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
   }
 }
 
+// ================================================================================================
+// Value / reward support heads wider than 32 bins (the paper's Atari support is 601):
+//   out[g] = h^-1( sum_i softmax(logits[g])_i * (support_min + i) ),  logits[g] = hidden[g, 0:512] . W2^T + b2
+// (networks.py:438-440, 477-483; config.py:27-33).  One CTA per tile of 128 games, M = 128 rows = games.
+//   A: the tile's float32 head hidden rows, rounded to bf16 (round-to-nearest-even) by the epilogue warps
+//      while they stage it into shared memory in the 128-byte-swizzle K-major layout: 8 K blocks of 64,
+//      128 KB, resident for the whole tile.  This is the only rounding of the hidden layer; fc1's epilogue
+//      keeps it float32 in global memory.
+//   B: W2 as plain row-major bf16 [bins][512] (rounded once at load_weights), streamed by TMA in chunks of
+//      128 outputs x 64 K through a 4-stage mbarrier ring; rows >= bins arrive as zeros (TMA out-of-bounds
+//      fill) and their columns get a -inf bias, so they add exp(-inf) = 0 to the softmax.
+//   D: float32 in TMEM, two 128-column accumulators: the epilogue of chunk c overlaps the MMAs of c + 1.
+// Epilogue = online softmax, one thread per game: running max m, denominator den and numerator num (sum of
+// e_i * support_i), rescaled by exp(m_old - m_new) whenever a group of 32 columns raises the max.  The
+// reduction order is fixed: columns in increasing order, one group of 32 at a time, each group's max first,
+// then its terms added one by one -- no cross-thread reduction, so a given input gives the same bits on
+// every run and at every grid size.
+// ================================================================================================
+constexpr int SH_K = 512;                      // head hidden width
+constexpr int SH_KB = SH_K / BK;               // 8 K blocks
+constexpr int SH_N = 128;                      // outputs per chunk (one accumulator)
+constexpr int SH_STAGES = 4;
+constexpr int SH_A_BYTES = BM * SH_K * 2;      // 128 KB
+constexpr int SH_A_KB_BYTES = BM * BK * 2;     // 16 KB per K block
+constexpr int SH_B_BYTES = SH_N * BK * 2;      // 16 KB per stage
+constexpr int SH_MIN_BINS = 33, SH_MAX_BINS = 1024;
+constexpr int SH_THREADS = 192;                // TMA producer, MMA issuer, 4 staging / epilogue warps
+
+__global__ void __launch_bounds__(SH_THREADS, 1)
+conv_support_head_tc_kernel(const __grid_constant__ CUtensorMap map_w, int G, const float* __restrict__ hidden,
+                            int ldh, const float* __restrict__ b2, int bins, int support_min, int no_tt,
+                            float* __restrict__ out, int ldo) {
+  extern __shared__ __align__(1024) uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
+  uint8_t* s_a = smem;                                  // [8 K blocks][128 rows][128 B]
+  uint8_t* s_b = smem + SH_A_BYTES;                     // [SH_STAGES][128 rows][128 B]
+  uint64_t* full = reinterpret_cast<uint64_t*>(s_b + SH_STAGES * SH_B_BYTES);
+  uint64_t* empty = full + SH_STAGES;
+  uint64_t* acc_full = empty + SH_STAGES;   // [2]
+  uint64_t* acc_empty = acc_full + 2;       // [2]
+  uint64_t* a_full = acc_empty + 2;         // [1]
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(a_full + 1);
+  float* s_bias = reinterpret_cast<float*>(tmem_ptr + 4);  // [nchunks * 128], -inf past `bins`
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int nchunks = (bins + SH_N - 1) / SH_N;
+  // weights only: nothing here depends on the previous kernel
+  for (int i = threadIdx.x; i < nchunks * SH_N; i += SH_THREADS) s_bias[i] = i < bins ? b2[i] : -INFINITY;
+
+  if (threadIdx.x == 0) {
+    for (int i = 0; i < SH_STAGES; ++i) {
+      mbar_init(&full[i], 1);
+      mbar_init(&empty[i], 1);
+    }
+    for (int i = 0; i < 2; ++i) {
+      mbar_init(&acc_full[i], 1);
+      mbar_init(&acc_empty[i], 4);  // one arrival per epilogue warp
+    }
+    mbar_init(a_full, 4);           // one arrival per staging warp
+    mbar_fence_init();
+    tma_prefetch_desc(&map_w);
+  }
+  if (warp == 0) {
+    tmem_alloc(tmem_ptr, 2 * SH_N);
+    tmem_relinquish();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = *tmem_ptr;
+
+  if (warp == 0) {
+    // ===== TMA producer: W2 is a weight, its loads may overlap the previous kernel's tail =====
+    for (int it = 0; it < nchunks * SH_KB; ++it) {
+      const int st = it % SH_STAGES, chunk = it / SH_KB, kb = it - chunk * SH_KB;
+      mbar_wait(&empty[st], ((it / SH_STAGES) & 1) ^ 1);
+      if (elect_one()) {
+        uint8_t* sb = s_b + st * SH_B_BYTES;
+        mbar_arrive_expect_tx(&full[st], (uint32_t)SH_B_BYTES);  // out-of-bounds rows count as loaded zeros
+        tma_load_2d(sb, &map_w, kb * BK, chunk * SH_N, &full[st]);
+        tma_load_2d(sb + 64 * BK * 2, &map_w, kb * BK, chunk * SH_N + 64, &full[st]);
+      }
+      __syncwarp();
+    }
+    pdl_wait();
+    pdl_trigger();
+  } else if (warp == 1) {
+    // ===== MMA issuer =====
+    pdl_wait();
+    pdl_trigger();
+    const uint32_t idesc = make_idesc_128xN(SH_N);
+    mbar_wait(a_full, 0);
+    tc_fence_after();
+    int it = 0;
+    for (int chunk = 0; chunk < nchunks; ++chunk) {
+      const int acc = chunk & 1;
+      mbar_wait(&acc_empty[acc], ((chunk >> 1) & 1) ^ 1);
+      tc_fence_after();
+      const uint32_t d = tmem + acc * SH_N;
+      for (int kb = 0; kb < SH_KB; ++kb, ++it) {
+        const int st = it % SH_STAGES;
+        mbar_wait(&full[st], (it / SH_STAGES) & 1);
+        tc_fence_after();
+        const uint64_t ad = make_desc_sw128(smem_u32(s_a + kb * SH_A_KB_BYTES));
+        const uint64_t bd = make_desc_sw128(smem_u32(s_b + st * SH_B_BYTES));
+        if (elect_one()) {
+          if (kb == 0) umma_ss<false>(d, ad, bd, idesc);
+          else umma_ss<true>(d, ad, bd, idesc);
+#pragma unroll
+          for (int ks = 1; ks < BK / 16; ++ks)  // +32 bytes along K inside the 128-byte swizzle row
+            umma_ss<true>(d, ad + (uint64_t)(ks * 2), bd + (uint64_t)(ks * 2), idesc);
+          tc_commit(&empty[st]);
+          if (kb == SH_KB - 1) tc_commit(&acc_full[acc]);
+        }
+        __syncwarp();
+      }
+    }
+  } else {
+    // ===== staging of A, then epilogue: thread = accumulator row = game =====
+    const int quarter = warp & 3;
+    const int row = quarter * 32 + lane;
+    const int g0 = blockIdx.x * BM;
+    pdl_wait();  // the hidden rows are the previous kernel's output
+    pdl_trigger();
+    // this warp's 32 rows, one row per step: lane l converts floats [8 q, 8 q + 8) for q = l and l + 32
+    // (coalesced 1 KB per row and step) into 16-byte chunk q % 8 of K block q / 8, at its swizzled place
+#pragma unroll 4
+    for (int i = 0; i < 32; ++i) {
+      const int r = quarter * 32 + i, g = g0 + r;
+      const float4* src = reinterpret_cast<const float4*>(hidden + (size_t)g * ldh);
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int q = lane + 32 * h;
+        uint4 v = make_uint4(0u, 0u, 0u, 0u);  // rows past the last game: zeros
+        if (g < G) {
+          const float4 lo = __ldg(src + 2 * q), hi = __ldg(src + 2 * q + 1);
+          v = make_uint4(pack_bf16(lo.x, lo.y), pack_bf16(lo.z, lo.w), pack_bf16(hi.x, hi.y), pack_bf16(hi.z, hi.w));
+        }
+        const uint32_t dst = smem_u32(s_a + (q >> 3) * SH_A_KB_BYTES + r * 128 + (((q & 7) ^ (r & 7)) << 4));
+        asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w)
+                     : "memory");
+      }
+    }
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy stores -> tensor core reads
+    __syncwarp();
+    if (lane == 0) mbar_arrive(a_full);
+
+    const uint32_t lane_addr = tmem + ((uint32_t)(quarter * 32) << 16);
+    float m = -INFINITY, den = 0.0f, num = 0.0f;
+    for (int chunk = 0; chunk < nchunks; ++chunk) {
+      const int acc = chunk & 1;
+      mbar_wait(&acc_full[acc], (chunk >> 1) & 1);
+      tc_fence_after();
+#pragma unroll 1
+      for (int c0 = 0; c0 < SH_N; c0 += 32) {
+        const int col0 = chunk * SH_N + c0;
+        if (col0 >= bins) break;  // uniform: whole groups past the support are never read
+        uint32_t v[32];
+        tmem_ld32(lane_addr + acc * SH_N + c0, v);
+        tmem_wait_ld();
+        float x[32];
+        float gm = -INFINITY;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          x[j] = __uint_as_float(v[j]) + s_bias[col0 + j];
+          gm = fmaxf(gm, x[j]);
+        }
+        const float nm = fmaxf(m, gm);   // finite: every group read holds at least one real bin
+        const float sc = expf(m - nm);   // 0 on the first group (m = -inf), 1 when the max holds
+        den *= sc;
+        num *= sc;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          const float e = expf(x[j] - nm);
+          den += e;
+          num = fmaf(e, (float)(support_min + col0 + j), num);
+        }
+        m = nm;
+      }
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0)
+        asm volatile("mbarrier.arrive.relaxed.cta.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&acc_empty[acc])) : "memory");
+    }
+    const int g = g0 + row;
+    if (g < G) {
+      float x = num / den;
+      if (!no_tt) {  // same h^-1 arithmetic as conv_head_kernel
+        const float eps = 0.001f;
+        const float sgn = x > 0.0f ? 1.0f : (x < 0.0f ? -1.0f : 0.0f);
+        const float t = (sqrtf(1.0f + 4.0f * eps * (fabsf(x) + 1.0f + eps)) - 1.0f) / (2.0f * eps);
+        x = sgn * (t * t - 1.0f);
+      }
+      out[(size_t)g * ldo] = x;
+    }
+  }
+
+  __syncthreads();
+  if (warp == 0) {
+    tc_fence_after();
+    tmem_dealloc(tmem, 2 * SH_N);
+  }
+}
+
 // ---- heads: relu(fc1) [G][512] -> Linear(512 -> bins) (+ softmax expectation + h^-1) --------------
 // One warp per game.  networks.py:438-440, 477-483; config.py:27-33.
 __global__ void conv_head_kernel(int G, const float* __restrict__ hidden, int ldh, const float* __restrict__ w2,
@@ -1216,6 +1419,36 @@ int mz_conv_head(int32_t games, const float* hidden, int32_t ldh, const float* w
   const int threads = 256, grid = (games * 32 + threads - 1) / threads;
   conv_head_kernel<<<grid, threads, 0, (cudaStream_t)stream>>>(games, hidden, ldh, w2, b2, outs, to_scalar,
                                                                support_min, no_target_transform, out, ldo);
+  MZ_LAUNCH_CHECK();
+  return MZ_OK;
+}
+
+// Value / reward head Linear(512 -> bins) on the tensor cores for 33 <= bins <= 1024, followed by
+// Config.inverse_transform (config.py:27-33): one float per game at out[g * ldo].  hidden: float32 rows
+// of stride ldh (16-byte aligned), w2: bf16 [bins][512] row-major (16-byte aligned), b2: float32 [bins].
+int mz_conv_support_head_tc(int32_t games, const float* hidden, int32_t ldh, const void* w2, const float* b2,
+                            int32_t bins, int32_t support_min, int32_t no_target_transform, float* out, int32_t ldo,
+                            void* stream) {
+  if (games < 1 || !hidden || !w2 || !b2 || !out || ldh < SH_K || (ldh % 4) || ldo < 1 ||
+      (reinterpret_cast<uintptr_t>(hidden) & 15) || (reinterpret_cast<uintptr_t>(w2) & 15))
+    return MZ_ERR_BAD_ARG;
+  if (bins < SH_MIN_BINS || bins > SH_MAX_BINS) return MZ_ERR_UNSUPPORTED;
+  static bool attr = false;
+  const size_t smem = 1024 + (size_t)SH_A_BYTES + (size_t)SH_STAGES * SH_B_BYTES +
+                      (2 * SH_STAGES + 5) * sizeof(uint64_t) + 16 + SH_MAX_BINS * sizeof(float);
+  if (!attr) {
+    cudaError_t e = cudaFuncSetAttribute(conv_support_head_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    attr = true;
+  }
+  CUtensorMap mw;
+  const int rc = make_map(&mw, w2, (uint64_t)bins, SH_K);
+  if (rc) return rc;
+  cudaError_t e = mz_launch(conv_support_head_tc_kernel, dim3((games + BM - 1) / BM), dim3(SH_THREADS), smem,
+                            (cudaStream_t)stream, true, mw, (int)games, hidden, (int)ldh, b2, (int)bins,
+                            (int)support_min, (int)no_target_transform, out, (int)ldo);
+  if (e != cudaSuccess) return (int)e;
   MZ_LAUNCH_CHECK();
   return MZ_OK;
 }

@@ -27,6 +27,8 @@ ROWS = 49         # rows per game: 7 zero | 6 x (6 pixels + 1 zero)
 K_FC = ROWS * CH  # 6272: flattened padded state
 RELU, RESIDUAL, ACTION, SCALE = 1, 2, 4, 8
 BN_EPS = 1e-5
+NARROW_HEAD_BINS = 32    # value / reward supports up to this width: mz_conv_head (one warp per game)
+MAX_SUPPORT_BINS = 1024  # wider ones: mz_conv_support_head_tc, which takes up to this many bins
 
 
 def to_padded(state):
@@ -94,6 +96,16 @@ class _StridedConv(object):
     self.bias = bias.to(device, torch.float32).contiguous()
 
 
+def _pack_support_head(weight, bias, device):
+  """Second layer Linear(512 -> bins) of a value or reward head: float32 [bins][512] for mz_conv_head up to
+  NARROW_HEAD_BINS bins, above that the bf16 [bins][512] B operand of mz_conv_support_head_tc (rounded here,
+  once).  The bias stays float32."""
+  w = weight.to(device, torch.float32)
+  if w.shape[0] > NARROW_HEAD_BINS:
+    w = w.to(torch.bfloat16)
+  return w.contiguous(), bias.to(device, torch.float32).contiguous()
+
+
 def _pack_fc(weight, device):
   """Linear(128*6*6 -> n) weight [n, c*36 + y*6 + x] -> [n, (7 + y*7 + x)*128 + c] bf16."""
   n = weight.shape[0]
@@ -133,6 +145,10 @@ class MuZeroNetwork(object):
   def load_weights(self, weights):
     """Accepts the reference's state dict (networks.py:549-550); folds BatchNorm (eval statistics)
     into the convolutions and packs everything for the tensor-core kernels."""
+    for name, bins in (('value', self.value_bins), ('reward', self.reward_bins)):
+      if bins > MAX_SUPPORT_BINS:
+        raise ValueError("the %s support has %d bins; MuZeroNetwork's support heads take at most %d"
+                         % (name, bins, MAX_SUPPORT_BINS))
     dev = self.device
     sd = {k: torch.as_tensor(v).detach() for k, v in weights.items()}
     # a snapshot (the reference hands weights over as `.cpu()` copies, networks.py:36-40): later in-place
@@ -180,12 +196,12 @@ class MuZeroNetwork(object):
     f32 = lambda k: sd[k].to(dev, torch.float32).contiguous()
     self.rew_fc1_w = _pack_fc(sd[d + '.fc1.weight'], dev)
     self.rew_fc1_b = f32(d + '.fc1.bias')
-    self.rew_fc2_w, self.rew_fc2_b = f32(d + '.fc2.weight'), f32(d + '.fc2.bias')
+    self.rew_fc2_w, self.rew_fc2_b = _pack_support_head(sd[d + '.fc2.weight'], sd[d + '.fc2.bias'], dev)
     # value and policy heads read the same state: one GEMM with 1024 outputs
     self.vp_fc1_w = torch.cat((_pack_fc(sd[q + '.fc_value.weight'], dev),
                                _pack_fc(sd[q + '.fc_policy.weight'], dev)), dim=0).contiguous()
     self.vp_fc1_b = torch.cat((f32(q + '.fc_value.bias'), f32(q + '.fc_policy.bias'))).contiguous()
-    self.val_fc2_w, self.val_fc2_b = f32(q + '.fc_value_o.weight'), f32(q + '.fc_value_o.bias')
+    self.val_fc2_w, self.val_fc2_b = _pack_support_head(sd[q + '.fc_value_o.weight'], sd[q + '.fc_value_o.bias'], dev)
     self.pol_fc2_w, self.pol_fc2_b = f32(q + '.fc_policy_o.weight'), f32(q + '.fc_policy_o.bias')
     if self.rew_fc2_w.shape[0] != self.reward_bins or self.val_fc2_w.shape[0] != self.value_bins or \
         self.pol_fc2_w.shape[0] != self.action_space:
@@ -254,6 +270,18 @@ class MuZeroNetwork(object):
       cur = o
     return cur
 
+  def _support_head(self, games, hidden, w2, b2, bins, support_min, out):
+    """Linear(512 -> bins) of the value or reward head over `hidden` (a view of the fc buffer, row stride 1536)
+    + softmax expectation + h^-1 -> out [games] f32.  Supports of up to NARROW_HEAD_BINS bins run on
+    mz_conv_head, wider ones on the tensor-core kernel."""
+    P, st, ntt = _lib.ptr, _lib.current_stream(), int(self.no_target_transform)
+    if bins <= NARROW_HEAD_BINS:
+      _lib.check(self.lib.mz_conv_head(games, C_ptr(hidden), 1536, P(w2), P(b2), bins, 1, support_min, ntt,
+                                       P(out), 1, st), "mz_conv_head")
+    else:
+      _lib.check(self.lib.mz_conv_support_head_tc(games, C_ptr(hidden), 1536, P(w2), P(b2), bins, support_min, ntt,
+                                                  P(out), 1, st), "mz_conv_support_head_tc")
+
   def run_recurrent(self, games, state, actions, value, reward, logits, pool_out=None, pool_base=None):
     """recurrent_inference (networks.py:31-34) for `games` games on the current stream.
       state      [games * 49][128] bf16 (flat padded layout)
@@ -271,9 +299,7 @@ class MuZeroNetwork(object):
                       pool_out=pool_out, pool_base=pool_base)
     _lib.check(self.lib.mz_conv_fc_tc(games, P(raw), P(self.rew_fc1_w), P(self.rew_fc1_b), 512, 1,
                                       P(b['fc']), 1536, st), "mz_conv_fc_tc")
-    _lib.check(self.lib.mz_conv_head(games, P(b['fc']), 1536, P(self.rew_fc2_w), P(self.rew_fc2_b),
-                                     self.reward_bins, 1, self.reward_min, int(self.no_target_transform),
-                                     P(reward), 1, st), "mz_conv_head")
+    self._support_head(games, b['fc'], self.rew_fc2_w, self.rew_fc2_b, self.reward_bins, self.reward_min, reward)
     self.launches += 2
     self.run_prediction(games, scaled, value, logits)  # prediction on the scaled state
     return scaled
@@ -287,9 +313,7 @@ class MuZeroNetwork(object):
     fc_vp = b['fc'][:, 512:]
     _lib.check(self.lib.mz_conv_fc_tc(games, P(out), P(self.vp_fc1_w), P(self.vp_fc1_b), 1024, 1,
                                       C_ptr(fc_vp), 1536, st), "mz_conv_fc_tc")
-    _lib.check(self.lib.mz_conv_head(games, C_ptr(fc_vp), 1536, P(self.val_fc2_w), P(self.val_fc2_b),
-                                     self.value_bins, 1, self.value_min, int(self.no_target_transform),
-                                     P(value), 1, st), "mz_conv_head")
+    self._support_head(games, fc_vp, self.val_fc2_w, self.val_fc2_b, self.value_bins, self.value_min, value)
     _lib.check(self.lib.mz_conv_head(games, C_ptr(b['fc'][:, 1024:]), 1536, P(self.pol_fc2_w),
                                      P(self.pol_fc2_b), self.action_space, 0, 0, 0, P(logits),
                                      self.action_space, st), "mz_conv_head")
