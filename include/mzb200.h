@@ -750,6 +750,23 @@ int64_t mz_chain_mask_words(int32_t rows, int32_t steps);
 int mz_chain_forward_tc(const mz_tc_chain* chain, void* stream);
 int mz_chain_backward_tc(const mz_tc_chain* chain, void* stream);
 
+/* ------------------------------------------------------------------------------------------- */
+/* The same four launches at float32 accuracy on the tensor cores (csrc/mz_learner_tf32.cu):     */
+/* every contraction is three TF32 products on split operands (hi x hi + hi x lo + lo x hi,       */
+/* float32 accumulation), as in mz_fc_*_tf32x3.  Same structs and shapes as the _tc entry points; */
+/* the images of mz_tc_head are packed by mz_learner_pack_tf32x3 (hi / lo TF32 B fragments of      */
+/* 8 (n) x 8 (k) blocks, mz_learner_packed_words_tf32x3(N, K) 32-bit words, zero padded), and the  */
+/* ReLU bits of the chain have the layout of mz_chain_mask_words.  MZ_ERR_UNSUPPORTED for a head   */
+/* with d_in > 1024 or d_out > 64 (a chain with d > 64 or d + num_actions > 128), MZ_ERR_BAD_ARG  */
+/* for a dX of a head wider than 128 and every other refused argument.                             */
+/* ------------------------------------------------------------------------------------------- */
+int64_t mz_learner_packed_words_tf32x3(int32_t n, int32_t k);
+int mz_learner_pack_tf32x3(int32_t njobs, const mz_pack_job* jobs, void* stream);
+int mz_heads_forward_tf32x3(int32_t njobs, const mz_tc_job* jobs, void* stream);
+int mz_heads_backward_tf32x3(int32_t njobs, const mz_tc_job* jobs, void* stream);
+int mz_chain_forward_tf32x3(const mz_tc_chain* chain, void* stream);
+int mz_chain_backward_tf32x3(const mz_tc_chain* chain, void* stream);
+
 #if defined(MZ_BUILDING) && defined(__GNUC__)
 #pragma GCC visibility pop
 #endif

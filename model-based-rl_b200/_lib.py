@@ -191,6 +191,12 @@ _SIGNATURES = {
     "mz_heads_backward_tc": (C.c_int, [C.c_int32, C.POINTER(TcJob), _V]),
     "mz_chain_forward_tc": (C.c_int, [C.POINTER(TcChain), _V]),
     "mz_chain_backward_tc": (C.c_int, [C.POINTER(TcChain), _V]),
+    "mz_learner_packed_words_tf32x3": (C.c_int64, [C.c_int32, C.c_int32]),
+    "mz_learner_pack_tf32x3": (C.c_int, [C.c_int32, C.POINTER(PackJob), _V]),
+    "mz_heads_forward_tf32x3": (C.c_int, [C.c_int32, C.POINTER(TcJob), _V]),
+    "mz_heads_backward_tf32x3": (C.c_int, [C.c_int32, C.POINTER(TcJob), _V]),
+    "mz_chain_forward_tf32x3": (C.c_int, [C.POINTER(TcChain), _V]),
+    "mz_chain_backward_tf32x3": (C.c_int, [C.POINTER(TcChain), _V]),
     "mz_sumtree_add_from": (C.c_int, [_V, C.c_int64, C.c_int64, _V, _V, C.c_int64, C.c_int32, C.c_int32, _V, _V, _V,
                                       _V, _V]),
     "mz_sumtree_sample": (C.c_int, [_V, C.c_int64, C.c_int32, _V, _V, _V, _V, C.c_int64, C.c_double,

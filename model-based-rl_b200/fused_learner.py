@@ -19,12 +19,24 @@ search kernels' `FCNetwork.load_weights` see the usual tensors.  `FusedLearner(p
   -- 10 kernels per step, 128 us at B = 512, K = 5 (7 800 steps/s on a B200; the torch-module step in a
   CUDA graph: 1 100 us).
 
+  precision='tf32x3' (csrc/mz_learner_tf32.cu: the same launches on the tensor cores at float32 accuracy -- every
+  contraction is three TF32 products on split operands, float32 accumulation -- held to the f32 path's bars)
+    mz_learner_pack_tf32x3    the 20 weight images as hi / lo TF32 B fragments + clears 1 launch
+    mz_chain_forward_tf32x3   representation -> LN -> K x (dynamics -> LN)               1 launch
+    mz_heads_forward_tf32x3   value / policy / reward heads over all K + 1 steps         1 launch
+    mz_unroll_loss            fused loss + logit gradients (or mz_scalar_unroll_loss)    2 launches
+    mz_heads_backward_tf32x3  the three output heads                                     1 launch
+    mz_chain_backward_tf32x3  the serial part: LN backward -> dH -> dX per step          1 launch
+    mz_heads_backward_tf32x3  parameter gradients of dynamics + representation           1 launch
+    mz_adam_step              AdamW / Adam over the flat buffer                          2 launches
+  The network allocates the hi / lo images when the first tf32x3 learner is built (FusedFCNetwork.tf32x3_images).
+
   precision='f32' (csrc/mz_learner.cu: float32 CUDA-core kernels, one launch per head evaluation; the parity baseline
   against the reference's goldens at float32 bars)
     transposes, 2 (K + 1) forward launches, 3 head launches, loss, 3 + 2 (K + 1) backward launches, optimiser.
 
-Both are captured in CUDA graphs.  SGD / RMSprop use the torch optimiser over the flat buffer (elementwise, the
-reference's arithmetic).  Observations of up to 1024 features (MAX_INPUT_DIM) train in both precisions: the
+All three are captured in CUDA graphs.  SGD / RMSprop use the torch optimiser over the flat buffer (elementwise, the
+reference's arithmetic).  Observations of up to 1024 features (MAX_INPUT_DIM) train in every precision: the
 representation head's input goes through the kernels' 128-feature input tiles in slices.  `--no_support` networks
 (one-unit value / reward heads, `config.scalar_loss` MSE or Huber, utils.py:61-70) run the same launches with
 d_out = 1 heads and the scalar loss kernel.  `save_state` writes the checkpoint dictionary of learners.py:72-83;
@@ -108,25 +120,41 @@ class FusedFCNetwork(object):
     # bf16 mma B-operand images of the same matrices for the tensor-core kernels (csrc/mz_learner_tc.cu), refreshed
     # every step from the float32 master weights by ONE launch.  w1tp only feeds dX, which a head wider than SLICE
     # (the representation head, whose input is the observation) never needs: no image for it.
-    words = lambda n, k: int(self.lib.mz_learner_packed_words(n, k))
-    # (N, K) of w1p w2p w2tp w1tp
-    shapes = lambda h: [(WIDTH, h.d_in), (h.d_out, WIDTH), (WIDTH, h.d_out), (h.d_in, WIDTH)][:4 if h.d_in <= SLICE else 3]
-    self.packed = torch.zeros(sum(words(n, k) for h in self.heads.values() for n, k in shapes(h)), dtype=torch.int32,
-                              device=self.device)
-    jobs, off = [], 0
-    for h in self.heads.values():
-      w1, w2 = h.p[0], h.p[2]
-      h.images = []
-      for (n, k), (src, sn, sk) in zip(shapes(h), [(w1, h.d_in, 1), (w2, WIDTH, 1), (w2, 1, WIDTH), (w1, 1, h.d_in)]):
-        dst = self.packed[off:off + words(n, k)]
-        off += words(n, k)
-        h.images.append(dst)
-        jobs.append(_lib.PackJob(src.data_ptr(), dst.data_ptr(), n, k, sn, sk))
-    self._pack_list = jobs
-    self._pack_jobs = (_lib.PackJob * len(jobs))(*jobs)
+    self.packed, self._pack_list = self._pack_images(self.lib.mz_learner_packed_words, 'images')
+    self._pack_jobs = (_lib.PackJob * len(self._pack_list))(*self._pack_list)
+    # hi / lo TF32 images for a precision='tf32x3' learner (csrc/mz_learner_tf32.cu): made by tf32x3_images() when such
+    # a learner is built, so a network that never trains at that precision does not hold them
+    self.packed_tf32x3 = self._pack_list_tf32x3 = None
     # the reference's initialisation: torch's defaults for nn.Linear / nn.LayerNorm
     ref = learners.FCNetworkTrain(self.input_dim, A, 'cpu', config)
     self.load_weights(ref.state_dict())
+
+  def _pack_images(self, words_fn, attr):
+    """One int32 buffer with the packed images of every head (h.<attr>: views into it) and the pack jobs that fill it
+    from the float32 master weights."""
+    words = lambda n, k: int(words_fn(n, k))
+    # (N, K) of w1p w2p w2tp w1tp
+    shapes = lambda h: [(WIDTH, h.d_in), (h.d_out, WIDTH), (WIDTH, h.d_out), (h.d_in, WIDTH)][:4 if h.d_in <= SLICE else 3]
+    packed = torch.zeros(sum(words(n, k) for h in self.heads.values() for n, k in shapes(h)), dtype=torch.int32,
+                         device=self.device)
+    jobs, off = [], 0
+    for h in self.heads.values():
+      w1, w2 = h.p[0], h.p[2]
+      images = []
+      for (n, k), (src, sn, sk) in zip(shapes(h), [(w1, h.d_in, 1), (w2, WIDTH, 1), (w2, 1, WIDTH), (w1, 1, h.d_in)]):
+        dst = packed[off:off + words(n, k)]
+        off += words(n, k)
+        images.append(dst)
+        jobs.append(_lib.PackJob(src.data_ptr(), dst.data_ptr(), n, k, sn, sk))
+      setattr(h, attr, images)
+    return packed, jobs
+
+  def tf32x3_images(self):
+    """The hi / lo TF32 fragment images of every weight matrix (mz_learner_pack_tf32x3), allocated on first use;
+    returns their pack jobs."""
+    if self.packed_tf32x3 is None:
+      self.packed_tf32x3, self._pack_list_tf32x3 = self._pack_images(self.lib.mz_learner_packed_words_tf32x3, 'images_tf32x3')
+    return self._pack_list_tf32x3
 
   # -- the reference's network interface ------------------------------------------------------------
   def load_weights(self, weights):
@@ -155,11 +183,13 @@ class FusedFCNetwork(object):
   def train(self, mode=True):
     return self
 
-  def tc_head(self, name):
-    """struct mz_tc_head of one head: packed images, float32 biases, gradient views."""
+  def tc_head(self, name, precision='bf16'):
+    """struct mz_tc_head of one head: packed images (bf16, or the 'tf32x3' hi / lo images), float32 biases, gradient
+    views."""
     h = self.heads[name]
-    w1tp = h.images[3].data_ptr() if len(h.images) > 3 else None
-    return _lib.TcHead(h.images[0].data_ptr(), h.images[1].data_ptr(), h.images[2].data_ptr(), w1tp,
+    images = h.images if precision == 'bf16' else h.images_tf32x3
+    w1tp = images[3].data_ptr() if len(images) > 3 else None
+    return _lib.TcHead(images[0].data_ptr(), images[1].data_ptr(), images[2].data_ptr(), w1tp,
                        h.p[1].data_ptr(), h.p[3].data_ptr(), h.g[0].data_ptr(), h.g[1].data_ptr(), h.g[2].data_ptr(),
                        h.g[3].data_ptr(), h.d_in, h.d_out)
 
@@ -186,9 +216,12 @@ class FusedLearner(object):
     _lib.require_cuda()
     if not isinstance(network, FusedFCNetwork):
       raise TypeError("FusedLearner trains a FusedFCNetwork")
-    if precision not in ('bf16', 'f32'):
-      raise ValueError("precision is 'bf16' (tensor cores, float32 accumulation and master weights) or 'f32'")
+    if precision not in ('bf16', 'tf32x3', 'f32'):
+      raise ValueError("precision is 'bf16' (tensor cores, float32 accumulation and master weights), 'tf32x3' (tensor "
+                       "cores at float32 accuracy) or 'f32' (CUDA cores)")
     self.precision = precision
+    if precision == 'tf32x3':
+      network.tf32x3_images()
     self.config, self.network, self.lib = config, network, _lib.load()
     self.device = network.device
     self.replay_buffer, self.search_network = replay_buffer, search_network
@@ -258,35 +291,44 @@ class FusedLearner(object):
     self.c_loss = _lib.LossCfg(B, K, A, self.loss_cfg['value_min'], self.loss_cfg['value_max'], self.loss_cfg['reward_min'],
                                self.loss_cfg['reward_max'], int(self.loss_cfg['no_target_transform']))
     self._shape, self._graphs = B, None
-    if self.precision == 'bf16':
+    if self.precision != 'f32':
       self._alloc_tc()
 
   def _alloc_tc(self):
-    """Argument structs of the four tensor-core launches (pointers into the buffers of this batch shape)."""
+    """Argument structs of the four tensor-core launches (pointers into the buffers of this batch shape) and the entry
+    points of this precision: mz_*_tc (bf16) or mz_*_tf32x3."""
     net, K, B, A, ldx = self.network, self.K, self.B, self.A, self.ldx
     P = lambda t: t.data_ptr()
+    tf = self.precision == 'tf32x3'
+    sfx = '_tf32x3' if tf else '_tc'
+    self.tc_fn = {k: (getattr(self.lib, k + sfx), k + sfx) for k in
+                  ('mz_chain_forward', 'mz_chain_backward', 'mz_heads_forward', 'mz_heads_backward')}
+    self.tc_fn['mz_learner_pack'] = ((self.lib.mz_learner_pack_tf32x3, 'mz_learner_pack_tf32x3') if tf else
+                                     (self.lib.mz_learner_pack, 'mz_learner_pack'))
+    tc_head = lambda name: net.tc_head(name, self.precision)
     self.relu_mask = torch.zeros(int(self.lib.mz_chain_mask_words(B, K + 1)), dtype=torch.int32, device=self.device)
     self.dyall = torch.zeros((K + 1, B, HIDDEN), dtype=torch.float32, device=self.device)
-    self.tc_chain = _lib.TcChain(net.tc_head('representation_head'), net.tc_head('transition_head'), B, K + 1, HIDDEN, A,
+    self.tc_chain = _lib.TcChain(tc_head('representation_head'), tc_head('transition_head'), B, K + 1, HIDDEN, A,
                                  P(self.s_obs), net.input_dim, P(self.s_actions), max(K, 1), K, P(net.views['LN.weight']),
                                  P(net.views['LN.bias']), P(self.xs), ldx, P(self.yall), P(self.mean), P(self.rstd),
                                  P(self.relu_mask), P(self.dxs), 0.5, P(net.grads['LN.weight']), P(net.grads['LN.bias']),
                                  P(self.dyall))
     # parameter gradients of the recurrent heads, off the chain: all K B + B rows in one launch
-    rec = [_lib.TcJob(net.tc_head('representation_head'), B, net.input_dim, HIDDEN, 0, P(self.s_obs), None, P(self.dyall[0]),
+    rec = [_lib.TcJob(tc_head('representation_head'), B, net.input_dim, HIDDEN, 0, P(self.s_obs), None, P(self.dyall[0]),
                       None)]
     if K > 0:
-      rec.append(_lib.TcJob(net.tc_head('transition_head'), K * B, ldx, HIDDEN, 0, P(self.xs), None, P(self.dyall[1]), None))
+      rec.append(_lib.TcJob(tc_head('transition_head'), K * B, ldx, HIDDEN, 0, P(self.xs), None, P(self.dyall[1]), None))
     self.tc_rec_jobs = (_lib.TcJob * len(rec))(*rec)
     # the step's first launch packs the weight images AND clears the two accumulation buffers (src NULL = zero n words)
-    first = list(net._pack_list) + [_lib.PackJob(None, P(net.grad), net.grad.numel(), 0, 0, 0),
-                                    _lib.PackJob(None, P(self.dxs), self.dxs.numel(), 0, 0, 0)]
+    first = list(net._pack_list_tf32x3 if tf else net._pack_list)
+    first += [_lib.PackJob(None, P(net.grad), net.grad.numel(), 0, 0, 0),
+              _lib.PackJob(None, P(self.dxs), self.dxs.numel(), 0, 0, 0)]
     self.tc_first_jobs = (_lib.PackJob * len(first))(*first)
     V, R = self.v.shape[2], self.r.shape[2]
-    jobs = [_lib.TcJob(net.tc_head('value_head'), (K + 1) * B, ldx, V, ldx, P(self.xs), P(self.v), P(self.dv), P(self.dxs)),
-            _lib.TcJob(net.tc_head('policy_head'), (K + 1) * B, ldx, A, ldx, P(self.xs), P(self.p), P(self.dp), P(self.dxs))]
+    jobs = [_lib.TcJob(tc_head('value_head'), (K + 1) * B, ldx, V, ldx, P(self.xs), P(self.v), P(self.dv), P(self.dxs)),
+            _lib.TcJob(tc_head('policy_head'), (K + 1) * B, ldx, A, ldx, P(self.xs), P(self.p), P(self.dp), P(self.dxs))]
     if K > 0:
-      jobs.append(_lib.TcJob(net.tc_head('reward_head'), K * B, ldx, R, ldx, P(self.xs), P(self.r), P(self.dr), P(self.dxs)))
+      jobs.append(_lib.TcJob(tc_head('reward_head'), K * B, ldx, R, ldx, P(self.xs), P(self.r), P(self.dr), P(self.dxs)))
     self.tc_jobs = (_lib.TcJob * len(jobs))(*jobs)
 
   # -- launch sequences --------------------------------------------------------------------------------
@@ -316,12 +358,13 @@ class FusedLearner(object):
     output heads (whose parameter gradients are then complete)."""
     net, lib, K, B, A, ldx = self.network, self.lib, self.K, self.B, self.A, self.ldx
     st = _lib.current_stream()
-    if self.precision == 'bf16':
-      _lib.check(lib.mz_learner_pack(len(self.tc_first_jobs), self.tc_first_jobs, st), "mz_learner_pack")
-      _lib.check(lib.mz_chain_forward_tc(self.tc_chain, st), "mz_chain_forward_tc")
-      _lib.check(lib.mz_heads_forward_tc(len(self.tc_jobs), self.tc_jobs, st), "mz_heads_forward_tc")
+    if self.precision != 'f32':
+      fn = self.tc_fn
+      _lib.check(fn['mz_learner_pack'][0](len(self.tc_first_jobs), self.tc_first_jobs, st), fn['mz_learner_pack'][1])
+      _lib.check(fn['mz_chain_forward'][0](self.tc_chain, st), fn['mz_chain_forward'][1])
+      _lib.check(fn['mz_heads_forward'][0](len(self.tc_jobs), self.tc_jobs, st), fn['mz_heads_forward'][1])
       self._loss(st)
-      _lib.check(lib.mz_heads_backward_tc(len(self.tc_jobs), self.tc_jobs, st), "mz_heads_backward_tc")
+      _lib.check(fn['mz_heads_backward'][0](len(self.tc_jobs), self.tc_jobs, st), fn['mz_heads_backward'][1])
       return
     ln_w, ln_b = net.views['LN.weight'], net.views['LN.bias']
     net.refresh_transposes()
@@ -350,9 +393,10 @@ class FusedLearner(object):
     of every hidden state the dynamics produced."""
     net, lib, K, B, ldx = self.network, self.lib, self.K, self.B, self.ldx
     st = _lib.current_stream()
-    if self.precision == 'bf16':
-      _lib.check(lib.mz_chain_backward_tc(self.tc_chain, st), "mz_chain_backward_tc")
-      _lib.check(lib.mz_heads_backward_tc(len(self.tc_rec_jobs), self.tc_rec_jobs, st), "mz_heads_backward_tc")
+    if self.precision != 'f32':
+      fn = self.tc_fn
+      _lib.check(fn['mz_chain_backward'][0](self.tc_chain, st), fn['mz_chain_backward'][1])
+      _lib.check(fn['mz_heads_backward'][0](len(self.tc_rec_jobs), self.tc_rec_jobs, st), fn['mz_heads_backward'][1])
       return
     ln_w = net.views['LN.weight']
     g_w, g_b = net.grads['LN.weight'], net.grads['LN.bias']
