@@ -674,7 +674,10 @@ int mz_adam_step(int64_t n, float* params, const float* grads, float* exp_avg, f
 /* accumulation, f32 master weights and gradients.  A training step is FOUR launches: the chain    */
 /* representation -> LN -> K x (dynamics -> LN) (learners.py:175-206), the three output heads      */
 /* over the stacked hidden states, their backward, and the chain's backward with the 0.5 gradient  */
-/* hook of learners.py:201.                                                                        */
+/* hook of learners.py:201.  These entry points and their _tf32x3 counterparts below return        */
+/* MZ_ERR_UNSUPPORTED for a head with d_in > 1024 or d_out > 64 (a chain with d > 64 or            */
+/* d + num_actions > 128), MZ_ERR_BAD_ARG for a dX of a head wider than 128 and every other        */
+/* refused argument.                                                                               */
 /* ------------------------------------------------------------------------------------------- */
 /* One matrix to pack as an mma B operand: B[k][n] = src[n * stride_n + k * stride_k] (n < N, k < K), as bf16
  * fragments of 8 (n) x 32 (k) blocks, mz_learner_packed_words(N, K) 32-bit words (zero padded). */
@@ -756,9 +759,7 @@ int mz_chain_backward_tc(const mz_tc_chain* chain, void* stream);
 /* float32 accumulation), as in mz_fc_*_tf32x3.  Same structs and shapes as the _tc entry points; */
 /* the images of mz_tc_head are packed by mz_learner_pack_tf32x3 (hi / lo TF32 B fragments of      */
 /* 8 (n) x 8 (k) blocks, mz_learner_packed_words_tf32x3(N, K) 32-bit words, zero padded), and the  */
-/* ReLU bits of the chain have the layout of mz_chain_mask_words.  MZ_ERR_UNSUPPORTED for a head   */
-/* with d_in > 1024 or d_out > 64 (a chain with d > 64 or d + num_actions > 128), MZ_ERR_BAD_ARG  */
-/* for a dX of a head wider than 128 and every other refused argument.                             */
+/* ReLU bits of the chain have the layout of mz_chain_mask_words.  Error codes as above.           */
 /* ------------------------------------------------------------------------------------------- */
 int64_t mz_learner_packed_words_tf32x3(int32_t n, int32_t k);
 int mz_learner_pack_tf32x3(int32_t njobs, const mz_pack_job* jobs, void* stream);

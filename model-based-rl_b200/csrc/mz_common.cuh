@@ -67,6 +67,17 @@ inline cudaError_t mz_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, si
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
+// ---- 3xTF32 operands ----------------------------------------------------------------------------
+// The split of the float32-accurate tensor-core products x w ~= x_lo w_hi + x_hi w_lo + x_hi w_hi (three TF32 mma,
+// float32 accumulation).  x = hi + lo: hi = x cut to TF32's 11 significant bits (one LOP3; `cvt.rna.tf32.f32` compiles to five
+// instructions on sm_100a), lo = the exact float32 remainder (|lo| < 2^-10 |x|), of which the tensor core reads the
+// top 11 bits (the low 13 mantissa bits of a .tf32 operand register are ignored).  What a product loses -- lo's own
+// cut and the x_lo * w_lo term -- is below 2^-20 of it.
+MZ_DEV void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
+  hi = __float_as_uint(x) & 0xffffe000u;
+  lo = __float_as_uint(x - __uint_as_float(hi));
+}
+
 // ---- 64-bit shuffles ---------------------------------------------------------------------------
 template <int W>
 MZ_DEV double shfl_f64(double v, int src) {

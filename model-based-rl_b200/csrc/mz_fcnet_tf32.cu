@@ -30,14 +30,6 @@ constexpr int LDA = 520;         // row stride of the first-layer activations: 8
 constexpr int LDO = 72;          // row stride of second-layer outputs (<= 64 columns)
 constexpr int LDR = 64;          // row stride of a partial-sum slot
 
-// x = hi + lo: hi = x cut to TF32's 11 significant bits (one LOP3; `cvt.rna.tf32.f32` compiles to five
-// instructions on sm_100a), lo = the exact float32 remainder (|lo| < 2^-10 |x|), of which the tensor core reads the
-// top 11 bits (the low 13 mantissa bits of a .tf32 operand register are ignored).  What a product loses -- lo's own
-// cut and the x_lo * w_lo term -- is below 2^-20 of it.
-MZ_DEV void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
-  hi = __float_as_uint(x) & 0xffffe000u;
-  lo = __float_as_uint(x - __uint_as_float(hi));
-}
 MZ_DEV void mma_tf32(float (&d)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]) {
   asm("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
       "{%0, %1, %2, %3};"

@@ -5,8 +5,8 @@ library's own kernels instead of torch modules on library GEMMs.
 its state dict is a set of views with the reference's keys and shapes, so checkpoints, `Learner.send_weights` and the
 search kernels' `FCNetwork.load_weights` see the usual tensors.  `FusedLearner(precision=...)` runs a step as
 
-  precision='bf16' (default; csrc/mz_learner_tc.cu: tensor cores, bf16 operands, float32 accumulation, float32 master
-  weights / gradients / optimiser state)
+  precision='bf16' (default; csrc/mz_learner_tc.cuh with csrc/mz_learner_tc.cu: tensor cores, bf16 operands, float32
+  accumulation, float32 master weights / gradients / optimiser state)
     mz_learner_pack           the 20 weight images as bf16 mma B fragments + clears     1 launch
     mz_chain_forward_tc       representation -> LN -> K x (dynamics -> LN)               1 launch
     mz_heads_forward_tc       value / policy / reward heads over all K + 1 steps         1 launch
@@ -19,8 +19,9 @@ search kernels' `FCNetwork.load_weights` see the usual tensors.  `FusedLearner(p
   -- 10 kernels per step, 128 us at B = 512, K = 5 (7 800 steps/s on a B200; the torch-module step in a
   CUDA graph: 1 100 us).
 
-  precision='tf32x3' (csrc/mz_learner_tf32.cu: the same launches on the tensor cores at float32 accuracy -- every
-  contraction is three TF32 products on split operands, float32 accumulation -- held to the f32 path's bars)
+  precision='tf32x3' (csrc/mz_learner_tc.cuh with csrc/mz_learner_tf32.cu: the same launches on the tensor cores at
+  float32 accuracy -- every contraction is three TF32 products on split operands, float32 accumulation -- held to the
+  f32 path's bars)
     mz_learner_pack_tf32x3    the 20 weight images as hi / lo TF32 B fragments + clears 1 launch
     mz_chain_forward_tf32x3   representation -> LN -> K x (dynamics -> LN)               1 launch
     mz_heads_forward_tf32x3   value / policy / reward heads over all K + 1 steps         1 launch
@@ -56,8 +57,8 @@ from . import _lib, checkpoints, learners, parallel
 from .networks import HIDDEN
 
 WIDTH = _lib.FC_WIDTH
-MAX_SUPPORT_BINS = 64  # widest value / reward head: LMAXOUT in csrc/mz_learner.cu, head_ok in csrc/mz_learner_tc.cu
-MAX_INPUT_DIM = 1024   # widest observation: LMAXD in csrc/mz_learner.cu, MAXIN in csrc/mz_learner_tc.cu
+MAX_SUPPORT_BINS = 64  # widest value / reward head: LMAXOUT in csrc/mz_learner.cu, head_check in csrc/mz_learner_tc.cuh
+MAX_INPUT_DIM = 1024   # widest observation: LMAXD in csrc/mz_learner.cu, MAXIN in csrc/mz_learner_tc.cuh
 SLICE = 128            # input features per pass of the kernels' X tile: a wider (representation) head has no dX image
 _P = lambda t: C.c_void_p(t.data_ptr())
 

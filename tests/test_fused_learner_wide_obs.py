@@ -15,7 +15,7 @@ import torch
 
 from test_fused_learner import _rel, _teacher_forced_check
 
-MZ_ERR_BAD_ARG = -1
+MZ_ERR_BAD_ARG, MZ_ERR_UNSUPPORTED = -1, -2
 WIDE = (129, 136, 147, 200, 256, 512, 1000, 1024)
 ROWS = (1, 33, 100, 513)
 CSRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "model-based-rl_b200", "csrc")
@@ -47,23 +47,23 @@ def _head(lib, _lib, d_in, d_out=50):
   return _lib.TcHead(*p, d_in, d_out)
 
 
-def test_c_abi_refuses_inputs_wider_than_1024_and_dx_of_wide_heads_without_a_gpu():
+def test_c_abi_refuses_inputs_wider_than_1024_as_unsupported_and_dx_of_wide_heads_as_bad_arg_without_a_gpu():
   from model_based_rl_b200 import _lib
   lib = _lib.load()
   buf = C.c_void_p(4096)
-  for d_in, dx in ((1025, None), (200, 8192)):
+  for d_in, dx, want in ((1025, None, MZ_ERR_UNSUPPORTED), (200, 8192, MZ_ERR_BAD_ARG)):
     job = _lib.TcJob(_head(lib, _lib, d_in), 1, d_in, 50, d_in, 4096, 4096, 4096, dx)
     arr = (_lib.TcJob * 1)(job)
     if dx is None:
-      assert lib.mz_heads_forward_tc(1, arr, None) == MZ_ERR_BAD_ARG
-    assert lib.mz_heads_backward_tc(1, arr, None) == MZ_ERR_BAD_ARG, d_in
+      assert lib.mz_heads_forward_tc(1, arr, None) == want
+    assert lib.mz_heads_backward_tc(1, arr, None) == want, d_in
     # mz_mlp2_backward(rows, d_in, ldx, X, W1T, b1, W1, W2, d_out, dY, ldy, dX, lddx, gW1, gb1, gW2, gb2, stream)
     assert lib.mz_mlp2_backward(1, d_in, d_in, buf, buf, buf, buf, buf, 50, buf, 50, None if dx is None else C.c_void_p(dx),
                                 d_in, buf, buf, buf, buf, None) == MZ_ERR_BAD_ARG, d_in
   assert lib.mz_mlp2_forward(1, 1025, 1025, buf, buf, buf, buf, buf, 50, buf, 50, None) == MZ_ERR_BAD_ARG
   chain = _lib.TcChain(_head(lib, _lib, 1025), _head(lib, _lib, 68), 16, 2, 50, 18, 4096, 1025, None, 1, 1, 4096, 4096,
                        4096, 68, 4096, 4096, 4096, None, None, 0.5, None, None, None)
-  assert lib.mz_chain_forward_tc(C.byref(chain), None) == MZ_ERR_BAD_ARG
+  assert lib.mz_chain_forward_tc(C.byref(chain), None) == MZ_ERR_UNSUPPORTED
 
 
 def test_fused_network_refuses_more_than_1024_features_before_touching_the_device():
